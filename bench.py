@@ -20,6 +20,11 @@ the m <-> ring exchange of the phases fused into the Legendre kernels over NVLin
 -> strong scaling.
 
 --impl reference times the CPU path (all host threads) on the same config/metric.
+
+--dump-outputs DIR (N = 1) writes the map and a_lm of the last timed step as DIR/map.npy and DIR/alm.npy (float64, a
+fixed seeded sample of columns at large sizes), so that two builds can be compared output for output.  The inputs are the
+same in every run; the outputs agree to rounding, not bit for bit, because the analysis kernels accumulate with atomics
+(two runs of the default workload: 1.1e-14 relative L2, B200 at 1000 W).
 """
 import argparse
 import json
@@ -350,6 +355,24 @@ def run_parity(args, info, comm, dev, world, m, alm_in):
     out["parity_ok"] = bool(out["parity"]["rel_l2"] <= 1e-10)
     return out
 
+
+DUMP_COLS = 1_000_000    # per dumped array: 3 x 1e6 float64 = 24 MB, so map + alm stay under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Writes each (ncomp, n) array as path/<name>.npy in float64.  An array with more than DUMP_COLS columns is
+    reduced to a seeded sample of DUMP_COLS columns, the same columns for every component and for every run of the
+    same size."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, x in arrays.items():
+        n = x.shape[-1]
+        if n > DUMP_COLS:
+            cols = np.sort(np.random.default_rng(20).choice(n, DUMP_COLS, replace=False))
+            x = x[:, torch.as_tensor(cols, device=x.device)]
+        np.save(os.path.join(path, name + ".npy"), x.cpu().numpy())
+
 # ------------------------------------------------------------------ GPU arm
 def run_ours(args):
     import numpy as np
@@ -363,6 +386,8 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (no CPU fallback); use --impl reference for the CPU arm")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of a single-GPU run")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     comm = None
@@ -421,6 +446,9 @@ def run_ours(args):
     ms_total = ev[0].elapsed_time(ev[1])
     leg = sharp.last_legendre_ms()
     sharp.set_profiling(False)
+    if args.dump_outputs:
+        # what the caller of the last timed step receives: the map of Y() and the a_lm of YtW()
+        dump_outputs(args.dump_outputs, {"map": m.map, "alm": m.alm})
     tmax = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
@@ -767,7 +795,12 @@ def main():
     ap.add_argument("--no-cg", action="store_true", help="skip the secondary CG iters/s measurement")
     ap.add_argument("--no-batch", action="store_true", help="skip the 30-band batch measurement (config 5)")
     ap.add_argument("--no-conviqt", action="store_true", help="skip the conviqt cube measurement (SURVEY 8f rank 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the map and a_lm of the last timed step as DIR/map.npy and DIR/alm.npy (float64; a fixed "
+                         f"seeded sample of {DUMP_COLS} columns when larger)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -5,6 +5,7 @@ import ctypes as C
 import math
 import os
 import re
+import shutil
 import subprocess
 import sys
 
@@ -32,7 +33,9 @@ def test_library_is_sm100a_only():
     lib = os.path.join(ROOT, "commander_b200", "lib", "libcmdr_sht.so")
     if not os.path.exists(lib):
         pytest.skip("library not built")
-    out = subprocess.run(["cuobjdump", "-lelf", lib], capture_output=True, text=True).stdout
+    # the toolkit commander_b200/csrc/Makefile builds with when it is not on PATH
+    cuobjdump = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
+    out = subprocess.run([cuobjdump, "-lelf", lib], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
