@@ -177,6 +177,9 @@ CMDR_HD void start_spin_s(int m, int s, double Ksm, const RingTrig &g, double &P
     double base = Ksm * split_scale(mant, ex, k);
     P = base * ipow(g.sh, 2 * s);
     M = base * ipow(g.ch, 2 * s);
+    // k was chosen from sin^(m-s) alone; Ksm (which carries 2^s) can lift the start values over the threshold.  Join
+    // now: the recurrences only check every 8 l, and with lmax - m < 8 they would never do it.
+    if (k < 0 && (needs_rescale(P) || needs_rescale(M))) { P *= pow2i(-SCALE_BITS); M *= pow2i(-SCALE_BITS); ++k; }
   } else {
     k = 0;
     P = Ksm * ipow(g.ch, s - m) * ipow(g.sh, s + m);

@@ -28,7 +28,10 @@ def _setup(nside, lmax, lmax_beam, nmaps, seed):
 
 
 @pytest.mark.parametrize("nside,lmax,lmax_beam,bmax,nmaps", [(8, 16, 16, 1, 3), (8, 16, 12, 3, 3), (16, 32, 32, 4, 1),
-                                                             (32, 64, 48, 6, 3), (16, 40, 40, 9, 3)])
+                                                             (32, 64, 48, 6, 3), (16, 40, 40, 9, 3),
+                                                             # up to CMDR_MAX_SPIN: 64 psi planes at bmax 32
+                                                             (16, 48, 48, 16, 3), (16, 48, 40, 31, 1),
+                                                             (16, 48, 48, 32, 3)])
 def test_cube_vs_oracle(shtlib, cpu_oracle, nside, lmax, lmax_beam, bmax, nmaps):
     import torch
     from commander_b200 import comm_map

@@ -247,6 +247,50 @@ def test_device_recurrence_math_arbitrary_spin(emul, spin):
                 assert abs(P[l] - rp) <= 1e-11 * sc + 1e-19 and abs(M[l] - rm) <= 1e-11 * sc + 1e-19, (m, north, l)
 
 
+@pytest.mark.parametrize("spin", [8, 17, 31, 32])
+def test_device_recurrence_math_high_spin(emul, spin):
+    """start_spin_s (plain powers of sin / cos(theta/2) for m < s) and the spin-s coefficient tables up to
+    CMDR_MAX_SPIN = 32 at lmax 1000, every l, against the independent mpmath reference of tests/slam_ref.py."""
+    import slam_ref as R
+    nside, lmax = 512, 1000
+    worst = 0.0
+    for m in sorted({0, 1, spin - 1, spin, spin + 1, 40, 500, 999, lmax}):
+        for north in (1, 3, 40, 256, 512, 700, 1024):
+            cth, sth = R.ring_trig(nside, north)
+            P, M = emul(spin, lmax, m, nside, north)
+            rp = R.slam_column(lmax, m, spin, cth, sth)
+            rm = R.slam_column(lmax, m, -spin, cth, sth)
+            sc = max(np.abs(rp).max(), np.abs(rm).max())
+            if sc == 0:
+                assert not P.any() and not M.any()
+                continue
+            l0 = max(m, spin)
+            assert not P[:l0].any() and not M[:l0].any()
+            err = max(np.abs(P - rp).max(), np.abs(M - rm).max())
+            # ring 1 (sin theta = 0.003): the start values use sin / cos(theta/2) of the exact ring, the recurrence the
+            # float64 z = cos(theta), whose rounding moves theta by up to 2^-53 / (1 - z) / 2 relative, i.e. up to
+            # ~(m + s) * 4e-11 here; the reference is evaluated at arccos(z)
+            eps = 2e-9 if sth < 0.01 else 1e-11
+            worst = max(worst, (err - 1e-19) / sc)
+            assert err <= eps * sc + 1e-19, (m, north, err / sc)
+    print(f"spin {spin}: worst |delta| / max|lambda| {worst:.2e}")
+
+
+@pytest.mark.parametrize("spin,m,north", [(31, 193, 63), (31, 199, 64), (16, 193, 63), (32, 200, 63)])
+def test_high_spin_start_above_threshold_joins(emul, spin, m, north):
+    """m >= s with fewer than 8 l left: Ksm (which carries 2^s) lifts the start values over the join threshold although
+    sin^(m-s) alone is below it.  start_spin_s must join at once -- the recurrences check only every 8 l, so these
+    values (up to 4e-11 at nside 64 / lmax 200) came out as 0 before."""
+    import slam_ref as R
+    nside, lmax = 64, 200
+    cth, sth = R.ring_trig(nside, north)
+    P, M = emul(spin, lmax, m, nside, north)
+    rp, rm = R.slam_column(lmax, m, spin, cth, sth), R.slam_column(lmax, m, -spin, cth, sth)
+    sc = max(np.abs(rp).max(), np.abs(rm).max())
+    assert sc > 1e-17
+    assert max(np.abs(P - rp).max(), np.abs(M - rm).max()) <= 1e-11 * sc + 1e-19
+
+
 @pytest.fixture(scope="module")
 def emul_fft():
     """tests/host_emul/emul_bluefft.cpp: the product's blue_fft.cuh executed on the host."""
