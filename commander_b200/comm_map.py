@@ -231,6 +231,18 @@ class comm_map:
         """exec_sharp_Y_EB, :491-509: every column as a spin-0 field."""
         self._exec_scalar(sharp.SHARP_Y)
 
+    def alm2map_der1(self, i=0):
+        """Gradient maps {dT/dtheta, (1/sin theta) dT/dphi} of a_lm column `i`, shape (2, np), on the T geometry
+        (SHARP_ALM2MAP_DERIV1).  On this object's device; collective on the info's communicator when distributed."""
+        info = self.info
+        if self.device is None:
+            grad = np.zeros((2, info.np))
+        else:
+            import torch
+            grad = torch.zeros((2, info.np), dtype=torch.float64, device=self.alm.device)
+        sharp.alm2map_der1(self.alm[i:i + 1], info.alm_info, grad, info.geom_info_T, comm=self._comm())
+        return grad
+
     # fused variants (additive; one library call for T and QU)
     def _exec_iqu(self, job):
         info = self.info

@@ -444,14 +444,16 @@ LegAlm make_legalm(sharp_alm_info *a, int spin, bool classic) {
 // handles components [comp0, comp0+ncomp) of it.
 void run_single(int type, int spin, double *const *alm, double *const *map, sharp_geom_info *g,
                 sharp_alm_info *a, int flags, cudaStream_t st, const XformOpts *opts, int comp_off) {
+  if (type < 0 || type > SHARP_ALM2MAP_DERIV1) { fprintf(stderr, "cmdr_sht: job type %d unsupported\n", type); abort(); }
+  spin = job_spin(type, spin);
   if (spin < 0 || spin > CMDR_MAX_SPIN) { fprintf(stderr, "cmdr_sht: spin %d unsupported (0..%d)\n", spin, CMDR_MAX_SPIN); abort(); }
-  if (type < 0 || type > 3) { fprintf(stderr, "cmdr_sht: job type %d unsupported\n", type); abort(); }
   if (flags & SHARP_NO_FFT) { fprintf(stderr, "cmdr_sht: SHARP_NO_FFT unsupported\n"); abort(); }
-  const int ncomp = spin == 0 ? 1 : 2;
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
+  const int ncomp = job_map_cols(type, spin);   // map columns and phase components (the a_lm side of a synthesis reads what it needs)
+  const bool synth = job_synth(type);
   const bool add = (flags & SHARP_ADD) != 0;
   ensure_geom_device(g);
   LegAlm A = make_legalm(a, spin);
+  A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
   const double *pixscale[2] = {nullptr, nullptr};
   if (opts)
     for (int c = 0; c < ncomp; ++c) { A.lscale[c] = opts->lscale[comp_off + c]; pixscale[c] = opts->pixscale[comp_off + c]; }
@@ -597,13 +599,16 @@ bool alm_m_chunks(const sharp_alm_info *a, long long nalm_d, int nch, std::vecto
 static bool try_pipelined(int type, int spin, double *const *alm, double *const *map, sharp_geom_info *g,
                           sharp_alm_info *a, int flags, cudaStream_t st) {
   static const bool disabled = getenv("CMDR_SHT_NO_PIPELINE") != nullptr;
-  const int ncomp = spin == 0 ? 1 : 2;
+  if (type < 0 || type > SHARP_ALM2MAP_DERIV1) return false;
+  spin = job_spin(type, spin);
+  const int nca = job_alm_cols(type, spin), ncomp = job_map_cols(type, spin);
   if (disabled || (flags & SHARP_ADD) || g->npix < (1 << 21) || a->nm == 0 || spin < 0 || spin > CMDR_MAX_SPIN) return false;
-  if (type < 0 || type > 3) return false;
   // host arrays of either kind: pinned ones are copied in place, pageable ones (what sharp.f90:219-224 passes)
   // go through the library's pinned arena and the copy threads (hostio.cu)
+  for (int c = 0; c < nca; ++c)
+    if (host_kind(alm[c]) == HostKind::Device) return false;
   for (int c = 0; c < ncomp; ++c)
-    if (host_kind(alm[c]) == HostKind::Device || host_kind(map[c]) == HostKind::Device) return false;
+    if (host_kind(map[c]) == HostKind::Device) return false;
   HostIO ioA, ioM;
   // tuning aid: CMDR_SHT_PIPE_TRACE=1 prints a timeline (ms since the call started) of the stream markers below
   static const bool trace = getenv("CMDR_SHT_PIPE_TRACE") != nullptr;
@@ -631,20 +636,22 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
   static const int nchunks = getenv("CMDR_SHT_CHUNKS") ? atoi(getenv("CMDR_SHT_CHUNKS")) : 8;
   ensure_subgeoms(g, nchunks);
   if (g->subs.empty()) return false;
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
+  const bool synth = job_synth(type);
   ensure_geom_device(g);
   LegAlm A = make_legalm(a, spin);
+  A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
-  double *alm_buf = static_cast<double *>(scratch_get("stage_alm", sizeof(double) * (size_t)nalm_d * ncomp));
+  double *alm_buf = static_cast<double *>(scratch_get("stage_alm", sizeof(double) * (size_t)nalm_d * nca));
   double *map_buf = static_cast<double *>(scratch_get("stage_map", sizeof(double) * (size_t)g->npix * ncomp));
   double4 *ph = static_cast<double4 *>(scratch_get("phase", sizeof(double4) * (size_t)ncomp * a->nm * g->npairs));
-  ioA.init("hstage_alm", alm, ncomp, nalm_d, true);
+  ioA.init("hstage_alm", alm, nca, nalm_d, true);
   ioM.init("hstage_map", map, ncomp, g->npix, true);
   size_t maxz = 0;
   for (sharp_geom_info *sub : g->subs) { ensure_geom_device(sub); maxz = std::max(maxz, ringfft_scratch_elems(sub)); }
   if (maxz) scratch_get("fftbuf", sizeof(double2) * maxz * ncomp);
   double *alm_dev[2], *map_dev[2];
-  for (int c = 0; c < ncomp; ++c) { alm_dev[c] = alm_buf + (size_t)c * nalm_d; map_dev[c] = map_buf + (size_t)c * g->npix; }
+  for (int c = 0; c < nca; ++c) alm_dev[c] = alm_buf + (size_t)c * nalm_d;
+  for (int c = 0; c < ncomp; ++c) map_dev[c] = map_buf + (size_t)c * g->npix;
   LegGeom G;
   G.nslots = g->npairs; G.NPL = g->npairs; G.nowners = 1; G.NML = a->nm; G.ncomp_tot = ncomp; G.comp0 = 0;
   G.trig = g->d_trig; G.mlim = ensure_mlim(g, a->lmax, spin);
@@ -661,7 +668,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
     std::vector<int> mcut;
     const int nmch = alm_m_chunks(a, nalm_d, NMCH, mstart, mcut) ? NMCH : 1;
     if (nmch == 1) {
-      for (int c = 0; c < ncomp; ++c) ioA.h2d(alm_dev[c], c, 0, nalm_d, st);
+      for (int c = 0; c < nca; ++c) ioA.h2d(alm_dev[c], c, 0, nalm_d, st);
     } else {
       cudaEvent_t e0 = pooled_event(ns + 1);               // earlier work on `st` may still read the staging buffer
       CMDR_CUDA_CHECK(cudaEventRecord(e0, st));
@@ -671,7 +678,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
     // this thread -- hence the kernels of chunk j are queued right behind its upload, not after all uploads)
     auto upload_mchunk = [&](int j) {
       const long long b = mstart[mcut[j]], e = mstart[mcut[j + 1]];
-      for (int c = 0; c < ncomp; ++c) ioA.h2d(alm_dev[c] + b, c, b, e - b, cs);
+      for (int c = 0; c < nca; ++c) ioA.h2d(alm_dev[c] + b, c, b, e - b, cs);
       CMDR_CUDA_CHECK(cudaEventRecord(pooled_event(ns + 2 + j), cs));
       mark("up", j, cs);
     };
@@ -795,33 +802,40 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
   return true;
 }
 
-unsigned long long nominal_flops(const sharp_geom_info *g, const sharp_alm_info *a, int spin) {
-  // (l,m) count over the local m's times ring pairs (an unpaired ring counts half)
+// (l,m) count over the local m's times ring pairs (an unpaired ring counts half), times `per` nominal flops
+static unsigned long long lm_pair_flops(const sharp_geom_info *g, const sharp_alm_info *a, double per) {
   double nlm = 0;
   for (int m : a->mval) nlm += a->lmax + 1 - m;
   double pairs = 0;
   for (int p = 0; p < g->npairs; ++p) pairs += (g->ofsN[p] >= 0 && g->ofsS[p] >= 0) ? 1.0 : 0.5;
-  return (unsigned long long)(nlm * pairs * (spin == 0 ? 8.0 : 28.0));
+  return (unsigned long long)(nlm * pairs * per);
+}
+unsigned long long nominal_flops(const sharp_geom_info *g, const sharp_alm_info *a, int spin) {
+  return lm_pair_flops(g, a, spin == 0 ? 8.0 : 28.0);
+}
+// `opcnt` of a job: DERIV1 counts 20 per (l, m, ring pair) -- 12 for the spin-1 recurrence, 4 accumulate FMAs (FMA = 2)
+unsigned long long job_opcnt(const sharp_geom_info *g, const sharp_alm_info *a, int type, int spin) {
+  return type == SHARP_ALM2MAP_DERIV1 ? lm_pair_flops(g, a, 20.0) : nominal_flops(g, a, spin);
 }
 
 void execute_any(int type, int spin, void *alm_v, void *map_v, sharp_geom_info *g, sharp_alm_info *a,
                  int flags, double *time, unsigned long long *opcnt, cudaStream_t st) {
   auto t0 = std::chrono::steady_clock::now();
-  const int ncomp = spin == 0 ? 1 : 2;
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
+  const int nca = job_alm_cols(type, spin), ncm = job_map_cols(type, spin);
+  const bool synth = job_synth(type);
   const bool add = (flags & SHARP_ADD) != 0;
   double *const *alm = static_cast<double *const *>(alm_v);
   double *const *map = static_cast<double *const *>(map_v);
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
   if (!try_pipelined(type, spin, alm, map, g, a, flags, st)) {
-    Staged sa = stage_in("stage_alm", alm, ncomp, nalm_d, synth || add, st);
-    Staged sm = stage_in("stage_map", map, ncomp, g->npix, !synth || add, st);
+    Staged sa = stage_in("stage_alm", alm, nca, nalm_d, synth || add, st);
+    Staged sm = stage_in("stage_map", map, ncm, g->npix, !synth || add, st);
     run_single(type, spin, sa.dev.data(), sm.dev.data(), g, a, flags, st);
     if (synth) stage_out(sm, g->npix, st); else stage_out(sa, nalm_d, st);
     if (sa.staged || sm.staged || time) CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
   }
   if (time) *time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-  if (opcnt) *opcnt = nominal_flops(g, a, spin);
+  if (opcnt) *opcnt = job_opcnt(g, a, type, spin);
 }
 
 }  // namespace cmdr
@@ -846,6 +860,7 @@ void cmdr_sht_execute_dev(int type, int spin, double *const *alm, double *const 
 void cmdr_sht_execute_iqu(int type, double *const *alm3, double *const *map3, const sharp_geom_info *geom_T,
                           const sharp_geom_info *geom_P, const sharp_alm_info *alm_info, int flags,
                           void *stream) {
+  require_iqu_job(type, "cmdr_sht_execute_iqu");
   cudaStream_t st = (cudaStream_t)stream;
   sharp_geom_info *gT = const_cast<sharp_geom_info *>(geom_T), *gP = const_cast<sharp_geom_info *>(geom_P);
   sharp_alm_info *a = const_cast<sharp_alm_info *>(alm_info);
@@ -868,6 +883,7 @@ void cmdr_sht_execute_iqu(int type, double *const *alm3, double *const *map3, co
 void cmdr_sht_execute_iqu_batch(int type, int nbatch, double *const *alm3, double *const *map3,
                                 const sharp_geom_info *geom_T, const sharp_geom_info *geom_P,
                                 const sharp_alm_info *alm_info, int flags, void *stream) {
+  require_iqu_job(type, "cmdr_sht_execute_iqu_batch");
   cudaStream_t st = (cudaStream_t)stream;
   sharp_geom_info *gT = const_cast<sharp_geom_info *>(geom_T), *gP = const_cast<sharp_geom_info *>(geom_P);
   sharp_alm_info *a = const_cast<sharp_alm_info *>(alm_info);

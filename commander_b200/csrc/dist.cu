@@ -425,8 +425,8 @@ struct Part {
 // share one phase buffer of ncomp_tot components and one exchange.
 static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int ncomp_tot, sharp_alm_info *a,
                      int flags, cudaStream_t st) {
-  if (type < 0 || type > 3) { fprintf(stderr, "cmdr_sht: job type %d unsupported\n", type); abort(); }
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
+  if (type < 0 || type > SHARP_ALM2MAP_DERIV1) { fprintf(stderr, "cmdr_sht: job type %d unsupported\n", type); abort(); }
+  const bool synth = job_synth(type);
   const bool add = (flags & SHARP_ADD) != 0;
   sharp_geom_info *g0 = parts[0].g;
   for (int i = 0; i < nparts; ++i) {
@@ -459,6 +459,7 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
       const Part &p = parts[i];
       LegAlm A = make_legalm(a, p.spin);
       A.lscale[0] = p.lscale[0]; A.lscale[1] = p.lscale[1];
+      A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
       G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.spin);
       prof_begin(p.spin, 0, st);
       launch_legendre_synth(p.spin, G, A, p.alm, reinterpret_cast<double4 *>(B.mine), st);
@@ -522,6 +523,7 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
       const Part &p = parts[i];
       LegAlm A = make_legalm(a, p.spin);
       A.lscale[0] = p.lscale[0]; A.lscale[1] = p.lscale[1];
+      A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
       G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.spin);
       prof_begin(p.spin, 0, st);
       launch_legendre_synth(p.spin, G, A, p.alm, reinterpret_cast<double4 *>(bufA), st);
@@ -574,17 +576,20 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
 static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *alm, double *const *map,
                                sharp_geom_info *g, sharp_alm_info *a, int flags, cudaStream_t st) {
   static const bool disabled = getenv("CMDR_SHT_NO_PIPELINE") != nullptr;
-  const int ncomp = spin == 0 ? 1 : 2;
-  if (disabled || (flags & SHARP_ADD) || !use_p2p(C) || type < 0 || type > 3) return false;
+  const int nca = job_alm_cols(type, spin), ncomp = job_map_cols(type, spin);
+  if (disabled || (flags & SHARP_ADD) || !use_p2p(C) || type < 0 || type > SHARP_ALM2MAP_DERIV1) return false;
+  spin = job_spin(type, spin);
   // Every rank must take the same decision (the chunked path has K + 1 exchange barriers, the plain one 2).
   // Global sizes are equal everywhere by construction; host-versus-device buffers is a property of the call
   // site, the same on all ranks of a collective call (pinned or pageable does not matter: both take this
   // path).  What can differ from rank to rank -- a rank without rings or m's, a ring list that is not
   // contiguous -- is agreed once per plan with an all-reduce (min) and cached there.
   if ((long long)g->nside * g->nside * 12 < (1LL << 20) * C->nranks) return false;
+  for (int c = 0; c < nca; ++c)
+    if (host_kind(alm[c]) == HostKind::Device) return false;
   for (int c = 0; c < ncomp; ++c)
-    if (host_kind(alm[c]) == HostKind::Device || host_kind(map[c]) == HostKind::Device) return false;
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
+    if (host_kind(map[c]) == HostKind::Device) return false;
+  const bool synth = job_synth(type);
   ensure_geom_device(g);
   ensure_alm_device(a);
   DistPlan *P = get_plan(C, g, a, st);
@@ -609,13 +614,14 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
   const size_t cap = sizeof(double) * (size_t)3 * P->NML * P->NPL * 4 * C->nranks;
   if (!(ensure_peerbuf(C, C->pb[0], cap, st) && ensure_peerbuf(C, C->pb[1], cap, st))) { C->p2p = 0; return false; }
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
-  double *alm_buf = static_cast<double *>(scratch_get("stage_alm", sizeof(double) * (size_t)nalm_d * ncomp));
+  double *alm_buf = static_cast<double *>(scratch_get("stage_alm", sizeof(double) * (size_t)nalm_d * nca));
   double *map_buf = static_cast<double *>(scratch_get("stage_map", sizeof(double) * (size_t)g->npix * ncomp));
   size_t maxz = 0;
   for (sharp_geom_info *sub : P->subs) if (sub) { ensure_geom_device(sub); maxz = std::max(maxz, ringfft_scratch_elems(sub)); }
   if (maxz) scratch_get("fftbuf", sizeof(double2) * maxz * ncomp);
   double *alm_dev[2], *map_dev[2];
-  for (int c = 0; c < ncomp; ++c) { alm_dev[c] = alm_buf + (size_t)c * nalm_d; map_dev[c] = map_buf + (size_t)c * g->npix; }
+  for (int c = 0; c < nca; ++c) alm_dev[c] = alm_buf + (size_t)c * nalm_d;
+  for (int c = 0; c < ncomp; ++c) map_dev[c] = map_buf + (size_t)c * g->npix;
   PhaseLayout L;
   L.NPL = P->NPL; L.NML = P->NML; L.ncomp_tot = ncomp; L.comp0 = 0; L.mmax = P->mmax;
   L.m2src = P->d_m2src; L.m2im = P->d_m2im; L.nm_total = P->nm_total;
@@ -627,10 +633,11 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
   G.npeer = C->nranks; G.src_rank = C->rank;
   for (int r = 0; r < C->nranks; ++r) G.peer[r] = reinterpret_cast<double4 *>(B.peer[r]);
   LegAlm A = make_legalm(a, spin);
+  A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
   cudaStream_t cs = copy_stream();
   const size_t ev0 = 32;                                  // events 0..31 belong to the single-GPU pipeline
   HostIO ioA, ioM;                                        // pageable caller arrays go through the pinned arena (hostio.cu)
-  ioA.init("hstage_alm", alm, ncomp, nalm_d);
+  ioA.init("hstage_alm", alm, nca, nalm_d);
   ioM.init("hstage_map", map, ncomp, g->npix);
   // The a_lm move in NMCH chunks of local m's beside the kernels of ONE work-slot chunk (rank-local: no barrier inside):
   // synthesis runs the first chunk's Legendre kernel m-chunk by m-chunk as the upload lands, analysis the last chunk's,
@@ -641,7 +648,7 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
   const int nmch = alm_m_chunks(a, nalm_d, NMCH, mstart, mcut) ? NMCH : 1;
   const size_t evm = 200;                                 // events of the m-chunks
   if (synth) {
-    if (nmch == 1) for (int c = 0; c < ncomp; ++c) ioA.h2d(alm_dev[c], c, 0, nalm_d, st);
+    if (nmch == 1) for (int c = 0; c < nca; ++c) ioA.h2d(alm_dev[c], c, 0, nalm_d, st);
     else {
       cudaEvent_t e0 = pooled_event(evm + 2 * NMCH);       // the staging a_lm may still be read by earlier work on `st`
       CMDR_CUDA_CHECK(cudaEventRecord(e0, st));
@@ -653,7 +660,7 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
       if (c == K - 1 && nmch > 1) {
         for (int j = 0; j < nmch; ++j) {
           const long long b = mstart[mcut[j]], e = mstart[mcut[j + 1]];
-          for (int k = 0; k < ncomp; ++k) ioA.h2d(alm_dev[k] + b, k, b, e - b, cs);
+          for (int k = 0; k < nca; ++k) ioA.h2d(alm_dev[k] + b, k, b, e - b, cs);
           cudaEvent_t ej = pooled_event(evm + j);
           CMDR_CUDA_CHECK(cudaEventRecord(ej, cs));
           CMDR_CUDA_CHECK(cudaStreamWaitEvent(st, ej, 0));
@@ -736,20 +743,23 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
 static void execute_dist_any(DistComm *C, int type, int nparts, const int *spins, double *const *alm,
                              double *const *map, sharp_geom_info *const *geoms, sharp_alm_info *a, int flags,
                              cudaStream_t st, const XformOpts *opts = nullptr) {
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
+  if (type == SHARP_ALM2MAP_DERIV1 && nparts != 1) require_iqu_job(type, "execute_dist_any");
+  const bool synth = job_synth(type);
   const bool add = (flags & SHARP_ADD) != 0;
-  int ncomp_tot = 0;
-  for (int i = 0; i < nparts; ++i) ncomp_tot += spins[i] == 0 ? 1 : 2;
+  // a_lm and map columns: equal except for DERIV1 (one part: 1 a_lm column, 2 maps)
+  int ncomp_tot = 0, nalm_tot = 0;
+  for (int i = 0; i < nparts; ++i) { ncomp_tot += job_map_cols(type, spins[i]); nalm_tot += job_alm_cols(type, spins[i]); }
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
   if (nparts == 1 && !opts && try_dist_pipelined(C, type, spins[0], alm, map, geoms[0], a, flags, st)) return;
-  Staged sa = stage_in("stage_alm", alm, ncomp_tot, nalm_d, synth || add, st);
+  Staged sa = stage_in("stage_alm", alm, nalm_tot, nalm_d, synth || add, st);
   Staged sm = stage_in("stage_map", map, ncomp_tot, geoms[0]->npix, !synth || add, st);
   Part parts[4];
-  int c0 = 0;
+  int c0 = 0, ca = 0;
   for (int i = 0; i < nparts; ++i) {
-    int nc = spins[i] == 0 ? 1 : 2;
-    if (spins[i] < 0 || spins[i] > CMDR_MAX_SPIN) { fprintf(stderr, "cmdr_sht: spin %d unsupported\n", spins[i]); abort(); }
-    parts[i] = Part{spins[i], c0, nc, geoms[i], sa.dev.data() + c0, sm.dev.data() + c0};
+    const int spin = job_spin(type, spins[i]), nc = job_map_cols(type, spins[i]);
+    if (spin < 0 || spin > CMDR_MAX_SPIN) { fprintf(stderr, "cmdr_sht: spin %d unsupported\n", spin); abort(); }
+    parts[i] = Part{spin, c0, nc, geoms[i], sa.dev.data() + ca, sm.dev.data() + c0};
+    ca += job_alm_cols(type, spins[i]);
     if (opts)
       for (int c = 0; c < nc; ++c) { parts[i].lscale[c] = opts->lscale[c0 + c]; parts[i].pixscale[c] = opts->pixscale[c0 + c]; }
     c0 += nc;
@@ -769,6 +779,7 @@ int effective_comm(int comm, const sharp_geom_info *g, const sharp_alm_info *a, 
 // on a registered communicator (cr.cu)
 void execute_iqu_opts(int comm, int type, int nmaps, double *const *alm, double *const *map, sharp_geom_info *gT,
                       sharp_geom_info *gP, sharp_alm_info *a, int flags, const XformOpts *opts, cudaStream_t st) {
+  require_iqu_job(type, "execute_iqu_opts");
   DistComm *C = comm_or_local(comm, gT, a, "cmdr_cr");
   if (!C) {
     run_single(type, 0, alm, map, gT, a, flags, st, opts, 0);
@@ -851,6 +862,7 @@ void cmdr_sht_execute_dist(int comm, int type, int spin, void *alm, void *map, c
 void cmdr_sht_execute_iqu_dist(int comm, int type, double *const *alm3, double *const *map3,
                                const sharp_geom_info *geom_T, const sharp_geom_info *geom_P,
                                const sharp_alm_info *alm_info, int flags, void *stream) {
+  require_iqu_job(type, "cmdr_sht_execute_iqu_dist");
   DistComm *C = comm_or_local(comm, geom_T, alm_info, "cmdr_sht_execute_iqu_dist");
   if (!C) {
     cmdr_sht_execute_iqu(type, alm3, map3, geom_T, geom_P, alm_info, flags, stream);
@@ -971,7 +983,7 @@ void sharp_execute_mpi_fortran(int comm, int type, int spin, void *alm, void *ma
                    flags, (cudaStream_t)0);
   if (time || opcnt) CMDR_CUDA_CHECK(cudaStreamSynchronize(0));
   if (time) *time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();   // wall seconds, as libsharp2 reports
-  if (opcnt) *opcnt = cmdr_sht_nominal_flops(geom_info, alm_info, spin);
+  if (opcnt) *opcnt = job_opcnt(geom_info, alm_info, type, spin);
 }
 
 }  // extern "C"

@@ -56,7 +56,21 @@ struct LegAlm {
   // a_lm on load (synthesis) and on store (analysis) -- how cr_matmulA's sqrt(S), beam and F_mean passes
   // (commander3/src/comm_cr_mod.f90:797-836, 957-1008; comm_B_bl_mod.f90:108-127) ride in the Legendre kernels
   const double *lscale[2] = {nullptr, nullptr};
+  bool deriv1 = false;             // SHARP_ALM2MAP_DERIV1 (spin 1 tables, one a_lm column): prep_d1 / synth_d1 kernels
 };
+
+// Column counts of a job.  SHARP_ALM2MAP_DERIV1 is a synthesis from ONE spin-0 a_lm column to TWO maps
+// {d_theta T, d_phi T / sin theta}; it runs on the spin-1 tables whatever spin the caller passes.
+inline bool job_synth(int type) { return type == SHARP_Y || type == SHARP_WY || type == SHARP_ALM2MAP_DERIV1; }
+inline int job_spin(int type, int spin) { return type == SHARP_ALM2MAP_DERIV1 ? 1 : spin; }
+inline int job_alm_cols(int type, int spin) { return type == SHARP_ALM2MAP_DERIV1 ? 1 : (spin == 0 ? 1 : 2); }
+inline int job_map_cols(int type, int spin) { return type == SHARP_ALM2MAP_DERIV1 ? 2 : (spin == 0 ? 1 : 2); }
+unsigned long long job_opcnt(const sharp_geom_info *g, const sharp_alm_info *a, int type, int spin);
+// The fused T + (Q,U) entry points (execute_iqu[_batch|_dist]) run the four map <-> a_lm jobs only: DERIV1 has one
+// a_lm column and two maps per transform, which their three-column pointer tables cannot carry.
+inline void require_iqu_job(int type, const char *who) {
+  if (type < SHARP_YtW || type > SHARP_WY) { fprintf(stderr, "cmdr_sht: %s: job type %d unsupported\n", who, type); abort(); }
+}
 
 // Optional element-wise factors fused into a transform (cr.cu): per l on the a_lm side, per local pixel on the map
 // side of a synthesis (N^-1 of commander3/src/comm_N_rms_mod.f90:264-273 in the ring-FFT epilogue).

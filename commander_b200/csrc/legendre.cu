@@ -496,6 +496,132 @@ __global__ void __launch_bounds__(32, MINB) synth2_kernel(KParams p) {
 }
 
 // ------------------------------------------------------------------------------------
+// SHARP_ALM2MAP_DERIV1: {d_theta T, d_phi T / sin theta} from one spin-0 a_lm column, as the spin-1 synthesis with
+// E = -sqrt(l(l+1)) a, B = 0 (cp = c, cm = -c; legendre_core.cuh, d1_accum / d1_combine).  Same structure as
+// synth2_kernel with a 32-byte tile row and half the accumulate FMAs.
+// ------------------------------------------------------------------------------------
+struct __align__(16) TileD1 { double A, C, cr, ci; };
+
+__global__ void __launch_bounds__(256) prep_d1_kernel(KParams p) {
+  const int im = p.im0 + blockIdx.y, m = p.mval[im];
+  const int l0 = max(m, 1);
+  const int j = blockIdx.x * blockDim.x + threadIdx.x, l = l0 + j;
+  const int npad = l0 <= p.lmax ? (p.lmax - l0 + 1 + 7) & ~7 : 0;
+  if (j >= npad) return;
+  TileD1 e{0.0, 0.0, 0.0, 0.0};
+  if (l <= p.lmax) {
+    const double *a = p.alm0;
+    const long long mvs = p.mvstart[im];
+    const double nrm = (p.real_packed && m > 0) ? 0.70710678118654752440 : 1.0;
+    const double4 c = reinterpret_cast<const double4 *>(p.coef + p.cofs[im])[l - l0];   // {A', C', g, 0}
+    double ar, ai = 0.0;
+    if (p.real_packed) {
+      if (m == 0) ar = a[mvs + l];
+      else { ar = a[mvs + 2 * (long long)l]; ai = a[mvs + 2 * (long long)l + 1]; }
+    } else {
+      ar = a[2 * (mvs + l)];
+      if (m > 0) ai = a[2 * (mvs + l) + 1];
+    }
+    const double f = -sqrt((double)l * (double)(l + 1)) * c.z * nrm;
+    e.A = c.x; e.C = c.y; e.cr = f * ar; e.ci = f * ai;
+  }
+  reinterpret_cast<TileD1 *>(p.trows)[p.tofs[im] + j] = e;
+}
+
+template <int MODE, int R>
+__device__ __forceinline__ void synth_d1_group(const TileD1 *t, const double (&x)[R], double (&P)[R],
+                                               double (&Pp)[R], double (&M)[R], double (&Mp)[R],
+                                               double (&s)[R][8], int (&k)[R]) {
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const double A = t[j].A, C = t[j].C, cr = t[j].cr, ci = t[j].ci;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+      if (MODE >= 1) {
+        const bool on = (MODE == 2 || k[r] == 0);
+        d1_accum(j & 1, on ? P[r] : 0.0, on ? M[r] : 0.0, cr, ci, s[r]);
+      }
+      double up = fma(A, x[r], C), um = fma(A, x[r], -C);
+      double np_ = fma(up, P[r], -Pp[r]), nm_ = fma(um, M[r], -Mp[r]);
+      Pp[r] = P[r]; P[r] = np_; Mp[r] = M[r]; M[r] = nm_;
+    }
+  }
+  if (MODE < 2) {
+#pragma unroll
+    for (int r = 0; r < R; ++r)
+      if (k[r] < 0 && (needs_rescale(P[r]) || needs_rescale(M[r]))) {
+        P[r] *= SCALE_DOWN; Pp[r] *= SCALE_DOWN; M[r] *= SCALE_DOWN; Mp[r] *= SCALE_DOWN; ++k[r];
+      }
+  }
+}
+
+template <int R, int MINB>
+__global__ void __launch_bounds__(32, MINB) synth_d1_kernel(KParams p) {
+  __shared__ __align__(16) TileD1 tile[2][TL];
+  const int im = p.im0 + blockIdx.y, m = p.mval[im];
+  const int lane = threadIdx.x;
+  const int chunk0 = p.slot_begin + blockIdx.x * (32 * R);
+  const int l0 = max(m, 1);
+  double x[R], P[R], Pp[R], M[R], Mp[R], s[R][8];
+  int k[R], slot[R];
+  bool any = false;
+  const double K = p.Kstart[m];
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    slot[r] = chunk0 + lane * R + r;
+    bool valid = slot[r] < p.nslots && m <= p.mlim[min(slot[r], p.nslots - 1)] && l0 <= p.lmax;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) s[r][q] = 0.0;
+    P[r] = M[r] = Pp[r] = Mp[r] = 0.0; k[r] = 0; x[r] = 0.0;
+    if (valid) {
+      const double4 tg = reinterpret_cast<const double4 *>(p.trig)[slot[r]];
+      RingTrig g{tg.x, tg.y, tg.z, tg.w};
+      x[r] = g.cth;
+      start_spin_s(m, 1, K, g, P[r], M[r], k[r]);
+      any = true;
+    }
+  }
+  if (__any_sync(FULL, any)) {
+    const TileD1 *rows = reinterpret_cast<const TileD1 *>(p.trows) + p.tofs[im];
+    auto issue_tile = [&](int b, int lt) {     // rows past this m's padded range are never used
+      const char *src = reinterpret_cast<const char *>(rows + (lt - l0));
+      char *dst = reinterpret_cast<char *>(tile[b]);
+#pragma unroll
+      for (int q = 0; q < (int)(TL * sizeof(TileD1)) / 512; ++q) cp_async16(dst + (q * 32 + lane) * 16, src + (q * 32 + lane) * 16);
+      cp_async_commit();
+    };
+    issue_tile(0, l0);
+    cp_async_wait_all();
+    __syncwarp();
+    int buf = 0;
+    for (int lt = l0; lt <= p.lmax; lt += TL, buf ^= 1) {
+      if (lt + TL <= p.lmax) issue_tile(buf ^ 1, lt + TL);
+      const int ngroups = min(TL, p.lmax - lt + 8) / 8;
+#pragma unroll 1
+      for (int g = 0; g < ngroups; ++g) {
+        bool all_on = true, none_on = true;
+#pragma unroll
+        for (int r = 0; r < R; ++r) { all_on &= (k[r] == 0); none_on &= (k[r] < 0); }
+        if (__all_sync(FULL, all_on)) synth_d1_group<2, R>(tile[buf] + 8 * g, x, P, Pp, M, Mp, s, k);
+        else if (__all_sync(FULL, none_on)) synth_d1_group<0, R>(tile[buf] + 8 * g, x, P, Pp, M, Mp, s, k);
+        else synth_d1_group<1, R>(tile[buf] + 8 * g, x, P, Pp, M, Mp, s, k);
+      }
+      cp_async_wait_all();
+      __syncwarp();
+    }
+  }
+  const double sg0 = ((l0 + m) & 1) ? -0.5 : 0.5;
+#pragma unroll
+  for (int r = 0; r < R; ++r)
+    if (slot[r] < p.nslots) {
+      double q[4], u[4];
+      d1_combine(s[r], sg0, q, u);
+      *ph_out(p, 0, im, slot[r]) = make_double4(q[0], q[1], q[2], q[3]);
+      *ph_out(p, 1, im, slot[r]) = make_double4(u[0], u[1], u[2], u[3]);
+    }
+}
+
+// ------------------------------------------------------------------------------------
 // Ring reduction for analysis.  Each lane holds 16 partial sums per group (the l of the group
 // times the real outputs per l); a 5-stage butterfly reduce-scatter over the warp leaves one
 // distinct total in every even lane: 16 double shuffles + 16 DADD per 16 outputs.
@@ -1049,7 +1175,7 @@ __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
 // launchers
 // ------------------------------------------------------------------------------------
 // Ring pairs per thread (register blocking).  Defaults were picked from the sweep recorded in
-// profiles/; CMDR_SHT_R_S0 / _S2 / _A0 / _A2 override them for tuning runs.
+// profiles/; CMDR_SHT_R_S0 / _S2 / _D1 / _A0 / _A2 (with _MINB_) override them for tuning runs.
 static int env_int(const char *name, int dflt) {
   const char *e = getenv(name);
   return (e && *e) ? atoi(e) : dflt;
@@ -1086,20 +1212,32 @@ void launch_legendre_synth(int spin, const LegGeom &g, const LegAlm &a, const do
   if (a.nm == 0 || g.nslots == 0) return;
   const int nmr = (a.im_end >= 0 ? a.im_end : a.nm) - a.im_begin;   // local m's of this launch
   if (nmr <= 0) return;
-  KParams p = make_params(g, a, const_cast<double *>(alm[0]), spin ? const_cast<double *>(alm[1]) : nullptr, ph);
+  if (a.deriv1 && spin != 1) { fprintf(stderr, "cmdr_sht: the DERIV1 synthesis runs on the spin-1 tables\n"); abort(); }
+  // DERIV1 reads one a_lm column: never touch alm[1]
+  KParams p = make_params(g, a, const_cast<double *>(alm[0]), (spin && !a.deriv1) ? const_cast<double *>(alm[1]) : nullptr, ph);
   // tile rows {A', [C',] g a_lm} for all local (m, l): written once per transform (`prep`), then
   // streamed by every warp of the Legendre kernel
-  const size_t rowbytes = spin == 0 ? sizeof(TileS0) : sizeof(TileS2);
+  const size_t rowbytes = spin == 0 ? sizeof(TileS0) : (a.deriv1 ? sizeof(TileD1) : sizeof(TileS2));
   p.tofs = a.tofs;
   p.trows = static_cast<double *>(scratch_get(spin == 0 ? "synth_rows0" : "synth_rows2", rowbytes * (size_t)(a.trows + TL)));
   if (prep) {
     dim3 pg((a.lmax + 8 + 255) / 256, nmr);
-    if (spin == 0) prep_s0_kernel<<<pg, 256, 0, st>>>(p); else prep_s2_kernel<<<pg, 256, 0, st>>>(p);
+    if (spin == 0) prep_s0_kernel<<<pg, 256, 0, st>>>(p);
+    else if (a.deriv1) prep_d1_kernel<<<pg, 256, 0, st>>>(p);
+    else prep_s2_kernel<<<pg, 256, 0, st>>>(p);
     count_launch();
   }
   static const int r0 = env_int("CMDR_SHT_R_S0", 4), r2 = env_int("CMDR_SHT_R_S2", 4);
   static const int b0 = env_int("CMDR_SHT_MINB_S0", 16), b2 = env_int("CMDR_SHT_MINB_S2", 8);
-  if (spin == 0) {
+  static const int rd = env_int("CMDR_SHT_R_D1", 2), bd = env_int("CMDR_SHT_MINB_D1", 16);
+  if (a.deriv1) {
+    switch (rd * 100 + bd) {
+      case 312: launch_w<3>(synth_d1_kernel<3, 12>, p, nmr, st); break;
+      case 412: launch_w<4>(synth_d1_kernel<4, 12>, p, nmr, st); break;
+      case 408: launch_w<4>(synth_d1_kernel<4, 8>, p, nmr, st); break;
+      default: launch_w<2>(synth_d1_kernel<2, 16>, p, nmr, st); break;
+    }
+  } else if (spin == 0) {
     switch (r0 * 100 + b0) {
       case 216: launch_w<2>(synth0_kernel<2, 16>, p, nmr, st); break;
       case 412: launch_w<4>(synth0_kernel<4, 12>, p, nmr, st); break;

@@ -187,6 +187,30 @@ CMDR_HD void start_spin_s(int m, int s, double Ksm, const RingTrig &g, double &P
   }
 }
 
+// ---- SHARP_ALM2MAP_DERIV1: gradient of a spin-0 map through the spin-1 functions ---------------------------
+// d_theta T = spin-1 synthesis with E = -sqrt(l(l+1)) a, B = 0, so both spin-1 coefficients are multiples of one
+// number c_l: cp = c, cm = -c.  The four phase sums of the spin-s kernels (north: sum cp P, sum cm M; south:
+// sum sg cp M, sum sg cm P, sg = (-1)^(l - l0) relative to l0) then follow from sum c P and sum c M, each split by
+// the parity of l - l0.  s[0..1] = even c P, s[2..3] = even c M, s[4..5] = odd c P, s[6..7] = odd c M (re, im):
+// 4 accumulate FMAs per l and ring pair instead of 8.
+CMDR_HD void d1_accum(bool odd, double P, double M, double cr, double ci, double (&s)[8]) {
+  if (odd) { s[4] = fma(P, cr, s[4]); s[5] = fma(P, ci, s[5]); s[6] = fma(M, cr, s[6]); s[7] = fma(M, ci, s[7]); }
+  else     { s[0] = fma(P, cr, s[0]); s[1] = fma(P, ci, s[1]); s[2] = fma(M, cr, s[2]); s[3] = fma(M, ci, s[3]); }
+}
+// Phases {N.re, N.im, S.re, S.im} of the two map components from the parity sums, in the combination of the spin-s
+// synthesis epilogue (a1 = sum cp P, a2 = sum cm M, a3 = sum sg cp M, a4 = sum sg cm P; Q = (a1 + a2)/2,
+// U = -i (a1 - a2)/2, south with sg0 = (-1)^(l0 + m) / 2).
+CMDR_HD void d1_combine(const double (&s)[8], double sg0, double (&q)[4], double (&u)[4]) {
+  const double a1r = s[0] + s[4], a1i = s[1] + s[5];
+  const double a2r = -(s[2] + s[6]), a2i = -(s[3] + s[7]);
+  const double a3r = s[2] - s[6], a3i = s[3] - s[7];
+  const double a4r = s[4] - s[0], a4i = s[5] - s[1];
+  q[0] = 0.5 * (a1r + a2r); q[1] = 0.5 * (a1i + a2i);
+  u[0] = 0.5 * (a1i - a2i); u[1] = -0.5 * (a1r - a2r);
+  q[2] = sg0 * (a3r + a4r); q[3] = sg0 * (a3i + a4i);
+  u[2] = sg0 * (a3i - a4i); u[3] = -sg0 * (a3r - a4r);
+}
+
 // libsharp-style per-ring m cut-off (contributions above it are far below FP64
 // resolution).  Same form as the oracle's get_mlim.
 inline int mlim_for_ring(int lmax, int spin, double sth, double cth) {

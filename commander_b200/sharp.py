@@ -217,12 +217,36 @@ def sharp_execute(type, spin, nmaps, alm, alm_info: sharp_alm_info, map, geom_in
     return None
 
 
+def alm2map_der1(alm, alm_info: sharp_alm_info, map, geom_info: sharp_geom_info, add=False, comm=None):
+    """Gradient maps of one spin-0 a_lm column (SHARP_ALM2MAP_DERIV1, healpy's alm2map_der1):
+    map[0] = dT/dtheta and map[1] = (1/sin theta) dT/dphi, where T is what SHARP_Y (spin 0) makes from
+    the same a_lm.  alm has shape (1, alm_info.n_local), map (2, geom_info.n_local); numpy or torch,
+    host or device.  No ring weights; `add` accumulates into both maps."""
+    L = lib()
+    flags = SHARP_DP | (SHARP_ADD if add else 0)
+    alm_ptr, _a = _col_ptrs(alm, 1, alm_info.n_local)
+    map_ptr, _m = _col_ptrs(map, 2, geom_info.n_local)
+    if comm is not None:
+        L.sharp_execute_mpi_fortran(int(comm), SHARP_ALM2MAP_DERIV1, 1, alm_ptr, map_ptr, geom_info.handle,
+                                    alm_info.handle, flags, None, None)
+    else:
+        L.sharp_execute(SHARP_ALM2MAP_DERIV1, 1, alm_ptr, map_ptr, geom_info.handle, alm_info.handle, flags,
+                        None, None)
+
+
 # ---- additive entry points (include/cmdr_sht.h part 2)
+
+def _check_iqu_job(type):
+    if type not in (SHARP_YtW, SHARP_Y, SHARP_Yt, SHARP_WY):
+        raise ValueError(f"job type {type} has no fused IQU form (SHARP_YtW, SHARP_Y, SHARP_Yt, SHARP_WY only)")
+
 
 def execute_iqu(type, alm, map, geom_T: sharp_geom_info, geom_P: sharp_geom_info, alm_info: sharp_alm_info,
                 add=False, stream=None, comm=None):
     """Fused T + (Q,U) transform: one call for what comm_map%Y etc. do in two
-    (commander3/src/comm_map_mod.f90:444-447).  alm (3, n_alm), map (3, n_pix)."""
+    (commander3/src/comm_map_mod.f90:444-447).  alm (3, n_alm), map (3, n_pix).  SHARP_YtW, SHARP_Y, SHARP_Yt or
+    SHARP_WY: the gradient job has no IQU form (use alm2map_der1)."""
+    _check_iqu_job(type)
     L = lib()
     flags = SHARP_DP | (SHARP_ADD if add else 0)
     alm_ptr, _a = _col_ptrs(alm, 3, alm_info.n_local)
@@ -239,6 +263,7 @@ def execute_iqu_batch(type, alms, maps, geom_T: sharp_geom_info, geom_P: sharp_g
                       add=False, stream=None):
     """nbatch fused IQU transforms with shared handles (one per frequency band); alms / maps are
     sequences of (3, n_alm) / (3, n_pix) arrays.  Host arrays are pipelined band against band."""
+    _check_iqu_job(type)
     L = lib()
     nb = len(alms)
     if nb != len(maps):

@@ -80,7 +80,14 @@ ptrdiff_t sharp_map_size(const sharp_geom_info *info);
  * double array.  The pointers may be host memory (pageable or pinned; the
  * Fortran case) or device memory (detected with cudaPointerGetAttributes).
  * spin 0, or any spin 1..32 (two components; conviqt calls spin j, comm_conviqt_mod.f90:254).  `time` (seconds) and `opcnt` (nominal flops) are
- * optional outputs. */
+ * optional outputs.
+ *
+ * SHARP_ALM2MAP_DERIV1 (healpy's alm2map_der1): `alm` holds ONE pointer, a spin-0 a_lm set with the SHARP_Y spin-0
+ * convention; `map` holds TWO, which receive d_theta T and (1/sin theta) d_phi T of the map T that SHARP_Y (spin 0)
+ * would make from it (theta colatitude, phi the ring's HEALPix azimuth).  `spin` is ignored.  No ring weights;
+ * SHARP_ADD adds to both maps; SHARP_NO_FFT aborts; l = 0 contributes nothing.  The same holds for
+ * sharp_execute_mpi_fortran, cmdr_sht_execute_dev and cmdr_sht_execute_dist.  `opcnt` counts 20 nominal flops per
+ * (l, m, ring pair): 12 for the spin-1 recurrence plus 4 accumulate FMAs, with FMA = 2 (spin 0: 8, spin s: 28). */
 void sharp_execute(int type, int spin, void *alm, void *map, const sharp_geom_info *geom_info,
                    const sharp_alm_info *alm_info, int flags, double *time,
                    unsigned long long *opcnt);
