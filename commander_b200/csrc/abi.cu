@@ -59,15 +59,6 @@ static void scratch_release() {
   g_scratch.clear();
 }
 
-template <typename T>
-static T *upload(const std::vector<T> &v) {  // (dist.cu has its own copy)
-  T *d = nullptr;
-  size_t n = v.size() ? v.size() : 1;
-  CMDR_CUDA_CHECK(cudaMalloc(&d, sizeof(T) * n));
-  if (v.size()) CMDR_CUDA_CHECK(cudaMemcpy(d, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
-  return d;
-}
-
 // ---------------------------------------------------------------- device residency
 void ensure_alm_device(sharp_alm_info *a) {
   int dev = 0;
@@ -419,8 +410,8 @@ void forget_layout(const sharp_alm_info *a) {
   g_idlayout.erase(it);
 }
 
-// `classic`: spin 0 with the one-step table {A', g} (invn.cu); the transforms use the two-l-per-step tables
-LegAlm make_legalm(sharp_alm_info *a, int spin, bool classic) {
+LegAlm make_legalm(sharp_alm_info *a, const Job &job, const double *const *lscale, bool classic) {
+  const int spin = job.spin;
   ensure_alm_device(a);
   const int key = (spin == 0 && !classic) ? COEF_KEY_S0X2 : spin;
   ensure_coef(a, key);
@@ -437,28 +428,26 @@ LegAlm make_legalm(sharp_alm_info *a, int spin, bool classic) {
     A.front_coef = a->coef[COEF_KEY_S0X2].tab; A.front_mix = a->coef[COEF_KEY_S0X2].tab2; A.front_cofs = a->coef[COEF_KEY_S0X2].ofs;
     A.front_K0 = ensure_start_norms(a, 0);
   }
+  A.deriv1 = job.deriv1;
+  if (lscale)
+    for (int c = 0; c < job.alm_cols; ++c) A.lscale[c] = lscale[c];
   return A;
 }
 
 // Single-GPU transform with device pointers.  `ph` holds ncomp_tot components; this call
 // handles components [comp0, comp0+ncomp) of it.
-void run_single(int type, int spin, double *const *alm, double *const *map, sharp_geom_info *g,
-                sharp_alm_info *a, int flags, cudaStream_t st, const XformOpts *opts, int comp_off) {
-  if (type < 0 || type > SHARP_ALM2MAP_DERIV1) { fprintf(stderr, "cmdr_sht: job type %d unsupported\n", type); abort(); }
-  spin = job_spin(type, spin);
-  if (spin < 0 || spin > CMDR_MAX_SPIN) { fprintf(stderr, "cmdr_sht: spin %d unsupported (0..%d)\n", spin, CMDR_MAX_SPIN); abort(); }
-  if (flags & SHARP_NO_FFT) { fprintf(stderr, "cmdr_sht: SHARP_NO_FFT unsupported\n"); abort(); }
-  const int ncomp = job_map_cols(type, spin);   // map columns and phase components (the a_lm side of a synthesis reads what it needs)
-  const bool synth = job_synth(type);
-  const bool add = (flags & SHARP_ADD) != 0;
+void run_single(const Job &job, double *const *alm, double *const *map, sharp_geom_info *g, sharp_alm_info *a,
+                cudaStream_t st, const XformOpts *opts, int comp_off) {
+  const int spin = job.spin;
+  const int ncomp = job.map_cols;   // map columns and phase components (the a_lm side of a synthesis reads what it needs)
+  const bool synth = job.synth;
   ensure_geom_device(g);
-  LegAlm A = make_legalm(a, spin);
-  A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
+  LegAlm A = make_legalm(a, job, opts ? opts->lscale + comp_off : nullptr);
   const double *pixscale[2] = {nullptr, nullptr};
   if (opts)
-    for (int c = 0; c < ncomp; ++c) { A.lscale[c] = opts->lscale[comp_off + c]; pixscale[c] = opts->pixscale[comp_off + c]; }
+    for (int c = 0; c < ncomp; ++c) pixscale[c] = opts->pixscale[comp_off + c];
   if (g->npairs == 0 || a->nm == 0) {
-    if (!add) {
+    if (!job.add) {
       if (synth) { for (int c = 0; c < ncomp; ++c) if (g->npix) CMDR_CUDA_CHECK(cudaMemsetAsync(map[c], 0, sizeof(double) * g->npix, st)); }
       else { for (int c = 0; c < ncomp; ++c) if (a->nalm) CMDR_CUDA_CHECK(cudaMemsetAsync(alm[c], 0, sizeof(double) * a->nalm * (a->real_packed ? 1 : 2), st)); }
     }
@@ -471,20 +460,20 @@ void run_single(int type, int spin, double *const *alm, double *const *map, shar
   double4 *ph = static_cast<double4 *>(scratch_get("phase", sizeof(double4) * (size_t)ncomp * a->nm * g->npairs));
   if (synth) {
     prof_begin(spin, 0, st);
-    launch_legendre_synth(spin, G, A, alm, ph, st);
+    launch_legendre_synth(G, A, alm, ph, st);
     prof_end(st);
     prof_begin(100 + spin, 0, st);
-    ringfft_synth(g, ncomp, L, ph, map, type == SHARP_WY, add, st, opts ? pixscale : nullptr);
+    ringfft_synth(g, ncomp, L, ph, map, job.weighted, job.add, st, opts ? pixscale : nullptr);
     prof_end(st);
   } else {
     prof_begin(100 + spin, 1, st);
-    ringfft_anal(g, ncomp, L, ph, map, type == SHARP_YtW, st);
+    ringfft_anal(g, ncomp, L, ph, map, job.weighted, st);
     prof_end(st);
-    if (!add)
+    if (!job.add)
       for (int c = 0; c < ncomp; ++c)
         CMDR_CUDA_CHECK(cudaMemsetAsync(alm[c], 0, sizeof(double) * a->nalm * (a->real_packed ? 1 : 2), st));
     prof_begin(spin, 1, st);
-    launch_legendre_anal(spin, G, A, alm, ph, st);
+    launch_legendre_anal(G, A, alm, ph, st);
     prof_end(st);
   }
 }
@@ -596,13 +585,11 @@ bool alm_m_chunks(const sharp_alm_info *a, long long nalm_d, int nch, std::vecto
   return true;
 }
 
-static bool try_pipelined(int type, int spin, double *const *alm, double *const *map, sharp_geom_info *g,
-                          sharp_alm_info *a, int flags, cudaStream_t st) {
+static bool try_pipelined(const Job &job, double *const *alm, double *const *map, sharp_geom_info *g,
+                          sharp_alm_info *a, cudaStream_t st) {
   static const bool disabled = getenv("CMDR_SHT_NO_PIPELINE") != nullptr;
-  if (type < 0 || type > SHARP_ALM2MAP_DERIV1) return false;
-  spin = job_spin(type, spin);
-  const int nca = job_alm_cols(type, spin), ncomp = job_map_cols(type, spin);
-  if (disabled || (flags & SHARP_ADD) || g->npix < (1 << 21) || a->nm == 0 || spin < 0 || spin > CMDR_MAX_SPIN) return false;
+  const int spin = job.spin, nca = job.alm_cols, ncomp = job.map_cols;
+  if (disabled || job.add || g->npix < (1 << 21) || a->nm == 0) return false;
   // host arrays of either kind: pinned ones are copied in place, pageable ones (what sharp.f90:219-224 passes)
   // go through the library's pinned arena and the copy threads (hostio.cu)
   for (int c = 0; c < nca; ++c)
@@ -622,7 +609,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
   };
   auto dump_marks = [&]() {
     if (!trace) return;
-    fprintf(stderr, "[cmdr_sht pipe] type %d spin %d:", type, spin);
+    fprintf(stderr, "[cmdr_sht pipe] type %d spin %d:", job.type, spin);
     for (size_t k = 1; k < marks.size(); ++k) {
       float ms = 0;
       cudaEventElapsedTime(&ms, marks[0].second, marks[k].second);
@@ -636,10 +623,8 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
   static const int nchunks = getenv("CMDR_SHT_CHUNKS") ? atoi(getenv("CMDR_SHT_CHUNKS")) : 8;
   ensure_subgeoms(g, nchunks);
   if (g->subs.empty()) return false;
-  const bool synth = job_synth(type);
   ensure_geom_device(g);
-  LegAlm A = make_legalm(a, spin);
-  A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
+  LegAlm A = make_legalm(a, job);
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
   double *alm_buf = static_cast<double *>(scratch_get("stage_alm", sizeof(double) * (size_t)nalm_d * nca));
   double *map_buf = static_cast<double *>(scratch_get("stage_map", sizeof(double) * (size_t)g->npix * ncomp));
@@ -659,7 +644,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
   cudaStream_t cs = copy_stream();
   const int ns = (int)g->subs.size();
   mark("start", 0, st);
-  if (synth) {
+  if (job.synth) {
     // a_lm upload in NMCH chunks of local m's (the packed columns of consecutive m's are contiguous): the
     // first ring-pair chunk runs its Legendre kernel m-chunk by m-chunk as the data lands, so only the
     // first quarter of the upload is exposed.  Falls back to one copy for layouts that are not dense.
@@ -690,7 +675,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
       sharp_geom_info *sub = g->subs[i];
       L.pair0 = sub->pair0;
       mark("leg", i, st);
-      ringfft_synth(sub, ncomp, L, ph, map_dev, type == SHARP_WY, false, st);
+      ringfft_synth(sub, ncomp, L, ph, map_dev, job.weighted, false, st);
       mark("fft", i, st);
       cudaEvent_t e = pooled_event(i);
       CMDR_CUDA_CHECK(cudaEventRecord(e, st));
@@ -715,7 +700,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
         Aj.im_begin = mcut[j]; Aj.im_end = mcut[j + 1];
         // one launch over the merged slot range of the first nj chunks (consecutive ring pairs; belt first)
         G.slot_begin = g->subs[ns - nj]->pair0; G.slot_end = g->subs[ns - 1]->pair0 + g->subs[ns - 1]->npairs;
-        launch_legendre_synth(spin, G, Aj, alm_dev, ph, sj, true);
+        launch_legendre_synth(G, Aj, alm_dev, ph, sj, true);
         mark("legm", j, sj);
       }
       if (as != st) {
@@ -728,7 +713,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
     for (int i = (nmch > 1 ? ns - nj : ns) - 1; i >= 0; --i) {
       sharp_geom_info *sub = g->subs[i];
       G.slot_begin = sub->pair0; G.slot_end = sub->pair0 + sub->npairs;
-      launch_legendre_synth(spin, G, A, alm_dev, ph, st, nmch == 1 && i == ns - 1);
+      launch_legendre_synth(G, A, alm_dev, ph, st, nmch == 1 && i == ns - 1);
       finish_chunk(i);
     }
     ioM.drain();                                   // pageable caller map: rows leave the arena as their chunks land
@@ -758,10 +743,10 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
       mark("up", i, cs);
       CMDR_CUDA_CHECK(cudaStreamWaitEvent(st, e, 0));
       L.pair0 = sub->pair0;
-      ringfft_anal(sub, ncomp, L, ph, map_dev, type == SHARP_YtW, st);
+      ringfft_anal(sub, ncomp, L, ph, map_dev, job.weighted, st);
       mark("fft", i, st);
       G.slot_begin = sub->pair0; G.slot_end = sub->pair0 + sub->npairs;
-      if (i < ns - nj) { launch_legendre_anal(spin, G, A, alm_dev, ph, st); mark("leg", i, st); }
+      if (i < ns - nj) { launch_legendre_anal(G, A, alm_dev, ph, st); mark("leg", i, st); }
     }
     // last `nj` ring-pair chunks: m-chunk by m-chunk over all of them, so that the finished a_lm columns go
     // back to the host while the next m-chunk is still being accumulated (nj chunks of compute per slice of
@@ -777,7 +762,7 @@ static bool try_pipelined(int type, int spin, double *const *alm, double *const 
       LegAlm Aj = A;
       if (nmch > 1) { Aj.im_begin = mcut[j]; Aj.im_end = mcut[j + 1]; }    // (mcut is empty when the m's are not chunkable)
       G.slot_begin = g->subs[ns - nj]->pair0; G.slot_end = g->subs[ns - 1]->pair0 + g->subs[ns - 1]->npairs;
-      launch_legendre_anal(spin, G, Aj, alm_dev, ph, sj);   // merged slot range of the last nj chunks
+      launch_legendre_anal(G, Aj, alm_dev, ph, sj);   // merged slot range of the last nj chunks
       if (nmch > 1) {
         cudaEvent_t e = pooled_event(ns + 2 + j);
         CMDR_CUDA_CHECK(cudaEventRecord(e, sj));
@@ -814,28 +799,26 @@ unsigned long long nominal_flops(const sharp_geom_info *g, const sharp_alm_info 
   return lm_pair_flops(g, a, spin == 0 ? 8.0 : 28.0);
 }
 // `opcnt` of a job: DERIV1 counts 20 per (l, m, ring pair) -- 12 for the spin-1 recurrence, 4 accumulate FMAs (FMA = 2)
-unsigned long long job_opcnt(const sharp_geom_info *g, const sharp_alm_info *a, int type, int spin) {
-  return type == SHARP_ALM2MAP_DERIV1 ? lm_pair_flops(g, a, 20.0) : nominal_flops(g, a, spin);
+unsigned long long job_opcnt(const sharp_geom_info *g, const sharp_alm_info *a, const Job &job) {
+  return job.deriv1 ? lm_pair_flops(g, a, 20.0) : nominal_flops(g, a, job.spin);
 }
 
-void execute_any(int type, int spin, void *alm_v, void *map_v, sharp_geom_info *g, sharp_alm_info *a,
-                 int flags, double *time, unsigned long long *opcnt, cudaStream_t st) {
+void execute_any(const Job &job, void *alm_v, void *map_v, sharp_geom_info *g, sharp_alm_info *a, double *time,
+                 unsigned long long *opcnt, cudaStream_t st) {
   auto t0 = std::chrono::steady_clock::now();
-  const int nca = job_alm_cols(type, spin), ncm = job_map_cols(type, spin);
-  const bool synth = job_synth(type);
-  const bool add = (flags & SHARP_ADD) != 0;
+  const bool synth = job.synth, add = job.add;
   double *const *alm = static_cast<double *const *>(alm_v);
   double *const *map = static_cast<double *const *>(map_v);
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
-  if (!try_pipelined(type, spin, alm, map, g, a, flags, st)) {
-    Staged sa = stage_in("stage_alm", alm, nca, nalm_d, synth || add, st);
-    Staged sm = stage_in("stage_map", map, ncm, g->npix, !synth || add, st);
-    run_single(type, spin, sa.dev.data(), sm.dev.data(), g, a, flags, st);
+  if (!try_pipelined(job, alm, map, g, a, st)) {
+    Staged sa = stage_in("stage_alm", alm, job.alm_cols, nalm_d, synth || add, st);
+    Staged sm = stage_in("stage_map", map, job.map_cols, g->npix, !synth || add, st);
+    run_single(job, sa.dev.data(), sm.dev.data(), g, a, st);
     if (synth) stage_out(sm, g->npix, st); else stage_out(sa, nalm_d, st);
     if (sa.staged || sm.staged || time) CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
   }
   if (time) *time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-  if (opcnt) *opcnt = job_opcnt(g, a, type, spin);
+  if (opcnt) *opcnt = job_opcnt(g, a, job);
 }
 
 }  // namespace cmdr
@@ -844,8 +827,9 @@ extern "C" {
 
 void sharp_execute(int type, int spin, void *alm, void *map, const sharp_geom_info *geom_info,
                    const sharp_alm_info *alm_info, int flags, double *time, unsigned long long *opcnt) {
-  execute_any(type, spin, alm, map, const_cast<sharp_geom_info *>(geom_info),
-              const_cast<sharp_alm_info *>(alm_info), flags, time, opcnt, (cudaStream_t)0);
+  const Job job = job_or_abort("sharp_execute", type, spin, flags);
+  execute_any(job, alm, map, const_cast<sharp_geom_info *>(geom_info), const_cast<sharp_alm_info *>(alm_info), time,
+              opcnt, (cudaStream_t)0);
 }
 
 int cmdr_sht_version(void) { return 100; }
@@ -853,24 +837,25 @@ int cmdr_sht_version(void) { return 100; }
 void cmdr_sht_execute_dev(int type, int spin, double *const *alm, double *const *map,
                           const sharp_geom_info *geom_info, const sharp_alm_info *alm_info, int flags,
                           void *stream) {
-  run_single(type, spin, alm, map, const_cast<sharp_geom_info *>(geom_info),
-             const_cast<sharp_alm_info *>(alm_info), flags, (cudaStream_t)stream);
+  const Job job = job_or_abort("cmdr_sht_execute_dev", type, spin, flags);
+  run_single(job, alm, map, const_cast<sharp_geom_info *>(geom_info), const_cast<sharp_alm_info *>(alm_info),
+             (cudaStream_t)stream);
 }
 
 void cmdr_sht_execute_iqu(int type, double *const *alm3, double *const *map3, const sharp_geom_info *geom_T,
                           const sharp_geom_info *geom_P, const sharp_alm_info *alm_info, int flags,
                           void *stream) {
-  require_iqu_job(type, "cmdr_sht_execute_iqu");
+  const Job jT = job_or_abort("cmdr_sht_execute_iqu", type, 0, flags, true);
+  const Job jP = job_or_abort("cmdr_sht_execute_iqu", type, 2, flags, true);
   cudaStream_t st = (cudaStream_t)stream;
   sharp_geom_info *gT = const_cast<sharp_geom_info *>(geom_T), *gP = const_cast<sharp_geom_info *>(geom_P);
   sharp_alm_info *a = const_cast<sharp_alm_info *>(alm_info);
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
-  const bool add = (flags & SHARP_ADD) != 0;
+  const bool synth = jT.synth, add = jT.add;
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
   Staged sa = stage_in("stage_alm", alm3, 3, nalm_d, synth || add, st);
   Staged sm = stage_in("stage_map", map3, 3, gT->npix, !synth || add, st);
-  run_single(type, 0, sa.dev.data(), sm.dev.data(), gT, a, flags, st);
-  run_single(type, 2, sa.dev.data() + 1, sm.dev.data() + 1, gP, a, flags, st);
+  run_single(jT, sa.dev.data(), sm.dev.data(), gT, a, st);
+  run_single(jP, sa.dev.data() + 1, sm.dev.data() + 1, gP, a, st);
   if (synth) stage_out(sm, gT->npix, st); else stage_out(sa, nalm_d, st);
   if (sa.staged || sm.staged) CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
 }
@@ -883,12 +868,12 @@ void cmdr_sht_execute_iqu(int type, double *const *alm3, double *const *map3, co
 void cmdr_sht_execute_iqu_batch(int type, int nbatch, double *const *alm3, double *const *map3,
                                 const sharp_geom_info *geom_T, const sharp_geom_info *geom_P,
                                 const sharp_alm_info *alm_info, int flags, void *stream) {
-  require_iqu_job(type, "cmdr_sht_execute_iqu_batch");
+  const Job jT = job_or_abort("cmdr_sht_execute_iqu_batch", type, 0, flags, true);
+  const Job jP = job_or_abort("cmdr_sht_execute_iqu_batch", type, 2, flags, true);
   cudaStream_t st = (cudaStream_t)stream;
   sharp_geom_info *gT = const_cast<sharp_geom_info *>(geom_T), *gP = const_cast<sharp_geom_info *>(geom_P);
   sharp_alm_info *a = const_cast<sharp_alm_info *>(alm_info);
-  const bool synth = (type == SHARP_Y || type == SHARP_WY);
-  const bool add = (flags & SHARP_ADD) != 0;
+  const bool synth = jT.synth, add = jT.add;
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
   const long long npix = gT->npix;
   if (nbatch <= 0) return;
@@ -947,8 +932,8 @@ void cmdr_sht_execute_iqu_batch(int type, int nbatch, double *const *alm3, doubl
     if (b >= 2) CMDR_CUDA_CHECK(cudaStreamWaitEvent(st, down[b - 2], 0));
     double *ap[3], *mp[3];
     for (int c = 0; c < 3; ++c) { ap[c] = abuf[s] + (size_t)c * nalm_d; mp[c] = mbuf[s] + (size_t)c * npix; }
-    run_single(type, 0, ap, mp, gT, a, flags, st);
-    run_single(type, 2, ap + 1, mp + 1, gP, a, flags, st);
+    run_single(jT, ap, mp, gT, a, st);
+    run_single(jP, ap + 1, mp + 1, gP, a, st);
     CMDR_CUDA_CHECK(cudaEventRecord(done[b], st));
     // download band b
     CMDR_CUDA_CHECK(cudaStreamWaitEvent(cout, done[b], 0));

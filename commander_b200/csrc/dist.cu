@@ -83,15 +83,6 @@ static NcclApi *nccl_api() {
   return &api;
 }
 
-template <typename T>
-static T *upload_v(const std::vector<T> &v) {
-  T *d = nullptr;
-  size_t n = v.size() ? v.size() : 1;
-  CMDR_CUDA_CHECK(cudaMalloc(&d, sizeof(T) * n));
-  if (v.size()) CMDR_CUDA_CHECK(cudaMemcpy(d, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
-  return d;
-}
-
 struct DistPlan {
   int NPL = 0, NML = 0, mmax = -1, nm_total = 0;
   int nslots = 0;
@@ -190,7 +181,7 @@ static DistComm *comm_or_local(int comm, const sharp_geom_info *g, const sharp_a
 static std::vector<int> allgather_ints(DistComm *C, const std::vector<int> &mine, int n, cudaStream_t st) {
   std::vector<int> pad(n, -1);
   std::copy(mine.begin(), mine.end(), pad.begin());
-  int *d_in = upload_v(pad), *d_out = nullptr;
+  int *d_in = upload(pad), *d_out = nullptr;
   CMDR_CUDA_CHECK(cudaMalloc(&d_out, sizeof(int) * (size_t)n * C->nranks));
   CMDR_NCCL_CHECK(nccl_api()->AllGather(d_in, d_out, n, ncclInt32, C->nccl, st));
   std::vector<int> out((size_t)n * C->nranks);
@@ -255,8 +246,8 @@ static DistPlan *get_plan(DistComm *C, sharp_geom_info *g, sharp_alm_info *a, cu
     while (ci < (int)P->wcut.size()) P->lcut[ci++] = mine;
   }
   for (int s2 = 0; s2 < P->nslots; ++s2) if (!used[s2]) wslot[w++] = s2;   // padding slots: zero-filled, never read
-  P->d_trig = upload_v(trig);
-  P->d_wslot = upload_v(wslot);
+  P->d_trig = upload(trig);
+  P->d_wslot = upload(wslot);
   // global m tables
   int mmax = -1;
   for (int r = 0; r < R; ++r) for (int i = 0; i < sz[4 * r]; ++i) mmax = std::max(mmax, all_m[(size_t)r * NML + i]);
@@ -270,8 +261,8 @@ static DistPlan *get_plan(DistComm *C, sharp_geom_info *g, sharp_alm_info *a, cu
       mlist.push_back(m); mlist_src.push_back(r); mlist_im.push_back(i);
     }
   P->nm_total = (int)mlist.size();
-  P->d_m2src = upload_v(m2src); P->d_m2im = upload_v(m2im);
-  P->d_mlist = upload_v(mlist); P->d_mlist_src = upload_v(mlist_src); P->d_mlist_im = upload_v(mlist_im);
+  P->d_m2src = upload(m2src); P->d_m2im = upload(m2im);
+  P->d_mlist = upload(mlist); P->d_mlist_src = upload(mlist_src); P->d_mlist_im = upload(mlist_im);
   C->plans[key] = P;
   return P;
 }
@@ -282,7 +273,7 @@ static const int *plan_mlim(DistPlan *P, int lmax, int spin) {
   std::vector<int> ml(P->nslots, -1);
   for (int s = 0; s < P->nslots; ++s)
     if (P->h_valid[s]) ml[s] = mlim_for_ring(lmax, spin, P->h_sth[s], P->h_cth[s]);
-  int *d = upload_v(ml);
+  int *d = upload(ml);
   P->d_mlim[spin] = d;
   return d;
 }
@@ -416,18 +407,16 @@ static void alltoall_blocks(DistComm *C, const double *send, double *recv, size_
 }
 
 struct Part {
-  int spin, comp0, ncomp; sharp_geom_info *g; double *const *alm; double *const *map;
+  Job job; int comp0; sharp_geom_info *g; double *const *alm; double *const *map;
   const double *lscale[2] = {nullptr, nullptr}, *pixscale[2] = {nullptr, nullptr};   // fused factors (XformOpts)
   bool has_ps() const { return pixscale[0] || pixscale[1]; }
 };
 
-// Distributed transform over `parts` (one part = one spin with its geometry); all parts
+// Distributed transform over `parts` (one part = one spin with its geometry; all of the same job type); all parts
 // share one phase buffer of ncomp_tot components and one exchange.
-static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int ncomp_tot, sharp_alm_info *a,
-                     int flags, cudaStream_t st) {
-  if (type < 0 || type > SHARP_ALM2MAP_DERIV1) { fprintf(stderr, "cmdr_sht: job type %d unsupported\n", type); abort(); }
-  const bool synth = job_synth(type);
-  const bool add = (flags & SHARP_ADD) != 0;
+static void run_dist(DistComm *C, const Part *parts, int nparts, int ncomp_tot, sharp_alm_info *a, cudaStream_t st) {
+  const Job &job = parts[0].job;
+  const bool synth = job.synth, add = job.add;
   sharp_geom_info *g0 = parts[0].g;
   for (int i = 0; i < nparts; ++i) {
     ensure_geom_device(parts[i].g);
@@ -457,12 +446,10 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
     prof_end(st);
     for (int i = 0; i < nparts; ++i) {
       const Part &p = parts[i];
-      LegAlm A = make_legalm(a, p.spin);
-      A.lscale[0] = p.lscale[0]; A.lscale[1] = p.lscale[1];
-      A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
-      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.spin);
-      prof_begin(p.spin, 0, st);
-      launch_legendre_synth(p.spin, G, A, p.alm, reinterpret_cast<double4 *>(B.mine), st);
+      LegAlm A = make_legalm(a, p.job, p.lscale);
+      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.job.spin);
+      prof_begin(p.job.spin, 0, st);
+      launch_legendre_synth(G, A, p.alm, reinterpret_cast<double4 *>(B.mine), st);
       prof_end(st);
     }
     prof_begin(201, 0, st);
@@ -472,8 +459,8 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
       const Part &p = parts[i];
       L.comp0 = p.comp0;
       if (p.g->npairs == 0) continue;
-      prof_begin(100 + p.spin, 0, st);
-      ringfft_synth(p.g, p.ncomp, L, reinterpret_cast<double4 *>(B.mine), p.map, type == SHARP_WY, add, st,
+      prof_begin(100 + p.job.spin, 0, st);
+      ringfft_synth(p.g, p.job.map_cols, L, reinterpret_cast<double4 *>(B.mine), p.map, job.weighted, add, st,
                     p.has_ps() ? p.pixscale : nullptr);
       prof_end(st);
     }
@@ -492,8 +479,8 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
       const Part &p = parts[i];
       L.comp0 = p.comp0;
       if (p.g->npairs == 0) continue;
-      prof_begin(100 + p.spin, 1, st);
-      ringfft_anal(p.g, p.ncomp, L, reinterpret_cast<double4 *>(B.mine), p.map, type == SHARP_YtW, st);
+      prof_begin(100 + p.job.spin, 1, st);
+      ringfft_anal(p.g, p.job.map_cols, L, reinterpret_cast<double4 *>(B.mine), p.map, job.weighted, st);
       prof_end(st);
     }
     prof_begin(201, 1, st);
@@ -501,14 +488,13 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
     prof_end(st);
     for (int i = 0; i < nparts; ++i) {
       const Part &p = parts[i];
-      LegAlm A = make_legalm(a, p.spin);
-      A.lscale[0] = p.lscale[0]; A.lscale[1] = p.lscale[1];
-      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.spin);
+      LegAlm A = make_legalm(a, p.job, p.lscale);
+      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.job.spin);
       const size_t nd = (size_t)a->nalm * (a->real_packed ? 1 : 2);
       if (!add && nd)
-        for (int c = 0; c < p.ncomp; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(p.alm[c], 0, sizeof(double) * nd, st));
-      prof_begin(p.spin, 1, st);
-      launch_legendre_anal(p.spin, G, A, p.alm, reinterpret_cast<const double4 *>(B.mine), st);
+        for (int c = 0; c < p.job.alm_cols; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(p.alm[c], 0, sizeof(double) * nd, st));
+      prof_begin(p.job.spin, 1, st);
+      launch_legendre_anal(G, A, p.alm, reinterpret_cast<const double4 *>(B.mine), st);
       prof_end(st);
     }
     return;
@@ -521,12 +507,10 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
     if (a->nm < P->NML) CMDR_CUDA_CHECK(cudaMemsetAsync(bufA, 0, sizeof(double) * block * C->nranks, st));
     for (int i = 0; i < nparts; ++i) {
       const Part &p = parts[i];
-      LegAlm A = make_legalm(a, p.spin);
-      A.lscale[0] = p.lscale[0]; A.lscale[1] = p.lscale[1];
-      A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
-      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.spin);
-      prof_begin(p.spin, 0, st);
-      launch_legendre_synth(p.spin, G, A, p.alm, reinterpret_cast<double4 *>(bufA), st);
+      LegAlm A = make_legalm(a, p.job, p.lscale);
+      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.job.spin);
+      prof_begin(p.job.spin, 0, st);
+      launch_legendre_synth(G, A, p.alm, reinterpret_cast<double4 *>(bufA), st);
       prof_end(st);
     }
     prof_begin(200, 0, st);
@@ -536,8 +520,8 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
       const Part &p = parts[i];
       L.comp0 = p.comp0;
       if (p.g->npairs == 0) continue;
-      prof_begin(100 + p.spin, 0, st);
-      ringfft_synth(p.g, p.ncomp, L, reinterpret_cast<double4 *>(bufB), p.map, type == SHARP_WY, add, st,
+      prof_begin(100 + p.job.spin, 0, st);
+      ringfft_synth(p.g, p.job.map_cols, L, reinterpret_cast<double4 *>(bufB), p.map, job.weighted, add, st,
                     p.has_ps() ? p.pixscale : nullptr);
       prof_end(st);
     }
@@ -547,8 +531,8 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
       const Part &p = parts[i];
       L.comp0 = p.comp0;
       if (p.g->npairs == 0) continue;
-      prof_begin(100 + p.spin, 1, st);
-      ringfft_anal(p.g, p.ncomp, L, reinterpret_cast<double4 *>(bufA), p.map, type == SHARP_YtW, st);
+      prof_begin(100 + p.job.spin, 1, st);
+      ringfft_anal(p.g, p.job.map_cols, L, reinterpret_cast<double4 *>(bufA), p.map, job.weighted, st);
       prof_end(st);
     }
     prof_begin(200, 1, st);
@@ -556,14 +540,13 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
     prof_end(st);
     for (int i = 0; i < nparts; ++i) {
       const Part &p = parts[i];
-      LegAlm A = make_legalm(a, p.spin);
-      A.lscale[0] = p.lscale[0]; A.lscale[1] = p.lscale[1];
-      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.spin);
+      LegAlm A = make_legalm(a, p.job, p.lscale);
+      G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.job.spin);
       const size_t nd = (size_t)a->nalm * (a->real_packed ? 1 : 2);
       if (!add && nd)
-        for (int c = 0; c < p.ncomp; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(p.alm[c], 0, sizeof(double) * nd, st));
-      prof_begin(p.spin, 1, st);
-      launch_legendre_anal(p.spin, G, A, p.alm, reinterpret_cast<const double4 *>(bufB), st);
+        for (int c = 0; c < p.job.alm_cols; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(p.alm[c], 0, sizeof(double) * nd, st));
+      prof_begin(p.job.spin, 1, st);
+      launch_legendre_anal(G, A, p.alm, reinterpret_cast<const double4 *>(bufB), st);
       prof_end(st);
     }
   }
@@ -573,12 +556,11 @@ static void run_dist(DistComm *C, int type, const Part *parts, int nparts, int n
 // the work slots are processed in chunks with one exchange barrier per chunk, so that the PCIe copy of the map
 // rows of chunk c runs beside the Legendre kernel of chunk c+-1 (synthesis: D2H after each chunk's FFT;
 // analysis: H2D ahead of each chunk's FFT).  Every rank walks the same chunks, so the barriers match.
-static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *alm, double *const *map,
-                               sharp_geom_info *g, sharp_alm_info *a, int flags, cudaStream_t st) {
+static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, double *const *map,
+                               sharp_geom_info *g, sharp_alm_info *a, cudaStream_t st) {
   static const bool disabled = getenv("CMDR_SHT_NO_PIPELINE") != nullptr;
-  const int nca = job_alm_cols(type, spin), ncomp = job_map_cols(type, spin);
-  if (disabled || (flags & SHARP_ADD) || !use_p2p(C) || type < 0 || type > SHARP_ALM2MAP_DERIV1) return false;
-  spin = job_spin(type, spin);
+  const int spin = job.spin, nca = job.alm_cols, ncomp = job.map_cols;
+  if (disabled || job.add || !use_p2p(C)) return false;
   // Every rank must take the same decision (the chunked path has K + 1 exchange barriers, the plain one 2).
   // Global sizes are equal everywhere by construction; host-versus-device buffers is a property of the call
   // site, the same on all ranks of a collective call (pinned or pageable does not matter: both take this
@@ -589,7 +571,7 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
     if (host_kind(alm[c]) == HostKind::Device) return false;
   for (int c = 0; c < ncomp; ++c)
     if (host_kind(map[c]) == HostKind::Device) return false;
-  const bool synth = job_synth(type);
+  const bool synth = job.synth;
   ensure_geom_device(g);
   ensure_alm_device(a);
   DistPlan *P = get_plan(C, g, a, st);
@@ -632,8 +614,7 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
   PeerBuf &B = C->pb[synth ? 1 : 0];
   G.npeer = C->nranks; G.src_rank = C->rank;
   for (int r = 0; r < C->nranks; ++r) G.peer[r] = reinterpret_cast<double4 *>(B.peer[r]);
-  LegAlm A = make_legalm(a, spin);
-  A.deriv1 = type == SHARP_ALM2MAP_DERIV1;
+  LegAlm A = make_legalm(a, job);
   cudaStream_t cs = copy_stream();
   const size_t ev0 = 32;                                  // events 0..31 belong to the single-GPU pipeline
   HostIO ioA, ioM;                                        // pageable caller arrays go through the pinned arena (hostio.cu)
@@ -666,16 +647,16 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
           CMDR_CUDA_CHECK(cudaStreamWaitEvent(st, ej, 0));
           LegAlm Aj = A;
           Aj.im_begin = mcut[j]; Aj.im_end = mcut[j + 1];
-          launch_legendre_synth(spin, G, Aj, alm_dev, reinterpret_cast<double4 *>(B.mine), st, true);
+          launch_legendre_synth(G, Aj, alm_dev, reinterpret_cast<double4 *>(B.mine), st, true);
         }
       } else {
-        launch_legendre_synth(spin, G, A, alm_dev, reinterpret_cast<double4 *>(B.mine), st, c == K - 1);
+        launch_legendre_synth(G, A, alm_dev, reinterpret_cast<double4 *>(B.mine), st, c == K - 1);
       }
       stream_barrier(C, st);                               // chunk c has landed everywhere
       sharp_geom_info *sub = P->subs[c];
       if (!sub) continue;
       L.pair0 = sub->pair0;
-      ringfft_synth(sub, ncomp, L, reinterpret_cast<double4 *>(B.mine), map_dev, type == SHARP_WY, false, st);
+      ringfft_synth(sub, ncomp, L, reinterpret_cast<double4 *>(B.mine), map_dev, job.weighted, false, st);
       cudaEvent_t e = pooled_event(ev0 + c);
       CMDR_CUDA_CHECK(cudaEventRecord(e, st));
       CMDR_CUDA_CHECK(cudaStreamWaitEvent(cs, e, 0));
@@ -709,7 +690,7 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
         CMDR_CUDA_CHECK(cudaEventRecord(e, cs));
         CMDR_CUDA_CHECK(cudaStreamWaitEvent(st, e, 0));
         L.pair0 = sub->pair0;
-        ringfft_anal(sub, ncomp, L, reinterpret_cast<double4 *>(B.mine), map_dev, type == SHARP_YtW, st);
+        ringfft_anal(sub, ncomp, L, reinterpret_cast<double4 *>(B.mine), map_dev, job.weighted, st);
       }
       stream_barrier(C, st);                               // chunk c is complete on every rank
       G.slot_begin = P->wcut[c]; G.slot_end = P->wcut[c + 1];
@@ -717,7 +698,7 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
         for (int j = 0; j < nmch; ++j) {
           LegAlm Aj = A;
           Aj.im_begin = mcut[j]; Aj.im_end = mcut[j + 1];
-          launch_legendre_anal(spin, G, Aj, alm_dev, reinterpret_cast<const double4 *>(B.mine), st);
+          launch_legendre_anal(G, Aj, alm_dev, reinterpret_cast<const double4 *>(B.mine), st);
           cudaEvent_t ej = pooled_event(evm + NMCH + j);
           CMDR_CUDA_CHECK(cudaEventRecord(ej, st));
           CMDR_CUDA_CHECK(cudaStreamWaitEvent(cs, ej, 0));
@@ -726,7 +707,7 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
           ioA.commit(cs);
         }
       } else {
-        launch_legendre_anal(spin, G, A, alm_dev, reinterpret_cast<const double4 *>(B.mine), st);
+        launch_legendre_anal(G, A, alm_dev, reinterpret_cast<const double4 *>(B.mine), st);
       }
     }
     if (nmch == 1) {
@@ -740,31 +721,29 @@ static bool try_dist_pipelined(DistComm *C, int type, int spin, double *const *a
   return true;
 }
 
-static void execute_dist_any(DistComm *C, int type, int nparts, const int *spins, double *const *alm,
-                             double *const *map, sharp_geom_info *const *geoms, sharp_alm_info *a, int flags,
-                             cudaStream_t st, const XformOpts *opts = nullptr) {
-  if (type == SHARP_ALM2MAP_DERIV1 && nparts != 1) require_iqu_job(type, "execute_dist_any");
-  const bool synth = job_synth(type);
-  const bool add = (flags & SHARP_ADD) != 0;
+// `jobs`: one per part, all of the same type (T alone, or T and P of a fused IQU call)
+static void execute_dist_any(DistComm *C, const Job *jobs, int nparts, double *const *alm, double *const *map,
+                             sharp_geom_info *const *geoms, sharp_alm_info *a, cudaStream_t st,
+                             const XformOpts *opts = nullptr) {
+  const bool synth = jobs[0].synth, add = jobs[0].add;
   // a_lm and map columns: equal except for DERIV1 (one part: 1 a_lm column, 2 maps)
   int ncomp_tot = 0, nalm_tot = 0;
-  for (int i = 0; i < nparts; ++i) { ncomp_tot += job_map_cols(type, spins[i]); nalm_tot += job_alm_cols(type, spins[i]); }
+  for (int i = 0; i < nparts; ++i) { ncomp_tot += jobs[i].map_cols; nalm_tot += jobs[i].alm_cols; }
   const long long nalm_d = a->nalm * (a->real_packed ? 1 : 2);
-  if (nparts == 1 && !opts && try_dist_pipelined(C, type, spins[0], alm, map, geoms[0], a, flags, st)) return;
+  if (nparts == 1 && !opts && try_dist_pipelined(C, jobs[0], alm, map, geoms[0], a, st)) return;
   Staged sa = stage_in("stage_alm", alm, nalm_tot, nalm_d, synth || add, st);
   Staged sm = stage_in("stage_map", map, ncomp_tot, geoms[0]->npix, !synth || add, st);
   Part parts[4];
   int c0 = 0, ca = 0;
   for (int i = 0; i < nparts; ++i) {
-    const int spin = job_spin(type, spins[i]), nc = job_map_cols(type, spins[i]);
-    if (spin < 0 || spin > CMDR_MAX_SPIN) { fprintf(stderr, "cmdr_sht: spin %d unsupported\n", spin); abort(); }
-    parts[i] = Part{spin, c0, nc, geoms[i], sa.dev.data() + ca, sm.dev.data() + c0};
-    ca += job_alm_cols(type, spins[i]);
+    const int nc = jobs[i].map_cols;
+    parts[i] = Part{jobs[i], c0, geoms[i], sa.dev.data() + ca, sm.dev.data() + c0};
+    ca += jobs[i].alm_cols;
     if (opts)
       for (int c = 0; c < nc; ++c) { parts[i].lscale[c] = opts->lscale[c0 + c]; parts[i].pixscale[c] = opts->pixscale[c0 + c]; }
     c0 += nc;
   }
-  run_dist(C, type, parts, nparts, ncomp_tot, a, flags, st);
+  run_dist(C, parts, nparts, ncomp_tot, a, st);
   if (synth) stage_out(sm, geoms[0]->npix, st); else stage_out(sa, nalm_d, st);
   if (sa.staged || sm.staged) CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
 }
@@ -779,16 +758,16 @@ int effective_comm(int comm, const sharp_geom_info *g, const sharp_alm_info *a, 
 // on a registered communicator (cr.cu)
 void execute_iqu_opts(int comm, int type, int nmaps, double *const *alm, double *const *map, sharp_geom_info *gT,
                       sharp_geom_info *gP, sharp_alm_info *a, int flags, const XformOpts *opts, cudaStream_t st) {
-  require_iqu_job(type, "execute_iqu_opts");
+  const Job jobs[2] = {job_or_abort("execute_iqu_opts", type, 0, flags, true),
+                       job_or_abort("execute_iqu_opts", type, 2, flags, true)};
   DistComm *C = comm_or_local(comm, gT, a, "cmdr_cr");
   if (!C) {
-    run_single(type, 0, alm, map, gT, a, flags, st, opts, 0);
-    if (nmaps == 3) run_single(type, 2, alm + 1, map + 1, gP, a, flags, st, opts, 1);
+    run_single(jobs[0], alm, map, gT, a, st, opts, 0);
+    if (nmaps == 3) run_single(jobs[1], alm + 1, map + 1, gP, a, st, opts, 1);
     return;
   }
-  int spins[2] = {0, 2};
   sharp_geom_info *gs[2] = {gT, gP};
-  execute_dist_any(C, type, nmaps == 3 ? 2 : 1, spins, alm, map, gs, a, flags, st, opts);
+  execute_dist_any(C, jobs, nmaps == 3 ? 2 : 1, alm, map, gs, a, st, opts);
 }
 
 // map *= F, the pixel-space mixing step between Y and YtW (HBM-bound: 24 bytes per pixel)
@@ -848,30 +827,30 @@ void cmdr_sht_comm_set_exchange(int comm, int mode) {
 
 void cmdr_sht_execute_dist(int comm, int type, int spin, void *alm, void *map, const sharp_geom_info *geom_info,
                            const sharp_alm_info *alm_info, int flags, void *stream) {
+  const Job job = job_or_abort("cmdr_sht_execute_dist", type, spin, flags);
   sharp_geom_info *g = const_cast<sharp_geom_info *>(geom_info);
   sharp_alm_info *a = const_cast<sharp_alm_info *>(alm_info);
   DistComm *C = comm_or_local(comm, g, a, "cmdr_sht_execute_dist");
   if (!C) {
-    execute_any(type, spin, alm, map, g, a, flags, nullptr, nullptr, (cudaStream_t)stream);
+    execute_any(job, alm, map, g, a, nullptr, nullptr, (cudaStream_t)stream);
     return;
   }
-  execute_dist_any(C, type, 1, &spin, static_cast<double *const *>(alm), static_cast<double *const *>(map), &g, a,
-                   flags, (cudaStream_t)stream);
+  execute_dist_any(C, &job, 1, static_cast<double *const *>(alm), static_cast<double *const *>(map), &g, a,
+                   (cudaStream_t)stream);
 }
 
 void cmdr_sht_execute_iqu_dist(int comm, int type, double *const *alm3, double *const *map3,
                                const sharp_geom_info *geom_T, const sharp_geom_info *geom_P,
                                const sharp_alm_info *alm_info, int flags, void *stream) {
-  require_iqu_job(type, "cmdr_sht_execute_iqu_dist");
+  const Job jobs[2] = {job_or_abort("cmdr_sht_execute_iqu_dist", type, 0, flags, true),
+                       job_or_abort("cmdr_sht_execute_iqu_dist", type, 2, flags, true)};
   DistComm *C = comm_or_local(comm, geom_T, alm_info, "cmdr_sht_execute_iqu_dist");
   if (!C) {
     cmdr_sht_execute_iqu(type, alm3, map3, geom_T, geom_P, alm_info, flags, stream);
     return;
   }
-  int spins[2] = {0, 2};
   sharp_geom_info *gs[2] = {const_cast<sharp_geom_info *>(geom_T), const_cast<sharp_geom_info *>(geom_P)};
-  execute_dist_any(C, type, 2, spins, alm3, map3, gs, const_cast<sharp_alm_info *>(alm_info), flags,
-                   (cudaStream_t)stream);
+  execute_dist_any(C, jobs, 2, alm3, map3, gs, const_cast<sharp_alm_info *>(alm_info), (cudaStream_t)stream);
 }
 
 void cmdr_sht_allreduce_sum(int comm, double *dev_buf, int n, void *stream) {
@@ -971,19 +950,20 @@ void cmdr_sht_mix(int comm, int nmaps, double *const *alm, const double *const *
 void sharp_execute_mpi_fortran(int comm, int type, int spin, void *alm, void *map,
                                const sharp_geom_info *geom_info, const sharp_alm_info *alm_info, int flags,
                                double *time, unsigned long long *opcnt) {
+  const Job job = job_or_abort("sharp_execute_mpi_fortran", type, spin, flags);
   sharp_geom_info *g = const_cast<sharp_geom_info *>(geom_info);
   sharp_alm_info *a = const_cast<sharp_alm_info *>(alm_info);
   DistComm *C = comm_or_local(comm, g, a, "sharp_execute_mpi_fortran");
   if (!C) {
-    execute_any(type, spin, alm, map, g, a, flags, time, opcnt, (cudaStream_t)0);
+    execute_any(job, alm, map, g, a, time, opcnt, (cudaStream_t)0);
     return;
   }
   auto t0 = std::chrono::steady_clock::now();
-  execute_dist_any(C, type, 1, &spin, static_cast<double *const *>(alm), static_cast<double *const *>(map), &g, a,
-                   flags, (cudaStream_t)0);
+  execute_dist_any(C, &job, 1, static_cast<double *const *>(alm), static_cast<double *const *>(map), &g, a,
+                   (cudaStream_t)0);
   if (time || opcnt) CMDR_CUDA_CHECK(cudaStreamSynchronize(0));
   if (time) *time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();   // wall seconds, as libsharp2 reports
-  if (opcnt) *opcnt = job_opcnt(geom_info, alm_info, type, spin);
+  if (opcnt) *opcnt = job_opcnt(geom_info, alm_info, job);
 }
 
 }  // extern "C"

@@ -212,7 +212,7 @@ void cmdr_sht_invn_diag(int nmaps, const double *const *a_l0, double npix, const
   for (auto &t : th) t.join();
 
   ensure_alm_device(a);
-  LegAlm A = make_legalm(a, 0, true);   // one-step spin-0 table {A', g}
+  LegAlm A = make_legalm(a, Job{}, nullptr, true);   // spin 0, one-step table {A', g}
   double *d_trig = static_cast<double *>(scratch_get("invn_trig", sizeof(double) * trig.size()));
   double *d_f = static_cast<double *>(scratch_get("invn_f", sizeof(double) * f.size()));
   CMDR_CUDA_CHECK(cudaMemcpyAsync(d_trig, trig.data(), sizeof(double) * trig.size(), cudaMemcpyHostToDevice, st));

@@ -6,12 +6,12 @@
 #include <cstdlib>
 #include <vector>
 
+#include "job.h"
 #include "sht_internal.h"
 
 namespace cmdr {
 
 constexpr int CMDR_MAX_PEERS = 8;
-constexpr int CMDR_MAX_SPIN = 32;   // start values use plain powers sh^(2s), ch^(2s): fine in FP64 up to here
 
 void count_launch(int n = 1);
 
@@ -59,18 +59,7 @@ struct LegAlm {
   bool deriv1 = false;             // SHARP_ALM2MAP_DERIV1 (spin 1 tables, one a_lm column): prep_d1 / synth_d1 kernels
 };
 
-// Column counts of a job.  SHARP_ALM2MAP_DERIV1 is a synthesis from ONE spin-0 a_lm column to TWO maps
-// {d_theta T, d_phi T / sin theta}; it runs on the spin-1 tables whatever spin the caller passes.
-inline bool job_synth(int type) { return type == SHARP_Y || type == SHARP_WY || type == SHARP_ALM2MAP_DERIV1; }
-inline int job_spin(int type, int spin) { return type == SHARP_ALM2MAP_DERIV1 ? 1 : spin; }
-inline int job_alm_cols(int type, int spin) { return type == SHARP_ALM2MAP_DERIV1 ? 1 : (spin == 0 ? 1 : 2); }
-inline int job_map_cols(int type, int spin) { return type == SHARP_ALM2MAP_DERIV1 ? 2 : (spin == 0 ? 1 : 2); }
-unsigned long long job_opcnt(const sharp_geom_info *g, const sharp_alm_info *a, int type, int spin);
-// The fused T + (Q,U) entry points (execute_iqu[_batch|_dist]) run the four map <-> a_lm jobs only: DERIV1 has one
-// a_lm column and two maps per transform, which their three-column pointer tables cannot carry.
-inline void require_iqu_job(int type, const char *who) {
-  if (type < SHARP_YtW || type > SHARP_WY) { fprintf(stderr, "cmdr_sht: %s: job type %d unsupported\n", who, type); abort(); }
-}
+unsigned long long job_opcnt(const sharp_geom_info *g, const sharp_alm_info *a, const Job &job);
 
 // Optional element-wise factors fused into a transform (cr.cu): per l on the a_lm side, per local pixel on the map
 // side of a synthesis (N^-1 of commander3/src/comm_N_rms_mod.f90:264-273 in the ring-FFT epilogue).
@@ -95,10 +84,9 @@ __host__ __device__ inline size_t ph_index(int block, int ncomp_tot, int comp, i
 // synthesis: alm (device, ncomp pointers) -> ph ; analysis: ph -> alm (atomic accumulate)
 // `prep`: (re)build the pre-scaled a_lm tile rows first; false when the same a_lm were already
 // prepared by an earlier launch of this transform (ring-pair chunks of the pipelined host path)
-void launch_legendre_synth(int spin, const LegGeom &g, const LegAlm &a, const double *const *alm,
-                           double4 *ph, cudaStream_t st, bool prep = true);
-void launch_legendre_anal(int spin, const LegGeom &g, const LegAlm &a, double *const *alm,
-                          const double4 *ph, cudaStream_t st);
+void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *const *alm, double4 *ph, cudaStream_t st,
+                           bool prep = true);
+void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm, const double4 *ph, cudaStream_t st);
 
 // Ring-FFT stage on the LOCAL rings of `geom` (ringfft.cu).
 // The phase buffer on this side is indexed
@@ -126,7 +114,9 @@ void ringfft_anal(sharp_geom_info *geom, int ncomp, const PhaseLayout &L, double
 void *scratch_get(const char *name, size_t bytes);
 void ensure_alm_device(sharp_alm_info *a);
 void ensure_geom_device(sharp_geom_info *g);
-LegAlm make_legalm(sharp_alm_info *a, int spin, bool classic = false);
+// The Legendre-stage view of `a` for `job`, with lscale[c] (nullptr: none) as the factor per l of a_lm component c.
+// `classic`: spin 0 with the one-step table {A', g} (invn.cu); the transforms use the two-l-per-step tables.
+LegAlm make_legalm(sharp_alm_info *a, const Job &job, const double *const *lscale = nullptr, bool classic = false);
 void ring_trig_ld(int nside, int north, long double &cth, long double &sth, long double &sh, long double &ch);
 bool is_device_ptr(const void *p);
 extern thread_local int g_profiling;
@@ -183,11 +173,11 @@ struct Staged {
 };
 Staged stage_in(const char *tag, double *const *ptrs, int n, long long count, bool copy_in, cudaStream_t st);
 void stage_out(Staged &s, long long count, cudaStream_t st);
-void execute_any(int type, int spin, void *alm_v, void *map_v, sharp_geom_info *g, sharp_alm_info *a,
-                 int flags, double *time, unsigned long long *opcnt, cudaStream_t st);
+void execute_any(const Job &job, void *alm_v, void *map_v, sharp_geom_info *g, sharp_alm_info *a, double *time,
+                 unsigned long long *opcnt, cudaStream_t st);
 // device-pointer transforms with fused factors (single GPU: abi.cu; any registered comm: dist.cu)
-void run_single(int type, int spin, double *const *alm, double *const *map, sharp_geom_info *g,
-                sharp_alm_info *a, int flags, cudaStream_t st, const XformOpts *opts = nullptr, int comp_off = 0);
+void run_single(const Job &job, double *const *alm, double *const *map, sharp_geom_info *g, sharp_alm_info *a,
+                cudaStream_t st, const XformOpts *opts = nullptr, int comp_off = 0);
 int effective_comm(int comm, const sharp_geom_info *g, const sharp_alm_info *a, const char *who);
 void execute_iqu_opts(int comm, int type, int nmaps, double *const *alm, double *const *map, sharp_geom_info *gT,
                       sharp_geom_info *gP, sharp_alm_info *a, int flags, const XformOpts *opts, cudaStream_t st);
@@ -203,3 +193,17 @@ void execute_iqu_opts(int comm, int type, int nmaps, double *const *alm, double 
       abort();                                                                               \
     }                                                                                        \
   } while (0)
+
+namespace cmdr {
+
+// device copy of a host vector (one element allocated for an empty one); the caller frees it
+template <typename T>
+T *upload(const std::vector<T> &v) {
+  T *d = nullptr;
+  size_t n = v.size() ? v.size() : 1;
+  CMDR_CUDA_CHECK(cudaMalloc(&d, sizeof(T) * n));
+  if (v.size()) CMDR_CUDA_CHECK(cudaMemcpy(d, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
+  return d;
+}
+
+}  // namespace cmdr

@@ -1207,12 +1207,12 @@ static void launch_w(K kernel, const KParams &p, int nm, cudaStream_t st) {   //
   kernel<<<grid, 32, 0, st>>>(p);
 }
 
-void launch_legendre_synth(int spin, const LegGeom &g, const LegAlm &a, const double *const *alm,
-                           double4 *ph, cudaStream_t st, bool prep) {
+void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *const *alm, double4 *ph, cudaStream_t st,
+                           bool prep) {
   if (a.nm == 0 || g.nslots == 0) return;
   const int nmr = (a.im_end >= 0 ? a.im_end : a.nm) - a.im_begin;   // local m's of this launch
   if (nmr <= 0) return;
-  if (a.deriv1 && spin != 1) { fprintf(stderr, "cmdr_sht: the DERIV1 synthesis runs on the spin-1 tables\n"); abort(); }
+  const int spin = a.spin;
   // DERIV1 reads one a_lm column: never touch alm[1]
   KParams p = make_params(g, a, const_cast<double *>(alm[0]), (spin && !a.deriv1) ? const_cast<double *>(alm[1]) : nullptr, ph);
   // tile rows {A', [C',] g a_lm} for all local (m, l): written once per transform (`prep`), then
@@ -1261,11 +1261,11 @@ void launch_legendre_synth(int spin, const LegGeom &g, const LegAlm &a, const do
   CMDR_CUDA_CHECK(cudaGetLastError());
 }
 
-void launch_legendre_anal(int spin, const LegGeom &g, const LegAlm &a, double *const *alm,
-                          const double4 *ph, cudaStream_t st) {
+void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm, const double4 *ph, cudaStream_t st) {
   if (a.nm == 0 || g.nslots == 0) return;
   const int nmr = (a.im_end >= 0 ? a.im_end : a.nm) - a.im_begin;   // local m's of this launch
   if (nmr <= 0) return;
+  const int spin = a.spin;
   KParams p = make_params(g, a, alm[0], spin ? alm[1] : nullptr, const_cast<double4 *>(ph));
   // spin 0: 8 ring pairs per thread since the two-l-per-step kernels (fewer registers per ring pair; the butterfly and the
   // per-tile flush are per warp, so their share halves): 8.71 -> 8.31 ms at nside 2048 / lmax 4000
