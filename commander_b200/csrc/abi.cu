@@ -279,6 +279,7 @@ ptrdiff_t sharp_alm_count(const sharp_alm_info *self) { return (ptrdiff_t)self->
 void sharp_destroy_alm_info(sharp_alm_info *a) {
   if (!a) return;
   dist_forget_handle(a);
+  seed_forget(a);
   if (a->device >= 0) {
     forget_layout(a);
     cudaFree(a->d_mval); cudaFree(a->d_mvstart); cudaFree(a->d_m2im);
@@ -327,6 +328,7 @@ void sharp_make_subset_healpix_geom_info(int nside, int stride, int nrings, cons
 void sharp_destroy_geom_info(sharp_geom_info *g) {
   if (!g) return;
   dist_forget_handle(g);
+  seed_forget(g);
   for (sharp_geom_info *sub : g->subs) sharp_destroy_geom_info(sub);
   g->subs.clear();
   if (g->device >= 0) {
@@ -456,6 +458,7 @@ void run_single(const Job &job, double *const *alm, double *const *map, sharp_ge
   LegGeom G;
   G.nslots = g->npairs; G.NPL = g->npairs; G.nowners = 1; G.NML = a->nm; G.ncomp_tot = ncomp; G.comp0 = 0;
   G.trig = g->d_trig; G.mlim = ensure_mlim(g, a->lmax, spin);
+  G.seed_geom = g; G.seed_alm = a;
   PhaseLayout L = single_layout(a, g->npairs, ncomp, 0);
   double4 *ph = static_cast<double4 *>(scratch_get("phase", sizeof(double4) * (size_t)ncomp * a->nm * g->npairs));
   if (synth) {
@@ -960,6 +963,6 @@ int cmdr_sht_last_legendre_ms(double *entries3, int max) {
 unsigned long long cmdr_sht_nominal_flops(const sharp_geom_info *g, const sharp_alm_info *a, int spin) {
   return nominal_flops(g, a, spin);
 }
-void cmdr_sht_release_caches(void) { scratch_release(); pinned_release(); }
+void cmdr_sht_release_caches(void) { scratch_release(); pinned_release(); seed_release(); }
 
 }  // extern "C"

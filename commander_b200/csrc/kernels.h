@@ -34,6 +34,9 @@ struct LegGeom {
   // No send buffer and no all-to-all in either direction.
   int npeer = 0, src_rank = 0;
   double4 *peer[CMDR_MAX_PEERS] = {};
+  // Handles that key the per-plan seed tables of the Legendre kernels (legendre.cu), set by a caller that launches every
+  // slot of the geometry on one GPU; nullptr: every warp starts from the closed-form start values.
+  const void *seed_geom = nullptr, *seed_alm = nullptr;
 };
 
 // alm side of the Legendre stage (local m's of this rank)
@@ -87,6 +90,9 @@ __host__ __device__ inline size_t ph_index(int block, int ncomp_tot, int comp, i
 void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *const *alm, double4 *ph, cudaStream_t st,
                            bool prep = true);
 void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm, const double4 *ph, cudaStream_t st);
+// Seed tables (legendre.cu): dropped with the geometry or alm handle they were built for, or all at once.
+void seed_forget(const void *h);
+void seed_release();
 
 // Ring-FFT stage on the LOCAL rings of `geom` (ringfft.cu).
 // The phase buffer on this side is indexed

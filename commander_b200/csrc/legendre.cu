@@ -21,6 +21,8 @@
 // butterfly and adds the sums to the a_lm with coalesced atomics (DESIGN.md 3.1).
 #include <cstdio>
 #include <cstdlib>
+#include <map>
+#include <tuple>
 
 #include "kernels.h"
 #include "legendre_core.cuh"
@@ -55,6 +57,11 @@ struct KParams {
   const double *trig;
   const int *mlim;
   const int *wslot;                  // work index -> storage slot (nullptr: identity)
+  // seeded kernels only (seed tables, see seed0_kernel / seed2_kernel): first row (spin 0) / l - l0 (spin 2) each warp
+  // accumulates at, per (local m, warp); recurrence state and scale exponent there, per (local m, slot)
+  const int *sl;
+  const double *ss;
+  const int *sk;
   double *alm0, *alm1;
   const double *lscale0, *lscale1;   // optional factor per l on component 0 / 1 (nullptr: 1)
   double4 *ph;
@@ -179,7 +186,9 @@ __global__ void __launch_bounds__(256) prep_s0_kernel(KParams p) {
 
 // Synthesis kernels: ONE WARP PER CTA like the analysis kernels (no block barriers; a thread owns R
 // adjacent ring pairs; whole warps beyond the m cut-off only write zeros).
-template <int R, int MINB>
+// SEED: start each ring from the seed table at the warp's first accumulating row instead of from the closed-form start
+// values at row 0 (the rows in between add exact zeros; seed0_kernel).
+template <int R, int MINB, bool SEED = false>
 __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
   __shared__ __align__(16) TileS0 tile[2][TL];
   const int im = p.im0 + blockIdx.y, m = p.mval[im];
@@ -190,6 +199,7 @@ __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
   int k[R], slot[R];
   bool any = false;
   const double K = p.Kstart[m];
+  const int j0 = SEED ? p.sl[(size_t)im * gridDim.x + blockIdx.x] : 0;
 #pragma unroll
   for (int r = 0; r < R; ++r) {
     slot[r] = chunk0 + lane * R + r;
@@ -200,11 +210,17 @@ __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
       const double4 tg = reinterpret_cast<const double4 *>(p.trig)[slot[r]];
       RingTrig g{tg.x, tg.y, tg.z, tg.w};
       x[r] = g.cth; x2[r] = g.cth * g.cth;
-      start_spin0(m, K, g, cur[r], k[r]);
+      if constexpr (SEED) {
+        const size_t s = (size_t)im * p.nslots + slot[r];
+        const double2 st = reinterpret_cast<const double2 *>(p.ss)[s];
+        cur[r] = st.x; prev[r] = st.y; k[r] = p.sk[s];
+      } else {
+        start_spin0(m, K, g, cur[r], k[r]);
+      }
       any = true;
     }
   }
-  if (__any_sync(FULL, any)) {
+  if (__any_sync(FULL, any) && (!SEED || j0 < J)) {
     const TileS0 *rows = reinterpret_cast<const TileS0 *>(p.trows) + p.tofs[im];
     auto issue_tile = [&](int b, int jt) {     // rows past this m's padded range are never used
       const char *src = reinterpret_cast<const char *>(rows + jt);
@@ -213,11 +229,11 @@ __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
       for (int q = 0; q < (int)(TL * sizeof(TileS0)) / 512; ++q) cp_async16(dst + (q * 32 + lane) * 16, src + (q * 32 + lane) * 16);
       cp_async_commit();
     };
-    issue_tile(0, 0);
+    issue_tile(0, j0);
     cp_async_wait_all();
     __syncwarp();
     int buf = 0;
-    for (int jt = 0; jt < J; jt += TL, buf ^= 1) {
+    for (int jt = j0; jt < J; jt += TL, buf ^= 1) {
       if (jt + TL < J) issue_tile(buf ^ 1, jt + TL);
       const int ngroups = min(TL, J - jt + 3) / 4;
 #pragma unroll 1
@@ -395,7 +411,7 @@ __global__ void __launch_bounds__(256) prep_s2_kernel(KParams p) {
   reinterpret_cast<TileS2 *>(p.trows)[p.tofs[im] + j] = e;
 }
 
-template <int R, int MINB>
+template <int R, int MINB, bool SEED = false>
 __global__ void __launch_bounds__(32, MINB) synth2_kernel(KParams p) {
   __shared__ __align__(16) TileS2 tile[2][TL];
   const int im = p.im0 + blockIdx.y, m = p.mval[im];
@@ -410,7 +426,7 @@ __global__ void __launch_bounds__(32, MINB) synth2_kernel(KParams p) {
   // is not too close to a pole; P / Pp hold the scalar state until the conversion
   unsigned vmask = 0;
   int mg[R];
-  bool front = p.fcoef != nullptr && m >= 4 && l0 <= p.lmax, fok = true;
+  bool front = !SEED && p.fcoef != nullptr && m >= 4 && l0 <= p.lmax, fok = true;
 #pragma unroll
   for (int r = 0; r < R; ++r) {
     slot[r] = chunk0 + lane * R + r;
@@ -423,14 +439,21 @@ __global__ void __launch_bounds__(32, MINB) synth2_kernel(KParams p) {
       RingTrig g{tg.x, tg.y, tg.z, tg.w};
       x[r] = g.cth;
       vmask |= 1u << r;
-      mg[r] = front_margin_bits(g.sth);
-      if (front) { start_spin0(m, p.fK0[m], g, P[r], k[r]); fok &= k[r] < 0 && g.sth >= FRONT_MIN_STH; }
+      if constexpr (SEED) {
+        const size_t s = (size_t)im * p.nslots + slot[r];
+        const double4 st = reinterpret_cast<const double4 *>(p.ss)[s];
+        P[r] = st.x; Pp[r] = st.y; M[r] = st.z; Mp[r] = st.w; k[r] = p.sk[s];
+      } else {
+        mg[r] = front_margin_bits(g.sth);
+        if (front) { start_spin0(m, p.fK0[m], g, P[r], k[r]); fok &= k[r] < 0 && g.sth >= FRONT_MIN_STH; }
+      }
       any = true;
     }
   }
   front = front && __all_sync(FULL, fok);
-  int lskip = 0;                        // l (counted from l0) the front phase has covered: whole tiles
-  if (__any_sync(FULL, any)) {
+  // l (counted from l0) the front phase has covered (whole tiles), or where the seed table starts the warp
+  int lskip = SEED ? p.sl[(size_t)im * gridDim.x + blockIdx.x] : 0;
+  if (__any_sync(FULL, any) && (!SEED || l0 + lskip <= p.lmax)) {
     if (front) {
       const int jb = spin2_front_phase<R, 4, FRONT_TR>(p, im, m, vmask, x, mg, P, Pp, k);
       lskip = 2 * jb;
@@ -443,7 +466,7 @@ __global__ void __launch_bounds__(32, MINB) synth2_kernel(KParams p) {
           spin2_front_finish(p, im, m, jb, x[r], sth, nu, nup, P[r], Pp[r], M[r], Mp[r]);
         } else k[r] = 0;
       }
-    } else {
+    } else if (!SEED) {
 #pragma unroll
       for (int r = 0; r < R; ++r)
         if ((vmask >> r) & 1) {
@@ -778,7 +801,7 @@ __device__ __forceinline__ void anal0_step(const TileA0 *tA, const double (&x2)[
 // shuffle latency hides behind FP64 work.  After each tile the reduced sums are read back row-major
 // from shared memory and added to the a_lm with fully coalesced atomics (other warps hold the
 // other rings of the same m).
-template <int R, int MINB>
+template <int R, int MINB, bool SEED = false>
 __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
   __shared__ __align__(16) TileA0 tile[2][TL];
   __shared__ __align__(16) double red[(TL + 1) * 4];   // row 0: T1 of the last row of the previous tile
@@ -801,7 +824,13 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
       const double4 tg = reinterpret_cast<const double4 *>(p.trig)[slot];
       RingTrig g{tg.x, tg.y, tg.z, tg.w};
       x2[r] = g.cth * g.cth;
-      start_spin0(m, K, g, cur[r], k[r]);
+      if constexpr (SEED) {
+        const size_t s = (size_t)im * p.nslots + slot;
+        const double2 st = reinterpret_cast<const double2 *>(p.ss)[s];
+        cur[r] = st.x; prev[r] = st.y; k[r] = p.sk[s];
+      } else {
+        start_spin0(m, K, g, cur[r], k[r]);
+      }
       double4 q = *ph_in(p, 0, im, slot);
       double z[4] = {q.x + q.z, q.y + q.w, g.cth * (q.x - q.z), g.cth * (q.y - q.w)};
       // w[i] = z[i ^ (swapT ? 2 : 0) ^ (swapRI ? 1 : 0)]
@@ -814,6 +843,10 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
     }
   }
   if (!__any_sync(FULL, any)) return;
+  // first row of the warp's tile loop: the rows before the seeded one add exact zeros (the T1 of row j0 - 1 that the
+  // first flush reads from red[0..3] is zero too)
+  const int j0 = SEED ? p.sl[(size_t)im * gridDim.x + blockIdx.x] : 0;
+  if (SEED && j0 >= J) return;
   const double *coef = p.coef + p.cofs[im];
   const double4 *mix = reinterpret_cast<const double4 *>(p.coef2 + 2 * p.cofs[im]);   // {u_j, v_j, h_j, v_{j-1}}
   const long long mvs = p.mvstart[im];
@@ -828,7 +861,7 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
     for (int q = 0; q < (int)(TL * sizeof(TileA0)) / 512; ++q) cp_async16(dst + (q * 32 + lane) * 16, src + (q * 32 + lane) * 16);
     cp_async_commit();
   };
-  issue_tile(0, 0);
+  issue_tile(0, j0);
   if (lane < 4) red[lane] = 0.0;
   cp_async_wait_all();
   __syncwarp();
@@ -836,7 +869,7 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
   bool steady = false;
   unsigned sidx = (unsigned)__cvta_generic_to_shared(red + 4 + store_index_s2(lane));
   asm volatile("mov.u32 %0, %0;" : "+r"(sidx));   // opaque: kept in a register instead of being recomputed per group
-  for (int jt = 0; jt < J; jt += TL, buf ^= 1) {
+  for (int jt = j0; jt < J; jt += TL, buf ^= 1) {
     if (jt + TL < J) issue_tile(buf ^ 1, jt + TL);
     const int ngroups = min(TL, J - jt + 3) / 4;
     const TileA0 *T = tile[buf];
@@ -999,7 +1032,7 @@ __device__ __forceinline__ void anal2_step(const TileA2 *t, const int csign, con
   }
 }
 
-template <int R, int MINB>
+template <int R, int MINB, bool SEED = false>
 __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
   __shared__ __align__(16) TileA2 tile[2][TL];
   __shared__ __align__(16) double red[TL * 4];
@@ -1018,7 +1051,7 @@ __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
   // scalar front phase (see synth2_kernel): Pa / Pap hold the scalar state until the conversion
   unsigned vmask = 0;
   int mg[R];
-  bool front = p.fcoef != nullptr && m >= 4, fok = true;
+  bool front = !SEED && p.fcoef != nullptr && m >= 4, fok = true;
 #pragma unroll
   for (int r = 0; r < R; ++r) {
     int slot = chunk0 + r * 32 + lane;
@@ -1031,15 +1064,26 @@ __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
       RingTrig g{tg.x, tg.y, tg.z, tg.w};
       x[r] = g.cth;
       vmask |= 1u << r;
-      mg[r] = front_margin_bits(g.sth);
-      if (front) { start_spin0(m, p.fK0[m], g, Pa[r], k[r]); fok &= k[r] < 0 && g.sth >= FRONT_MIN_STH; }
+      if constexpr (SEED) {   // the table holds P / M roles (seed2_kernel)
+        const size_t s = (size_t)im * p.nslots + slot;
+        const double4 st = reinterpret_cast<const double4 *>(p.ss)[s];
+        Pa[r] = swapPM ? st.z : st.x; Pb[r] = swapPM ? st.x : st.z;
+        Pap[r] = swapPM ? st.w : st.y; Pbp[r] = swapPM ? st.y : st.w;
+        k[r] = p.sk[s];
+      } else {
+        mg[r] = front_margin_bits(g.sth);
+        if (front) { start_spin0(m, p.fK0[m], g, Pa[r], k[r]); fok &= k[r] < 0 && g.sth >= FRONT_MIN_STH; }
+      }
       any = true;
     }
   }
   if (!__any_sync(FULL, any)) return;
   front = front && __all_sync(FULL, fok);
-  int lskip = 0;                        // l (counted from l0) the front phase has covered: whole tiles, which
-  if (front) {                          // contribute nothing to the a_lm
+  // l (counted from l0) the front phase has covered (whole tiles, which contribute nothing to the a_lm), or where the
+  // seed table starts the warp
+  int lskip = SEED ? p.sl[(size_t)im * gridDim.x + blockIdx.x] : 0;
+  if (SEED && l0 + lskip > p.lmax) return;
+  if (front) {
     const int jb = spin2_front_phase<R, 2, FRONT_TR>(p, im, m, vmask, x, mg, Pa, Pap, k);
     lskip = 2 * jb;
 #pragma unroll
@@ -1054,7 +1098,7 @@ __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
         Pap[r] = swapPM ? Mp0 : Pp0; Pbp[r] = swapPM ? Pp0 : Mp0;
       } else k[r] = 0;
     }
-  } else {
+  } else if (!SEED) {
 #pragma unroll
     for (int r = 0; r < R; ++r)
       if ((vmask >> r) & 1) {
@@ -1172,6 +1216,163 @@ __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
 }
 
 // ------------------------------------------------------------------------------------
+// Seed tables.  Before the first ring of a warp reaches the accumulation threshold, a Legendre kernel only advances the
+// recurrence (and, for spin 2, the scalar front phase); nothing it adds to the phases or the a_lm there is non-zero.
+// That part depends on the geometry, lmax, the m set, the spin and the kernel's slot-to-warp mapping only, so it is run
+// once per plan by the seed kernels below and the Legendre kernels start from where it ends.  A seed kernel repeats
+// its Legendre kernel's prologue and its group loop without the accumulation, on the same slots per lane, with the same
+// start values, steps, rescaling points and front-phase hand-over, and stops at the first group at which a valid ring
+// of the warp is on (k == 0).  It records that group's first row (spin 0) or l - l0 (spin 2) per (m, warp) and the
+// state of every ring there, per (m, slot).  The groups it skips add exact zeros in the Legendre kernel (nothing while
+// no ring is on; products with 0.0 when only invalid slots of the warp are "on"), so a seeded synthesis is bit-for-bit
+// the unseeded one and a seeded analysis only loses atomic additions of zeros.
+// ------------------------------------------------------------------------------------
+// spin 0: synth0 (R = 4) and anal0 (R = 8), ring pair r of lane `lane` = slot chunk0 + lane R + r, groups of 4 rows
+template <int R>
+__global__ void __launch_bounds__(32) seed0_kernel(KParams p) {
+  const int im = blockIdx.y, m = p.mval[im];
+  const int lane = threadIdx.x;
+  const int chunk0 = blockIdx.x * (32 * R);
+  const int J = p.lmax >= m ? (p.lmax - m) / 2 + 1 : 0;
+  double x2[R], cur[R], prev[R];
+  int k[R];
+  unsigned vmask = 0;
+  const double K = p.Kstart[m];
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int slot = chunk0 + lane * R + r;
+    const bool valid = slot < p.nslots && m <= p.mlim[min(slot, p.nslots - 1)];
+    prev[r] = cur[r] = x2[r] = 0.0; k[r] = 0;
+    if (valid) {
+      const double4 tg = reinterpret_cast<const double4 *>(p.trig)[slot];
+      RingTrig g{tg.x, tg.y, tg.z, tg.w};
+      x2[r] = g.cth * g.cth;
+      start_spin0(m, K, g, cur[r], k[r]);
+      vmask |= 1u << r;
+    }
+  }
+  const double2 *rec = reinterpret_cast<const double2 *>(p.coef + p.cofs[im]);   // {A_j, B_j}, the tiles' rows
+  int j = 0;
+  if (__any_sync(FULL, vmask != 0)) {
+#pragma unroll 1
+    for (; j < J; j += 4) {
+      bool on = false;
+#pragma unroll
+      for (int r = 0; r < R; ++r) on |= ((vmask >> r) & 1) && k[r] == 0;
+      if (__any_sync(FULL, on)) break;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const double2 ab = rec[j + q];
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+          const double nxt = step0x2(ab.x, ab.y, x2[r], cur[r], prev[r]);
+          prev[r] = cur[r]; cur[r] = nxt;
+        }
+      }
+#pragma unroll
+      for (int r = 0; r < R; ++r)
+        if (k[r] < 0 && needs_rescale(cur[r])) { cur[r] *= SCALE_DOWN; prev[r] *= SCALE_DOWN; ++k[r]; }
+    }
+  }
+  if (lane == 0) const_cast<int *>(p.sl)[(size_t)im * gridDim.x + blockIdx.x] = j;
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int slot = chunk0 + lane * R + r;
+    if (slot < p.nslots) {
+      const size_t s = (size_t)im * p.nslots + slot;
+      reinterpret_cast<double2 *>(const_cast<double *>(p.ss))[s] = make_double2(cur[r], prev[r]);
+      const_cast<int *>(p.sk)[s] = k[r];
+    }
+  }
+}
+
+// spin 2: synth2 (lane-major slots, front phase rows GR = 4 at a time, groups of GL = 8 l) and anal2 (slots 32 apart,
+// GR = 2, GL = 4).  The state is stored in the P / M roles {P, P_prev, M, M_prev}.
+template <int R, int GR, int GL, bool STRIDED>
+__global__ void __launch_bounds__(32) seed2_kernel(KParams p) {
+  const int im = blockIdx.y, m = p.mval[im];
+  const int lane = threadIdx.x;
+  const int chunk0 = blockIdx.x * (32 * R);
+  const int l0 = max(m, p.spin);
+  auto slot_of = [&](int r) { return STRIDED ? chunk0 + r * 32 + lane : chunk0 + lane * R + r; };
+  double x[R], P[R], Pp[R], M[R], Mp[R];
+  int k[R], mg[R];
+  unsigned vmask = 0;
+  bool front = p.fcoef != nullptr && m >= 4 && l0 <= p.lmax, fok = true;
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int slot = slot_of(r);
+    const bool valid = slot < p.nslots && m <= p.mlim[min(slot, p.nslots - 1)] && l0 <= p.lmax;
+    P[r] = M[r] = Pp[r] = Mp[r] = 0.0; k[r] = 0; x[r] = 0.0; mg[r] = 0;
+    if (valid) {
+      const double4 tg = reinterpret_cast<const double4 *>(p.trig)[slot];
+      RingTrig g{tg.x, tg.y, tg.z, tg.w};
+      x[r] = g.cth;
+      vmask |= 1u << r;
+      mg[r] = front_margin_bits(g.sth);
+      if (front) { start_spin0(m, p.fK0[m], g, P[r], k[r]); fok &= k[r] < 0 && g.sth >= FRONT_MIN_STH; }
+    }
+  }
+  int lt = 0;   // l - l0
+  if (__any_sync(FULL, vmask != 0)) {
+    if (__all_sync(FULL, fok) && front) {
+      const int jb = spin2_front_phase<R, GR, FRONT_TR>(p, im, m, vmask, x, mg, P, Pp, k);
+      lt = 2 * jb;
+#pragma unroll
+      for (int r = 0; r < R; ++r) {
+        const double nu = P[r], nup = Pp[r];
+        P[r] = Pp[r] = 0.0;
+        if ((vmask >> r) & 1) {
+          const double sth = reinterpret_cast<const double4 *>(p.trig)[slot_of(r)].y;
+          spin2_front_finish(p, im, m, jb, x[r], sth, nu, nup, P[r], Pp[r], M[r], Mp[r]);
+        } else k[r] = 0;
+      }
+    } else {
+#pragma unroll
+      for (int r = 0; r < R; ++r)
+        if ((vmask >> r) & 1) {
+          const double4 tg = reinterpret_cast<const double4 *>(p.trig)[slot_of(r)];
+          RingTrig g{tg.x, tg.y, tg.z, tg.w};
+          start_spin2(m, p.Kstart[m], g, P[r], M[r], k[r]);
+        }
+    }
+    const double4 *coef = reinterpret_cast<const double4 *>(p.coef + p.cofs[im]);   // {A', C', g, 0} from l0
+#pragma unroll 1
+    for (; l0 + lt <= p.lmax; lt += GL) {
+      bool on = false;
+#pragma unroll
+      for (int r = 0; r < R; ++r) on |= ((vmask >> r) & 1) && k[r] == 0;
+      if (__any_sync(FULL, on)) break;
+#pragma unroll
+      for (int j = 0; j < GL; ++j) {
+        const double4 c = coef[lt + j];
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+          const double up = fma(c.x, x[r], c.y), um = fma(c.x, x[r], -c.y);
+          const double np_ = fma(up, P[r], -Pp[r]), nm_ = fma(um, M[r], -Mp[r]);
+          Pp[r] = P[r]; P[r] = np_; Mp[r] = M[r]; M[r] = nm_;
+        }
+      }
+#pragma unroll
+      for (int r = 0; r < R; ++r)
+        if (k[r] < 0 && (needs_rescale(P[r]) || needs_rescale(M[r]))) {
+          P[r] *= SCALE_DOWN; Pp[r] *= SCALE_DOWN; M[r] *= SCALE_DOWN; Mp[r] *= SCALE_DOWN; ++k[r];
+        }
+    }
+  }
+  if (lane == 0) const_cast<int *>(p.sl)[(size_t)im * gridDim.x + blockIdx.x] = lt;
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int slot = slot_of(r);
+    if (slot < p.nslots) {
+      const size_t s = (size_t)im * p.nslots + slot;
+      reinterpret_cast<double4 *>(const_cast<double *>(p.ss))[s] = make_double4(P[r], Pp[r], M[r], Mp[r]);
+      const_cast<int *>(p.sk)[s] = k[r];
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------
 // Ring pairs per thread (register blocking).  Defaults were picked from the sweep recorded in
@@ -1190,6 +1391,7 @@ static KParams make_params(const LegGeom &g, const LegAlm &a, double *alm0, doub
   p.mval = a.mval; p.mvstart = a.mvstart; p.coef = a.coef; p.coef2 = a.coef2; p.cofs = a.cofs; p.Kstart = a.Kstart;
   p.fcoef = a.front_coef; p.fmix = a.front_mix; p.fcofs = a.front_cofs; p.fK0 = a.front_K0;
   p.tofs = nullptr; p.trows = nullptr;
+  p.sl = nullptr; p.ss = nullptr; p.sk = nullptr;
   p.im0 = a.im_begin;
   p.trig = g.trig; p.mlim = g.mlim; p.wslot = g.wslot;
   p.alm0 = alm0; p.alm1 = alm1; p.ph = ph;
@@ -1206,6 +1408,73 @@ static void launch_w(K kernel, const KParams &p, int nm, cudaStream_t st) {   //
   dim3 grid((n + 32 * R - 1) / (32 * R), nm);
   kernel<<<grid, 32, 0, st>>>(p);
 }
+
+// ---- seed tables: one per (geometry handle, alm handle, kernel), built on first use ----
+enum SeedKind { SEED_S0, SEED_A0, SEED_S2, SEED_A2 };
+struct SeedTab { int *sl = nullptr; double *ss = nullptr; int *sk = nullptr; size_t bytes = 0; };
+static std::map<std::tuple<const void *, const void *, int>, SeedTab> g_seeds;
+static bool g_seeds_on = true;
+static size_t g_seed_bytes = 0;
+
+static void seed_free(SeedTab &t) {
+  cudaFree(t.sl); cudaFree(t.ss); cudaFree(t.sk);
+  g_seed_bytes -= t.bytes;
+}
+void seed_forget(const void *h) {
+  for (auto it = g_seeds.begin(); it != g_seeds.end();) {
+    if (std::get<0>(it->first) == h || std::get<1>(it->first) == h) {
+      CMDR_CUDA_CHECK(cudaDeviceSynchronize());   // queued kernels may still read the table
+      seed_free(it->second);
+      it = g_seeds.erase(it);
+    } else {
+      ++it;
+    }
+  }
+}
+void seed_release() {
+  if (g_seeds.empty()) return;
+  CMDR_CUDA_CHECK(cudaDeviceSynchronize());
+  for (auto &kv : g_seeds) seed_free(kv.second);
+  g_seeds.clear();
+}
+
+// The seed table of `kind` for a launch with parameters `p` (nullptr: start from the closed-form values).  Used when
+// the launch covers every slot of a single-GPU geometry (the tables follow the warps of a launch from slot 0) and the
+// table takes at most 1/32 of the device memory: at nside 2048 / lmax 4000, 20 B (spin 0) or 36 B (spin 2) per
+// (m, ring pair) = 0.33 / 0.59 GB per kernel.
+static const SeedTab *seed_table(const LegGeom &g, SeedKind kind, int R, const KParams &p, int nm, cudaStream_t st) {
+  if (!g_seeds_on || !g.seed_geom || p.slot_begin != 0 || p.nslots != g.nslots || g.wslot) return nullptr;
+  const auto key = std::make_tuple(g.seed_geom, g.seed_alm, (int)kind);
+  auto it = g_seeds.find(key);
+  if (it != g_seeds.end()) return &it->second;
+  const int nwarps = (g.nslots + 32 * R - 1) / (32 * R);
+  const size_t nst = (size_t)nm * g.nslots, nsl = (size_t)nm * nwarps;
+  const size_t sbytes = (kind == SEED_S0 || kind == SEED_A0 ? 2 : 4) * sizeof(double);
+  const size_t bytes = nst * (sbytes + sizeof(int)) + nsl * sizeof(int);
+  static size_t cap = 0;
+  if (!cap) { size_t fr, tot; CMDR_CUDA_CHECK(cudaMemGetInfo(&fr, &tot)); cap = tot / 32; }
+  if (bytes > cap) return nullptr;
+  SeedTab t;
+  t.bytes = bytes;
+  CMDR_CUDA_CHECK(cudaMalloc(&t.sl, nsl * sizeof(int)));
+  CMDR_CUDA_CHECK(cudaMalloc(&t.ss, nst * sbytes));
+  CMDR_CUDA_CHECK(cudaMalloc(&t.sk, nst * sizeof(int)));
+  KParams q = p;   // all local m's, from slot 0
+  q.im0 = 0; q.sl = t.sl; q.ss = t.ss; q.sk = t.sk;
+  const dim3 grid(nwarps, nm);
+  switch (kind) {
+    case SEED_S0: seed0_kernel<4><<<grid, 32, 0, st>>>(q); break;
+    case SEED_A0: seed0_kernel<8><<<grid, 32, 0, st>>>(q); break;
+    case SEED_S2: seed2_kernel<4, 4, 8, false><<<grid, 32, 0, st>>>(q); break;
+    case SEED_A2: seed2_kernel<4, 2, 4, true><<<grid, 32, 0, st>>>(q); break;
+  }
+  count_launch();
+  CMDR_CUDA_CHECK(cudaGetLastError());
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));   // once per plan: other streams may use the table next
+  g_seed_bytes += bytes;
+  return &(g_seeds[key] = t);
+}
+static void use_seed(KParams &p, const SeedTab *t) { p.sl = t->sl; p.ss = t->ss; p.sk = t->sk; }
 
 void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *const *alm, double4 *ph, cudaStream_t st,
                            bool prep) {
@@ -1244,7 +1513,10 @@ void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *cons
       case 612: launch_w<6>(synth0_kernel<6, 12>, p, nmr, st); break;
       case 812: launch_w<8>(synth0_kernel<8, 12>, p, nmr, st); break;
       case 808: launch_w<8>(synth0_kernel<8, 8>, p, nmr, st); break;
-      default: launch_w<4>(synth0_kernel<4, 16>, p, nmr, st); break;
+      default:
+        if (const SeedTab *t = seed_table(g, SEED_S0, 4, p, a.nm, st)) { use_seed(p, t); launch_w<4>(synth0_kernel<4, 16, true>, p, nmr, st); }
+        else launch_w<4>(synth0_kernel<4, 16>, p, nmr, st);
+        break;
     }
   } else {
     switch (r2 * 100 + b2) {
@@ -1253,7 +1525,13 @@ void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *cons
       case 312: launch_w<3>(synth2_kernel<3, 12>, p, nmr, st); break;
       case 308: launch_w<3>(synth2_kernel<3, 8>, p, nmr, st); break;
       case 412: launch_w<4>(synth2_kernel<4, 12>, p, nmr, st); break;
-      case 408: launch_w<4>(synth2_kernel<4, 8>, p, nmr, st); break;
+      case 408:
+        if (const SeedTab *t = spin == 2 ? seed_table(g, SEED_S2, 4, p, a.nm, st) : nullptr) {
+          use_seed(p, t); launch_w<4>(synth2_kernel<4, 12, true>, p, nmr, st);   // 12: the 8 of the unseeded kernel lets the seeded one take 170 registers, one warp per SM fewer
+        } else {
+          launch_w<4>(synth2_kernel<4, 8>, p, nmr, st);
+        }
+        break;
       default: launch_w<2>(synth2_kernel<2, 16>, p, nmr, st); break;
     }
   }
@@ -1278,7 +1556,10 @@ void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm,
       case 408: launch_w<4>(anal0_kernel<4, 8>, p, nmr, st); break;
       case 612: launch_w<6>(anal0_kernel<6, 12>, p, nmr, st); break;
       case 608: launch_w<6>(anal0_kernel<6, 8>, p, nmr, st); break;
-      case 812: launch_w<8>(anal0_kernel<8, 12>, p, nmr, st); break;
+      case 812:
+        if (const SeedTab *t = seed_table(g, SEED_A0, 8, p, a.nm, st)) { use_seed(p, t); launch_w<8>(anal0_kernel<8, 12, true>, p, nmr, st); }
+        else launch_w<8>(anal0_kernel<8, 12>, p, nmr, st);
+        break;
       case 808: launch_w<8>(anal0_kernel<8, 8>, p, nmr, st); break;
       default: launch_w<4>(anal0_kernel<4, 12>, p, nmr, st); break;
     }
@@ -1288,7 +1569,13 @@ void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm,
       case 308: launch_w<3>(anal2_kernel<3, 8>, p, nmr, st); break;
       case 216: launch_w<2>(anal2_kernel<2, 16>, p, nmr, st); break;
       case 212: launch_w<2>(anal2_kernel<2, 12>, p, nmr, st); break;
-      case 412: launch_w<4>(anal2_kernel<4, 12>, p, nmr, st); break;
+      case 412:
+        if (const SeedTab *t = spin == 2 ? seed_table(g, SEED_A2, 4, p, a.nm, st) : nullptr) {
+          use_seed(p, t); launch_w<4>(anal2_kernel<4, 12, true>, p, nmr, st);
+        } else {
+          launch_w<4>(anal2_kernel<4, 12>, p, nmr, st);
+        }
+        break;
       case 410: launch_w<4>(anal2_kernel<4, 10>, p, nmr, st); break;
       default: launch_w<4>(anal2_kernel<4, 8>, p, nmr, st); break;
     }
@@ -1298,3 +1585,8 @@ void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm,
 }
 
 }  // namespace cmdr
+
+extern "C" {
+void cmdr_sht_set_legendre_seeds(int on) { cmdr::g_seeds_on = on != 0; }
+size_t cmdr_sht_legendre_seed_bytes(void) { return cmdr::g_seed_bytes; }
+}

@@ -37,7 +37,7 @@ ABI_SYMBOLS = [
     "cmdr_sht_execute_iqu_dist", "cmdr_sht_mix", "cmdr_sht_invn_diag", "cmdr_sht_conviqt_cube", "cmdr_sht_allreduce_sum", "cmdr_sht_launch_count",
     "cmdr_sht_set_profiling", "cmdr_sht_last_legendre_ms", "cmdr_sht_nominal_flops",
     "cmdr_sht_release_caches", "cmdr_sht_measure_fp64_tflops", "cmdr_sht_measure_fp64_tflops_3op",
-    "cmdr_sht_measure_host_copy", "cmdr_sht_host_copy_threads",
+    "cmdr_sht_measure_host_copy", "cmdr_sht_host_copy_threads", "cmdr_sht_set_legendre_seeds", "cmdr_sht_legendre_seed_bytes",
     "cmdr_cr_setup", "cmdr_cr_destroy", "cmdr_cr_matmulA", "cmdr_cr_invM", "cmdr_cr_set_precond_diag",
     "cmdr_cr_get_precond_diag", "cmdr_cr_compute_rhs", "cmdr_cr_solve", "cmdr_cr_matmul_count",
 ]
@@ -93,6 +93,8 @@ def lib() -> C.CDLL:
     L.cmdr_sht_measure_host_copy.argtypes = [C.c_size_t, ci, ci, ci]
     L.cmdr_sht_measure_host_copy.restype = C.c_double
     L.cmdr_sht_host_copy_threads.restype = ci
+    L.cmdr_sht_set_legendre_seeds.argtypes = [ci]
+    L.cmdr_sht_legendre_seed_bytes.restype = C.c_size_t
     L.cmdr_cr_setup.argtypes = [ci, ci, ci, vp, vp, vp, vp, vp, vp, ci]
     L.cmdr_cr_setup.restype = vp
     L.cmdr_cr_destroy.argtypes = [vp]
@@ -348,6 +350,16 @@ def launch_count() -> int:
 
 def set_profiling(on: bool) -> None:
     lib().cmdr_sht_set_profiling(1 if on else 0)
+
+
+def set_legendre_seeds(on: bool) -> None:
+    """Seed tables of the Legendre kernels on (default) or off; see cmdr_sht.h."""
+    lib().cmdr_sht_set_legendre_seeds(1 if on else 0)
+
+
+def legendre_seed_bytes() -> int:
+    """Device bytes held by the seed tables built so far."""
+    return int(lib().cmdr_sht_legendre_seed_bytes())
 
 
 def last_legendre_ms():
