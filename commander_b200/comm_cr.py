@@ -685,3 +685,155 @@ class cr_native_system:
         it = self.L.cmdr_cr_solve(self.handle, bp, xp, 1 if x0 is not None else 0, int(maxiter), float(cg_tol),
                                   0 if cg_conv_crit == "residual" else 1, int(cg_miniter), int(cg_check_conv_freq), hist, None)
         return x, int(it), [float(hist[i]) for i in range(it + 1)]
+
+
+# =====================================================================================================
+# The general system behind the C ABI (cmdr_cr_setup_multi, commander_b200/csrc/cr_multi.cu): the components and bands
+# of cr_system, F_mean mixing, the block-diagonal preconditioner; vectors in cr_system's flat layout.
+# =====================================================================================================
+
+class cr_native_multi_system:
+    """Several diffuse components seen through bands of their own nside, lmax, beam and noise: the handle of
+    cmdr_cr_setup_multi.  `comps` / `bands` are the cr_component / cr_band objects of cr_system (F_mean mixing only);
+    vectors are flat float64 arrays of length ncr in cr_system's layout (component after component, each
+    (nmaps, nalm)), numpy or torch.  precond: 'diagonal' (the block-diagonal preconditioner of
+    cr_system.initDiffPrecond_diagonal) or 'none'."""
+
+    def __init__(self, comps, bands, precond: str = "diagonal"):
+        import ctypes as C
+        from . import sharp
+        self.comps, self.bands = list(comps), list(bands)
+        if not self.comps or not self.bands:
+            raise ValueError("at least one component and one band")
+        if precond not in ("diagonal", "none"):
+            raise ValueError("Preconditioner type not supported: " + str(precond))
+        nb, nc = len(self.bands), len(self.comps)
+        for b in self.bands:
+            if not isinstance(b, cr_band):
+                raise ValueError("bands must be cr_band objects")
+            nm = b.info.nmaps
+            if tuple(b.invN.shape) != (nm, b.info.np):
+                raise ValueError(f"band invN has shape {tuple(b.invN.shape)}, expected {(nm, b.info.np)}")
+            if b.b_l.ndim != 2 or b.b_l.shape[0] < b.info.lmax + 1 or b.b_l.shape[1] < nm:
+                raise ValueError(f"band b_l has shape {b.b_l.shape}, expected at least {(b.info.lmax + 1, nm)}")
+        F = np.zeros((nb, nc, 3))
+        for k, c in enumerate(self.comps):
+            if not isinstance(c, cr_component):
+                raise ValueError("comps must be cr_component objects")
+            if c.F is not None and any(f is not None for f in c.F):
+                raise ValueError("per-pixel mixing F is not supported by the native system (use cr_system)")
+            if c.F_mean.ndim != 2 or c.F_mean.shape[0] != nb or c.F_mean.shape[1] < c.nmaps:
+                raise ValueError(f"component F_mean has shape {c.F_mean.shape}, expected ({nb}, {c.nmaps})")
+            F[:, k, :c.nmaps] = c.F_mean[:, :c.nmaps]
+            if c.Cl is not None and (c.Cl.ndim != 2 or c.Cl.shape[0] < c.lmax_amp + 1 or c.Cl.shape[1] < c.nmaps):
+                raise ValueError(f"component Cl has shape {c.Cl.shape}, expected at least {(c.lmax_amp + 1, c.nmaps)}")
+        self.off = [0]
+        for c in self.comps:
+            self.off.append(self.off[-1] + c.nmaps * c.x_info.nalm)
+        self.ncr = self.off[-1]
+        self._F = np.ascontiguousarray(F)
+        # host columns the library reads during setup
+        sS = []
+        for c in self.comps:
+            for j in range(c.nmaps):
+                sS.append(None if c.Cl is None else np.ascontiguousarray(np.sqrt(np.maximum(c.Cl[:c.lmax_amp + 1, j], 0.0))))
+        bl = [np.ascontiguousarray(b.b_l[:b.info.lmax + 1, j]) for b in self.bands for j in range(b.info.nmaps)]
+        icols = [b.invN[j] for b in self.bands for j in range(b.info.nmaps)]
+        ip, _k1 = _ptrs(icols)
+        bp, _k2 = _ptrs(bl)
+        sp = (C.c_void_p * len(sS))(*[None if a is None else a.ctypes.data for a in sS])
+
+        def handles(hs):
+            return (C.c_void_p * len(hs))(*[None if h is None else h.handle.value for h in hs])
+        comp_alm = handles([c.x_info.alm_info for c in self.comps])
+        comp_nm = (C.c_int * nc)(*[c.nmaps for c in self.comps])
+        gT = handles([b.info.geom_info_T for b in self.bands])
+        gP = handles([b.info.geom_info_P if b.info.nmaps == 3 else None for b in self.bands])
+        band_alm = handles([b.info.alm_info for b in self.bands])
+        band_nm = (C.c_int * nb)(*[b.info.nmaps for b in self.bands])
+        info = self.bands[0].info
+        comm = info.comm.handle if (info.dist and info.comm.size > 1) else -1
+        self.L = sharp.lib()
+        self.handle = self.L.cmdr_cr_setup_multi(comm, nc, comp_alm, comp_nm, sp, nb, gT, gP, band_alm, band_nm, ip, bp,
+                                                 self._F.ctypes.data, 1 if precond == "diagonal" else 0)
+
+    def __del__(self):
+        if getattr(self, "handle", None):
+            self.L.cmdr_cr_destroy(self.handle)
+            self.handle = None
+
+    @property
+    def n_matmul(self):
+        return int(self.L.cmdr_cr_matmul_count(self.handle))
+
+    def _cols(self, v):
+        """Column pointers of a flat vector of length ncr (component-major, each (nmaps, nalm))."""
+        shape = tuple(v.shape)
+        if shape != (self.ncr,):
+            raise ValueError(f"vector of shape {shape}, expected ({self.ncr},)")
+        cols = []
+        for k, c in enumerate(self.comps):
+            n = c.x_info.nalm
+            cols += [v[self.off[k] + j * n:self.off[k] + (j + 1) * n] for j in range(c.nmaps)]
+        return _ptrs(cols)
+
+    def _like(self, v):
+        if isinstance(v, np.ndarray):
+            return np.empty(self.ncr)
+        import torch
+        return torch.empty(self.ncr, dtype=torch.float64, device=v.device)
+
+    def _band_cols(self, maps, what):
+        if len(maps) != len(self.bands):
+            raise ValueError(f"{what}: one map array per band")
+        cols = []
+        for b, m in zip(self.bands, maps):
+            if tuple(m.shape) != (b.info.nmaps, b.info.np):
+                raise ValueError(f"{what}: shape {tuple(m.shape)}, expected {(b.info.nmaps, b.info.np)}")
+            cols += [m[j] for j in range(b.info.nmaps)]
+        return _ptrs(cols)
+
+    def matmulA(self, x):
+        """cr_matmulA, commander3/src/comm_cr_mod.f90:771-1024"""
+        y = self._like(x)
+        xp, _a = self._cols(x)
+        yp, _b = self._cols(y)
+        self.L.cmdr_cr_matmulA(self.handle, xp, yp, None)
+        return y
+
+    def invM(self, r):
+        """cr_invM with the block-diagonal preconditioner (comm_diffuse_comp_mod.f90:2186-2235), or the identity"""
+        z = self._like(r)
+        rp, _a = self._cols(r)
+        zp, _b = self._cols(z)
+        self.L.cmdr_cr_invM(self.handle, rp, zp, None)
+        return z
+
+    def computeRHS(self, data, eta_pix=None, eta_alm=None):
+        """cr_computeRHS, commander3/src/comm_cr_mod.f90:542-769; data / eta_pix: lists (per band) of (nmaps, np) arrays,
+        eta_alm: a flat vector (used on the components with a prior)."""
+        b = self._like(data[0])
+        dp, _a = self._band_cols(data, "data")
+        ep = ap = None
+        if eta_pix is not None:
+            ep, _b = self._band_cols(eta_pix, "eta_pix")
+        if eta_alm is not None:
+            ap, _c = self._cols(eta_alm)
+        bp, _d = self._cols(b)
+        self.L.cmdr_cr_compute_rhs(self.handle, dp, ep, ap, bp, None)
+        return b
+
+    def solve(self, b, x0=None, maxiter=300, cg_tol=1e-8, cg_conv_crit="residual", cg_miniter=5, cg_check_conv_freq=1):
+        """solve_cr_eqn_by_CG, commander3/src/comm_cr_mod.f90:201-348.  Returns (x, iterations done, residual history)."""
+        import ctypes as C
+        if cg_conv_crit not in ("residual", "fixed_iter"):
+            raise ValueError("Unsupported convergence criterion = " + cg_conv_crit)
+        x = self._like(b)
+        if x0 is not None:
+            x[...] = x0
+        bp, _a = self._cols(b)
+        xp, _b = self._cols(x)
+        hist = (C.c_double * (maxiter + 1))()
+        it = self.L.cmdr_cr_solve(self.handle, bp, xp, 1 if x0 is not None else 0, int(maxiter), float(cg_tol),
+                                  0 if cg_conv_crit == "residual" else 1, int(cg_miniter), int(cg_check_conv_freq), hist, None)
+        return x, int(it), [float(hist[i]) for i in range(it + 1)]

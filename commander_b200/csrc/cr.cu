@@ -51,6 +51,9 @@ struct cmdr_cr_system {
   double *h_sc = nullptr;      // pinned host mirror of the scalars
   unsigned long long n_matmul = 0;
   std::vector<double> h_lsc;   // host copy of lsc (preconditioner build)
+  std::vector<long long> col;  // a_lm per column of a CG vector: nmaps x nalm, or those of every component (multi)
+  cmdr::CrMulti *multi = nullptr;   // several components and bands (cmdr_cr_setup_multi, cr_multi.cu)
+  double *vs = nullptr;        // M^-1 r of the block preconditioner (multi)
 };
 
 namespace {
@@ -185,6 +188,11 @@ void reduce_and_step(cmdr_cr_system *s, int what, int it, cudaStream_t st) {
 
 // y = A x on device vectors ([nmaps][nalm] contiguous)
 void matmulA_dev(cmdr_cr_system *s, const double *x, double *y, cudaStream_t st) {
+  if (s->multi) {
+    cr_multi_matmulA(s->multi, x, y, st);
+    ++s->n_matmul;
+    return;
+  }
   if (s->prior) CMDR_CUDA_CHECK(cudaMemcpyAsync(y, x, sizeof(double) * s->n, cudaMemcpyDeviceToDevice, st));   // P = 1
   else CMDR_CUDA_CHECK(cudaMemsetAsync(y, 0, sizeof(double) * s->n, st));
   double *xa[3], *ya[3], *mp[3];
@@ -208,15 +216,75 @@ void matmulA_dev(cmdr_cr_system *s, const double *x, double *y, cudaStream_t st)
 }
 
 void copy_in(cmdr_cr_system *s, double *dst, const double *const *src, cudaStream_t st) {
-  for (int c = 0; c < s->nmaps; ++c)
-    if (s->nalm) CMDR_CUDA_CHECK(cudaMemcpyAsync(dst + (size_t)c * s->nalm, src[c], sizeof(double) * s->nalm, cudaMemcpyDefault, st));
+  size_t o = 0;
+  for (size_t c = 0; c < s->col.size(); o += s->col[c++])
+    if (s->col[c]) CMDR_CUDA_CHECK(cudaMemcpyAsync(dst + o, src[c], sizeof(double) * s->col[c], cudaMemcpyDefault, st));
 }
 void copy_out(cmdr_cr_system *s, double *const *dst, const double *src, cudaStream_t st) {
-  for (int c = 0; c < s->nmaps; ++c)
-    if (s->nalm) CMDR_CUDA_CHECK(cudaMemcpyAsync(dst[c], src + (size_t)c * s->nalm, sizeof(double) * s->nalm, cudaMemcpyDefault, st));
+  size_t o = 0;
+  for (size_t c = 0; c < s->col.size(); o += s->col[c++])
+    if (s->col[c]) CMDR_CUDA_CHECK(cudaMemcpyAsync(dst[c], src + o, sizeof(double) * s->col[c], cudaMemcpyDefault, st));
+}
+
+// CG vectors, device scalars and their host mirror, for a system of s->n unknowns
+void alloc_work(cmdr_cr_system *s, cudaStream_t st) {
+  s->vx = dalloc<double>(s->n); s->vr = dalloc<double>(s->n); s->vd = dalloc<double>(s->n);
+  s->vq = dalloc<double>(s->n); s->vb = dalloc<double>(s->n);
+  s->sc = dalloc<double>(S_COUNT);
+  CMDR_CUDA_CHECK(cudaMemsetAsync(s->sc, 0, sizeof(double) * S_COUNT, st));
+  s->partial = dalloc<double>(NBLK);
+  CMDR_CUDA_CHECK(cudaHostAlloc(&s->h_sc, sizeof(double) * S_COUNT, cudaHostAllocDefault));
+}
+
+// the preconditioner step of the CG: z = M^-1 r with the block preconditioner of a multi system
+bool block_precond(const cmdr_cr_system *s) { return s->multi && cr_multi_has_precond(s->multi); }
+
+void no_diag_precond(const cmdr_cr_system *s, const char *who) {
+  if (!s->multi) return;
+  fprintf(stderr, "%s: a system of several components has a block preconditioner, not a diagonal one\n", who);
+  abort();
 }
 
 }  // namespace
+
+namespace cmdr {
+
+void cr_rhs_map(double *m, const double *invN, const double *d, const double *eta, long long n, cudaStream_t st) {
+  k_rhs_map<<<NBLK, NTHR, 0, st>>>(m, invN, d, eta, n);
+  count_launch(1);
+}
+
+// compute_invN_lm (comm_N_mod.f90:127-197): YtW_scalar of every N^-1 column on geom_info_T (:146), its m = 0
+// coefficients to every rank, then the 3j sum (evaluated as a quadrature on the device, invn.cu)
+void cr_invn_lm(int comm, int nmaps, double *invN, sharp_geom_info *gT, sharp_geom_info *gP, sharp_alm_info *a, double *nlm,
+                cudaStream_t st) {
+  const int nl = a->lmax + 1;
+  for (int c = 0; c < nmaps; ++c) {
+    double *ap[1] = {nlm + (size_t)c * a->nalm};
+    double *mp[1] = {invN + (size_t)c * gT->npix};
+    execute_iqu_opts(comm, SHARP_YtW, 1, ap, mp, gT, gP, a, SHARP_DP, nullptr, st);
+  }
+  double *al0_d = dalloc<double>((size_t)nmaps * nl);
+  std::vector<double> al0((size_t)nmaps * nl);
+  int im0 = -1;
+  for (int im = 0; im < a->nm; ++im) if (a->mval[im] == 0) im0 = im;
+  CMDR_CUDA_CHECK(cudaMemsetAsync(al0_d, 0, sizeof(double) * nmaps * nl, st));
+  if (im0 >= 0)
+    for (int c = 0; c < nmaps; ++c)
+      CMDR_CUDA_CHECK(cudaMemcpyAsync(al0_d + (size_t)c * nl, nlm + (size_t)c * a->nalm + a->mvstart[im0], sizeof(double) * nl,
+                                      cudaMemcpyDeviceToDevice, st));
+  cmdr_sht_allreduce_sum(comm, al0_d, nmaps * nl, st);   // the mpi_bcast from the owner of m = 0 (:147-152): zero elsewhere
+  CMDR_CUDA_CHECK(cudaMemcpyAsync(al0.data(), al0_d, sizeof(double) * nmaps * nl, cudaMemcpyDeviceToHost, st));
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+  const double *ap[3];
+  double *op[3];
+  for (int c = 0; c < nmaps; ++c) { ap[c] = al0.data() + (size_t)c * nl; op[c] = nlm + (size_t)c * a->nalm; }
+  cmdr_sht_invn_diag(nmaps, ap, 12.0 * (double)gT->nside * (double)gT->nside, a, op, st);
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+  cudaFree(al0_d);
+}
+
+}  // namespace cmdr
 
 extern "C" {
 
@@ -252,12 +320,8 @@ cmdr_cr_system *cmdr_cr_setup(int comm, int nbands, int nmaps, const sharp_geom_
   s->lsc = dalloc<double>(s->h_lsc.size());
   CMDR_CUDA_CHECK(cudaMemcpyAsync(s->lsc, s->h_lsc.data(), sizeof(double) * s->h_lsc.size(), cudaMemcpyHostToDevice, st));
   s->map = dalloc<double>((size_t)nmaps * s->npix);
-  s->vx = dalloc<double>(s->n); s->vr = dalloc<double>(s->n); s->vd = dalloc<double>(s->n);
-  s->vq = dalloc<double>(s->n); s->vb = dalloc<double>(s->n);
-  s->sc = dalloc<double>(S_COUNT);
-  CMDR_CUDA_CHECK(cudaMemsetAsync(s->sc, 0, sizeof(double) * S_COUNT, st));
-  s->partial = dalloc<double>(NBLK);
-  CMDR_CUDA_CHECK(cudaHostAlloc(&s->h_sc, sizeof(double) * S_COUNT, cudaHostAllocDefault));
+  s->col.assign(nmaps, s->nalm);
+  alloc_work(s, st);
   CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
   if (precond == 1) {
     // diagonal preconditioner (initDiffPrecond_diagonal / updateDiffPrecond_diagonal for npre = 1,
@@ -277,28 +341,8 @@ cmdr_cr_system *cmdr_cr_setup(int comm, int nbands, int nmaps, const sharp_geom_
     int *d_lof = dalloc<int>(s->nalm);
     if (s->nalm) CMDR_CUDA_CHECK(cudaMemcpyAsync(d_lof, l_of.data(), sizeof(int) * s->nalm, cudaMemcpyHostToDevice, st));
     double *nlm = s->vq;                               // [nmaps][nalm] scratch
-    double *al0_d = dalloc<double>((size_t)nmaps * nl);
-    std::vector<double> al0((size_t)nmaps * nl);
-    int im0 = -1;
-    for (int im = 0; im < s->a->nm; ++im) if (s->a->mval[im] == 0) im0 = im;
     for (int b = 0; b < nbands; ++b) {
-      for (int c = 0; c < nmaps; ++c) {                // YtW_scalar: every column as a spin-0 field on geom_info_T (:146)
-        double *ap[1] = {nlm + (size_t)c * s->nalm};
-        double *mp[1] = {s->invN + ((size_t)b * nmaps + c) * s->npix};
-        execute_iqu_opts(comm, SHARP_YtW, 1, ap, mp, s->gT, s->gP, s->a, SHARP_DP, nullptr, st);
-      }
-      CMDR_CUDA_CHECK(cudaMemsetAsync(al0_d, 0, sizeof(double) * nmaps * nl, st));
-      if (im0 >= 0)
-        for (int c = 0; c < nmaps; ++c)
-          CMDR_CUDA_CHECK(cudaMemcpyAsync(al0_d + (size_t)c * nl, nlm + (size_t)c * s->nalm + s->a->mvstart[im0], sizeof(double) * nl,
-                                          cudaMemcpyDeviceToDevice, st));
-      cmdr_sht_allreduce_sum(comm, al0_d, nmaps * nl, st);   // the mpi_bcast from the owner of m = 0 (:147-152): zero elsewhere
-      CMDR_CUDA_CHECK(cudaMemcpyAsync(al0.data(), al0_d, sizeof(double) * nmaps * nl, cudaMemcpyDeviceToHost, st));
-      CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
-      const double *ap[3];
-      double *op[3];
-      for (int c = 0; c < nmaps; ++c) { ap[c] = al0.data() + (size_t)c * nl; op[c] = nlm + (size_t)c * s->nalm; }
-      cmdr_sht_invn_diag(nmaps, ap, 12.0 * (double)s->gT->nside * (double)s->gT->nside, s->a, op, st);
+      cr_invn_lm(comm, nmaps, s->invN + (size_t)b * nmaps * s->npix, s->gT, s->gP, s->a, nlm, st);
       for (int c = 0; c < nmaps; ++c)
         k_precond_acc<<<NBLK, NTHR, 0, st>>>(s->Minv + (size_t)c * s->nalm, nlm + (size_t)c * s->nalm,
                                             s->lsc + ((size_t)b * nmaps + c) * nl, d_lof, s->nalm);
@@ -308,8 +352,34 @@ cmdr_cr_system *cmdr_cr_setup(int comm, int nbands, int nmaps, const sharp_geom_
     count_launch(1);
     CMDR_CUDA_CHECK(cudaGetLastError());
     CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
-    cudaFree(d_lof); cudaFree(al0_d);
+    cudaFree(d_lof);
   }
+  return s;
+}
+
+cmdr_cr_system *cmdr_cr_setup_multi(int comm, int ncomp, const sharp_alm_info *const *comp_alm, const int *comp_nmaps,
+                                    const double *const *sqrtS, int nbands, const sharp_geom_info *const *band_geom_T,
+                                    const sharp_geom_info *const *band_geom_P, const sharp_alm_info *const *band_alm,
+                                    const int *band_nmaps, const double *const *invN, const double *const *b_l,
+                                    const double *F_mean, int precond) {
+  size_t free_b = 0, total_b = 0;
+  CMDR_CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+  const CrPlan plan = plan_cr_multi(ncomp, comp_alm, comp_nmaps, sqrtS, nbands, band_geom_T, band_geom_P, band_alm, band_nmaps,
+                                    invN, b_l, F_mean, precond, free_b);
+  if (!plan.error.empty()) { fprintf(stderr, "cmdr_sht: cmdr_cr_setup_multi: %s\n", plan.error.c_str()); abort(); }
+  int c = comm;
+  for (int q = 0; q < nbands; ++q) c = effective_comm(comm, band_geom_T[q], band_alm[q], "cmdr_cr_setup_multi");
+  cudaStream_t st = 0;
+  cmdr_cr_system *s = new cmdr_cr_system;
+  s->comm = c;
+  s->nbands = nbands;
+  s->multi = cr_multi_create(c, plan, comp_nmaps, sqrtS, band_geom_T, band_geom_P, band_alm, band_nmaps, invN, b_l, F_mean,
+                             precond, st);
+  cr_multi_columns(s->multi, s->col);
+  s->n = cr_multi_length(s->multi);
+  alloc_work(s, st);
+  if (block_precond(s)) s->vs = dalloc<double>(s->n);
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
   return s;
 }
 
@@ -318,13 +388,15 @@ void cmdr_cr_destroy(cmdr_cr_system *s) {
   cudaDeviceSynchronize();
   cudaFree(s->invN); cudaFree(s->lsc); cudaFree(s->blF); cudaFree(s->Minv); cudaFree(s->map);
   cudaFree(s->vx); cudaFree(s->vr); cudaFree(s->vd); cudaFree(s->vq); cudaFree(s->vb);
-  cudaFree(s->sc); cudaFree(s->partial); cudaFree(s->hist);
+  cudaFree(s->sc); cudaFree(s->partial); cudaFree(s->hist); cudaFree(s->vs);
   if (s->h_sc) cudaFreeHost(s->h_sc);
+  if (s->multi) cr_multi_destroy(s->multi);
   delete s;
 }
 
 // Replaces the caller-visible preconditioner: Minv[c] -> nalm doubles (host or device), or nullptr for the identity.
 void cmdr_cr_set_precond_diag(cmdr_cr_system *s, const double *const *Minv) {
+  no_diag_precond(s, "cmdr_cr_set_precond_diag");
   if (!Minv) { cudaFree(s->Minv); s->Minv = nullptr; return; }
   if (!s->Minv) s->Minv = dalloc<double>(s->n);
   for (int c = 0; c < s->nmaps; ++c)
@@ -333,6 +405,7 @@ void cmdr_cr_set_precond_diag(cmdr_cr_system *s, const double *const *Minv) {
 
 // Copies the diagonal preconditioner out (1 / (P + sum_nu S b_l^2 N^-1_lm)); out[c] -> nalm doubles, host or device.
 void cmdr_cr_get_precond_diag(const cmdr_cr_system *s, double *const *out) {
+  no_diag_precond(s, "cmdr_cr_get_precond_diag");
   for (int c = 0; c < s->nmaps; ++c)
     if (s->nalm) {
       if (s->Minv) CMDR_CUDA_CHECK(cudaMemcpy(out[c], s->Minv + (size_t)c * s->nalm, sizeof(double) * s->nalm, cudaMemcpyDefault));
@@ -350,8 +423,12 @@ void cmdr_cr_matmulA(cmdr_cr_system *s, const double *const *x, double *const *y
 void cmdr_cr_invM(cmdr_cr_system *s, const double *const *r, double *const *z, void *stream) {
   cudaStream_t st = (cudaStream_t)stream;
   copy_in(s, s->vd, r, st);
-  k_mul<<<NBLK, NTHR, 0, st>>>(s->vq, s->vd, s->Minv, s->n);
-  count_launch(1);
+  if (block_precond(s)) {
+    cr_multi_precond(s->multi, s->vd, s->vq, st);
+  } else {
+    k_mul<<<NBLK, NTHR, 0, st>>>(s->vq, s->vd, s->Minv, s->n);
+    count_launch(1);
+  }
   copy_out(s, z, s->vq, st);
   CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
 }
@@ -360,6 +437,13 @@ void cmdr_cr_invM(cmdr_cr_system *s, const double *const *r, double *const *z, v
 void cmdr_cr_compute_rhs(cmdr_cr_system *s, const double *const *data, const double *const *eta_pix,
                          const double *const *eta_alm, double *const *b, void *stream) {
   cudaStream_t st = (cudaStream_t)stream;
+  if (s->multi) {
+    if (eta_alm) copy_in(s, s->vq, eta_alm, st);
+    cr_multi_rhs(s->multi, data, eta_pix, eta_alm ? s->vq : nullptr, s->vb, st);
+    copy_out(s, b, s->vb, st);
+    CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+    return;
+  }
   CMDR_CUDA_CHECK(cudaMemsetAsync(s->vb, 0, sizeof(double) * s->n, st));
   double *ba[3], *mp[3];
   cols(s->vb, s->nalm, s->nmaps, ba);
@@ -407,10 +491,19 @@ int cmdr_cr_solve(cmdr_cr_system *s, const double *const *b, double *const *x, i
     CMDR_CUDA_CHECK(cudaMemcpyAsync(s->vr, s->vb, sizeof(double) * s->n, cudaMemcpyDeviceToDevice, st));
     ++s->n_matmul;
   }
-  k_direction<<<NBLK, NTHR, 0, st>>>(s->vd, s->vr, s->Minv, s->n, s->sc, 1);   // d = invM r           (:202)
+  // the block preconditioner is one more kernel (z = M^-1 r into s->vs) before the dot products that the diagonal one
+  // fuses into k_update / k_direction / k_dot
+  const bool block = block_precond(s);
+  if (block) cr_multi_precond(s->multi, s->vr, s->vd, st);                     // d = invM r           (:202)
+  else k_direction<<<NBLK, NTHR, 0, st>>>(s->vd, s->vr, s->Minv, s->n, s->sc, 1);
   k_dot<<<NBLK, NTHR, 0, st>>>(s->vr, s->vd, nullptr, s->n, s->partial);       // delta_new = r.d      (:205)
   reduce_and_step(s, 0, 0, st);
-  k_dot<<<NBLK, NTHR, 0, st>>>(s->vb, s->vb, s->Minv, s->n, s->partial);       // delta0 = b.invM b    (:207)
+  if (block) {                                                                 // delta0 = b.invM b    (:207)
+    cr_multi_precond(s->multi, s->vb, s->vs, st);
+    k_dot<<<NBLK, NTHR, 0, st>>>(s->vb, s->vs, nullptr, s->n, s->partial);
+  } else {
+    k_dot<<<NBLK, NTHR, 0, st>>>(s->vb, s->vb, s->Minv, s->n, s->partial);
+  }
   reduce_and_step(s, 1, 0, st);
   count_launch(4);
   CMDR_CUDA_CHECK(cudaMemcpyAsync(s->h_sc, s->sc, sizeof(double) * S_COUNT, cudaMemcpyDeviceToHost, st));
@@ -435,8 +528,13 @@ int cmdr_cr_solve(cmdr_cr_system *s, const double *const *b, double *const *x, i
     k_dot<<<NBLK, NTHR, 0, st>>>(s->vd, s->vq, nullptr, s->n, s->partial);     // alpha = delta_new / d.q  (:253)
     reduce_and_step(s, 2, i, st);
     k_update<<<NBLK, NTHR, 0, st>>>(s->vx, s->vr, s->vd, s->vq, s->Minv, s->n, s->sc, s->partial);   // :254-270
+    if (block) {
+      cr_multi_precond(s->multi, s->vr, s->vs, st);
+      k_dot<<<NBLK, NTHR, 0, st>>>(s->vr, s->vs, nullptr, s->n, s->partial);
+      count_launch(1);
+    }
     reduce_and_step(s, 3, i, st);
-    k_direction<<<NBLK, NTHR, 0, st>>>(s->vd, s->vr, s->Minv, s->n, s->sc, 0); // d = s + beta d       (:272)
+    k_direction<<<NBLK, NTHR, 0, st>>>(s->vd, block ? s->vs : s->vr, s->Minv, s->n, s->sc, 0);   // d = s + beta d (:272)
     count_launch(3);
     it = i;
   }

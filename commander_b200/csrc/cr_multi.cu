@@ -1,0 +1,372 @@
+// cr_multi.cu -- the constrained-realisation operator of several diffuse components seen through bands of their own
+// nside, lmax, beam and noise (cr_matmulA and cr_computeRHS of commander3/src/comm_cr_mod.f90:542-1024 as written), and
+// its block-diagonal preconditioner (comm_diffuse_comp_mod.f90:1167-1557, 2186-2235).  The entry point and the CG loop
+// are those of cr.cu; this file holds what differs from the one-component system:
+//   * band gather: a_q = sum_k F_mean[q][k] b_q sqrt(S_k) x_k on the band's transform layout at
+//     L_q = min(lmax_q, max_k lmax_k) -- evalDiffuseBand(alm_out) over the components, then alm_equal (:858-882);
+//   * Y with N^-1 fused into the ring-FFT epilogue, then Y^t into the band buffer (:888-918);
+//   * component gather: y_k = sum_q (the same factor) a'_q + P x_k, one pass per component over every band buffer
+//     (projectDiffuseBand(alm_in), :926-1008), written as a gather per component slot: no atomics, deterministic;
+//   * block preconditioner: npre x npre per (map, l, m) slot of info_pre, built from N_lm of every band and applied
+//     once per CG iteration.
+// Every re-pack is rank-local because all handles list the same m's (cr_plan.h).
+#include <cmath>
+#include <vector>
+
+#include "cr_block.cuh"
+#include "kernels.h"
+
+namespace cmdr {
+
+namespace {
+
+constexpr int NTHR = 256;
+
+// What the kernels read of the system: layouts (cr_plan.h), component and band descriptors, per-l factors.
+struct CrDev {
+  int nm = 0, ncomp = 0, nbands = 0, nl = 0;   // nl = lmax_all + 1: stride of the per-l tables
+  const int *mval = nullptr;
+  const long long *bstart = nullptr;           // [layout][im]
+  const long long *off = nullptr, *cnalm = nullptr;   // per component: offset in a CG vector, a_lm per map
+  const int *cnm = nullptr, *clmax = nullptr;
+  double *const *buf = nullptr;                // per band: a_lm at L_q, [nmaps_q][nalm]
+  const long long *bnalm = nullptr;
+  const int *bnm = nullptr, *L = nullptr;
+  const double *g = nullptr;                   // [k][q][j][l]: F_mean b_l sqrt(S), 0 where the pair has no such slot
+  int xform0 = 0, pre = 0;                     // layout index of band 0 at L_0, of the preconditioner slots
+  __device__ long long start(int layout, int im) const { return bstart[(size_t)layout * nm + im]; }
+  __device__ double fac(const double *tab, int k, int q, int j, int l) const {
+    return tab[(((size_t)k * nbands + q) * 3 + j) * nl + l];
+  }
+};
+
+// The slot of this thread in an m-block launch over a layout of lmax `L`: grid.y = common m index, t = offset in the
+// m block, the map index is grid.z.  False outside the layout.
+__device__ __forceinline__ bool mslot(const CrDev &D, int L, int &l, int &t) {
+  const int m = D.mval[blockIdx.y];
+  t = blockIdx.x * NTHR + threadIdx.x;
+  if (m > L) return false;
+  if (t >= (m == 0 ? L + 1 : 2 * (L + 1 - m))) return false;
+  l = m == 0 ? t : m + (t >> 1);
+  return true;
+}
+
+// a_q[j, slot] = sum_k g[k][q][j][l] x_k[j, slot_k]
+__global__ void __launch_bounds__(NTHR) k_cr_band_gather(CrDev D, int q, const double *__restrict__ x) {
+  int l, t;
+  if (!mslot(D, D.L[q], l, t)) return;
+  const int j = blockIdx.z, im = blockIdx.y;
+  double acc = 0.0;
+  for (int k = 0; k < D.ncomp; ++k) {
+    if (j >= D.cnm[k] || l > D.clmax[k]) continue;
+    acc = fma(D.fac(D.g, k, q, j, l), x[D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t], acc);
+  }
+  D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t] = acc;
+}
+
+// y_k[j, slot] = sum_q g[k][q][j][l] a'_q[j, slot_q] (+ add[slot] when add != nullptr)
+__global__ void __launch_bounds__(NTHR) k_cr_comp_gather(CrDev D, int k, const double *__restrict__ add, double *__restrict__ y) {
+  int l, t;
+  if (!mslot(D, D.clmax[k], l, t)) return;
+  const int j = blockIdx.z, im = blockIdx.y;
+  double acc = 0.0;
+  for (int q = 0; q < D.nbands; ++q) {
+    if (j >= D.bnm[q] || l > D.L[q]) continue;
+    acc = fma(D.fac(D.g, k, q, j, l), D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t], acc);
+  }
+  const long long i = D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t;
+  y[i] = add ? acc + add[i] : acc;
+}
+
+// M[j, slot, k1 <= k2] += N_lm b_l^2 F_k1 F_k2 of band q (f = F_mean b_l, zero beyond either lmax)
+__global__ void __launch_bounds__(NTHR) k_cr_pre_acc(CrDev D, int q, const double *__restrict__ nlm, long long nalm_band,
+                                                    int band_layout, const double *__restrict__ f, double *__restrict__ M,
+                                                    long long ntot, long long nalm_pre) {
+  int l, t;
+  if (!mslot(D, D.L[q], l, t)) return;
+  const int j = blockIdx.z, im = blockIdx.y;
+  const double w = nlm[(long long)j * nalm_band + D.start(band_layout, im) + t];
+  double r[CR_MAX_NPRE];
+#pragma unroll
+  for (int k = 0; k < CR_MAX_NPRE; ++k) r[k] = k < D.ncomp ? D.fac(f, k, q, j, l) : 0.0;
+  double *m = M + (long long)j * nalm_pre + D.start(D.pre, im) + t;
+#pragma unroll
+  for (int k1 = 0; k1 < CR_MAX_NPRE; ++k1)
+#pragma unroll
+    for (int k2 = k1; k2 < CR_MAX_NPRE; ++k2)
+      if (k2 < D.ncomp && r[k1] != 0.0 && r[k2] != 0.0) m[(long long)cr_tri(k1, k2, D.ncomp) * ntot] += w * r[k1] * r[k2];
+}
+
+// sqrt(S) on both sides, the prior, the inversion: one thread per (map, preconditioner slot)
+__global__ void __launch_bounds__(NTHR) k_cr_pre_finish(CrDev D, int lmax_pre, const double *__restrict__ sS, unsigned prior,
+                                                       double *M, long long ntot, long long nalm_pre) {
+  int l, t;
+  if (!mslot(D, lmax_pre, l, t)) return;
+  const int j = blockIdx.z, im = blockIdx.y;
+  double s[CR_MAX_NPRE];
+  bool pr[CR_MAX_NPRE];
+  for (int k = 0; k < D.ncomp; ++k) {
+    pr[k] = (prior >> k) & 1u;
+    s[k] = sS[((size_t)k * 3 + j) * D.nl + l];
+  }
+  cr_block_finish_invert<CR_MAX_NPRE>(M + (long long)j * nalm_pre + D.start(D.pre, im) + t, ntot, D.ncomp, s, pr);
+}
+
+// z = M r on every preconditioner slot: gather r from each component (zero where it has no such slot), one block
+// product, z back to each component's slot.  A preconditioner slot maps to at most one slot per component, so the
+// writes do not conflict.
+template <int NMAX>
+__global__ void __launch_bounds__(NTHR) k_cr_pre_apply(CrDev D, int lmax_pre, const double *__restrict__ M, long long ntot,
+                                                      long long nalm_pre, const double *__restrict__ r, double *__restrict__ z) {
+  int l, t;
+  if (!mslot(D, lmax_pre, l, t)) return;
+  const int j = blockIdx.z, im = blockIdx.y;
+  double rv[NMAX], zv[NMAX];
+  long long idx[NMAX];
+#pragma unroll
+  for (int k = 0; k < NMAX; ++k) {
+    idx[k] = -1;
+    rv[k] = 0.0;
+    if (k < D.ncomp && j < D.cnm[k] && l <= D.clmax[k]) {
+      idx[k] = D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t;
+      rv[k] = r[idx[k]];
+    }
+  }
+  cr_block_apply<NMAX>(M + (long long)j * nalm_pre + D.start(D.pre, im) + t, ntot, D.ncomp, rv, zv);
+#pragma unroll
+  for (int k = 0; k < NMAX; ++k)
+    if (idx[k] >= 0) z[idx[k]] = zv[k];
+}
+
+template <typename T>
+T *dalloc(size_t n) {
+  T *p = nullptr;
+  CMDR_CUDA_CHECK(cudaMalloc(&p, sizeof(T) * (n ? n : 1)));
+  return p;
+}
+
+// grid of an m-block launch over a layout of lmax L
+dim3 mgrid(int L, int nm, int nmaps) { return dim3((unsigned)((2 * (L + 1) + NTHR - 1) / NTHR), (unsigned)nm, (unsigned)nmaps); }
+
+}  // namespace
+
+struct CrMulti {
+  CrPlan p;
+  int comm = -1;
+  std::vector<int> cnm, bnm;
+  std::vector<long long> off;            // per component: offset in a CG vector (ncomp + 1 entries)
+  unsigned prior = 0;                    // bit k: component k has a prior
+  std::vector<sharp_geom_info *> gT, gP;
+  std::vector<sharp_alm_info *> xa;      // per band: the transform handle at L_q
+  std::vector<bool> own_xa;              // built here (L_q < lmax_q)
+  std::vector<long long> npix;
+  std::vector<double *> invN, buf;       // per band: [nmaps_q][npix_q], [nmaps_q][nalm at L_q]
+  double *map = nullptr;                 // [3][max npix]
+  CrDev D;
+  int *d_mval = nullptr, *d_cnm = nullptr, *d_clmax = nullptr, *d_bnm = nullptr, *d_L = nullptr;
+  long long *d_bstart = nullptr, *d_off = nullptr, *d_cnalm = nullptr, *d_bnalm = nullptr;
+  double **d_buf = nullptr;
+  double *d_g = nullptr;
+  double *Mtri = nullptr;                // block table, nullptr without preconditioner
+  long long ntot = 0;                    // nmaps_pre * nalm_pre: stride of the triangle elements
+};
+
+long long cr_multi_length(const CrMulti *S) { return S->off.back(); }
+bool cr_multi_has_precond(const CrMulti *S) { return S->Mtri != nullptr; }
+void cr_multi_columns(const CrMulti *S, std::vector<long long> &len) {
+  len.clear();
+  for (int k = 0; k < S->p.ncomp; ++k) len.insert(len.end(), S->cnm[k], S->p.nalm[S->p.comp(k)]);
+}
+
+CrMulti *cr_multi_create(int comm, const CrPlan &plan, const int *comp_nmaps, const double *const *sqrtS,
+                         const sharp_geom_info *const *band_geom_T, const sharp_geom_info *const *band_geom_P,
+                         const sharp_alm_info *const *band_alm, const int *band_nmaps, const double *const *invN,
+                         const double *const *b_l, const double *F_mean, int precond, cudaStream_t st) {
+  CrMulti *S = new CrMulti;
+  S->p = plan;
+  S->comm = comm;
+  const CrPlan &p = S->p;
+  const int nc = p.ncomp, nb = p.nbands, nl = p.lmax_all + 1, nm = p.nm();
+  S->cnm.assign(comp_nmaps, comp_nmaps + nc);
+  S->bnm.assign(band_nmaps, band_nmaps + nb);
+  S->off.assign(nc + 1, 0);
+  std::vector<int> clmax(nc), cofs(nc + 1, 0), bofs(nb + 1, 0);   // first sqrtS / b_l / invN column of each
+  std::vector<long long> cnalm(nc);
+  for (int k = 0; k < nc; ++k) {
+    clmax[k] = p.lmax[p.comp(k)];
+    cnalm[k] = p.nalm[p.comp(k)];
+    S->off[k + 1] = S->off[k] + S->cnm[k] * cnalm[k];
+    cofs[k + 1] = cofs[k] + S->cnm[k];
+    if (sqrtS && sqrtS[cofs[k]]) S->prior |= 1u << k;
+  }
+  for (int q = 0; q < nb; ++q) bofs[q + 1] = bofs[q] + S->bnm[q];
+  // per-l factors: sS[k][j][l] = sqrt(C_l) (0 for l < 2 in polarisation) or 1 without prior, 0 beyond lmax_k;
+  // f[k][q][j][l] = F_mean b_l where both the component and the band transform hold (j, l); g = f sS
+  std::vector<double> sS((size_t)nc * 3 * nl, 0.0), f((size_t)nc * nb * 3 * nl, 0.0), g(f.size(), 0.0);
+  for (int k = 0; k < nc; ++k)
+    for (int j = 0; j < S->cnm[k]; ++j)
+      for (int l = 0; l <= clmax[k]; ++l) {
+        double v = 1.0;
+        if ((S->prior >> k) & 1u) v = (j > 0 && l < 2) ? 0.0 : sqrtS[cofs[k] + j][l];
+        sS[((size_t)k * 3 + j) * nl + l] = v;
+      }
+  for (int k = 0; k < nc; ++k)
+    for (int q = 0; q < nb; ++q)
+      for (int j = 0; j < std::min(S->cnm[k], S->bnm[q]); ++j) {
+        const double F = F_mean[((size_t)q * nc + k) * 3 + j];
+        for (int l = 0; l <= std::min(clmax[k], p.L[q]); ++l) {
+          const size_t i = (((size_t)k * nb + q) * 3 + j) * nl + l;
+          f[i] = F * b_l[bofs[q] + j][l];
+          g[i] = f[i] * sS[((size_t)k * 3 + j) * nl + l];
+        }
+      }
+  // bands: handles, N^-1, buffers
+  long long maxpix = 0;
+  for (int q = 0; q < nb; ++q) {
+    S->gT.push_back(const_cast<sharp_geom_info *>(band_geom_T[q]));
+    S->gP.push_back(const_cast<sharp_geom_info *>(band_geom_P[q]));
+    sharp_alm_info *a = const_cast<sharp_alm_info *>(band_alm[q]);
+    const bool own = p.L[q] < a->lmax;
+    if (own) {
+      std::vector<int> ms;
+      for (int m : a->mval) if (m <= p.L[q]) ms.push_back(m);
+      sharp_make_mmajor_real_packed_alm_info(p.L[q], 1, (int)ms.size(), ms.data(), &a);
+    }
+    S->xa.push_back(a);
+    S->own_xa.push_back(own);
+    const long long np = S->gT[q]->npix;
+    S->npix.push_back(np);
+    maxpix = std::max(maxpix, np);
+    double *d = dalloc<double>((size_t)S->bnm[q] * np);
+    for (int j = 0; j < S->bnm[q]; ++j)
+      if (np) CMDR_CUDA_CHECK(cudaMemcpyAsync(d + (size_t)j * np, invN[bofs[q] + j], sizeof(double) * np, cudaMemcpyDefault, st));
+    S->invN.push_back(d);
+    S->buf.push_back(dalloc<double>((size_t)S->bnm[q] * p.nalm[p.xform(q)]));
+  }
+  S->map = dalloc<double>((size_t)3 * maxpix);
+  std::vector<int> bnm(S->bnm), L(p.L);
+  std::vector<long long> bnalm(nb);
+  for (int q = 0; q < nb; ++q) bnalm[q] = p.nalm[p.xform(q)];
+  S->d_mval = upload(p.mval); S->d_bstart = upload(p.bstart);
+  S->d_off = upload(S->off); S->d_cnalm = upload(cnalm); S->d_cnm = upload(S->cnm); S->d_clmax = upload(clmax);
+  S->d_buf = upload(S->buf); S->d_bnalm = upload(bnalm); S->d_bnm = upload(bnm); S->d_L = upload(L);
+  S->d_g = upload(g);
+  CrDev &D = S->D;
+  D.nm = nm; D.ncomp = nc; D.nbands = nb; D.nl = nl;
+  D.mval = S->d_mval; D.bstart = S->d_bstart; D.off = S->d_off; D.cnalm = S->d_cnalm; D.cnm = S->d_cnm; D.clmax = S->d_clmax;
+  D.buf = S->d_buf; D.bnalm = S->d_bnalm; D.bnm = S->d_bnm; D.L = S->d_L; D.g = S->d_g;
+  D.xform0 = p.xform(0); D.pre = p.pre();
+  if (precond == 1) {
+    // initDiffPrecond_diagonal / updateDiffPrecond_diagonal (comm_diffuse_comp_mod.f90:1167-1557) for npre = ncomp:
+    // N^-1_{lm,lm} of every band on its own layout, accumulated into the blocks, then finished and inverted per slot
+    const long long nalm_pre = p.nalm[p.pre()];
+    S->ntot = (long long)p.nmaps_pre * nalm_pre;
+    S->Mtri = dalloc<double>(p.precond_bytes / sizeof(double));
+    CMDR_CUDA_CHECK(cudaMemsetAsync(S->Mtri, 0, p.precond_bytes, st));
+    double *d_f = upload(f), *d_sS = upload(sS);
+    for (int q = 0; q < nb; ++q) {
+      const long long na = p.nalm[p.band(q)];
+      double *nlm = dalloc<double>((size_t)S->bnm[q] * na);
+      cr_invn_lm(comm, S->bnm[q], S->invN[q], S->gT[q], S->gP[q], const_cast<sharp_alm_info *>(band_alm[q]), nlm, st);
+      if (nm) {
+        k_cr_pre_acc<<<mgrid(p.L[q], nm, std::min(S->bnm[q], p.nmaps_pre)), NTHR, 0, st>>>(D, q, nlm, na, p.band(q), d_f, S->Mtri,
+                                                                                             S->ntot, nalm_pre);
+        count_launch(1);
+      }
+      CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+      cudaFree(nlm);
+    }
+    if (nm) {
+      k_cr_pre_finish<<<mgrid(p.lmax_pre, nm, p.nmaps_pre), NTHR, 0, st>>>(D, p.lmax_pre, d_sS, S->prior, S->Mtri, S->ntot, nalm_pre);
+      count_launch(1);
+    }
+    CMDR_CUDA_CHECK(cudaGetLastError());
+    CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+    cudaFree(d_f); cudaFree(d_sS);
+  }
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+  return S;
+}
+
+void cr_multi_destroy(CrMulti *S) {
+  for (size_t q = 0; q < S->xa.size(); ++q) {
+    if (S->own_xa[q]) sharp_destroy_alm_info(S->xa[q]);
+    cudaFree(S->invN[q]); cudaFree(S->buf[q]);
+  }
+  cudaFree(S->map); cudaFree(S->Mtri);
+  cudaFree(S->d_mval); cudaFree(S->d_bstart); cudaFree(S->d_off); cudaFree(S->d_cnalm); cudaFree(S->d_cnm); cudaFree(S->d_clmax);
+  cudaFree(S->d_buf); cudaFree(S->d_bnalm); cudaFree(S->d_bnm); cudaFree(S->d_L); cudaFree(S->d_g);
+  delete S;
+}
+
+namespace {
+void band_cols(CrMulti *S, int q, double **alm, double **map) {
+  for (int j = 0; j < S->bnm[q]; ++j) {
+    alm[j] = S->buf[q] + (size_t)j * S->p.nalm[S->p.xform(q)];
+    map[j] = S->map + (size_t)j * S->npix[q];
+  }
+}
+
+// y_k = sum_q g a'_q (+ add on the components with a prior), every component
+void comp_gather(CrMulti *S, const double *add, double *y, cudaStream_t st) {
+  if (!S->p.nm()) return;
+  for (int k = 0; k < S->p.ncomp; ++k) {
+    k_cr_comp_gather<<<mgrid(S->p.lmax[S->p.comp(k)], S->p.nm(), S->cnm[k]), NTHR, 0, st>>>(
+        S->D, k, ((S->prior >> k) & 1u) ? add : nullptr, y);
+    count_launch(1);
+  }
+}
+}  // namespace
+
+// y = A x on device vectors in the layout of cr_system.extract_comp
+void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st) {
+  double *alm[3], *map[3];
+  for (int q = 0; q < S->p.nbands; ++q) {
+    if (S->p.nm()) {
+      k_cr_band_gather<<<mgrid(S->p.L[q], S->p.nm(), S->bnm[q]), NTHR, 0, st>>>(S->D, q, x);
+      count_launch(1);
+    }
+    band_cols(S, q, alm, map);
+    XformOpts o;                                                   // N^-1 as the map is written   (:888-905)
+    for (int j = 0; j < S->bnm[q]; ++j) o.pixscale[j] = S->invN[q] + (size_t)j * S->npix[q];
+    execute_iqu_opts(S->comm, SHARP_Y, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, &o, st);
+    execute_iqu_opts(S->comm, SHARP_Yt, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, nullptr, st);   // :913-918
+  }
+  comp_gather(S, x, y, st);                                        // :926-1008, + P x
+}
+
+// b = sum_q g Y^t (N^-1 d_q + N^-1/2 eta_q) (+ eta_alm on the components with a prior); eta_alm: device vector or nullptr
+void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *eta_pix, const double *eta_alm, double *b,
+                  cudaStream_t st) {
+  double *alm[3], *map[3];
+  long long maxpix = 1;
+  for (long long np : S->npix) maxpix = std::max(maxpix, np);
+  double *tmp = static_cast<double *>(scratch_get("cr_rhs_in", sizeof(double) * (size_t)2 * maxpix));
+  int col = 0;
+  for (int q = 0; q < S->p.nbands; ++q) {
+    band_cols(S, q, alm, map);
+    const long long np = S->npix[q];
+    for (int j = 0; j < S->bnm[q]; ++j, ++col) {
+      if (!np) continue;
+      CMDR_CUDA_CHECK(cudaMemcpyAsync(tmp, data[col], sizeof(double) * np, cudaMemcpyDefault, st));
+      if (eta_pix) CMDR_CUDA_CHECK(cudaMemcpyAsync(tmp + np, eta_pix[col], sizeof(double) * np, cudaMemcpyDefault, st));
+      cr_rhs_map(map[j], S->invN[q] + (size_t)j * np, tmp, eta_pix ? tmp + np : nullptr, np, st);
+    }
+    execute_iqu_opts(S->comm, SHARP_Yt, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, nullptr, st);
+  }
+  comp_gather(S, eta_alm, b, st);
+}
+
+// z = M^-1 r with the block preconditioner
+void cr_multi_precond(CrMulti *S, const double *r, double *z, cudaStream_t st) {
+  const CrPlan &p = S->p;
+  if (!p.nm()) return;
+  const dim3 grid = mgrid(p.lmax_pre, p.nm(), p.nmaps_pre);
+  const long long nalm_pre = p.nalm[p.pre()];
+  if (p.ncomp <= 4) k_cr_pre_apply<4><<<grid, NTHR, 0, st>>>(S->D, p.lmax_pre, S->Mtri, S->ntot, nalm_pre, r, z);
+  else if (p.ncomp <= 8) k_cr_pre_apply<8><<<grid, NTHR, 0, st>>>(S->D, p.lmax_pre, S->Mtri, S->ntot, nalm_pre, r, z);
+  else k_cr_pre_apply<CR_MAX_NPRE><<<grid, NTHR, 0, st>>>(S->D, p.lmax_pre, S->Mtri, S->ntot, nalm_pre, r, z);
+  count_launch(1);
+}
+
+}  // namespace cmdr

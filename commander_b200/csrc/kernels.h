@@ -6,6 +6,7 @@
 #include <cstdlib>
 #include <vector>
 
+#include "cr_plan.h"
 #include "job.h"
 #include "sht_internal.h"
 
@@ -187,6 +188,26 @@ void run_single(const Job &job, double *const *alm, double *const *map, sharp_ge
 int effective_comm(int comm, const sharp_geom_info *g, const sharp_alm_info *a, const char *who);
 void execute_iqu_opts(int comm, int type, int nmaps, double *const *alm, double *const *map, sharp_geom_info *gT,
                       sharp_geom_info *gP, sharp_alm_info *a, int flags, const XformOpts *opts, cudaStream_t st);
+
+// constrained-realisation pieces shared by the one-component system (cr.cu) and the multi-component one (cr_multi.cu)
+// m = N^-1 d (+ sqrt(N^-1) eta): the map of one band and map column in cr_computeRHS
+void cr_rhs_map(double *m, const double *invN, const double *d, const double *eta, long long n, cudaStream_t st);
+// nlm ([nmaps][nalm] device) = N^-1_{lm,lm} of one band from its N^-1 maps ([nmaps][npix] device): compute_invN_lm
+void cr_invn_lm(int comm, int nmaps, double *invN, sharp_geom_info *gT, sharp_geom_info *gP, sharp_alm_info *a, double *nlm,
+                cudaStream_t st);
+struct CrMulti;
+CrMulti *cr_multi_create(int comm, const CrPlan &plan, const int *comp_nmaps, const double *const *sqrtS,
+                         const sharp_geom_info *const *band_geom_T, const sharp_geom_info *const *band_geom_P,
+                         const sharp_alm_info *const *band_alm, const int *band_nmaps, const double *const *invN,
+                         const double *const *b_l, const double *F_mean, int precond, cudaStream_t st);
+void cr_multi_destroy(CrMulti *S);
+long long cr_multi_length(const CrMulti *S);
+void cr_multi_columns(const CrMulti *S, std::vector<long long> &len);   // a_lm per column of a CG vector
+bool cr_multi_has_precond(const CrMulti *S);
+void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st);
+void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *eta_pix, const double *eta_alm, double *b,
+                  cudaStream_t st);
+void cr_multi_precond(CrMulti *S, const double *r, double *z, cudaStream_t st);
 
 }  // namespace cmdr
 
