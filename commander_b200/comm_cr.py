@@ -694,12 +694,13 @@ class cr_native_system:
 
 class cr_native_multi_system:
     """Several diffuse components seen through bands of their own nside, lmax, beam and noise: the handle of
-    cmdr_cr_setup_multi.  `comps` / `bands` are the cr_component / cr_band objects of cr_system (F_mean mixing only);
-    vectors are flat float64 arrays of length ncr in cr_system's layout (component after component, each
-    (nmaps, nalm)), numpy or torch.  precond: 'diagonal' (the block-diagonal preconditioner of
-    cr_system.initDiffPrecond_diagonal) or 'none'."""
+    cmdr_cr_setup_multi.  `comps` / `bands` are the cr_component / cr_band objects of cr_system; vectors are flat
+    float64 arrays of length ncr in cr_system's layout (component after component, each (nmaps, nalm)), numpy or torch.
+    precond: 'diagonal' (the block-diagonal preconditioner of cr_system.initDiffPrecond_diagonal, from F_mean) or 'none'.
+    pixel_mixing: install every per-pixel mixing map c.F[q] that is not None (cmdr_cr_set_mixing_map); without it a
+    component that carries one is refused.  set_mixing_map replaces or removes one between solves."""
 
-    def __init__(self, comps, bands, precond: str = "diagonal"):
+    def __init__(self, comps, bands, precond: str = "diagonal", pixel_mixing: bool = False):
         import ctypes as C
         from . import sharp
         self.comps, self.bands = list(comps), list(bands)
@@ -721,7 +722,10 @@ class cr_native_multi_system:
             if not isinstance(c, cr_component):
                 raise ValueError("comps must be cr_component objects")
             if c.F is not None and any(f is not None for f in c.F):
-                raise ValueError("per-pixel mixing F is not supported by the native system (use cr_system)")
+                if not pixel_mixing:
+                    raise ValueError("per-pixel mixing F is not supported by the native system (use cr_system)")
+                if len(c.F) != nb:
+                    raise ValueError(f"component F has {len(c.F)} entries, expected one per band ({nb})")
             if c.F_mean.ndim != 2 or c.F_mean.shape[0] != nb or c.F_mean.shape[1] < c.nmaps:
                 raise ValueError(f"component F_mean has shape {c.F_mean.shape}, expected ({nb}, {c.nmaps})")
             F[:, k, :c.nmaps] = c.F_mean[:, :c.nmaps]
@@ -732,6 +736,12 @@ class cr_native_multi_system:
             self.off.append(self.off[-1] + c.nmaps * c.x_info.nalm)
         self.ncr = self.off[-1]
         self._F = np.ascontiguousarray(F)
+        mixing = []                                           # (q, k, columns), checked before anything is allocated
+        if pixel_mixing:
+            for k, c in enumerate(self.comps):
+                for q, f in enumerate(c.F or []):
+                    if f is not None:
+                        mixing.append((q, k, self._mixing_cols(q, k, f)))
         # host columns the library reads during setup
         sS = []
         for c in self.comps:
@@ -756,6 +766,41 @@ class cr_native_multi_system:
         self.L = sharp.lib()
         self.handle = self.L.cmdr_cr_setup_multi(comm, nc, comp_alm, comp_nm, sp, nb, gT, gP, band_alm, band_nm, ip, bp,
                                                  self._F.ctypes.data, 1 if precond == "diagonal" else 0)
+        for q, k, cols in mixing:
+            fp, _keep = _ptrs(cols)
+            self.L.cmdr_cr_set_mixing_map(self.handle, q, k, fp, None)
+
+    def set_mixing_map(self, q, k, F):
+        """Per-pixel mixing of component k in band q (the Y, x F, YtW branch of evalDiffuseBand / projectDiffuseBand,
+        commander3/src/comm_diffuse_comp_mod.f90:2070-2083, 2142-2151): F of shape (>= min(nmaps_q, nmaps_k), np_q),
+        this rank's pixels of the band, numpy or torch; None returns the pair to F_mean mixing.  Collective."""
+        if F is None:
+            self._mixing_cols(q, k, None)
+            self.L.cmdr_cr_set_mixing_map(self.handle, q, k, None, None)
+            return
+        fp, _keep = _ptrs(self._mixing_cols(q, k, F))
+        self.L.cmdr_cr_set_mixing_map(self.handle, q, k, fp, None)
+
+    def _mixing_cols(self, q, k, F):
+        """The min(nmaps_q, nmaps_k) float64 columns of a mixing map, after the range and shape checks."""
+        nb, nc = len(self.bands), len(self.comps)
+        if not 0 <= q < nb:
+            raise ValueError(f"band {q} out of range ({nb} bands)")
+        if not 0 <= k < nc:
+            raise ValueError(f"component {k} out of range ({nc} components)")
+        if F is None:
+            return None
+        if not hasattr(F, "data_ptr"):
+            F = np.asarray(F, dtype=np.float64)
+        info = self.bands[q].info
+        n = min(info.nmaps, self.comps[k].nmaps)
+        shape = tuple(F.shape)
+        if len(shape) != 2 or shape[0] < n or shape[1] != info.np:
+            raise ValueError(f"F of component {k} in band {q} has shape {shape}, expected ({n} or more, {info.np})")
+        if isinstance(F, np.ndarray):
+            return [np.ascontiguousarray(F[j], dtype=np.float64) for j in range(n)]
+        import torch
+        return [F[j].to(torch.float64).contiguous() for j in range(n)]
 
     def __del__(self):
         if getattr(self, "handle", None):

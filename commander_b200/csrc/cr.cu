@@ -373,7 +373,7 @@ cmdr_cr_system *cmdr_cr_setup_multi(int comm, int ncomp, const sharp_alm_info *c
   cmdr_cr_system *s = new cmdr_cr_system;
   s->comm = c;
   s->nbands = nbands;
-  s->multi = cr_multi_create(c, plan, comp_nmaps, sqrtS, band_geom_T, band_geom_P, band_alm, band_nmaps, invN, b_l, F_mean,
+  s->multi = cr_multi_create(c, plan, comp_alm, comp_nmaps, sqrtS, band_geom_T, band_geom_P, band_alm, band_nmaps, invN, b_l, F_mean,
                              precond, st);
   cr_multi_columns(s->multi, s->col);
   s->n = cr_multi_length(s->multi);
@@ -381,6 +381,15 @@ cmdr_cr_system *cmdr_cr_setup_multi(int comm, int ncomp, const sharp_alm_info *c
   if (block_precond(s)) s->vs = dalloc<double>(s->n);
   CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
   return s;
+}
+
+// Per-pixel mixing of one (band, component) pair of a cmdr_cr_setup_multi handle, or F_mean again with F = NULL.
+void cmdr_cr_set_mixing_map(cmdr_cr_system *s, int band, int comp, const double *const *F, void *stream) {
+  if (!s->multi) {
+    fprintf(stderr, "cmdr_sht: cmdr_cr_set_mixing_map: %s\n", check_cr_mixing(false, 0, 0, nullptr, nullptr, band, comp, F).c_str());
+    abort();
+  }
+  cr_multi_set_mixing(s->multi, band, comp, F, (cudaStream_t)stream);
 }
 
 void cmdr_cr_destroy(cmdr_cr_system *s) {

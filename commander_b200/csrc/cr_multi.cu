@@ -8,7 +8,10 @@
 //   * component gather: y_k = sum_q (the same factor) a'_q + P x_k, one pass per component over every band buffer
 //     (projectDiffuseBand(alm_in), :926-1008), written as a gather per component slot: no atomics, deterministic;
 //   * block preconditioner: npre x npre per (map, l, m) slot of info_pre, built from N_lm of every band and applied
-//     once per CG iteration.
+//     once per CG iteration;
+//   * spatially varying mixing of a (band, component) pair (cmdr_cr_set_mixing_map): evalDiffuseBand's Y, x F, YtW
+//     (comm_diffuse_comp_mod.f90:2070-2083) before the band gather, and projectDiffuseBand's (:2142-2151) after the
+//     band transform, F fused into the ring-FFT epilogue of the Y, b_l and sqrt(S) into the Legendre load and store.
 // Every re-pack is rank-local because all handles list the same m's (cr_plan.h).
 #include <cmath>
 #include <vector>
@@ -34,6 +37,8 @@ struct CrDev {
   const int *bnm = nullptr, *L = nullptr;
   const double *g = nullptr;                   // [k][q][j][l]: F_mean b_l sqrt(S), 0 where the pair has no such slot
   int xform0 = 0, pre = 0;                     // layout index of band 0 at L_0, of the preconditioner slots
+  double *const *mix = nullptr;                // per pair q * ncomp + k: its mixing buffer, nullptr for F_mean mixing
+  const int *mlay = nullptr;                   // per pair: layout of the buffer after the backward mix
   __device__ long long start(int layout, int im) const { return bstart[(size_t)layout * nm + im]; }
   __device__ double fac(const double *tab, int k, int q, int j, int l) const {
     return tab[(((size_t)k * nbands + q) * 3 + j) * nl + l];
@@ -51,20 +56,28 @@ __device__ __forceinline__ bool mslot(const CrDev &D, int L, int &l, int &t) {
   return true;
 }
 
-// a_q[j, slot] = sum_k g[k][q][j][l] x_k[j, slot_k]
+// a_q[j, slot] = sum_k g[k][q][j][l] x_k[j, slot_k]; with MIX, the mixed pairs add their buffer (b_l Y^t W F Y sqrt(S)
+// x_k on the band's transform layout) instead
+template <bool MIX>
 __global__ void __launch_bounds__(NTHR) k_cr_band_gather(CrDev D, int q, const double *__restrict__ x) {
   int l, t;
   if (!mslot(D, D.L[q], l, t)) return;
   const int j = blockIdx.z, im = blockIdx.y;
   double acc = 0.0;
   for (int k = 0; k < D.ncomp; ++k) {
+    if (MIX && D.mix[q * D.ncomp + k]) {          // every l <= L_q: F spreads the component beyond its lmax
+      if (j < D.cnm[k]) acc += D.mix[q * D.ncomp + k][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t];
+      continue;
+    }
     if (j >= D.cnm[k] || l > D.clmax[k]) continue;
     acc = fma(D.fac(D.g, k, q, j, l), x[D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t], acc);
   }
   D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t] = acc;
 }
 
-// y_k[j, slot] = sum_q g[k][q][j][l] a'_q[j, slot_q] (+ add[slot] when add != nullptr)
+// y_k[j, slot] = sum_q g[k][q][j][l] a'_q[j, slot_q] (+ add[slot] when add != nullptr); with MIX, the mixed pairs add
+// their buffer (sqrt(S) Y^t W F Y b_l a'_q, on layout mlay, l <= min(lmax_k, L_q)) instead
+template <bool MIX>
 __global__ void __launch_bounds__(NTHR) k_cr_comp_gather(CrDev D, int k, const double *__restrict__ add, double *__restrict__ y) {
   int l, t;
   if (!mslot(D, D.clmax[k], l, t)) return;
@@ -72,10 +85,21 @@ __global__ void __launch_bounds__(NTHR) k_cr_comp_gather(CrDev D, int k, const d
   double acc = 0.0;
   for (int q = 0; q < D.nbands; ++q) {
     if (j >= D.bnm[q] || l > D.L[q]) continue;
-    acc = fma(D.fac(D.g, k, q, j, l), D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t], acc);
+    const int ip = q * D.ncomp + k;
+    if (MIX && D.mix[ip]) acc += D.mix[ip][(long long)j * D.bnalm[q] + D.start(D.mlay[ip], im) + t];
+    else acc = fma(D.fac(D.g, k, q, j, l), D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t], acc);
   }
   const long long i = D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t;
   y[i] = add ? acc + add[i] : acc;
+}
+
+// the component-side input of a mixed pair whose component has the larger lmax: x_k truncated at L_q = lmax_q on the
+// band's transform layout (the buffer of the pair)
+__global__ void __launch_bounds__(NTHR) k_cr_mix_pack(CrDev D, int q, int k, const double *__restrict__ x, double *__restrict__ out) {
+  int l, t;
+  if (!mslot(D, D.L[q], l, t)) return;
+  const int j = blockIdx.z, im = blockIdx.y;
+  out[(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t] = x[D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t];
 }
 
 // M[j, slot, k1 <= k2] += N_lm b_l^2 F_k1 F_k2 of band q (f = F_mean b_l, zero beyond either lmax)
@@ -157,6 +181,7 @@ struct CrMulti {
   std::vector<long long> off;            // per component: offset in a CG vector (ncomp + 1 entries)
   unsigned prior = 0;                    // bit k: component k has a prior
   std::vector<sharp_geom_info *> gT, gP;
+  std::vector<sharp_alm_info *> ca;      // per component: its amplitude handle
   std::vector<sharp_alm_info *> xa;      // per band: the transform handle at L_q
   std::vector<bool> own_xa;              // built here (L_q < lmax_q)
   std::vector<long long> npix;
@@ -169,6 +194,18 @@ struct CrMulti {
   double *d_g = nullptr;
   double *Mtri = nullptr;                // block table, nullptr without preconditioner
   long long ntot = 0;                    // nmaps_pre * nalm_pre: stride of the triangle elements
+  // spatially varying mixing, per pair q * ncomp + k (cmdr_cr_set_mixing_map)
+  std::vector<double *> F;               // [nmin][npix_q] on the device, nullptr: F_mean mixing
+  std::vector<double *> mix;             // [nmin][nalm at L_q]: the pair's forward, then backward, mix
+  int nmixed = 0;
+  std::vector<double> h_sS, h_bl;        // [k][j][l] sqrt(S), [q][j][l] b_l: the lscale of the mixing transforms
+  double *d_sS = nullptr, *d_bl = nullptr;
+  double **d_mix = nullptr;
+  int *d_mlay = nullptr;
+  int nmin(int q, int k) const { return std::min(bnm[q], cnm[k]); }
+  // lmax_k <= lmax_q: the component side of the mix runs on the component's own handle (reads x_k, writes its layout);
+  // else on the band's transform handle at L_q = lmax_q, through k_cr_mix_pack
+  bool direct(int q, int k) const { return p.lmax[p.comp(k)] <= p.lmax[p.band(q)]; }
 };
 
 long long cr_multi_length(const CrMulti *S) { return S->off.back(); }
@@ -178,7 +215,8 @@ void cr_multi_columns(const CrMulti *S, std::vector<long long> &len) {
   for (int k = 0; k < S->p.ncomp; ++k) len.insert(len.end(), S->cnm[k], S->p.nalm[S->p.comp(k)]);
 }
 
-CrMulti *cr_multi_create(int comm, const CrPlan &plan, const int *comp_nmaps, const double *const *sqrtS,
+CrMulti *cr_multi_create(int comm, const CrPlan &plan, const sharp_alm_info *const *comp_alm, const int *comp_nmaps,
+                         const double *const *sqrtS,
                          const sharp_geom_info *const *band_geom_T, const sharp_geom_info *const *band_geom_P,
                          const sharp_alm_info *const *band_alm, const int *band_nmaps, const double *const *invN,
                          const double *const *b_l, const double *F_mean, int precond, cudaStream_t st) {
@@ -190,6 +228,9 @@ CrMulti *cr_multi_create(int comm, const CrPlan &plan, const int *comp_nmaps, co
   S->cnm.assign(comp_nmaps, comp_nmaps + nc);
   S->bnm.assign(band_nmaps, band_nmaps + nb);
   S->off.assign(nc + 1, 0);
+  for (int k = 0; k < nc; ++k) S->ca.push_back(const_cast<sharp_alm_info *>(comp_alm[k]));
+  S->F.assign((size_t)nc * nb, nullptr);
+  S->mix.assign((size_t)nc * nb, nullptr);
   std::vector<int> clmax(nc), cofs(nc + 1, 0), bofs(nb + 1, 0);   // first sqrtS / b_l / invN column of each
   std::vector<long long> cnalm(nc);
   for (int k = 0; k < nc; ++k) {
@@ -220,6 +261,11 @@ CrMulti *cr_multi_create(int comm, const CrPlan &plan, const int *comp_nmaps, co
           g[i] = f[i] * sS[((size_t)k * 3 + j) * nl + l];
         }
       }
+  S->h_sS = sS;
+  S->h_bl.assign((size_t)nb * 3 * nl, 0.0);
+  for (int q = 0; q < nb; ++q)
+    for (int j = 0; j < S->bnm[q]; ++j)
+      for (int l = 0; l <= p.L[q]; ++l) S->h_bl[((size_t)q * 3 + j) * nl + l] = b_l[bofs[q] + j][l];
   // bands: handles, N^-1, buffers
   long long maxpix = 0;
   for (int q = 0; q < nb; ++q) {
@@ -293,6 +339,8 @@ void cr_multi_destroy(CrMulti *S) {
     if (S->own_xa[q]) sharp_destroy_alm_info(S->xa[q]);
     cudaFree(S->invN[q]); cudaFree(S->buf[q]);
   }
+  for (size_t i = 0; i < S->F.size(); ++i) { cudaFree(S->F[i]); cudaFree(S->mix[i]); }
+  cudaFree(S->d_sS); cudaFree(S->d_bl); cudaFree(S->d_mix); cudaFree(S->d_mlay);
   cudaFree(S->map); cudaFree(S->Mtri);
   cudaFree(S->d_mval); cudaFree(S->d_bstart); cudaFree(S->d_off); cudaFree(S->d_cnalm); cudaFree(S->d_cnm); cudaFree(S->d_clmax);
   cudaFree(S->d_buf); cudaFree(S->d_bnalm); cudaFree(S->d_bnm); cudaFree(S->d_L); cudaFree(S->d_g);
@@ -311,9 +359,75 @@ void band_cols(CrMulti *S, int q, double **alm, double **map) {
 void comp_gather(CrMulti *S, const double *add, double *y, cudaStream_t st) {
   if (!S->p.nm()) return;
   for (int k = 0; k < S->p.ncomp; ++k) {
-    k_cr_comp_gather<<<mgrid(S->p.lmax[S->p.comp(k)], S->p.nm(), S->cnm[k]), NTHR, 0, st>>>(
-        S->D, k, ((S->prior >> k) & 1u) ? add : nullptr, y);
+    const dim3 grid = mgrid(S->p.lmax[S->p.comp(k)], S->p.nm(), S->cnm[k]);
+    const double *a = ((S->prior >> k) & 1u) ? add : nullptr;
+    if (S->nmixed) k_cr_comp_gather<true><<<grid, NTHR, 0, st>>>(S->D, k, a, y);
+    else k_cr_comp_gather<false><<<grid, NTHR, 0, st>>>(S->D, k, a, y);
     count_launch(1);
+  }
+}
+
+// The map columns of a mixing transform of band q and its fused factors: F as the map is written, `ls` per l
+void mix_opts(CrMulti *S, int q, int k, const double *ls, int nl, double **map, XformOpts &o) {
+  const int ip = q * S->p.ncomp + k;
+  for (int j = 0; j < S->nmin(q, k); ++j) {
+    map[j] = S->map + (size_t)j * S->npix[q];
+    o.pixscale[j] = S->F[ip] + (size_t)j * S->npix[q];
+    o.lscale[j] = ls + (size_t)j * nl;
+  }
+}
+
+// evalDiffuseBand's mixing of pair (q, k) (:2070-2083, 2086): mix = b_l Y^t W (F Y (sqrt(S) x_k)) at L_q.  The Y runs at
+// min(lmax_k, L_q): its input holds no more.
+void mix_forward(CrMulti *S, int q, int k, const double *x, cudaStream_t st) {
+  const CrPlan &p = S->p;
+  const int ip = q * p.ncomp + k, n = S->nmin(q, k), nl = p.lmax_all + 1;
+  const long long na = p.nalm[p.xform(q)];
+  double *alm[3], *map[3];
+  XformOpts o;
+  mix_opts(S, q, k, S->d_sS + (size_t)k * 3 * nl, nl, map, o);
+  sharp_alm_info *ac = S->xa[q];
+  if (S->direct(q, k)) {
+    ac = S->ca[k];
+    for (int j = 0; j < n; ++j) alm[j] = const_cast<double *>(x) + S->off[k] + (size_t)j * p.nalm[p.comp(k)];
+  } else {
+    if (p.nm()) {
+      k_cr_mix_pack<<<mgrid(p.L[q], p.nm(), n), NTHR, 0, st>>>(S->D, q, k, x, S->mix[ip]);
+      count_launch(1);
+    }
+    for (int j = 0; j < n; ++j) alm[j] = S->mix[ip] + (size_t)j * na;
+  }
+  execute_iqu_opts(S->comm, SHARP_Y, n, alm, map, S->gT[q], S->gP[q], ac, SHARP_DP, &o, st);
+  XformOpts ob;
+  for (int j = 0; j < n; ++j) {
+    alm[j] = S->mix[ip] + (size_t)j * na;
+    ob.lscale[j] = S->d_bl + ((size_t)q * 3 + j) * nl;
+  }
+  execute_iqu_opts(S->comm, SHARP_YtW, n, alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, &ob, st);
+}
+
+// Y^t of band q's map into its buffer (:913-918), then projectDiffuseBand's mixing of every mixed pair (:2142-2152):
+// mix = sqrt(S) Y^t W (F Y (b_l a'_q)), its Y^t W at min(lmax_k, L_q) on the layout the component gather reads
+void band_back(CrMulti *S, int q, double **alm, double **map, cudaStream_t st) {
+  execute_iqu_opts(S->comm, SHARP_Yt, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, nullptr, st);
+  if (!S->nmixed) return;
+  const CrPlan &p = S->p;
+  const int nl = p.lmax_all + 1;
+  const long long na = p.nalm[p.xform(q)];
+  for (int k = 0; k < p.ncomp; ++k) {
+    const int ip = q * p.ncomp + k, n = S->nmin(q, k);
+    if (!S->F[ip]) continue;
+    double *a[3], *mp[3];
+    XformOpts o;
+    mix_opts(S, q, k, S->d_bl + (size_t)q * 3 * nl, nl, mp, o);
+    for (int j = 0; j < n; ++j) a[j] = S->buf[q] + (size_t)j * na;
+    execute_iqu_opts(S->comm, SHARP_Y, n, a, mp, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, &o, st);
+    XformOpts os;
+    for (int j = 0; j < n; ++j) {
+      a[j] = S->mix[ip] + (size_t)j * na;
+      os.lscale[j] = S->d_sS + ((size_t)k * 3 + j) * nl;
+    }
+    execute_iqu_opts(S->comm, SHARP_YtW, n, a, mp, S->gT[q], S->gP[q], S->direct(q, k) ? S->ca[k] : S->xa[q], SHARP_DP, &os, st);
   }
 }
 }  // namespace
@@ -322,15 +436,20 @@ void comp_gather(CrMulti *S, const double *add, double *y, cudaStream_t st) {
 void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st) {
   double *alm[3], *map[3];
   for (int q = 0; q < S->p.nbands; ++q) {
+    if (S->nmixed)
+      for (int k = 0; k < S->p.ncomp; ++k)
+        if (S->F[q * S->p.ncomp + k]) mix_forward(S, q, k, x, st);
     if (S->p.nm()) {
-      k_cr_band_gather<<<mgrid(S->p.L[q], S->p.nm(), S->bnm[q]), NTHR, 0, st>>>(S->D, q, x);
+      const dim3 grid = mgrid(S->p.L[q], S->p.nm(), S->bnm[q]);
+      if (S->nmixed) k_cr_band_gather<true><<<grid, NTHR, 0, st>>>(S->D, q, x);
+      else k_cr_band_gather<false><<<grid, NTHR, 0, st>>>(S->D, q, x);
       count_launch(1);
     }
     band_cols(S, q, alm, map);
     XformOpts o;                                                   // N^-1 as the map is written   (:888-905)
     for (int j = 0; j < S->bnm[q]; ++j) o.pixscale[j] = S->invN[q] + (size_t)j * S->npix[q];
     execute_iqu_opts(S->comm, SHARP_Y, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, &o, st);
-    execute_iqu_opts(S->comm, SHARP_Yt, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, nullptr, st);   // :913-918
+    band_back(S, q, alm, map, st);                                 // :913-918, 2142-2151
   }
   comp_gather(S, x, y, st);                                        // :926-1008, + P x
 }
@@ -352,9 +471,55 @@ void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *et
       if (eta_pix) CMDR_CUDA_CHECK(cudaMemcpyAsync(tmp + np, eta_pix[col], sizeof(double) * np, cudaMemcpyDefault, st));
       cr_rhs_map(map[j], S->invN[q] + (size_t)j * np, tmp, eta_pix ? tmp + np : nullptr, np, st);
     }
-    execute_iqu_opts(S->comm, SHARP_Yt, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, nullptr, st);
+    band_back(S, q, alm, map, st);
   }
   comp_gather(S, eta_alm, b, st);
+}
+
+// Installs (F != nullptr) or removes the per-pixel mixing map of pair (band, comp); the arguments are checked
+void cr_multi_set_mixing(CrMulti *S, int band, int comp, const double *const *F, cudaStream_t st) {
+  const CrPlan &p = S->p;
+  const std::string err = check_cr_mixing(true, p.ncomp, p.nbands, S->cnm.data(), S->bnm.data(), band, comp, F);
+  // every rank learns whether all passed the same (band, comp, NULL-ness) and all were valid before any of them aborts
+  const int code = err.empty() ? (band * p.ncomp + comp) * 2 + (F != nullptr) : -1;
+  const bool same = comm_all_equal(S->comm, code, st);
+  if (!err.empty()) { fprintf(stderr, "cmdr_sht: cmdr_cr_set_mixing_map: %s\n", err.c_str()); abort(); }
+  if (!same) {
+    fprintf(stderr, "cmdr_sht: cmdr_cr_set_mixing_map: the ranks passed different (band, comp, F == NULL) or one of them an "
+                    "invalid argument; every rank of the communicator must make the same call\n");
+    abort();
+  }
+  const int ip = band * p.ncomp + comp, n = S->nmin(band, comp);
+  const long long np = S->npix[band];
+  if (!F) {
+    if (S->F[ip]) {
+      CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+      cudaFree(S->F[ip]); cudaFree(S->mix[ip]);
+      S->F[ip] = S->mix[ip] = nullptr;
+      --S->nmixed;
+    }
+  } else {
+    if (!S->F[ip]) {
+      S->F[ip] = dalloc<double>((size_t)n * np);
+      S->mix[ip] = dalloc<double>((size_t)n * p.nalm[p.xform(band)]);
+      ++S->nmixed;
+    }
+    for (int j = 0; j < n; ++j)
+      if (np) CMDR_CUDA_CHECK(cudaMemcpyAsync(S->F[ip] + (size_t)j * np, F[j], sizeof(double) * np, cudaMemcpyDefault, st));
+  }
+  if (!S->d_mix) {
+    S->d_sS = upload(S->h_sS);
+    S->d_bl = upload(S->h_bl);
+    std::vector<int> mlay((size_t)p.ncomp * p.nbands);
+    for (int q = 0; q < p.nbands; ++q)
+      for (int k = 0; k < p.ncomp; ++k) mlay[(size_t)q * p.ncomp + k] = S->direct(q, k) ? p.comp(k) : p.xform(q);
+    S->d_mlay = upload(mlay);
+    S->d_mix = dalloc<double *>(S->mix.size());
+    S->D.mlay = S->d_mlay;
+    S->D.mix = S->d_mix;
+  }
+  CMDR_CUDA_CHECK(cudaMemcpyAsync(S->d_mix, S->mix.data(), sizeof(double *) * S->mix.size(), cudaMemcpyHostToDevice, st));
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
 }
 
 // z = M^-1 r with the block preconditioner

@@ -141,4 +141,21 @@ inline CrPlan plan_cr_multi(int ncomp, const sharp_alm_info *const *comp_alm, co
   return p;
 }
 
+// Checks the arguments of cmdr_cr_set_mixing_map (same names and meaning) on one rank.  `multi`: the handle comes from
+// cmdr_cr_setup_multi (the other arguments are read only then); comp_nmaps / band_nmaps as given to it.  Returns the
+// reason of a refusal, or an empty string.
+inline std::string check_cr_mixing(bool multi, int ncomp, int nbands, const int *comp_nmaps, const int *band_nmaps, int band,
+                                   int comp, const double *const *F) {
+  if (!multi) return "needs a handle of cmdr_cr_setup_multi (a cmdr_cr_setup handle has one component and no mixing)";
+  if (band < 0 || band >= nbands) return "band " + std::to_string(band) + " out of range (nbands " + std::to_string(nbands) + ")";
+  if (comp < 0 || comp >= ncomp) return "comp " + std::to_string(comp) + " out of range (ncomp " + std::to_string(ncomp) + ")";
+  if (!F) return "";
+  const int n = std::min(band_nmaps[band], comp_nmaps[comp]);
+  for (int j = 0; j < n; ++j)
+    if (!F[j])
+      return "F[" + std::to_string(j) + "] is NULL: give all " + std::to_string(n) +
+             " columns (min(nmaps_band, nmaps_comp)), or F = NULL for F_mean mixing";
+  return "";
+}
+
 }  // namespace cmdr

@@ -770,6 +770,21 @@ void execute_iqu_opts(int comm, int type, int nmaps, double *const *alm, double 
   execute_dist_any(C, jobs, nmaps == 3 ? 2 : 1, alm, map, gs, a, st, opts);
 }
 
+bool comm_all_equal(int comm, int v, cudaStream_t st) {
+  DistComm *C = find_comm(comm);
+  if (!C || C->nranks == 1) return true;
+  const int h[2] = {v, -v};
+  int *d = nullptr, r[2];
+  CMDR_CUDA_CHECK(cudaMalloc(&d, sizeof(h)));
+  CMDR_CUDA_CHECK(cudaMemcpyAsync(d, h, sizeof(h), cudaMemcpyHostToDevice, st));
+  CMDR_NCCL_CHECK(nccl_api()->AllReduce(d, d, 2, ncclInt32, ncclMax, C->nccl, st));
+  CMDR_CUDA_CHECK(cudaMemcpyAsync(r, d, sizeof(r), cudaMemcpyDeviceToHost, st));
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+  cudaFree(d);
+  count_launch(1);
+  return r[0] == -r[1];   // max v == min v
+}
+
 // map *= F, the pixel-space mixing step between Y and YtW (HBM-bound: 24 bytes per pixel)
 __global__ void __launch_bounds__(256) scale_map_kernel(double *__restrict__ m, const double *__restrict__ f, long long n) {
   const long long stride = (long long)gridDim.x * blockDim.x;

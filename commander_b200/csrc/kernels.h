@@ -196,7 +196,8 @@ void cr_rhs_map(double *m, const double *invN, const double *d, const double *et
 void cr_invn_lm(int comm, int nmaps, double *invN, sharp_geom_info *gT, sharp_geom_info *gP, sharp_alm_info *a, double *nlm,
                 cudaStream_t st);
 struct CrMulti;
-CrMulti *cr_multi_create(int comm, const CrPlan &plan, const int *comp_nmaps, const double *const *sqrtS,
+CrMulti *cr_multi_create(int comm, const CrPlan &plan, const sharp_alm_info *const *comp_alm, const int *comp_nmaps,
+                         const double *const *sqrtS,
                          const sharp_geom_info *const *band_geom_T, const sharp_geom_info *const *band_geom_P,
                          const sharp_alm_info *const *band_alm, const int *band_nmaps, const double *const *invN,
                          const double *const *b_l, const double *F_mean, int precond, cudaStream_t st);
@@ -208,6 +209,10 @@ void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st);
 void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *eta_pix, const double *eta_alm, double *b,
                   cudaStream_t st);
 void cr_multi_precond(CrMulti *S, const double *r, double *z, cudaStream_t st);
+// cmdr_cr_set_mixing_map on a multi-component handle: checks (collectively), then installs or removes the map
+void cr_multi_set_mixing(CrMulti *S, int band, int comp, const double *const *F, cudaStream_t st);
+// true when every rank of `comm` passed the same v (one 8-byte max all-reduce of (v, -v)); true on one GPU
+bool comm_all_equal(int comm, int v, cudaStream_t st);
 
 }  // namespace cmdr
 

@@ -1,9 +1,10 @@
 """Time the native multi-component constrained-realisation solve (cmdr_cr_setup_multi) against the torch mirror
 comm_cr.cr_system on the sampling group of tests/test_gpu_cr_multi_native.py::real_size_problem: bands (nside / lmax)
 512 / 1500, 1024 / 2000, 1024 / 2000; components CMB (3 maps, lmax 2000, prior), dust (3, 1500, prior) and a 1-map
-low-l component without prior.
+low-l component without prior.  With --pixel-F the dust component is mixed per pixel in every band
+(cmdr_cr_set_mixing_map; the mirror gets the same maps) and the result goes to cr_mix_bench[_nN].json.
 
-  python tools/cr_multi_bench.py --out DIR                 (one GPU)
+  python tools/cr_multi_bench.py --out DIR [--pixel-F]     (one GPU)
   python -m torch.distributed.run --nproc-per-node N tools/cr_multi_bench.py --out DIR
 
 Each solve runs `fixed_iter` iterations after a warm-up solve and is timed with CUDA events around work that ends in a
@@ -33,12 +34,14 @@ def nalm(lmax, ms):
     return int(sum((lmax + 1 - m) * (1 if m == 0 else 2) for m in ms if m <= lmax))
 
 
-def kernel_bytes(comps, bands, ms):
-    """Bytes each new kernel moves per CG iteration (one matmulA + one preconditioner apply), from the shapes."""
+def kernel_bytes(comps, bands, ms, mixed=()):
+    """Bytes each new kernel moves per CG iteration (one matmulA + one preconditioner apply), from the shapes.  `mixed`:
+    the (band, component) pairs mixed per pixel, whose band-gather input is their buffer at the band's L_q."""
     lmax_pre = max(c["lmax"] for c in comps)
     L = [min(b["lmax"], lmax_pre) for b in bands]
     bnm = [b.get("nmaps", 3) for b in bands]
-    band = sum(8 * (bnm[q] * nalm(L[q], ms) + sum(min(c["nmaps"], bnm[q]) * nalm(min(c["lmax"], L[q]), ms) for c in comps))
+    band = sum(8 * (bnm[q] * nalm(L[q], ms) + sum(min(c["nmaps"], bnm[q]) * nalm(L[q] if (q, k) in mixed else min(c["lmax"], L[q]), ms)
+                                                  for k, c in enumerate(comps)))
                for q in range(len(bands)))
     comp = sum(8 * (c["nmaps"] * nalm(c["lmax"], ms) * (2 if c["Cl"] is not None else 1)
                     + sum(min(c["nmaps"], bnm[q]) * nalm(min(c["lmax"], L[q]), ms) for q in range(len(bands))))
@@ -53,6 +56,7 @@ def main():
     ap.add_argument("--out", required=True, help="directory for the JSON result")
     ap.add_argument("--iters", type=int, default=50)
     ap.add_argument("--mirror-iters", type=int, default=10)
+    ap.add_argument("--pixel-F", action="store_true", help="mix the dust component per pixel in every band")
     args = ap.parse_args()
     import torch
     from commander_b200 import comm_mapinfo
@@ -75,9 +79,15 @@ def main():
     bands, comps = real_size_problem(np.random.default_rng(15))
     binfo = [comm_mapinfo(comm, b["nside"], b["lmax"], 3, True) for b in bands]
     cb = [cr_band(i, torch.as_tensor(np.ascontiguousarray(b["invN"][:, i.pix]), device=dev), b["b_l"]) for i, b in zip(binfo, bands)]
-    cc = [cr_component(comm_mapinfo(comm, c["nside"], c["lmax"], c["nmaps"], c["nmaps"] == 3), Cl=c["Cl"], F_mean=c["F_mean"])
-          for c in comps]
-    nat = cr_native_multi_system(cc, cb)
+    mixed = ()
+    if args.pixel_F:                                            # dust, F_mean times a smooth-ish per-pixel factor
+        frng = np.random.default_rng(17)
+        comps[1]["F"] = [torch.as_tensor(np.ascontiguousarray((f[0] * (1.0 + 0.3 * frng.uniform(size=(3, 12 * b["nside"] ** 2))))[:, i.pix]),
+                                         device=dev) for f, b, i in zip(comps[1]["F_mean"], bands, binfo)]
+        mixed = tuple((q, 1) for q in range(len(bands)))
+    cc = [cr_component(comm_mapinfo(comm, c["nside"], c["lmax"], c["nmaps"], c["nmaps"] == 3), Cl=c["Cl"], F_mean=c["F_mean"],
+                       F=c.get("F")) for c in comps]
+    nat = cr_native_multi_system(cc, cb, pixel_mixing=args.pixel_F)
     rng = np.random.default_rng(16)
     data = [torch.as_tensor(rng.standard_normal((3, i.np)), device=dev) for i in binfo]
     b = nat.computeRHS(data)
@@ -115,22 +125,25 @@ def main():
             continue
         t = ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total
         tot += t
-        for k in ("k_cr_band_gather", "k_cr_comp_gather", "k_cr_pre_apply"):
+        for k in ("k_cr_band_gather", "k_cr_comp_gather", "k_cr_pre_apply", "k_cr_mix_pack"):
             if k in ev.name:
                 per[k] = per.get(k, 0.0) + t
     ms_local = cc[0].x_info.ms                                  # the largest lmax: every local m
-    nbytes = kernel_bytes(comps, bands, ms_local)
+    nbytes = kernel_bytes(comps, bands, ms_local, mixed)
     iters = nprof + 1                                           # the solve's matmulA / precond count: one extra at the start
     kern = {}
     for k, us in per.items():
-        kern[k] = {"ms_per_iter": us / 1e3 / iters, "GB_per_iter": nbytes[k] / 1e9,
-                   "GB_per_s": nbytes[k] / (us / 1e6 / iters) / 1e9 if us > 0 else None}
+        kern[k] = {"ms_per_iter": us / 1e3 / iters}
+        if k in nbytes:
+            kern[k].update(GB_per_iter=nbytes[k] / 1e9, GB_per_s=nbytes[k] / (us / 1e6 / iters) / 1e9 if us > 0 else None)
     res["kernels"] = kern
+    res["pixel_F"] = [f"dust in band {q}" for q, _ in mixed]
     res["profiled_gpu_ms_per_iter"] = tot / 1e3 / iters
     res["new_kernel_share"] = sum(per.values()) / tot if tot > 0 else None
     if rank == 0:
         os.makedirs(args.out, exist_ok=True)
-        path = os.path.join(args.out, "cr_multi_bench.json" if world == 1 else f"cr_multi_bench_n{world}.json")
+        name = "cr_mix_bench" if args.pixel_F else "cr_multi_bench"
+        path = os.path.join(args.out, f"{name}.json" if world == 1 else f"{name}_n{world}.json")
         with open(path, "w") as f:
             json.dump(res, f, indent=1)
         print(json.dumps(res))
