@@ -4,7 +4,8 @@ cube used for sidelobe corrections of time-ordered data.
     comm_conviqt(...)       constructor,    :60-153   beam table, psi grid, cube, then precompute_sky
     %precompute_sky(map)    :207-292                  bmax+1 spin-j syntheses + a psi FFT per pixel
     %get_alms(m_b, map)     :294-357                  (kept for inspection; the library does it on the device)
-    %interp(pix, psi)       :155-205                  psi lookup / linear interpolation
+    %interp(pix, psi)       :155-205                  psi lookup / linear interpolation (host restatement; on the
+                                                      device: make_sampler() -> conviqt_sampler.interp)
 
 In the reference precompute_sky loops `sharp_execute(SHARP_Y, j, 2, ...)` over host arrays and then runs FFTW
 c2r per pixel on the host.  Here it is ONE library call (`cmdr_sht_conviqt_cube`): the coefficient products,
@@ -155,7 +156,77 @@ class comm_conviqt:
         with np.errstate(divide="ignore", invalid="ignore"):
             return ((c[psii, loc] * (x1 - unwrap) + c[psiu, loc] * (unwrap - x0)) / (x1 - x0)).astype(f)
 
+    def make_sampler(self):
+        """The cube of ALL ranks on every GPU of the group, ready for interp at any pixel: the device counterpart of the
+        reference's node-shared window (:140-141).  Collective on the communicator of self.info; build it after
+        precompute_sky (later updates of self.c do not reach it)."""
+        return conviqt_sampler(self.c, self.bmax, self.npix, self.optim, self.info.geom_info_T, comm=self._comm())
+
     def dealloc(self):
         """:360-368"""
         self.c = None
         self.alm_beam = None
+
+
+class conviqt_sampler:
+    """interp (:155-205) on the device (cmdr_sht_conviqt_interp), bit for bit the single-precision arithmetic of the
+    reference, for any global RING pixel on any rank."""
+
+    def __init__(self, cube, bmax, npix, optim, geom_T, comm=None):
+        import torch
+        self.npix, self.optim = npix, optim
+        self.device = torch.device("cuda", torch.cuda.current_device()) if isinstance(cube, np.ndarray) else cube.device
+        with torch.cuda.device(self.device):
+            st = None if isinstance(cube, np.ndarray) else torch.cuda.current_stream().cuda_stream
+            self.handle = sharp.conviqt_sampler(cube, bmax, geom_T, stream=st, comm=comm)
+
+    def interp(self, pix, psi, out=None):
+        """Samples at global RING pixels `pix` and angles `psi` (broadcast together): numpy in, numpy out; torch in, torch
+        out (on the sampler's device, or host tensors).  psi is rounded to float32 first, as the mirror does.  A pixel
+        outside 0 .. 12 nside^2 - 1 raises IndexError after the call (its entry of `out` is NaN)."""
+        import torch
+        if isinstance(pix, torch.Tensor) or isinstance(psi, torch.Tensor):
+            p = torch.as_tensor(pix)
+            p, q = torch.broadcast_tensors(p, torch.as_tensor(psi, device=p.device))
+            if p.is_cuda and p.device != self.device:
+                raise ValueError(f"samples on {p.device}, sampler on {self.device}")
+            shape = p.shape
+            p, q = p.reshape(-1), q.reshape(-1)
+            if p.dtype != torch.int32:
+                p = torch.where((p < 0) | (p >= self.npix), -1, p).to(torch.int32)
+            p, q = p.contiguous(), q.to(torch.float32).contiguous()
+            if out is None:
+                out = torch.empty(shape, dtype=torch.float32, device=p.device)
+            st = torch.cuda.current_stream(self.device).cuda_stream if p.is_cuda else None
+        else:
+            p, q = np.broadcast_arrays(np.atleast_1d(np.asarray(pix)), np.atleast_1d(np.asarray(psi)))
+            shape = p.shape
+            p = p.reshape(-1)
+            if p.dtype != np.int32:
+                p = np.where((p < 0) | (p >= self.npix), -1, p).astype(np.int32)
+            p, q = np.ascontiguousarray(p), np.ascontiguousarray(q.reshape(-1), dtype=np.float32)
+            if out is None:
+                out = np.empty(shape, dtype=np.float32)
+            st = None
+        if tuple(out.shape) != tuple(shape) or not (out.flags.c_contiguous if isinstance(out, np.ndarray)
+                                                    else out.is_contiguous()):
+            raise ValueError(f"out must be contiguous with shape {tuple(shape)}")
+        with torch.cuda.device(self.device):
+            nbad = sharp.conviqt_interp(self.handle, p, q, self.optim, out.reshape(-1), stream=st)
+        if nbad:
+            raise IndexError(f"{nbad} pixel(s) outside 0..{self.npix - 1}")
+        return out
+
+    def close(self):
+        if getattr(self, "handle", None):
+            sharp.conviqt_sampler_destroy(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        self.close()

@@ -785,6 +785,20 @@ bool comm_all_equal(int comm, int v, cudaStream_t st) {
   return r[0] == -r[1];   // max v == min v
 }
 
+bool comm_group(int comm, int &rank, int &nranks) {
+  DistComm *C = find_comm(comm);
+  rank = 0; nranks = 1;
+  if (!C || C->nranks == 1) return false;
+  rank = C->rank; nranks = C->nranks;
+  return true;
+}
+
+void comm_allgather(int comm, const void *in, void *out, size_t bytes, cudaStream_t st) {
+  DistComm *C = find_comm(comm);
+  CMDR_NCCL_CHECK(nccl_api()->AllGather(in, out, bytes, ncclChar, C->nccl, st));
+  count_launch(1);
+}
+
 // map *= F, the pixel-space mixing step between Y and YtW (HBM-bound: 24 bytes per pixel)
 __global__ void __launch_bounds__(256) scale_map_kernel(double *__restrict__ m, const double *__restrict__ f, long long n) {
   const long long stride = (long long)gridDim.x * blockDim.x;

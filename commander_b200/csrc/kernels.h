@@ -213,6 +213,11 @@ void cr_multi_precond(CrMulti *S, const double *r, double *z, cudaStream_t st);
 void cr_multi_set_mixing(CrMulti *S, int band, int comp, const double *const *F, cudaStream_t st);
 // true when every rank of `comm` passed the same v (one 8-byte max all-reduce of (v, -v)); true on one GPU
 bool comm_all_equal(int comm, int v, cudaStream_t st);
+// rank and size of `comm` when it is a registered group of several ranks (true); else rank 0 of 1 (false)
+bool comm_group(int comm, int &rank, int &nranks);
+// NCCL all-gather of `bytes` per rank on a registered group of several ranks: out (device) receives the ranks' blocks
+// in rank order
+void comm_allgather(int comm, const void *in, void *out, size_t bytes, cudaStream_t st);
 
 }  // namespace cmdr
 

@@ -34,7 +34,8 @@ ABI_SYMBOLS = [
     # part 2: additive
     "cmdr_sht_version", "cmdr_sht_execute_dev", "cmdr_sht_execute_iqu", "cmdr_sht_execute_iqu_batch", "cmdr_sht_get_unique_id",
     "cmdr_sht_comm_register", "cmdr_sht_comm_destroy", "cmdr_sht_comm_set_exchange", "cmdr_sht_execute_dist",
-    "cmdr_sht_execute_iqu_dist", "cmdr_sht_mix", "cmdr_sht_invn_diag", "cmdr_sht_conviqt_cube", "cmdr_sht_allreduce_sum", "cmdr_sht_launch_count",
+    "cmdr_sht_execute_iqu_dist", "cmdr_sht_mix", "cmdr_sht_invn_diag", "cmdr_sht_conviqt_cube", "cmdr_sht_conviqt_sampler",
+    "cmdr_sht_conviqt_interp", "cmdr_sht_conviqt_sampler_destroy", "cmdr_sht_allreduce_sum", "cmdr_sht_launch_count",
     "cmdr_sht_set_profiling", "cmdr_sht_last_legendre_ms", "cmdr_sht_nominal_flops",
     "cmdr_sht_release_caches", "cmdr_sht_measure_fp64_tflops", "cmdr_sht_measure_fp64_tflops_3op",
     "cmdr_sht_measure_host_copy", "cmdr_sht_host_copy_threads", "cmdr_sht_set_legendre_seeds", "cmdr_sht_legendre_seed_bytes",
@@ -80,6 +81,11 @@ def lib() -> C.CDLL:
     L.cmdr_sht_mix.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp]
     L.cmdr_sht_invn_diag.argtypes = [ci, vp, C.c_double, vp, vp, vp]
     L.cmdr_sht_conviqt_cube.argtypes = [ci, ci, ci, vp, vp, vp, vp, vp, ci, vp]
+    L.cmdr_sht_conviqt_sampler.argtypes = [ci, ci, vp, ci, vp, vp]
+    L.cmdr_sht_conviqt_sampler.restype = vp
+    L.cmdr_sht_conviqt_interp.argtypes = [vp, C.c_longlong, vp, vp, ci, vp, vp]
+    L.cmdr_sht_conviqt_interp.restype = C.c_longlong
+    L.cmdr_sht_conviqt_sampler_destroy.argtypes = [vp]
     L.cmdr_sht_allreduce_sum.argtypes = [ci, vp, ci, vp]
     L.cmdr_sht_launch_count.restype = C.c_ulonglong
     L.cmdr_sht_set_profiling.argtypes = [ci]
@@ -333,19 +339,61 @@ def conviqt_cube(sky_alm, beam, bmax, geom_T: sharp_geom_info, alm_info: sharp_a
         if beam.dtype != torch.complex64 or not beam.is_contiguous() or tuple(beam.shape) != (ntri, nmaps):
             raise ValueError("beam must be a contiguous complex64 tensor of shape (ntri, nmaps)")
         bptr = beam.data_ptr()
-    shape = (2 * bmax, geom_T.n_local)
-    if isinstance(cube, np.ndarray):
-        if cube.dtype not in (np.float32, np.float64) or not cube.flags.c_contiguous or cube.shape != shape:
-            raise ValueError(f"cube must be a C-contiguous float32/float64 array of shape {shape}")
-        cptr, f64 = cube.ctypes.data, cube.dtype == np.float64
-    else:
-        import torch
-        if cube.dtype not in (torch.float32, torch.float64) or not cube.is_contiguous() or tuple(cube.shape) != shape:
-            raise ValueError(f"cube must be a contiguous float32/float64 tensor of shape {shape}")
-        cptr, f64 = cube.data_ptr(), cube.dtype == torch.float64
+    cptr, f64 = _cube_arg(cube, (2 * bmax, geom_T.n_local))
     st = C.c_void_p(stream) if stream else None
     L.cmdr_sht_conviqt_cube(int(comm) if comm is not None else -1, nmaps, int(bmax), alm_ptr, bptr,
                             geom_T.handle, alm_info.handle, cptr, 1 if f64 else 0, st)
+
+
+def _cube_arg(cube, shape):
+    """(pointer, is float64) of a conviqt cube (2*bmax, n_pix), float32 or float64, numpy or torch."""
+    if isinstance(cube, np.ndarray):
+        if cube.dtype not in (np.float32, np.float64) or not cube.flags.c_contiguous or cube.shape != shape:
+            raise ValueError(f"cube must be a C-contiguous float32/float64 array of shape {shape}")
+        return cube.ctypes.data, cube.dtype == np.float64
+    import torch
+    if cube.dtype not in (torch.float32, torch.float64) or not cube.is_contiguous() or tuple(cube.shape) != shape:
+        raise ValueError(f"cube must be a contiguous float32/float64 tensor of shape {shape}")
+    return cube.data_ptr(), cube.dtype == torch.float64
+
+
+def conviqt_sampler(cube, bmax, geom_T: sharp_geom_info, stream=None, comm=None) -> int:
+    """The full-sky float table of the conviqt cube on the current device (cmdr_sht_conviqt_sampler; collective on
+    `comm`).  cube (2*bmax, n_pix) float32 or float64, as conviqt_cube wrote it on this rank, numpy or torch.
+    Returns the handle for conviqt_interp; free it with conviqt_sampler_destroy."""
+    cptr, f64 = _cube_arg(cube, (2 * bmax, geom_T.n_local))
+    st = C.c_void_p(stream) if stream else None
+    return lib().cmdr_sht_conviqt_sampler(int(comm) if comm is not None else -1, int(bmax), cptr, 1 if f64 else 0,
+                                          geom_T.handle, st)
+
+
+def _flat_arg(a, np_dtype, name):
+    """(pointer, length) of a contiguous 1-d numpy array or torch tensor of dtype np_dtype."""
+    if isinstance(a, np.ndarray):
+        if a.dtype != np_dtype or a.ndim != 1 or not a.flags.c_contiguous:
+            raise ValueError(f"{name} must be a contiguous 1-d {np.dtype(np_dtype).name} array")
+        return a.ctypes.data, a.size
+    import torch
+    if a.dtype != getattr(torch, np.dtype(np_dtype).name) or a.dim() != 1 or not a.is_contiguous():
+        raise ValueError(f"{name} must be a contiguous 1-d {np.dtype(np_dtype).name} tensor")
+    return a.data_ptr(), a.numel()
+
+
+def conviqt_interp(sampler, pix, psi, optim, out, stream=None) -> int:
+    """out <- comm_conviqt%interp(pix, psi) (commander3/src/comm_conviqt_mod.f90:155-205) from the sampler's table
+    (cmdr_sht_conviqt_interp).  pix int32 global RING pixels, psi float32, out float32: 1-d, one length, numpy or torch,
+    host or device.  Returns the number of pixels outside the sky (their out is NaN)."""
+    pp, n = _flat_arg(pix, np.int32, "pix")
+    qp, nq = _flat_arg(psi, np.float32, "psi")
+    op, no = _flat_arg(out, np.float32, "out")
+    if not n == nq == no:
+        raise ValueError("pix, psi and out must have the same length")
+    st = C.c_void_p(stream) if stream else None
+    return int(lib().cmdr_sht_conviqt_interp(sampler, n, pp, qp, int(optim), op, st))
+
+
+def conviqt_sampler_destroy(sampler) -> None:
+    lib().cmdr_sht_conviqt_sampler_destroy(sampler)
 
 
 def launch_count() -> int:
