@@ -698,7 +698,8 @@ class cr_native_multi_system:
     float64 arrays of length ncr in cr_system's layout (component after component, each (nmaps, nalm)), numpy or torch.
     precond: 'diagonal' (the block-diagonal preconditioner of cr_system.initDiffPrecond_diagonal, from F_mean) or 'none'.
     pixel_mixing: install every per-pixel mixing map c.F[q] that is not None (cmdr_cr_set_mixing_map); without it a
-    component that carries one is refused.  set_mixing_map replaces or removes one between solves."""
+    component that carries one is refused.  set_mixing_map replaces or removes one between solves; set_pseudoinv switches
+    to the pseudo-inverse preconditioner and back."""
 
     def __init__(self, comps, bands, precond: str = "diagonal", pixel_mixing: bool = False):
         import ctypes as C
@@ -781,6 +782,12 @@ class cr_native_multi_system:
         fp, _keep = _ptrs(self._mixing_cols(q, k, F))
         self.L.cmdr_cr_set_mixing_map(self.handle, q, k, fp, None)
 
+    def set_pseudoinv(self, on=True):
+        """Selects the pseudo-inverse preconditioner (cr_system's precond = 'pseudoinv': applyDiffPrecond_pseudoinv,
+        commander3/src/comm_diffuse_comp_mod.f90:2237-2380) for invM and solve, built on the device the first time; on=False
+        returns to the preconditioner chosen at construction.  Collective; invM is collective while it is selected."""
+        self.L.cmdr_cr_set_pseudoinv(self.handle, 1 if on else 0, None)
+
     def _mixing_cols(self, q, k, F):
         """The min(nmaps_q, nmaps_k) float64 columns of a mixing map, after the range and shape checks."""
         nb, nc = len(self.bands), len(self.comps)
@@ -847,7 +854,8 @@ class cr_native_multi_system:
         return y
 
     def invM(self, r):
-        """cr_invM with the block-diagonal preconditioner (comm_diffuse_comp_mod.f90:2186-2235), or the identity"""
+        """cr_invM with the block-diagonal preconditioner (comm_diffuse_comp_mod.f90:2186-2235), the identity, or the
+        pseudo-inverse after set_pseudoinv()"""
         z = self._like(r)
         rp, _a = self._cols(r)
         zp, _b = self._cols(z)

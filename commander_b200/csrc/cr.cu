@@ -53,7 +53,7 @@ struct cmdr_cr_system {
   std::vector<double> h_lsc;   // host copy of lsc (preconditioner build)
   std::vector<long long> col;  // a_lm per column of a CG vector: nmaps x nalm, or those of every component (multi)
   cmdr::CrMulti *multi = nullptr;   // several components and bands (cmdr_cr_setup_multi, cr_multi.cu)
-  double *vs = nullptr;        // M^-1 r of the block preconditioner (multi)
+  double *vs = nullptr;        // M^-1 r of the block or pseudo-inverse preconditioner (multi)
 };
 
 namespace {
@@ -236,7 +236,7 @@ void alloc_work(cmdr_cr_system *s, cudaStream_t st) {
   CMDR_CUDA_CHECK(cudaHostAlloc(&s->h_sc, sizeof(double) * S_COUNT, cudaHostAllocDefault));
 }
 
-// the preconditioner step of the CG: z = M^-1 r with the block preconditioner of a multi system
+// the preconditioner step of the CG: z = M^-1 r with the block or pseudo-inverse preconditioner of a multi system
 bool block_precond(const cmdr_cr_system *s) { return s->multi && cr_multi_has_precond(s->multi); }
 
 void no_diag_precond(const cmdr_cr_system *s, const char *who) {
@@ -392,6 +392,16 @@ void cmdr_cr_set_mixing_map(cmdr_cr_system *s, int band, int comp, const double 
   cr_multi_set_mixing(s->multi, band, comp, F, (cudaStream_t)stream);
 }
 
+// Selects (on != 0) the pseudo-inverse preconditioner of a cmdr_cr_setup_multi handle, or the one chosen at setup.
+void cmdr_cr_set_pseudoinv(cmdr_cr_system *s, int on, void *stream) {
+  if (!s->multi) {
+    fprintf(stderr, "cmdr_sht: cmdr_cr_set_pseudoinv: %s\n", check_cr_pseudoinv(false, 0, 0, 0).c_str());
+    abort();
+  }
+  cr_multi_set_pseudoinv(s->multi, on, (cudaStream_t)stream);
+  if (block_precond(s) && !s->vs) s->vs = dalloc<double>(s->n);   // a handle built with precond 0
+}
+
 void cmdr_cr_destroy(cmdr_cr_system *s) {
   if (!s) return;
   cudaDeviceSynchronize();
@@ -500,8 +510,8 @@ int cmdr_cr_solve(cmdr_cr_system *s, const double *const *b, double *const *x, i
     CMDR_CUDA_CHECK(cudaMemcpyAsync(s->vr, s->vb, sizeof(double) * s->n, cudaMemcpyDeviceToDevice, st));
     ++s->n_matmul;
   }
-  // the block preconditioner is one more kernel (z = M^-1 r into s->vs) before the dot products that the diagonal one
-  // fuses into k_update / k_direction / k_dot
+  // the block and pseudo-inverse preconditioners are one more step (z = M^-1 r into s->vs) before the dot products that
+  // the diagonal one fuses into k_update / k_direction / k_dot
   const bool block = block_precond(s);
   if (block) cr_multi_precond(s->multi, s->vr, s->vd, st);                     // d = invM r           (:202)
   else k_direction<<<NBLK, NTHR, 0, st>>>(s->vd, s->vr, s->Minv, s->n, s->sc, 1);

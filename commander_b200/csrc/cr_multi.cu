@@ -11,13 +11,19 @@
 //     once per CG iteration;
 //   * spatially varying mixing of a (band, component) pair (cmdr_cr_set_mixing_map): evalDiffuseBand's Y, x F, YtW
 //     (comm_diffuse_comp_mod.f90:2070-2083) before the band gather, and projectDiffuseBand's (:2142-2151) after the
-//     band transform, F fused into the ring-FFT epilogue of the Y, b_l and sqrt(S) into the Legendre load and store.
+//     band transform, F fused into the ring-FFT epilogue of the Y, b_l and sqrt(S) into the Legendre load and store;
+//   * pseudo-inverse preconditioner (cmdr_cr_set_pseudoinv, applyDiffPrecond_pseudoinv :2237-2380): the band gather
+//     with U+ instead of g, WY with N = 1 / N^-1 fused into the ring-FFT epilogue, YtW, the component gather with
+//     alpha^2 U+, plus P P^t r on every preconditioner slot (tables from cr_pinv.h).
 // Every re-pack is rank-local because all handles list the same m's (cr_plan.h).
 #include <cmath>
 #include <vector>
 
 #include "cr_block.cuh"
+#include "cr_pinv.h"
 #include "kernels.h"
+
+extern "C" void cmdr_sht_allreduce_sum(int comm, double *dev_buf, int n, void *stream);
 
 namespace cmdr {
 
@@ -56,10 +62,10 @@ __device__ __forceinline__ bool mslot(const CrDev &D, int L, int &l, int &t) {
   return true;
 }
 
-// a_q[j, slot] = sum_k g[k][q][j][l] x_k[j, slot_k]; with MIX, the mixed pairs add their buffer (b_l Y^t W F Y sqrt(S)
-// x_k on the band's transform layout) instead
+// a_q[j, slot] = sum_k tab[k][q][j][l] x_k[j, slot_k] (tab: g, or U+ of the pseudo-inverse); with MIX, the mixed pairs
+// add their buffer (b_l Y^t W F Y sqrt(S) x_k on the band's transform layout) instead
 template <bool MIX>
-__global__ void __launch_bounds__(NTHR) k_cr_band_gather(CrDev D, int q, const double *__restrict__ x) {
+__global__ void __launch_bounds__(NTHR) k_cr_band_gather(CrDev D, int q, const double *__restrict__ tab, const double *__restrict__ x) {
   int l, t;
   if (!mslot(D, D.L[q], l, t)) return;
   const int j = blockIdx.z, im = blockIdx.y;
@@ -70,15 +76,17 @@ __global__ void __launch_bounds__(NTHR) k_cr_band_gather(CrDev D, int q, const d
       continue;
     }
     if (j >= D.cnm[k] || l > D.clmax[k]) continue;
-    acc = fma(D.fac(D.g, k, q, j, l), x[D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t], acc);
+    acc = fma(D.fac(tab, k, q, j, l), x[D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t], acc);
   }
   D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t] = acc;
 }
 
-// y_k[j, slot] = sum_q g[k][q][j][l] a'_q[j, slot_q] (+ add[slot] when add != nullptr); with MIX, the mixed pairs add
-// their buffer (sqrt(S) Y^t W F Y b_l a'_q, on layout mlay, l <= min(lmax_k, L_q)) instead
+// y_k[j, slot] = sum_q tab[k][q][j][l] a'_q[j, slot_q] (+ add[slot] when add != nullptr; tab: g, or alpha^2 U+ of the
+// pseudo-inverse); with MIX, the mixed pairs add their buffer (sqrt(S) Y^t W F Y b_l a'_q, on layout mlay,
+// l <= min(lmax_k, L_q)) instead
 template <bool MIX>
-__global__ void __launch_bounds__(NTHR) k_cr_comp_gather(CrDev D, int k, const double *__restrict__ add, double *__restrict__ y) {
+__global__ void __launch_bounds__(NTHR) k_cr_comp_gather(CrDev D, int k, const double *__restrict__ tab, const double *__restrict__ add,
+                                                        double *__restrict__ y) {
   int l, t;
   if (!mslot(D, D.clmax[k], l, t)) return;
   const int j = blockIdx.z, im = blockIdx.y;
@@ -87,7 +95,7 @@ __global__ void __launch_bounds__(NTHR) k_cr_comp_gather(CrDev D, int k, const d
     if (j >= D.bnm[q] || l > D.L[q]) continue;
     const int ip = q * D.ncomp + k;
     if (MIX && D.mix[ip]) acc += D.mix[ip][(long long)j * D.bnalm[q] + D.start(D.mlay[ip], im) + t];
-    else acc = fma(D.fac(D.g, k, q, j, l), D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t], acc);
+    else acc = fma(D.fac(tab, k, q, j, l), D.buf[q][(long long)j * D.bnalm[q] + D.start(D.xform0 + q, im) + t], acc);
   }
   const long long i = D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t;
   y[i] = add ? acc + add[i] : acc;
@@ -162,6 +170,71 @@ __global__ void __launch_bounds__(NTHR) k_cr_pre_apply(CrDev D, int lmax_pre, co
     if (idx[k] >= 0) z[idx[k]] = zv[k];
 }
 
+// N = 1 / N^-1 where N^-1 > 0, else 0: the noise covariance N%N of the pseudo-inverse (masked pixels carry no information)
+__global__ void __launch_bounds__(NTHR) k_cr_noise_cov(double *__restrict__ N, const double *__restrict__ invN, long long n) {
+  for (long long i = (long long)blockIdx.x * NTHR + threadIdx.x; i < n; i += (long long)gridDim.x * NTHR)
+    N[i] = invN[i] > 0.0 ? 1.0 / invN[i] : 0.0;
+}
+
+// partial[2 b], partial[2 b + 1] = sum of v, sum of v^2 over block b's elements (compute_alpha_nu's sums, first stage)
+__global__ void __launch_bounds__(NTHR) k_cr_sum2_partial(const double *__restrict__ v, long long n, double *__restrict__ partial) {
+  __shared__ double sh[2][NTHR];
+  double s1 = 0.0, s2 = 0.0;
+  for (long long i = (long long)blockIdx.x * NTHR + threadIdx.x; i < n; i += (long long)gridDim.x * NTHR) {
+    const double t = v[i];
+    s1 += t;
+    s2 = fma(t, t, s2);
+  }
+  sh[0][threadIdx.x] = s1; sh[1][threadIdx.x] = s2;
+  __syncthreads();
+  for (int o = NTHR / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) { sh[0][threadIdx.x] += sh[0][threadIdx.x + o]; sh[1][threadIdx.x] += sh[1][threadIdx.x + o]; }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) { partial[2 * blockIdx.x] = sh[0][0]; partial[2 * blockIdx.x + 1] = sh[1][0]; }
+}
+
+// out[0..1] = the block partials summed in a fixed order (second stage)
+__global__ void __launch_bounds__(NTHR) k_cr_sum2_finish(const double *__restrict__ partial, int nblk, double *__restrict__ out) {
+  __shared__ double sh[2][NTHR];
+  double s1 = 0.0, s2 = 0.0;
+  for (int b = threadIdx.x; b < nblk; b += NTHR) { s1 += partial[2 * b]; s2 += partial[2 * b + 1]; }
+  sh[0][threadIdx.x] = s1; sh[1][threadIdx.x] = s2;
+  __syncthreads();
+  for (int o = NTHR / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) { sh[0][threadIdx.x] += sh[0][threadIdx.x + o]; sh[1][threadIdx.x] += sh[1][threadIdx.x + o]; }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) { out[0] = sh[0][0]; out[1] = sh[1][0]; }
+}
+
+// The prior term of the pseudo-inverse (:2322-2346) on every preconditioner slot: out_k = sum_k2 (P P^t)[k][k2] r_k2
+// with P P^t of this slot's (map, l) from PP ([j][l][cr_tri], cr_pinv_tables).  One thread per (map, slot); each
+// component slot is written by exactly one thread, and every one of them is written.
+template <int NMAX>
+__global__ void __launch_bounds__(NTHR) k_cr_pinv_prior(CrDev D, int lmax_pre, const double *__restrict__ PP,
+                                                       const double *__restrict__ r, double *__restrict__ out) {
+  int l, t;
+  if (!mslot(D, lmax_pre, l, t)) return;
+  const int j = blockIdx.z, im = blockIdx.y;
+  double rv[NMAX], zv[NMAX];
+  long long idx[NMAX];
+#pragma unroll
+  for (int k = 0; k < NMAX; ++k) {
+    idx[k] = -1;
+    rv[k] = 0.0;
+    if (k < D.ncomp && j < D.cnm[k] && l <= D.clmax[k]) {
+      idx[k] = D.off[k] + (long long)j * D.cnalm[k] + D.start(k, im) + t;
+      rv[k] = r[idx[k]];
+    }
+  }
+  const int ntri = D.ncomp * (D.ncomp + 1) / 2;
+  cr_block_apply<NMAX>(PP + ((long long)j * (lmax_pre + 1) + l) * ntri, 1, D.ncomp, rv, zv);
+#pragma unroll
+  for (int k = 0; k < NMAX; ++k)
+    if (idx[k] >= 0) out[idx[k]] = zv[k];
+}
+
 template <typename T>
 T *dalloc(size_t n) {
   T *p = nullptr;
@@ -199,9 +272,17 @@ struct CrMulti {
   std::vector<double *> mix;             // [nmin][nalm at L_q]: the pair's forward, then backward, mix
   int nmixed = 0;
   std::vector<double> h_sS, h_bl;        // [k][j][l] sqrt(S), [q][j][l] b_l: the lscale of the mixing transforms
+  std::vector<double> h_g;               // [k][q][j][l] F_mean b_l sqrt(S): what the pseudo-inverse's V is made of
   double *d_sS = nullptr, *d_bl = nullptr;
   double **d_mix = nullptr;
   int *d_mlay = nullptr;
+  // pseudo-inverse preconditioner (cmdr_cr_set_pseudoinv), built on first use
+  std::vector<sharp_alm_info *> ba;      // per band: its own handle (alpha_nu runs at lmax_q)
+  bool pinv = false;                     // selected for invM / solve
+  std::vector<double *> Ncov;            // per band: [nmaps_q][npix_q] N = 1 / N^-1 (0 where N^-1 <= 0), empty until built
+  double *d_U = nullptr, *d_UA = nullptr;   // [k][q][j][l] U+ and alpha^2 U+
+  double *d_PP = nullptr;                // [nmaps_pre][lmax_pre + 1][ncomp (ncomp + 1) / 2] P P^t
+  double *pt = nullptr;                  // prior term P P^t r: a CG vector
   int nmin(int q, int k) const { return std::min(bnm[q], cnm[k]); }
   // lmax_k <= lmax_q: the component side of the mix runs on the component's own handle (reads x_k, writes its layout);
   // else on the band's transform handle at L_q = lmax_q, through k_cr_mix_pack
@@ -209,7 +290,7 @@ struct CrMulti {
 };
 
 long long cr_multi_length(const CrMulti *S) { return S->off.back(); }
-bool cr_multi_has_precond(const CrMulti *S) { return S->Mtri != nullptr; }
+bool cr_multi_has_precond(const CrMulti *S) { return S->pinv || S->Mtri != nullptr; }
 void cr_multi_columns(const CrMulti *S, std::vector<long long> &len) {
   len.clear();
   for (int k = 0; k < S->p.ncomp; ++k) len.insert(len.end(), S->cnm[k], S->p.nalm[S->p.comp(k)]);
@@ -241,27 +322,11 @@ CrMulti *cr_multi_create(int comm, const CrPlan &plan, const sharp_alm_info *con
     if (sqrtS && sqrtS[cofs[k]]) S->prior |= 1u << k;
   }
   for (int q = 0; q < nb; ++q) bofs[q + 1] = bofs[q] + S->bnm[q];
-  // per-l factors: sS[k][j][l] = sqrt(C_l) (0 for l < 2 in polarisation) or 1 without prior, 0 beyond lmax_k;
-  // f[k][q][j][l] = F_mean b_l where both the component and the band transform hold (j, l); g = f sS
-  std::vector<double> sS((size_t)nc * 3 * nl, 0.0), f((size_t)nc * nb * 3 * nl, 0.0), g(f.size(), 0.0);
-  for (int k = 0; k < nc; ++k)
-    for (int j = 0; j < S->cnm[k]; ++j)
-      for (int l = 0; l <= clmax[k]; ++l) {
-        double v = 1.0;
-        if ((S->prior >> k) & 1u) v = (j > 0 && l < 2) ? 0.0 : sqrtS[cofs[k] + j][l];
-        sS[((size_t)k * 3 + j) * nl + l] = v;
-      }
-  for (int k = 0; k < nc; ++k)
-    for (int q = 0; q < nb; ++q)
-      for (int j = 0; j < std::min(S->cnm[k], S->bnm[q]); ++j) {
-        const double F = F_mean[((size_t)q * nc + k) * 3 + j];
-        for (int l = 0; l <= std::min(clmax[k], p.L[q]); ++l) {
-          const size_t i = (((size_t)k * nb + q) * 3 + j) * nl + l;
-          f[i] = F * b_l[bofs[q] + j][l];
-          g[i] = f[i] * sS[((size_t)k * 3 + j) * nl + l];
-        }
-      }
+  // per-l factors sqrt(S), F_mean b_l and their product g (cr_pinv.h)
+  std::vector<double> sS, f, g;
+  cr_factor_tables(nc, nb, nl, S->cnm.data(), clmax.data(), S->bnm.data(), p.L.data(), S->prior, sqrtS, b_l, F_mean, sS, f, g);
   S->h_sS = sS;
+  S->h_g = g;
   S->h_bl.assign((size_t)nb * 3 * nl, 0.0);
   for (int q = 0; q < nb; ++q)
     for (int j = 0; j < S->bnm[q]; ++j)
@@ -272,6 +337,7 @@ CrMulti *cr_multi_create(int comm, const CrPlan &plan, const sharp_alm_info *con
     S->gT.push_back(const_cast<sharp_geom_info *>(band_geom_T[q]));
     S->gP.push_back(const_cast<sharp_geom_info *>(band_geom_P[q]));
     sharp_alm_info *a = const_cast<sharp_alm_info *>(band_alm[q]);
+    S->ba.push_back(a);
     const bool own = p.L[q] < a->lmax;
     if (own) {
       std::vector<int> ms;
@@ -340,6 +406,8 @@ void cr_multi_destroy(CrMulti *S) {
     cudaFree(S->invN[q]); cudaFree(S->buf[q]);
   }
   for (size_t i = 0; i < S->F.size(); ++i) { cudaFree(S->F[i]); cudaFree(S->mix[i]); }
+  for (double *n : S->Ncov) cudaFree(n);
+  cudaFree(S->d_U); cudaFree(S->d_UA); cudaFree(S->d_PP); cudaFree(S->pt);
   cudaFree(S->d_sS); cudaFree(S->d_bl); cudaFree(S->d_mix); cudaFree(S->d_mlay);
   cudaFree(S->map); cudaFree(S->Mtri);
   cudaFree(S->d_mval); cudaFree(S->d_bstart); cudaFree(S->d_off); cudaFree(S->d_cnalm); cudaFree(S->d_cnm); cudaFree(S->d_clmax);
@@ -355,14 +423,16 @@ void band_cols(CrMulti *S, int q, double **alm, double **map) {
   }
 }
 
-// y_k = sum_q g a'_q (+ add on the components with a prior), every component
-void comp_gather(CrMulti *S, const double *add, double *y, cudaStream_t st) {
+// y_k = sum_q g a'_q (+ add on the components with a prior), every component; with `pinv`, y_k = sum_q alpha^2 U+ a'_q
+// + add on every component, F_mean mixing on every pair
+void comp_gather(CrMulti *S, const double *add, double *y, cudaStream_t st, bool pinv = false) {
   if (!S->p.nm()) return;
   for (int k = 0; k < S->p.ncomp; ++k) {
     const dim3 grid = mgrid(S->p.lmax[S->p.comp(k)], S->p.nm(), S->cnm[k]);
-    const double *a = ((S->prior >> k) & 1u) ? add : nullptr;
-    if (S->nmixed) k_cr_comp_gather<true><<<grid, NTHR, 0, st>>>(S->D, k, a, y);
-    else k_cr_comp_gather<false><<<grid, NTHR, 0, st>>>(S->D, k, a, y);
+    const double *a = (pinv || ((S->prior >> k) & 1u)) ? add : nullptr;
+    if (pinv) k_cr_comp_gather<false><<<grid, NTHR, 0, st>>>(S->D, k, S->d_UA, a, y);
+    else if (S->nmixed) k_cr_comp_gather<true><<<grid, NTHR, 0, st>>>(S->D, k, S->d_g, a, y);
+    else k_cr_comp_gather<false><<<grid, NTHR, 0, st>>>(S->D, k, S->d_g, a, y);
     count_launch(1);
   }
 }
@@ -441,8 +511,8 @@ void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st) {
         if (S->F[q * S->p.ncomp + k]) mix_forward(S, q, k, x, st);
     if (S->p.nm()) {
       const dim3 grid = mgrid(S->p.L[q], S->p.nm(), S->bnm[q]);
-      if (S->nmixed) k_cr_band_gather<true><<<grid, NTHR, 0, st>>>(S->D, q, x);
-      else k_cr_band_gather<false><<<grid, NTHR, 0, st>>>(S->D, q, x);
+      if (S->nmixed) k_cr_band_gather<true><<<grid, NTHR, 0, st>>>(S->D, q, S->d_g, x);
+      else k_cr_band_gather<false><<<grid, NTHR, 0, st>>>(S->D, q, S->d_g, x);
       count_launch(1);
     }
     band_cols(S, q, alm, map);
@@ -522,9 +592,126 @@ void cr_multi_set_mixing(CrMulti *S, int band, int comp, const double *const *F,
   CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
 }
 
-// z = M^-1 r with the block preconditioner
+namespace {
+// Builds what the pseudo-inverse needs (initDiffPrecond_pseudoinv, comm_diffuse_comp_mod.f90:1255-1294, 1560-1658):
+// N per band, alpha_nu per band and map group, the U+ / alpha^2 U+ / P P^t tables.  Collective (transforms and one
+// all-reduce); synchronises the stream.
+void pinv_build(CrMulti *S, cudaStream_t st) {
+  const CrPlan &p = S->p;
+  const int nc = p.ncomp, nb = p.nbands, nl = p.lmax_all + 1;
+  constexpr int NBLK = 592;
+  double *partial = dalloc<double>(2 * NBLK);
+  double *sums = dalloc<double>((size_t)4 * nb);   // [q][T, QU][sum tau, sum tau^2]
+  CMDR_CUDA_CHECK(cudaMemsetAsync(sums, 0, sizeof(double) * 4 * nb, st));
+  for (int q = 0; q < nb; ++q) {
+    const long long np = S->npix[q];
+    double *N = dalloc<double>((size_t)S->bnm[q] * np);
+    if (np) {
+      k_cr_noise_cov<<<NBLK, NTHR, 0, st>>>(N, S->invN[q], (long long)S->bnm[q] * np);
+      count_launch(1);
+    }
+    S->Ncov.push_back(N);
+    // compute_alpha_nu (comm_N_rms_mod.f90:218-247): tau = Y Yt (N^-1) on the band's own handle, into the work map
+    const long long na = p.nalm[p.band(q)];
+    double *alm_d = dalloc<double>((size_t)S->bnm[q] * na);
+    double *alm[3], *in[3], *map[3];
+    for (int j = 0; j < S->bnm[q]; ++j) {
+      alm[j] = alm_d + (size_t)j * na;
+      in[j] = S->invN[q] + (size_t)j * np;
+      map[j] = S->map + (size_t)j * np;
+    }
+    execute_iqu_opts(S->comm, SHARP_Yt, S->bnm[q], alm, in, S->gT[q], S->gP[q], S->ba[q], SHARP_DP, nullptr, st);
+    execute_iqu_opts(S->comm, SHARP_Y, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->ba[q], SHARP_DP, nullptr, st);
+    for (int grp = 0; grp < (S->bnm[q] == 3 ? 2 : 1); ++grp) {   // T alone, Q and U together
+      if (!np) continue;
+      k_cr_sum2_partial<<<NBLK, NTHR, 0, st>>>(S->map + (size_t)grp * np, (grp ? 2 : 1) * np, partial);
+      k_cr_sum2_finish<<<1, NTHR, 0, st>>>(partial, NBLK, sums + 4 * q + 2 * grp);
+      count_launch(2);
+    }
+    CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+    cudaFree(alm_d);
+  }
+  cmdr_sht_allreduce_sum(S->comm, sums, 4 * nb, st);
+  std::vector<double> h(4 * nb), alpha((size_t)3 * nb, 0.0);
+  CMDR_CUDA_CHECK(cudaMemcpyAsync(h.data(), sums, sizeof(double) * 4 * nb, cudaMemcpyDeviceToHost, st));
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+  cudaFree(partial); cudaFree(sums);
+  for (int q = 0; q < nb; ++q)
+    for (int j = 0; j < S->bnm[q]; ++j) {
+      const double s1 = h[4 * q + 2 * (j > 0)], s2 = h[4 * q + 2 * (j > 0) + 1];
+      alpha[(size_t)q * 3 + j] = s1 > 0.0 ? std::sqrt(s2 / s1) : 0.0;
+    }
+  std::vector<int> clmax(nc);
+  for (int k = 0; k < nc; ++k) clmax[k] = p.lmax[p.comp(k)];
+  std::vector<double> U, UA, PP;
+  cr_pinv_tables(nc, nb, nl, p.nmaps_pre, p.lmax_pre, S->cnm.data(), clmax.data(), S->prior, S->h_g, alpha.data(), U, UA, PP);
+  S->d_U = upload(U);
+  S->d_UA = upload(UA);
+  S->d_PP = upload(PP);
+  S->pt = dalloc<double>(S->off.back());
+}
+
+// z = M^-1 r with the pseudo-inverse (applyDiffPrecond_pseudoinv, :2237-2380).  buf[q] and map are scratch here:
+// cr_multi_matmulA and cr_multi_rhs rewrite both before they read them.
+void pinv_apply(CrMulti *S, const double *r, double *z, cudaStream_t st) {
+  const CrPlan &p = S->p;
+  if (p.nm()) {                                                    // P P^t r, :2322-2346
+    const dim3 grid = mgrid(p.lmax_pre, p.nm(), p.nmaps_pre);
+    if (p.ncomp <= 4) k_cr_pinv_prior<4><<<grid, NTHR, 0, st>>>(S->D, p.lmax_pre, S->d_PP, r, S->pt);
+    else if (p.ncomp <= 8) k_cr_pinv_prior<8><<<grid, NTHR, 0, st>>>(S->D, p.lmax_pre, S->d_PP, r, S->pt);
+    else k_cr_pinv_prior<CR_MAX_NPRE><<<grid, NTHR, 0, st>>>(S->D, p.lmax_pre, S->d_PP, r, S->pt);
+    count_launch(1);
+  }
+  double *alm[3], *map[3];
+  for (int q = 0; q < p.nbands; ++q) {
+    if (p.nm()) {                                                  // sum over (U+)^t, :2270-2285
+      k_cr_band_gather<false><<<mgrid(p.L[q], p.nm(), S->bnm[q]), NTHR, 0, st>>>(S->D, q, S->d_U, r);
+      count_launch(1);
+    }
+    band_cols(S, q, alm, map);
+    XformOpts o;                                                   // N%N as the map is written, :2288-2290
+    for (int j = 0; j < S->bnm[q]; ++j) o.pixscale[j] = S->Ncov[q] + (size_t)j * S->npix[q];
+    execute_iqu_opts(S->comm, SHARP_WY, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, &o, st);
+    execute_iqu_opts(S->comm, SHARP_YtW, S->bnm[q], alm, map, S->gT[q], S->gP[q], S->xa[q], SHARP_DP, nullptr, st);   // :2292
+  }
+  comp_gather(S, S->pt, z, st, true);                              // alpha^2, sum over U+, :2293-2315
+}
+}  // namespace
+
+// Selects (on) or deselects the pseudo-inverse preconditioner; the tables are built on the first selection
+void cr_multi_set_pseudoinv(CrMulti *S, int on, cudaStream_t st) {
+  const CrPlan &p = S->p;
+  size_t need = 0;
+  if (on && S->Ncov.empty() && p.ncomp <= CR_MAX_NPRE) {
+    const size_t ntab = (size_t)p.ncomp * p.nbands * 3 * (p.lmax_all + 1);
+    size_t pix = 0, alm = 0;
+    for (int q = 0; q < p.nbands; ++q) {
+      pix += (size_t)S->bnm[q] * S->npix[q];
+      alm = std::max(alm, (size_t)S->bnm[q] * (size_t)p.nalm[p.band(q)]);
+    }
+    need = sizeof(double) * (2 * ntab + (size_t)p.nmaps_pre * (p.lmax_pre + 1) * (p.ncomp * (p.ncomp + 1) / 2) + pix + alm +
+                             (size_t)S->off.back());
+  }
+  size_t free_b = 0, total_b = 0;
+  CMDR_CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+  const std::string err = check_cr_pseudoinv(true, p.ncomp, need, free_b);
+  // every rank learns whether all passed the same `on` and all were valid before any of them aborts
+  const bool same = comm_all_equal(S->comm, err.empty() ? (on != 0) : -1, st);
+  if (!err.empty()) { fprintf(stderr, "cmdr_sht: cmdr_cr_set_pseudoinv: %s\n", err.c_str()); abort(); }
+  if (!same) {
+    fprintf(stderr, "cmdr_sht: cmdr_cr_set_pseudoinv: the ranks passed different `on` or one of them was refused; every rank "
+                    "of the communicator must make the same call\n");
+    abort();
+  }
+  if (on && S->Ncov.empty()) pinv_build(S, st);
+  S->pinv = on != 0;
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+}
+
+// z = M^-1 r with the selected preconditioner: the pseudo-inverse, or the block diagonal
 void cr_multi_precond(CrMulti *S, const double *r, double *z, cudaStream_t st) {
   const CrPlan &p = S->p;
+  if (S->pinv) { pinv_apply(S, r, z, st); return; }
   if (!p.nm()) return;
   const dim3 grid = mgrid(p.lmax_pre, p.nm(), p.nmaps_pre);
   const long long nalm_pre = p.nalm[p.pre()];

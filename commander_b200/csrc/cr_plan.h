@@ -158,4 +158,18 @@ inline std::string check_cr_mixing(bool multi, int ncomp, int nbands, const int 
   return "";
 }
 
+// Checks a cmdr_cr_set_pseudoinv call on one rank.  `multi`: the handle comes from cmdr_cr_setup_multi; `need_bytes`:
+// device memory the tables still need (0 once they are built), `free_bytes`: what the device has free.  Returns the
+// reason of a refusal, or an empty string.
+inline std::string check_cr_pseudoinv(bool multi, int ncomp, size_t need_bytes, size_t free_bytes) {
+  if (!multi)
+    return "needs a handle of cmdr_cr_setup_multi (give a one-component system to cmdr_cr_setup_multi with ncomp = 1)";
+  if (ncomp > CR_MAX_NPRE)
+    return "ncomp " + std::to_string(ncomp) + " above the pseudo-inverse preconditioner's limit of " + std::to_string(CR_MAX_NPRE);
+  if (need_bytes > free_bytes)
+    return "the pseudo-inverse preconditioner needs " + std::to_string(need_bytes) + " bytes of device memory, " +
+           std::to_string(free_bytes) + " are free";
+  return "";
+}
+
 }  // namespace cmdr

@@ -204,11 +204,14 @@ CrMulti *cr_multi_create(int comm, const CrPlan &plan, const sharp_alm_info *con
 void cr_multi_destroy(CrMulti *S);
 long long cr_multi_length(const CrMulti *S);
 void cr_multi_columns(const CrMulti *S, std::vector<long long> &len);   // a_lm per column of a CG vector
-bool cr_multi_has_precond(const CrMulti *S);
+bool cr_multi_has_precond(const CrMulti *S);   // a preconditioner other than the identity is selected
 void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st);
 void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *eta_pix, const double *eta_alm, double *b,
                   cudaStream_t st);
+// z = M^-1 r with the selected preconditioner (pseudo-inverse or block diagonal; collective with the pseudo-inverse)
 void cr_multi_precond(CrMulti *S, const double *r, double *z, cudaStream_t st);
+// cmdr_cr_set_pseudoinv on a multi-component handle: checks (collectively), builds the tables on first use, selects
+void cr_multi_set_pseudoinv(CrMulti *S, int on, cudaStream_t st);
 // cmdr_cr_set_mixing_map on a multi-component handle: checks (collectively), then installs or removes the map
 void cr_multi_set_mixing(CrMulti *S, int band, int comp, const double *const *F, cudaStream_t st);
 // true when every rank of `comm` passed the same v (one 8-byte max all-reduce of (v, -v)); true on one GPU

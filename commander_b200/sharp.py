@@ -41,7 +41,7 @@ ABI_SYMBOLS = [
     "cmdr_sht_measure_host_copy", "cmdr_sht_host_copy_threads", "cmdr_sht_set_legendre_seeds", "cmdr_sht_legendre_seed_bytes",
     "cmdr_cr_setup", "cmdr_cr_destroy", "cmdr_cr_matmulA", "cmdr_cr_invM", "cmdr_cr_set_precond_diag",
     "cmdr_cr_get_precond_diag", "cmdr_cr_compute_rhs", "cmdr_cr_solve", "cmdr_cr_matmul_count", "cmdr_cr_setup_multi",
-    "cmdr_cr_set_mixing_map",
+    "cmdr_cr_set_mixing_map", "cmdr_cr_set_pseudoinv",
 ]
 
 
@@ -107,6 +107,7 @@ def lib() -> C.CDLL:
     L.cmdr_cr_setup_multi.argtypes = [ci, ci, vp, vp, vp, ci, vp, vp, vp, vp, vp, vp, vp, ci]
     L.cmdr_cr_setup_multi.restype = vp
     L.cmdr_cr_set_mixing_map.argtypes = [vp, ci, ci, vp, vp]
+    L.cmdr_cr_set_pseudoinv.argtypes = [vp, ci, vp]
     L.cmdr_cr_destroy.argtypes = [vp]
     L.cmdr_cr_matmulA.argtypes = [vp, vp, vp, vp]
     L.cmdr_cr_invM.argtypes = [vp, vp, vp, vp]

@@ -2,9 +2,13 @@
 comm_cr.cr_system on the sampling group of tests/test_gpu_cr_multi_native.py::real_size_problem: bands (nside / lmax)
 512 / 1500, 1024 / 2000, 1024 / 2000; components CMB (3 maps, lmax 2000, prior), dust (3, 1500, prior) and a 1-map
 low-l component without prior.  With --pixel-F the dust component is mixed per pixel in every band
-(cmdr_cr_set_mixing_map; the mirror gets the same maps) and the result goes to cr_mix_bench[_nN].json.
+(cmdr_cr_set_mixing_map; the mirror gets the same maps) and the result goes to cr_mix_bench[_nN].json.  With
+--precond pseudoinv both solvers use the pseudo-inverse preconditioner (cmdr_cr_set_pseudoinv on the native handle,
+precond = 'pseudoinv' on the mirror), the switch's setup time is recorded, and the result goes to
+cr_pinv_bench[_nN].json.  Either preconditioner also records the iterations (and time) to cg_tol = 1e-8 in 'residual'
+mode, which with the per-iteration rate settles what a preconditioner buys on this group.
 
-  python tools/cr_multi_bench.py --out DIR [--pixel-F]     (one GPU)
+  python tools/cr_multi_bench.py --out DIR [--pixel-F] [--precond {diagonal,pseudoinv}]     (one GPU)
   python -m torch.distributed.run --nproc-per-node N tools/cr_multi_bench.py --out DIR
 
 Each solve runs `fixed_iter` iterations after a warm-up solve and is timed with CUDA events around work that ends in a
@@ -57,6 +61,10 @@ def main():
     ap.add_argument("--iters", type=int, default=50)
     ap.add_argument("--mirror-iters", type=int, default=10)
     ap.add_argument("--pixel-F", action="store_true", help="mix the dust component per pixel in every band")
+    ap.add_argument("--precond", choices=("diagonal", "pseudoinv"), default="diagonal",
+                    help="block-diagonal (default) or pseudo-inverse preconditioner")
+    ap.add_argument("--residual-maxiter", type=int, default=2000,
+                    help="iteration cap of the 'residual' solve to cg_tol = 1e-8 (0: skip it)")
     args = ap.parse_args()
     import torch
     from commander_b200 import comm_mapinfo
@@ -91,6 +99,13 @@ def main():
     rng = np.random.default_rng(16)
     data = [torch.as_tensor(rng.standard_normal((3, i.np)), device=dev) for i in binfo]
     b = nat.computeRHS(data)
+    setup_ms = None
+    if args.precond == "pseudoinv":                             # the call synchronises: a host clock is exact here
+        import time
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        nat.set_pseudoinv(True)
+        setup_ms = 1e3 * (time.perf_counter() - t0)
 
     def timed(fn, n):
         fn(2)                                                   # warm-up: every shape of the timed window
@@ -103,10 +118,25 @@ def main():
         return e0.elapsed_time(e1)
 
     ms_nat = timed(lambda n: nat.solve(b, maxiter=n, cg_conv_crit="fixed_iter"), args.iters)
-    res = {"world": world, "card": card(), "iters_native": args.iters,
+    res = {"world": world, "card": card(), "precond": args.precond, "iters_native": args.iters,
            "native_ms_per_iter": ms_nat / args.iters, "native_iter_per_s": 1e3 * args.iters / ms_nat}
+    if setup_ms is not None:
+        res["pseudoinv_setup_ms"] = setup_ms
+    if args.residual_maxiter > 0:
+        # a data-like right-hand side: noise-weighted white data, so the residual solve sees the signal-to-noise of a
+        # real run rather than the unit-variance maps of the timing loop
+        dres = [torch.as_tensor(rng.standard_normal((3, i.np)), device=dev) / torch.sqrt(c.invN) for i, c in zip(binfo, cb)]
+        bres = nat.computeRHS(dres)
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        _, it_res, _ = nat.solve(bres, maxiter=args.residual_maxiter, cg_tol=1e-8, cg_conv_crit="residual")
+        e1.record()
+        torch.cuda.synchronize()
+        res.update(residual_cg_tol=1e-8, residual_iters=it_res, residual_ms=e0.elapsed_time(e1),
+                   residual_maxiter=args.residual_maxiter)
     if args.mirror_iters > 0:
-        mir = cr_system(cc, cb, dev)
+        mir = cr_system(cc, cb, dev, precond=args.precond)
         ms_mir = timed(lambda n: solve_cr_eqn_by_CG(mir, b.clone(), maxiter=n, cg_conv_crit="fixed_iter"), args.mirror_iters)
         res.update(iters_mirror=args.mirror_iters, mirror_ms_per_iter=ms_mir / args.mirror_iters,
                    mirror_iter_per_s=1e3 * args.mirror_iters / ms_mir)
@@ -125,7 +155,7 @@ def main():
             continue
         t = ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total
         tot += t
-        for k in ("k_cr_band_gather", "k_cr_comp_gather", "k_cr_pre_apply", "k_cr_mix_pack"):
+        for k in ("k_cr_band_gather", "k_cr_comp_gather", "k_cr_pre_apply", "k_cr_mix_pack", "k_cr_pinv_prior"):
             if k in ev.name:
                 per[k] = per.get(k, 0.0) + t
     ms_local = cc[0].x_info.ms                                  # the largest lmax: every local m
@@ -134,7 +164,7 @@ def main():
     kern = {}
     for k, us in per.items():
         kern[k] = {"ms_per_iter": us / 1e3 / iters}
-        if k in nbytes:
+        if k in nbytes and args.precond == "diagonal":       # the byte model counts one gather pass per iteration
             kern[k].update(GB_per_iter=nbytes[k] / 1e9, GB_per_s=nbytes[k] / (us / 1e6 / iters) / 1e9 if us > 0 else None)
     res["kernels"] = kern
     res["pixel_F"] = [f"dust in band {q}" for q, _ in mixed]
@@ -142,7 +172,7 @@ def main():
     res["new_kernel_share"] = sum(per.values()) / tot if tot > 0 else None
     if rank == 0:
         os.makedirs(args.out, exist_ok=True)
-        name = "cr_mix_bench" if args.pixel_F else "cr_multi_bench"
+        name = "cr_mix_bench" if args.pixel_F else ("cr_pinv_bench" if args.precond == "pseudoinv" else "cr_multi_bench")
         path = os.path.join(args.out, f"{name}.json" if world == 1 else f"{name}_n{world}.json")
         with open(path, "w") as f:
             json.dump(res, f, indent=1)
