@@ -100,7 +100,7 @@ struct DistPlan {
   std::vector<int> lcut;                      // this rank's local pair boundaries, size nchunk + 1
   std::vector<sharp_geom_info *> subs;        // per chunk (nullptr when this rank has no pair in it)
   bool subs_built = false;
-  int pipe_ok = -1;                           // chunked host pipeline usable on EVERY rank (agreed once; -1 = not yet)
+  int pipe_ok = 0;                            // chunked host pipeline usable on EVERY rank (agreed in get_plan)
 };
 
 struct PeerBuf {                       // one receive buffer per rank, mapped by every rank
@@ -197,14 +197,19 @@ static DistPlan *get_plan(DistComm *C, sharp_geom_info *g, sharp_alm_info *a, cu
   if (it != C->plans.end()) return it->second;
   DistPlan *P = new DistPlan;
   const int R = C->nranks;
-  // sizes: {nm, npairs, nside, lmax}
-  std::vector<int> sz = allgather_ints(C, {a->nm, g->npairs, g->nside, a->lmax}, 4, st);
+  // sizes: {nm, npairs, nside, lmax, this rank can take the chunked host pipeline}.  The last entry is agreed here,
+  // where every rank is anyway, rather than in try_dist_pipelined: a rank without rings or m's gets null columns, which
+  // look like device arrays, and must not skip a collective the other ranks enter.
+  const int pipe_mine = (g->npairs > 0 && a->nm > 0 && pairs_contiguous(g)) ? 1 : 0;
+  std::vector<int> sz = allgather_ints(C, {a->nm, g->npairs, g->nside, a->lmax, pipe_mine}, 5, st);
   int NML = 1, NPL = 1;
+  P->pipe_ok = 1;
   for (int r = 0; r < R; ++r) {
-    if (sz[4 * r + 2] != g->nside || sz[4 * r + 3] != a->lmax) {
+    if (sz[5 * r + 2] != g->nside || sz[5 * r + 3] != a->lmax) {
       fprintf(stderr, "cmdr_sht: ranks disagree on nside/lmax\n"); abort();
     }
-    NML = std::max(NML, sz[4 * r]); NPL = std::max(NPL, sz[4 * r + 1]);
+    NML = std::max(NML, sz[5 * r]); NPL = std::max(NPL, sz[5 * r + 1]);
+    P->pipe_ok = std::min(P->pipe_ok, sz[5 * r + 4]);
   }
   P->NML = NML; P->NPL = NPL; P->nslots = R * NPL;
   std::vector<int> all_m = allgather_ints(C, a->mval, NML, st);
@@ -212,7 +217,7 @@ static DistPlan *get_plan(DistComm *C, sharp_geom_info *g, sharp_alm_info *a, cu
   // global slot geometry in work order
   std::vector<std::pair<int, int>> order;   // (north ring, storage slot)
   for (int r = 0; r < R; ++r)
-    for (int j = 0; j < sz[4 * r + 1]; ++j) order.emplace_back(all_north[(size_t)r * NPL + j], r * NPL + j);
+    for (int j = 0; j < sz[5 * r + 1]; ++j) order.emplace_back(all_north[(size_t)r * NPL + j], r * NPL + j);
   std::sort(order.begin(), order.end());
   std::vector<int> wslot(P->nslots, 0);
   std::vector<char> used(P->nslots, 0);
@@ -250,11 +255,11 @@ static DistPlan *get_plan(DistComm *C, sharp_geom_info *g, sharp_alm_info *a, cu
   P->d_wslot = upload(wslot);
   // global m tables
   int mmax = -1;
-  for (int r = 0; r < R; ++r) for (int i = 0; i < sz[4 * r]; ++i) mmax = std::max(mmax, all_m[(size_t)r * NML + i]);
+  for (int r = 0; r < R; ++r) for (int i = 0; i < sz[5 * r]; ++i) mmax = std::max(mmax, all_m[(size_t)r * NML + i]);
   P->mmax = mmax;
   std::vector<int> m2src(mmax + 2, -1), m2im(mmax + 2, -1), mlist, mlist_src, mlist_im;
   for (int r = 0; r < R; ++r)
-    for (int i = 0; i < sz[4 * r]; ++i) {
+    for (int i = 0; i < sz[5 * r]; ++i) {
       int m = all_m[(size_t)r * NML + i];
       if (m2src[m] >= 0) { fprintf(stderr, "cmdr_sht: m=%d owned by two ranks\n", m); abort(); }
       m2src[m] = r; m2im[m] = i;
@@ -562,31 +567,21 @@ static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, 
   const int spin = job.spin, nca = job.alm_cols, ncomp = job.map_cols;
   if (disabled || job.add || !use_p2p(C)) return false;
   // Every rank must take the same decision (the chunked path has K + 1 exchange barriers, the plain one 2).
-  // Global sizes are equal everywhere by construction; host-versus-device buffers is a property of the call
-  // site, the same on all ranks of a collective call (pinned or pageable does not matter: both take this
-  // path).  What can differ from rank to rank -- a rank without rings or m's, a ring list that is not
-  // contiguous -- is agreed once per plan with an all-reduce (min) and cached there.
+  // Global sizes are equal everywhere by construction.  What can differ from rank to rank -- a rank without
+  // rings or m's, a ring list that is not contiguous -- was agreed when the plan was built (get_plan, which
+  // every rank reaches here).  Once that holds, every rank has non-null columns, and host-versus-device buffers
+  // is a property of the call site, the same on all ranks of a collective call (pinned or pageable does not
+  // matter: both take this path).
   if ((long long)g->nside * g->nside * 12 < (1LL << 20) * C->nranks) return false;
-  for (int c = 0; c < nca; ++c)
-    if (host_kind(alm[c]) == HostKind::Device) return false;
-  for (int c = 0; c < ncomp; ++c)
-    if (host_kind(map[c]) == HostKind::Device) return false;
   const bool synth = job.synth;
   ensure_geom_device(g);
   ensure_alm_device(a);
   DistPlan *P = get_plan(C, g, a, st);
-  if (P->pipe_ok < 0) {
-    int ok = (g->npairs > 0 && a->nm > 0 && pairs_contiguous(g)) ? 1 : 0;
-    int *d_ok = nullptr;
-    CMDR_CUDA_CHECK(cudaMalloc(&d_ok, sizeof(int)));
-    CMDR_CUDA_CHECK(cudaMemcpyAsync(d_ok, &ok, sizeof(int), cudaMemcpyHostToDevice, st));
-    CMDR_NCCL_CHECK(nccl_api()->AllReduce(d_ok, d_ok, 1, ncclInt32, ncclMin, C->nccl, st));
-    CMDR_CUDA_CHECK(cudaMemcpyAsync(&ok, d_ok, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
-    cudaFree(d_ok);
-    P->pipe_ok = ok;
-  }
   if (!P->pipe_ok) return false;
+  for (int c = 0; c < nca; ++c)
+    if (host_kind(alm[c]) == HostKind::Device) return false;
+  for (int c = 0; c < ncomp; ++c)
+    if (host_kind(map[c]) == HostKind::Device) return false;
   const int K = (int)P->wcut.size() - 1;
   if (!P->subs_built) {
     P->subs_built = true;
@@ -675,7 +670,7 @@ static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, 
     cudaEvent_t e0 = pooled_event(ev0 + K);                // staging rows may still be read by earlier work on `st`
     CMDR_CUDA_CHECK(cudaEventRecord(e0, st));
     CMDR_CUDA_CHECK(cudaStreamWaitEvent(cs, e0, 0));
-    for (int c = 0; c < ncomp; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(alm_dev[c], 0, sizeof(double) * nalm_d, st));
+    for (int c = 0; c < nca; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(alm_dev[c], 0, sizeof(double) * nalm_d, st));
     stream_barrier(C, st);                                 // every rank has finished reading my buffer
     for (int c = 0; c < K; ++c) {                          // polar chunks (short rows) first
       sharp_geom_info *sub = P->subs[c];
@@ -703,7 +698,7 @@ static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, 
           CMDR_CUDA_CHECK(cudaEventRecord(ej, st));
           CMDR_CUDA_CHECK(cudaStreamWaitEvent(cs, ej, 0));
           const long long b = mstart[mcut[j]], e = mstart[mcut[j + 1]];
-          for (int k = 0; k < ncomp; ++k) ioA.d2h(alm_dev[k] + b, k, b, e - b, cs);
+          for (int k = 0; k < nca; ++k) ioA.d2h(alm_dev[k] + b, k, b, e - b, cs);
           ioA.commit(cs);
         }
       } else {
@@ -711,7 +706,7 @@ static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, 
       }
     }
     if (nmch == 1) {
-      for (int c = 0; c < ncomp; ++c) ioA.d2h(alm_dev[c], c, 0, nalm_d, st);
+      for (int c = 0; c < nca; ++c) ioA.d2h(alm_dev[c], c, 0, nalm_d, st);
       ioA.commit(st);
     }
     ioA.drain();
