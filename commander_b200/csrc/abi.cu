@@ -90,12 +90,13 @@ void ensure_coef(sharp_alm_info *a, int spin) {
   if (c.ready) return;
   std::vector<double> tab; std::vector<long long> ofs;
   std::vector<long long> tofs(a->nm + 1, 0);
-  if (spin == COEF_KEY_S0X2) {   // spin 0 in steps of two l: one tile row per step
+  if (spin == COEF_KEY_S0X2 || spin == COEF_KEY_S0X2P2) {   // spin 0 in steps of two l: one tile row per step
+    const int lmax = spin == COEF_KEY_S0X2 ? a->lmax : a->lmax + 2;
     std::vector<double> mix;
-    build_coef_table_x2(a->lmax, a->mval, tab, mix, ofs);
+    build_coef_table_x2(lmax, a->mval, tab, mix, ofs);
     c.tab2 = upload(mix);
     for (int i = 0; i < a->nm; ++i) {
-      long long n = a->lmax >= a->mval[i] ? (a->lmax - a->mval[i]) / 2 + 1 : 0;
+      long long n = lmax >= a->mval[i] ? (lmax - a->mval[i]) / 2 + 1 : 0;
       tofs[i + 1] = tofs[i] + ((n + 7) & ~7LL);
     }
   } else {
@@ -110,6 +111,7 @@ void ensure_coef(sharp_alm_info *a, int spin) {
   c.ofs = upload(ofs);
   c.tofs = upload(tofs);
   c.trows = tofs[a->nm];
+  c.nofs = ofs[a->nm];
   c.ready = true;
 }
 
@@ -459,6 +461,15 @@ void run_single(const Job &job, double *const *alm, double *const *map, sharp_ge
   G.nslots = g->npairs; G.NPL = g->npairs; G.nowners = 1; G.NML = a->nm; G.ncomp_tot = ncomp; G.comp0 = 0;
   G.trig = g->d_trig; G.mlim = ensure_mlim(g, a->lmax, spin);
   G.seed_geom = g; G.seed_alm = a;
+  if (spin == 2 && !job.deriv1 && spin2_scalar_on()) {   // spin 2 as scalar sums (legendre.cu, launch_s2s_*)
+    ensure_coef(a, COEF_KEY_S0X2P2);
+    const CoefDev &c = a->coef[COEF_KEY_S0X2P2];
+    A.s2s_coef = c.tab; A.s2s_mix = c.tab2; A.s2s_cofs = c.ofs; A.s2s_tofs = c.tofs; A.s2s_trows = c.trows; A.s2s_nl = c.nofs;
+    A.s2s_K0 = ensure_start_norms(a, 0);
+    int np = 0;   // pairs are sorted by colatitude: the polar ones come first
+    while (np < g->npairs && g->sth[np] < S2S_MIN_STH) ++np;
+    G.s2s_npolar = np;
+  }
   PhaseLayout L = single_layout(a, g->npairs, ncomp, 0);
   double4 *ph = static_cast<double4 *>(scratch_get("phase", sizeof(double4) * (size_t)ncomp * a->nm * g->npairs));
   if (synth) {

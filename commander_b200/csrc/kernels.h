@@ -38,6 +38,9 @@ struct LegGeom {
   // Handles that key the per-plan seed tables of the Legendre kernels (legendre.cu), set by a caller that launches every
   // slot of the geometry on one GPU; nullptr: every warp starts from the closed-form start values.
   const void *seed_geom = nullptr, *seed_alm = nullptr;
+  // spin 2 as scalar sums (legendre.cu, launch_s2s_*): slots [0, s2s_npolar) have sin(theta) < S2S_MIN_STH and stay on
+  // the spin-2 kernels; -1: the route is off.  Set by a caller that launches every slot of the geometry on one GPU.
+  int s2s_npolar = -1;
 };
 
 // alm side of the Legendre stage (local m's of this rank)
@@ -61,7 +64,14 @@ struct LegAlm {
   // (commander3/src/comm_cr_mod.f90:797-836, 957-1008; comm_B_bl_mod.f90:108-127) ride in the Legendre kernels
   const double *lscale[2] = {nullptr, nullptr};
   bool deriv1 = false;             // SHARP_ALM2MAP_DERIV1 (spin 1 tables, one a_lm column): prep_d1 / synth_d1 kernels
+  // spin 2 as scalar sums: the two-l-per-step spin-0 tables up to lmax + 2 (rec, mix, offsets in doubles, tile rows),
+  // the spin-0 start norms and the number of l slots of the table (nullptr: the route is off)
+  const double *s2s_coef = nullptr, *s2s_mix = nullptr, *s2s_K0 = nullptr;
+  const long long *s2s_cofs = nullptr, *s2s_tofs = nullptr;
+  long long s2s_trows = 0, s2s_nl = 0;
 };
+// spin 2 as scalar sums on (default) or off (cmdr_sht_set_spin2_scalar)
+bool spin2_scalar_on();
 
 unsigned long long job_opcnt(const sharp_geom_info *g, const sharp_alm_info *a, const Job &job);
 

@@ -17,6 +17,7 @@
 //   spin 0: 1 (recurrence) + 2 (accumulate) -- two l per step, recurrence in x^2 (coef.cpp) ; spin s: 4 + 8.
 // Spin 2 runs that scalar recurrence too while every ring of a warp is still far below the accumulation threshold
 // (1 instead of 4 per l and ring pair) and converts to the two spin-2 recurrences at the hand-over (spin2_front_phase).
+// On one GPU, spin 2 runs as two scalar sums of premixed coefficients everywhere but near the poles (launch_s2s_*).
 // Analysis reduces over the rings of the warp with a select-free, software-pipelined register
 // butterfly and adds the sums to the a_lm with coalesced atomics (DESIGN.md 3.1).
 #include <cstdio>
@@ -57,6 +58,10 @@ struct KParams {
   const double *trig;
   const int *mlim;
   const int *wslot;                  // work index -> storage slot (nullptr: identity)
+  // spin-0 kernels running a spin-2 job as scalar sums (launch_s2s_*; -1: off): the phases are scaled by 1 / sin^2 on
+  // store (synthesis) or load (analysis), the slots below this one are left to the spin-2 kernels (analysis: weight 0),
+  // and the analysis writes the unnormalised sums per (m, l) into a scratch buffer laid out like the coefficient table
+  int s2s_npolar;
   // seeded kernels only (seed tables, see seed0_kernel / seed2_kernel): first row (spin 0) / l - l0 (spin 2) each warp
   // accumulates at, per (local m, warp); recurrence state and scale exponent there, per (local m, slot)
   const int *sl;
@@ -251,9 +256,14 @@ __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
   }
 #pragma unroll
   for (int r = 0; r < R; ++r)
-    if (slot[r] < p.nslots)
-      *ph_out(p, 0, im, slot[r]) =
-          make_double4(fma(x[r], por[r], per[r]), fma(x[r], poi[r], pei[r]), fma(-x[r], por[r], per[r]), fma(-x[r], poi[r], pei[r]));
+    if (slot[r] < p.nslots) {
+      double4 v = make_double4(fma(x[r], por[r], per[r]), fma(x[r], poi[r], pei[r]), fma(-x[r], por[r], per[r]), fma(-x[r], poi[r], pei[r]));
+      if (p.s2s_npolar >= 0) {   // spin 2 as scalar sums: sum d lam = sin^2 x (the spin-2 sum)
+        const double s = reinterpret_cast<const double4 *>(p.trig)[slot[r]].y, f = 1.0 / (s * s);
+        v.x *= f; v.y *= f; v.z *= f; v.w *= f;
+      }
+      *ph_out(p, 0, im, slot[r]) = v;
+    }
 }
 
 // ------------------------------------------------------------------------------------
@@ -832,6 +842,10 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
         start_spin0(m, K, g, cur[r], k[r]);
       }
       double4 q = *ph_in(p, 0, im, slot);
+      if (p.s2s_npolar >= 0) {   // spin 2 as scalar sums: phases / sin^2; the polar rings are anal2_kernel's
+        const double f = slot < p.s2s_npolar ? 0.0 : 1.0 / (g.sth * g.sth);
+        q.x *= f; q.y *= f; q.z *= f; q.w *= f;
+      }
       double z[4] = {q.x + q.z, q.y + q.w, g.cth * (q.x - q.z), g.cth * (q.y - q.w)};
       // w[i] = z[i ^ (swapT ? 2 : 0) ^ (swapRI ? 1 : 0)]
 #pragma unroll
@@ -852,7 +866,8 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
   const long long mvs = p.mvstart[im];
   // real-packed: orthonormal real basis (sqrt2 both ways).  complex a_lm: the phases carry the
   // factor 2 of the m>0 terms, so the adjoint needs 1/2 to return sum conj(Y) x as libsharp2 does
-  const double nrm = m > 0 ? (p.real_packed ? 0.70710678118654752440 : 0.5) : 1.0;
+  const double nrm = p.s2s_npolar >= 0 ? 1.0 : (m > 0 ? (p.real_packed ? 0.70710678118654752440 : 0.5) : 1.0);
+  const long long xofs = 2 * (p.cofs[im] - m);   // s2s scratch: {re, im} of l at 2 (cofs + l - m)
   // rows past the last one belong to the next m (or the table's zero padding): finite, never used
   auto issue_tile = [&](int b, int jt) {
     const char *src = reinterpret_cast<const char *>(coef + 2 * (size_t)jt);
@@ -926,7 +941,8 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
                          : fma(mx.x, red[4 * (li + 1) + part], mx.w * red[4 * li + part]);
         val *= nrm;
         if (p.lscale0) val *= p.lscale0[l];
-        const long long idx = p.real_packed ? (m == 0 ? mvs + l : mvs + 2 * (long long)l + part) : 2 * (mvs + l) + part;
+        const long long idx = p.s2s_npolar >= 0 ? xofs + 2 * (long long)l + part
+                            : p.real_packed ? (m == 0 ? mvs + l : mvs + 2 * (long long)l + part) : 2 * (mvs + l) + part;
         atomicAdd(&a[idx], val);
       }
     }
@@ -1373,6 +1389,94 @@ __global__ void __launch_bounds__(32) seed2_kernel(KParams p) {
 }
 
 // ------------------------------------------------------------------------------------
+// Spin 2 as scalar sums (legendre_core.cuh, s2s_coefs): sum_l c_l (+-2)lam_l = (1 / sin^2) sum_{l'} d_l' lam_l' with d a
+// banded map of the a_lm up to l' = lmax + 2, so a spin-2 synthesis is a prep kernel that forms the scalar sequences of
+// the two map components plus two spin-0 syntheses (phases scaled by 1 / sin^2 on store), and an analysis is two spin-0
+// analyses (phases scaled on load) into a scratch buffer plus the transposed map.  1 + 2 FP64 ops per (l, ring pair)
+// and component instead of 4 + 8 for both.  `p` is the spin-0 view (lmax + 2 and the two-l-per-step tables of that
+// range); `crow`: tile rows between the two components' tables.
+// ------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) prep_s2s_kernel(KParams p, long long crow) {
+  const int im = p.im0 + blockIdx.y, m = p.mval[im];
+  const int lmax = p.lmax - 2, l0 = max(m, 2);
+  const int j = blockIdx.x * blockDim.x + threadIdx.x, lj = m + 2 * j;
+  const int J = (p.lmax - m) / 2 + 1;
+  const int npad = (J + 7) & ~7;
+  if (j >= npad) return;
+  TileS0 e[2] = {{0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}};
+  if (j < J) {
+    const double *aE = p.alm0, *aB = p.alm1;
+    const long long mvs = p.mvstart[im];
+    const double nrm = (p.real_packed && m > 0) ? 0.70710678118654752440 : 1.0;
+    double d[2][3][2] = {};   // [component][l_j + t][re, im]
+#pragma unroll
+    for (int dl = -2; dl <= 4; ++dl) {   // sources l_j - 2 .. l_j + 4 reach l_j .. l_j + 2
+      const int l = lj + dl;
+      if (l < l0 || l > lmax) continue;
+      double er, ei = 0.0, br, bi = 0.0;
+      if (p.real_packed) {
+        if (m == 0) { er = aE[mvs + l]; br = aB[mvs + l]; }
+        else {
+          er = aE[mvs + 2 * (long long)l]; ei = aE[mvs + 2 * (long long)l + 1];
+          br = aB[mvs + 2 * (long long)l]; bi = aB[mvs + 2 * (long long)l + 1];
+        }
+      } else {
+        er = aE[2 * (mvs + l)]; br = aB[2 * (mvs + l)];
+        if (m > 0) { ei = aE[2 * (mvs + l) + 1]; bi = aB[2 * (mvs + l) + 1]; }
+      }
+      const double fE = p.lscale0 ? nrm * p.lscale0[l] : nrm, fB = p.lscale1 ? nrm * p.lscale1[l] : nrm;
+      double s[2][5][2] = {};
+      s2s_scatter(l, m, fE * er, fE * ei, fB * br, fB * bi, s);
+#pragma unroll
+      for (int t = 0; t < 3; ++t) {
+        const int i = t - dl + 2;
+#pragma unroll
+        for (int c = 0; c < 2; ++c)
+          if (i >= 0 && i < 5) { d[c][t][0] += s[c][i][0]; d[c][t][1] += s[c][i][1]; }
+      }
+    }
+    const double2 rc = reinterpret_cast<const double2 *>(p.coef + p.cofs[im])[j];        // {A_j, B_j}
+    const double4 mx = reinterpret_cast<const double4 *>(p.coef2 + 2 * p.cofs[im])[j];   // {u_j, v_j, h_j, v_{j-1}}
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+      e[c].A = rc.x; e[c].B = rc.y;
+      e[c].c1r = fma(mx.x, d[c][0][0], mx.y * d[c][2][0]); e[c].c1i = fma(mx.x, d[c][0][1], mx.y * d[c][2][1]);
+      e[c].c2r = mx.z * d[c][1][0]; e[c].c2i = mx.z * d[c][1][1];
+    }
+  }
+  TileS0 *rows = reinterpret_cast<TileS0 *>(p.trows) + p.tofs[im] + j;
+  rows[0] = e[0];
+  rows[crow] = e[1];
+}
+
+// E, B from the scalar sums T (component c at T + c * ctot, {re, im} of (m, l) at 2 (xcofs[im] + l - m)), added to the
+// a_lm after the real-packed norm and the per-l factors of the spin-2 analysis kernel.  `p` is the spin-2 view.
+__global__ void __launch_bounds__(256) post_s2s_kernel(KParams p, const double *T, const long long *xcofs, long long ctot) {
+  const int im = p.im0 + blockIdx.y, m = p.mval[im];
+  const int l = blockIdx.x * blockDim.x + threadIdx.x;
+  if (l < max(m, 2) || l > p.lmax) return;
+  const double *tq = T + 2 * (xcofs[im] - m), *tu = tq + ctot;
+  double q[5][2], u[5][2];
+#pragma unroll
+  for (int i = 0; i < 5; ++i) {
+    const int t = l - 2 + i;
+    const bool ok = t >= m;
+    q[i][0] = ok ? tq[2 * t] : 0.0; q[i][1] = ok ? tq[2 * t + 1] : 0.0;
+    u[i][0] = ok ? tu[2 * t] : 0.0; u[i][1] = ok ? tu[2 * t + 1] : 0.0;
+  }
+  double er, ei, br, bi;
+  s2s_gather(l, m, q, u, er, ei, br, bi);
+  // real-packed: orthonormal real basis (sqrt2 both ways); complex a_lm: 1/2 as in anal2_kernel
+  const double nrm = m > 0 ? (p.real_packed ? 0.70710678118654752440 : 0.5) : 1.0;
+  const double fE = p.lscale0 ? nrm * p.lscale0[l] : nrm, fB = p.lscale1 ? nrm * p.lscale1[l] : nrm;
+  double *aE = p.alm0, *aB = p.alm1;
+  const long long mvs = p.mvstart[im];
+  const long long i0 = p.real_packed ? (m == 0 ? mvs + l : mvs + 2 * (long long)l) : 2 * (mvs + l);
+  aE[i0] += fE * er; aB[i0] += fB * br;
+  if (m > 0) { aE[i0 + 1] += fE * ei; aB[i0 + 1] += fB * bi; }
+}
+
+// ------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------
 // Ring pairs per thread (register blocking).  Defaults were picked from the sweep recorded in
@@ -1392,6 +1496,7 @@ static KParams make_params(const LegGeom &g, const LegAlm &a, double *alm0, doub
   p.fcoef = a.front_coef; p.fmix = a.front_mix; p.fcofs = a.front_cofs; p.fK0 = a.front_K0;
   p.tofs = nullptr; p.trows = nullptr;
   p.sl = nullptr; p.ss = nullptr; p.sk = nullptr;
+  p.s2s_npolar = -1;
   p.im0 = a.im_begin;
   p.trig = g.trig; p.mlim = g.mlim; p.wslot = g.wslot;
   p.alm0 = alm0; p.alm1 = alm1; p.ph = ph;
@@ -1410,7 +1515,7 @@ static void launch_w(K kernel, const KParams &p, int nm, cudaStream_t st) {   //
 }
 
 // ---- seed tables: one per (geometry handle, alm handle, kernel), built on first use ----
-enum SeedKind { SEED_S0, SEED_A0, SEED_S2, SEED_A2 };
+enum SeedKind { SEED_S0, SEED_A0, SEED_S2, SEED_A2, SEED_S0X, SEED_A0X };   // ..X: spin-0 kernels of the s2s route
 struct SeedTab { int *sl = nullptr; double *ss = nullptr; int *sk = nullptr; size_t bytes = 0; };
 static std::map<std::tuple<const void *, const void *, int>, SeedTab> g_seeds;
 static bool g_seeds_on = true;
@@ -1449,7 +1554,7 @@ static const SeedTab *seed_table(const LegGeom &g, SeedKind kind, int R, const K
   if (it != g_seeds.end()) return &it->second;
   const int nwarps = (g.nslots + 32 * R - 1) / (32 * R);
   const size_t nst = (size_t)nm * g.nslots, nsl = (size_t)nm * nwarps;
-  const size_t sbytes = (kind == SEED_S0 || kind == SEED_A0 ? 2 : 4) * sizeof(double);
+  const size_t sbytes = (kind == SEED_S2 || kind == SEED_A2 ? 4 : 2) * sizeof(double);
   const size_t bytes = nst * (sbytes + sizeof(int)) + nsl * sizeof(int);
   static size_t cap = 0;
   if (!cap) { size_t fr, tot; CMDR_CUDA_CHECK(cudaMemGetInfo(&fr, &tot)); cap = tot / 32; }
@@ -1463,8 +1568,8 @@ static const SeedTab *seed_table(const LegGeom &g, SeedKind kind, int R, const K
   q.im0 = 0; q.sl = t.sl; q.ss = t.ss; q.sk = t.sk;
   const dim3 grid(nwarps, nm);
   switch (kind) {
-    case SEED_S0: seed0_kernel<4><<<grid, 32, 0, st>>>(q); break;
-    case SEED_A0: seed0_kernel<8><<<grid, 32, 0, st>>>(q); break;
+    case SEED_S0: case SEED_S0X: seed0_kernel<4><<<grid, 32, 0, st>>>(q); break;
+    case SEED_A0: case SEED_A0X: seed0_kernel<8><<<grid, 32, 0, st>>>(q); break;
     case SEED_S2: seed2_kernel<4, 4, 8, false><<<grid, 32, 0, st>>>(q); break;
     case SEED_A2: seed2_kernel<4, 2, 4, true><<<grid, 32, 0, st>>>(q); break;
   }
@@ -1475,6 +1580,84 @@ static const SeedTab *seed_table(const LegGeom &g, SeedKind kind, int R, const K
   return &(g_seeds[key] = t);
 }
 static void use_seed(KParams &p, const SeedTab *t) { p.sl = t->sl; p.ss = t->ss; p.sk = t->sk; }
+
+// ---- spin 2 as scalar sums (prep_s2s_kernel / post_s2s_kernel above) ----
+static bool g_s2s_on = true;
+bool spin2_scalar_on() { return g_s2s_on; }
+
+static bool s2s_route(const LegGeom &g, const LegAlm &a) { return a.spin == 2 && !a.deriv1 && a.s2s_coef && g.s2s_npolar >= 0; }
+
+// spin-0 view of a spin-2 launch: lmax + 2 and the two-l-per-step tables of that range, spin-2 m cut-off and slots
+static KParams s2s_params(const LegGeom &g, const LegAlm &a, const KParams &p) {
+  KParams q = p;
+  q.lmax = a.lmax + 2; q.spin = 0;
+  q.coef = a.s2s_coef; q.coef2 = a.s2s_mix; q.cofs = a.s2s_cofs; q.Kstart = a.s2s_K0; q.tofs = a.s2s_tofs;
+  q.fcoef = nullptr;
+  q.s2s_npolar = g.s2s_npolar;
+  return q;
+}
+
+// Every slot runs the spin-0 kernels (so that their seed tables apply); the spin-2 kernel then overwrites the polar
+// slots' phases.  `p`: the spin-2 parameters with the spin-2 tile rows.
+static void launch_s2s_synth(const LegGeom &g, const LegAlm &a, const KParams &p, int nmr, cudaStream_t st, bool prep) {
+  KParams q = s2s_params(g, a, p);
+  const long long crow = a.s2s_trows + TL;   // tile rows per component
+  q.trows = static_cast<double *>(scratch_get("synth_rows_s2s", sizeof(TileS0) * 2 * (size_t)crow));
+  if (prep) {
+    prep_s2s_kernel<<<dim3((a.lmax + 2 + 8 + 255) / 256, nmr), 256, 0, st>>>(q, crow);
+    count_launch();
+  }
+  const SeedTab *t = seed_table(g, SEED_S0X, 4, q, a.nm, st);
+  if (t) use_seed(q, t);
+  for (int c = 0; c < 2; ++c) {
+    KParams qc = q;
+    qc.comp0 = p.comp0 + c;
+    qc.trows = q.trows + (size_t)c * crow * (sizeof(TileS0) / sizeof(double));
+    if (t) launch_w<4>(synth0_kernel<4, 16, true>, qc, nmr, st);
+    else launch_w<4>(synth0_kernel<4, 16>, qc, nmr, st);
+    count_launch();
+  }
+  if (g.s2s_npolar > 0) {
+    KParams pp = p;
+    pp.nslots = min(p.nslots, g.s2s_npolar);
+    if (prep) {
+      prep_s2_kernel<<<dim3((a.lmax + 8 + 255) / 256, nmr), 256, 0, st>>>(pp);
+      count_launch();
+    }
+    launch_w<4>(synth2_kernel<4, 8>, pp, nmr, st);
+    count_launch();
+  }
+  CMDR_CUDA_CHECK(cudaGetLastError());
+}
+
+// Polar rings contribute to the scalar sums with weight 0 and go through the spin-2 kernel instead; the post kernel
+// then adds the transposed map of the sums to the a_lm.
+static void launch_s2s_anal(const LegGeom &g, const LegAlm &a, const KParams &p, int nmr, cudaStream_t st) {
+  KParams q = s2s_params(g, a, p);
+  q.lscale0 = q.lscale1 = nullptr;   // applied by the post kernel
+  const long long ctot = 2 * a.s2s_nl;   // doubles per component
+  double *T = static_cast<double *>(scratch_get("anal_s2s", sizeof(double) * 2 * (size_t)ctot));
+  CMDR_CUDA_CHECK(cudaMemsetAsync(T, 0, sizeof(double) * 2 * (size_t)ctot, st));
+  const SeedTab *t = seed_table(g, SEED_A0X, 8, q, a.nm, st);
+  if (t) use_seed(q, t);
+  for (int c = 0; c < 2; ++c) {
+    KParams qc = q;
+    qc.comp0 = p.comp0 + c;
+    qc.alm0 = T + (size_t)c * ctot;
+    if (t) launch_w<8>(anal0_kernel<8, 12, true>, qc, nmr, st);
+    else launch_w<8>(anal0_kernel<8, 12>, qc, nmr, st);
+    count_launch();
+  }
+  if (g.s2s_npolar > 0) {
+    KParams pp = p;
+    pp.nslots = min(p.nslots, g.s2s_npolar);
+    launch_w<4>(anal2_kernel<4, 12>, pp, nmr, st);
+    count_launch();
+  }
+  post_s2s_kernel<<<dim3((a.lmax + 1 + 255) / 256, nmr), 256, 0, st>>>(p, T, a.s2s_cofs, ctot);
+  count_launch();
+  CMDR_CUDA_CHECK(cudaGetLastError());
+}
 
 void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *const *alm, double4 *ph, cudaStream_t st,
                            bool prep) {
@@ -1489,6 +1672,7 @@ void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *cons
   const size_t rowbytes = spin == 0 ? sizeof(TileS0) : (a.deriv1 ? sizeof(TileD1) : sizeof(TileS2));
   p.tofs = a.tofs;
   p.trows = static_cast<double *>(scratch_get(spin == 0 ? "synth_rows0" : "synth_rows2", rowbytes * (size_t)(a.trows + TL)));
+  if (s2s_route(g, a)) { launch_s2s_synth(g, a, p, nmr, st, prep); return; }
   if (prep) {
     dim3 pg((a.lmax + 8 + 255) / 256, nmr);
     if (spin == 0) prep_s0_kernel<<<pg, 256, 0, st>>>(p);
@@ -1545,6 +1729,7 @@ void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm,
   if (nmr <= 0) return;
   const int spin = a.spin;
   KParams p = make_params(g, a, alm[0], spin ? alm[1] : nullptr, const_cast<double4 *>(ph));
+  if (s2s_route(g, a)) { launch_s2s_anal(g, a, p, nmr, st); return; }
   // spin 0: 8 ring pairs per thread since the two-l-per-step kernels (fewer registers per ring pair; the butterfly and the
   // per-tile flush are per warp, so their share halves): 8.71 -> 8.31 ms at nside 2048 / lmax 4000
   static const int r0 = env_int("CMDR_SHT_R_A0", 8), r2 = env_int("CMDR_SHT_R_A2", 4);
@@ -1588,5 +1773,6 @@ void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm,
 
 extern "C" {
 void cmdr_sht_set_legendre_seeds(int on) { cmdr::g_seeds_on = on != 0; }
+void cmdr_sht_set_spin2_scalar(int on) { cmdr::g_s2s_on = on != 0; }
 size_t cmdr_sht_legendre_seed_bytes(void) { return cmdr::g_seed_bytes; }
 }

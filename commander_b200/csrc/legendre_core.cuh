@@ -132,6 +132,63 @@ CMDR_HD void spin2_from_scalar(int l, int m, double x, double sth, double lam, d
   P = f * ((a - b) * lam + e * (x + dm) * lam1);
   M = f * ((a + b) * lam + e * (x - dm) * lam1);
 }
+// The same relations as a banded map onto the scalar functions (spin-2 Legendre sums run as scalar sums).  With
+// S_l = ((+2)lam_l + (-2)lam_l) / 2, A_l = ((+2)lam_l - (-2)lam_l) / 2, the W/X form above and the three-term relation
+// x lam_k = eps_{k+1} lam_{k+1} + eps_k lam_{k-1} (eps_k = sqrt((k^2 - m^2) / (4k^2 - 1)); e = (2l+1) eps_l above):
+//   sin^2 S_l = kS[0] lam_{l-2} + kS[1] lam_l + kS[2] lam_{l+2},    sin^2 A_l = kA[0] lam_{l-1} + kA[1] lam_{l+1}
+//   F = 2 / sqrt((l-1) l (l+1) (l+2)),  kS[0] = F (l+1)(l+2)/2 eps_l eps_{l-1},  kS[2] = F l(l-1)/2 eps_{l+1} eps_{l+2},
+//   kS[1] = F [-(l - m^2) - l(l-1)/2 + l(l-1)/2 (eps_{l+1}^2 + eps_l^2) + (2l+1) eps_l^2],
+//   kA[0] = F m (l+2) eps_l,  kA[1] = -F m (l-1) eps_{l+1}                                                (l >= 2)
+// The identity is polynomial in x = cos(theta), so it holds on the southern mirror too; the 1/sin^2 it leaves costs
+// digits near the poles only: ring pairs with sin(theta) < S2S_MIN_STH stay on the spin-2 recurrences.
+constexpr double S2S_MIN_STH = 0.05;
+CMDR_HD double s2s_eps(int l, int m) {
+  const double dl = l, dm = m;
+  return l > m ? sqrt((dl * dl - dm * dm) / (4.0 * dl * dl - 1.0)) : 0.0;
+}
+CMDR_HD void s2s_coefs(int l, int m, double (&kS)[3], double (&kA)[2]) {
+  const double dl = l, dm = m;
+  const double F = 2.0 / sqrt((dl - 1.0) * dl * (dl + 1.0) * (dl + 2.0));
+  const double e0 = s2s_eps(l, m), em = s2s_eps(l - 1, m), e1 = s2s_eps(l + 1, m), e2 = s2s_eps(l + 2, m);
+  const double h = 0.5 * dl * (dl - 1.0);
+  kS[0] = F * 0.5 * (dl + 1.0) * (dl + 2.0) * e0 * em;
+  kS[1] = F * (-(dl - dm * dm) - h + h * (e1 * e1 + e0 * e0) + (2.0 * dl + 1.0) * e0 * e0);
+  kS[2] = F * h * e1 * e2;
+  kA[0] = F * dm * (dl + 2.0) * e0;
+  kA[1] = -F * dm * (dl - 1.0) * e1;
+}
+// Synthesis of spin 2 (E, B of one l, after the per-l factor and the real-packed norm ns) as the two scalar sequences
+// of the map components (Q: dq, U: du) on the slots l-2 .. l+2 (index 0 .. 4), in the combination of synth2_kernel:
+//   Q = -sum_l [E_l S_l + i B_l A_l],  U = -sum_l [B_l S_l - i E_l A_l]   (north; the south is the same at -x).
+// d[c][i] += {re, im}.
+CMDR_HD void s2s_scatter(int l, int m, double er, double ei, double br, double bi, double (&d)[2][5][2]) {
+  double kS[3], kA[2];
+  s2s_coefs(l, m, kS, kA);
+  // S coefficients: Q -E, U -B ; A coefficients: Q -iB = (bi, -br), U +iE = (-ei, er)
+  for (int t = 0; t < 3; ++t) {
+    d[0][2 * t][0] -= kS[t] * er; d[0][2 * t][1] -= kS[t] * ei;
+    d[1][2 * t][0] -= kS[t] * br; d[1][2 * t][1] -= kS[t] * bi;
+  }
+  for (int t = 0; t < 2; ++t) {
+    d[0][2 * t + 1][0] += kA[t] * bi; d[0][2 * t + 1][1] -= kA[t] * br;
+    d[1][2 * t + 1][0] -= kA[t] * ei; d[1][2 * t + 1][1] += kA[t] * er;
+  }
+}
+// Its exact transpose for analysis: from the scalar sums Tq_{l+i-2}, Tu_{l+i-2} (i = 0 .. 4; {re, im}) to
+//   E_l = -[sum kS Tq + i sum kA Tu],  B_l = -sum kS Tu + i sum kA Tq      (before the real-packed norm and the per-l factor)
+CMDR_HD void s2s_gather(int l, int m, const double (&tq)[5][2], const double (&tu)[5][2], double &er, double &ei, double &br,
+                        double &bi) {
+  double kS[3], kA[2];
+  s2s_coefs(l, m, kS, kA);
+  double sq[2] = {0.0, 0.0}, su[2] = {0.0, 0.0}, aq[2] = {0.0, 0.0}, au[2] = {0.0, 0.0};
+  for (int t = 0; t < 3; ++t)
+    for (int c = 0; c < 2; ++c) { sq[c] = fma(kS[t], tq[2 * t][c], sq[c]); su[c] = fma(kS[t], tu[2 * t][c], su[c]); }
+  for (int t = 0; t < 2; ++t)
+    for (int c = 0; c < 2; ++c) { aq[c] = fma(kA[t], tq[2 * t + 1][c], aq[c]); au[c] = fma(kA[t], tu[2 * t + 1][c], au[c]); }
+  er = -(sq[0] - au[1]); ei = -(sq[1] + au[0]);
+  br = -su[0] - aq[1];   bi = -su[1] + aq[0];
+}
+
 // switch from the scalar to the spin-2 recurrences once a ring's scalar value (stored as true * 2^(-512 k)) is within
 // `margin` bits of the accumulation threshold.  The spin-2 functions are larger than the scalar one by at most
 // ~2 / sin^2(theta) (the m^2 / sin^2 term of W with m <= l), and a few bits of growth until the next check are allowed for.

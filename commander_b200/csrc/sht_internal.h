@@ -16,6 +16,7 @@ void build_coef_table(int lmax, int spin, const std::vector<int> &mval, std::vec
 void build_coef_table_x2(int lmax, const std::vector<int> &mval, std::vector<double> &rec, std::vector<double> &mix,
                          std::vector<long long> &ofs);
 constexpr int COEF_KEY_S0X2 = -1;   // key of that table in sharp_alm_info::coef (key 0 stays the one-step table of invn.cu)
+constexpr int COEF_KEY_S0X2P2 = -2; // the same up to lmax + 2: spin 2 run as scalar sums (legendre.cu, launch_s2s_*)
 void build_start_norms(int mmax, std::vector<double> &K0, std::vector<double> &K2);
 void build_start_norms_spin(int mmax, int spin, std::vector<double> &Ks);
 
@@ -26,6 +27,7 @@ struct CoefDev {            // device copy of one (alm_info, spin) coefficient t
   long long *ofs = nullptr; // per local m: offset (in doubles) of l = l0
   long long *tofs = nullptr; // per local m: first synthesis tile row (rows padded to a multiple of 8)
   long long trows = 0;       // total synthesis tile rows
+  long long nofs = 0;        // offset past the last local m (doubles)
 };
 
 // Region of the ring-FFT work buffer: pairs [first, first+np) share one FFT length.
