@@ -54,13 +54,13 @@ struct KParams {
   const double *fcoef, *fmix, *fK0;   // rec rows {a_j, b'_j}, mix rows {u, v, h, v_prev}, spin-0 start norms
   const long long *fcofs;
   const long long *tofs;             // synthesis: first tile row of each local m (rows padded to 8 per m)
-  double *trows;                     // synthesis: tile rows (TileS0 / TileS2), written by the prep kernels
+  double *trows;                     // synthesis: tile rows (TileS0<NC> / TileS2), written by the prep kernels
   const double *trig;
   const int *mlim;
   const int *wslot;                  // work index -> storage slot (nullptr: identity)
   // spin-0 kernels running a spin-2 job as scalar sums (launch_s2s_*; -1: off): the phases are scaled by 1 / sin^2 on
-  // store (synthesis) or load (analysis), the slots below this one are left to the spin-2 kernels (analysis: weight 0),
-  // and the analysis writes the unnormalised sums per (m, l) into a scratch buffer laid out like the coefficient table
+  // store (synthesis, synth0_kernel<2, ...>) or load (analysis), the slots below this one are left to the spin-2 kernels
+  // (analysis: weight 0), and the analysis writes the unnormalised sums per (m, l) into a scratch buffer laid out like the coefficient table
   int s2s_npolar;
   // seeded kernels only (seed tables, see seed0_kernel / seed2_kernel): first row (spin 0) / l - l0 (spin 2) each warp
   // accumulates at, per (local m, warp); recurrence state and scale exponent there, per (local m, slot)
@@ -74,7 +74,10 @@ struct KParams {
   double4 *peer[CMDR_MAX_PEERS];     // phase buffer of each ring owner (all = ph without the fused exchange)
 };
 
-struct __align__(16) TileS0 { double A, B, c1r, c1i, c2r, c2i; };   // one row = two l (l_j = m + 2j, l_j + 1)
+// one row = two l (l_j = m + 2j, l_j + 1): the shared recurrence coefficients and {c1r, c1i, c2r, c2i} of each of NC
+// components (1: T; 2: Q and U of a spin-2 job run as scalar sums)
+template <int NC>
+struct __align__(16) TileS0 { double A, B, c[NC][4]; };
 struct __align__(16) TileS2 { double A, C, cpr, cpi, cmr, cmi; };
 struct __align__(16) TileA0 { double A, B; };
 struct __align__(16) TileA2 { double A, C, g, pad; };
@@ -124,22 +127,28 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 // spin-0 synthesis, two l per recurrence step (coef.cpp, fill_spin0_x2):
 //   nu_{j+1} = (A_j x^2 + B_j) nu_j - nu_{j-1};  sum_l a_l lam_l = sum_j nu_j c1_j + x sum_j nu_j c2_j
 //   c1_j = u_j a_{l_j} + v_j a_{l_j+2} (even l - m),  c2_j = h_j a_{l_j+1} (odd l - m);  south ring: x -> -x.
-// One group = 4 rows = 8 l.
+// One group = 4 rows = 8 l.  NC components share the recurrence: each row's nu feeds 4 NC accumulate FMAs, and every
+// component's chain is the same fma sequence whatever NC and R are.
 // ------------------------------------------------------------------------------------
-template <int MODE, int R>
-__device__ __forceinline__ void synth0_group(const TileS0 *t, const double (&x2)[R], double (&cur)[R],
-                                             double (&prev)[R], double (&per)[R], double (&pei)[R],
-                                             double (&por)[R], double (&poi)[R], int (&k)[R], unsigned ron = ~0u) {
+template <int MODE, int NC, int R>
+__device__ __forceinline__ void synth0_group(const TileS0<NC> *t, const double (&x2)[R], double (&cur)[R],
+                                             double (&prev)[R], double (&acc)[NC][4][R], int (&k)[R]) {
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     const double A = t[j].A, B = t[j].B;
-    const double c1r = t[j].c1r, c1i = t[j].c1i, c2r = t[j].c2r, c2i = t[j].c2i;
+    double c[NC][4];
+#pragma unroll
+    for (int n = 0; n < NC; ++n)
+#pragma unroll
+      for (int i = 0; i < 4; ++i) c[n][i] = t[j].c[n][i];
 #pragma unroll
     for (int r = 0; r < R; ++r) {
-      if (MODE == 2 || (MODE == 1 && ((ron >> r) & 1))) {
+      if (MODE != 0) {
         double v = (MODE == 2 || k[r] == 0) ? cur[r] : 0.0;
-        per[r] = fma(v, c1r, per[r]); pei[r] = fma(v, c1i, pei[r]);
-        por[r] = fma(v, c2r, por[r]); poi[r] = fma(v, c2i, poi[r]);
+#pragma unroll
+        for (int n = 0; n < NC; ++n)
+#pragma unroll
+          for (int i = 0; i < 4; ++i) acc[n][i][r] = fma(v, c[n][i], acc[n][i][r]);
       }
       double nxt = step0x2(A, B, x2[r], cur[r], prev[r]);
       prev[r] = cur[r]; cur[r] = nxt;
@@ -161,7 +170,7 @@ __global__ void __launch_bounds__(256) prep_s0_kernel(KParams p) {
   const int J = p.lmax >= m ? (p.lmax - m) / 2 + 1 : 0;
   const int npad = (J + 7) & ~7;
   if (j >= npad) return;
-  TileS0 e{0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+  TileS0<1> e{0.0, 0.0, {{0.0, 0.0, 0.0, 0.0}}};
   if (j < J) {
     const double2 rc = reinterpret_cast<const double2 *>(p.coef + p.cofs[im])[j];        // {A_j, B_j}
     const double4 mx = reinterpret_cast<const double4 *>(p.coef2 + 2 * p.cofs[im])[j];   // {u_j, v_j, h_j, v_{j-1}}
@@ -183,24 +192,31 @@ __global__ void __launch_bounds__(256) prep_s0_kernel(KParams p) {
     double r0, i0, r1, i1, r2, i2;
     load(l, r0, i0); load(l + 1, r1, i1); load(l + 2, r2, i2);
     e.A = rc.x; e.B = rc.y;
-    e.c1r = fma(mx.x, r0, mx.y * r2); e.c1i = fma(mx.x, i0, mx.y * i2);
-    e.c2r = mx.z * r1; e.c2i = mx.z * i1;
+    e.c[0][0] = fma(mx.x, r0, mx.y * r2); e.c[0][1] = fma(mx.x, i0, mx.y * i2);
+    e.c[0][2] = mx.z * r1; e.c[0][3] = mx.z * i1;
   }
-  reinterpret_cast<TileS0 *>(p.trows)[p.tofs[im] + j] = e;
+  reinterpret_cast<TileS0<1> *>(p.trows)[p.tofs[im] + j] = e;
 }
 
 // Synthesis kernels: ONE WARP PER CTA like the analysis kernels (no block barriers; a thread owns R
 // adjacent ring pairs; whole warps beyond the m cut-off only write zeros).
 // SEED: start each ring from the seed table at the warp's first accumulating row instead of from the closed-form start
 // values at row 0 (the rows in between add exact zeros; seed0_kernel).
-template <int R, int MINB, bool SEED = false>
+// NC = 2 runs a spin-2 job as scalar sums (launch_s2s_synth): components comp0 and comp0 + 1, phases scaled by
+// 1 / sin^2 on store (sum d lam = sin^2 x the spin-2 sum).  Its 80-byte rows take tiles of TL_S2S rows: 2 x 128 rows
+// would be 20 KB of shared memory per one-warp CTA, 10 CTAs per SM instead of the 12 the 160 registers allow
+// (measured: 64 and 96 rows alike, 128 rows 1.3 % and 32 rows 0.6 % slower).
+constexpr int TL_S2S = 64;
+template <int NC, int R, int MINB, bool SEED = false>
 __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
-  __shared__ __align__(16) TileS0 tile[2][TL];
+  constexpr int TLN = NC == 1 ? TL : TL_S2S;
+  static_assert(TLN * sizeof(TileS0<NC>) % 512 == 0, "a tile is staged in whole 16-byte copies of the warp");
+  __shared__ __align__(16) TileS0<NC> tile[2][TLN];
   const int im = p.im0 + blockIdx.y, m = p.mval[im];
   const int lane = threadIdx.x;
   const int chunk0 = p.slot_begin + blockIdx.x * (32 * R);
   const int J = p.lmax >= m ? (p.lmax - m) / 2 + 1 : 0;   // rows (steps of two l) of this m
-  double x[R], x2[R], cur[R], prev[R], per[R], pei[R], por[R], poi[R];
+  double x[R], x2[R], cur[R], prev[R], acc[NC][4][R];
   int k[R], slot[R];
   bool any = false;
   const double K = p.Kstart[m];
@@ -209,7 +225,8 @@ __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
   for (int r = 0; r < R; ++r) {
     slot[r] = chunk0 + lane * R + r;
     bool valid = slot[r] < p.nslots && m <= p.mlim[min(slot[r], p.nslots - 1)];
-    per[r] = pei[r] = por[r] = poi[r] = 0.0;
+#pragma unroll
+    for (int n = 0; n < NC; ++n) acc[n][0][r] = acc[n][1][r] = acc[n][2][r] = acc[n][3][r] = 0.0;
     prev[r] = 0.0; cur[r] = 0.0; k[r] = 0; x[r] = 0.0; x2[r] = 0.0;
     if (valid) {
       const double4 tg = reinterpret_cast<const double4 *>(p.trig)[slot[r]];
@@ -226,29 +243,29 @@ __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
     }
   }
   if (__any_sync(FULL, any) && (!SEED || j0 < J)) {
-    const TileS0 *rows = reinterpret_cast<const TileS0 *>(p.trows) + p.tofs[im];
+    const TileS0<NC> *rows = reinterpret_cast<const TileS0<NC> *>(p.trows) + p.tofs[im];
     auto issue_tile = [&](int b, int jt) {     // rows past this m's padded range are never used
       const char *src = reinterpret_cast<const char *>(rows + jt);
       char *dst = reinterpret_cast<char *>(tile[b]);
 #pragma unroll
-      for (int q = 0; q < (int)(TL * sizeof(TileS0)) / 512; ++q) cp_async16(dst + (q * 32 + lane) * 16, src + (q * 32 + lane) * 16);
+      for (int q = 0; q < (int)(TLN * sizeof(TileS0<NC>)) / 512; ++q) cp_async16(dst + (q * 32 + lane) * 16, src + (q * 32 + lane) * 16);
       cp_async_commit();
     };
     issue_tile(0, j0);
     cp_async_wait_all();
     __syncwarp();
     int buf = 0;
-    for (int jt = j0; jt < J; jt += TL, buf ^= 1) {
-      if (jt + TL < J) issue_tile(buf ^ 1, jt + TL);
-      const int ngroups = min(TL, J - jt + 3) / 4;
+    for (int jt = j0; jt < J; jt += TLN, buf ^= 1) {
+      if (jt + TLN < J) issue_tile(buf ^ 1, jt + TLN);
+      const int ngroups = min(TLN, J - jt + 3) / 4;
 #pragma unroll 1
       for (int g = 0; g < ngroups; ++g) {
         bool all_on = true, none_on = true;
 #pragma unroll
         for (int r = 0; r < R; ++r) { all_on &= (k[r] == 0); none_on &= (k[r] < 0); }
-        if (__all_sync(FULL, all_on)) synth0_group<2, R>(tile[buf] + 4 * g, x2, cur, prev, per, pei, por, poi, k);
-        else if (__all_sync(FULL, none_on)) synth0_group<0, R>(tile[buf] + 4 * g, x2, cur, prev, per, pei, por, poi, k);
-        else synth0_group<1, R>(tile[buf] + 4 * g, x2, cur, prev, per, pei, por, poi, k);
+        if (__all_sync(FULL, all_on)) synth0_group<2, NC, R>(tile[buf] + 4 * g, x2, cur, prev, acc, k);
+        else if (__all_sync(FULL, none_on)) synth0_group<0, NC, R>(tile[buf] + 4 * g, x2, cur, prev, acc, k);
+        else synth0_group<1, NC, R>(tile[buf] + 4 * g, x2, cur, prev, acc, k);
       }
       cp_async_wait_all();
       __syncwarp();
@@ -257,12 +274,18 @@ __global__ void __launch_bounds__(32, MINB) synth0_kernel(KParams p) {
 #pragma unroll
   for (int r = 0; r < R; ++r)
     if (slot[r] < p.nslots) {
-      double4 v = make_double4(fma(x[r], por[r], per[r]), fma(x[r], poi[r], pei[r]), fma(-x[r], por[r], per[r]), fma(-x[r], poi[r], pei[r]));
-      if (p.s2s_npolar >= 0) {   // spin 2 as scalar sums: sum d lam = sin^2 x (the spin-2 sum)
-        const double s = reinterpret_cast<const double4 *>(p.trig)[slot[r]].y, f = 1.0 / (s * s);
-        v.x *= f; v.y *= f; v.z *= f; v.w *= f;
+      double f = 1.0;
+      if constexpr (NC == 2) {
+        const double s = reinterpret_cast<const double4 *>(p.trig)[slot[r]].y;
+        f = 1.0 / (s * s);
       }
-      *ph_out(p, 0, im, slot[r]) = v;
+#pragma unroll
+      for (int n = 0; n < NC; ++n) {
+        const double per = acc[n][0][r], pei = acc[n][1][r], por = acc[n][2][r], poi = acc[n][3][r];
+        double4 v = make_double4(fma(x[r], por, per), fma(x[r], poi, pei), fma(-x[r], por, per), fma(-x[r], poi, pei));
+        if constexpr (NC == 2) { v.x *= f; v.y *= f; v.z *= f; v.w *= f; }
+        *ph_out(p, n, im, slot[r]) = v;
+      }
     }
 }
 
@@ -1393,17 +1416,17 @@ __global__ void __launch_bounds__(32) seed2_kernel(KParams p) {
 // banded map of the a_lm up to l' = lmax + 2, so a spin-2 synthesis is a prep kernel that forms the scalar sequences of
 // the two map components plus two spin-0 syntheses (phases scaled by 1 / sin^2 on store), and an analysis is two spin-0
 // analyses (phases scaled on load) into a scratch buffer plus the transposed map.  1 + 2 FP64 ops per (l, ring pair)
-// and component instead of 4 + 8 for both.  `p` is the spin-0 view (lmax + 2 and the two-l-per-step tables of that
-// range); `crow`: tile rows between the two components' tables.
+// and component instead of 4 + 8 for both; the synthesis runs the recurrence once for both components (synth0_kernel<2>),
+// so 1 + 4 for Q and U together.  `p` is the spin-0 view (lmax + 2 and the two-l-per-step tables of that range).
 // ------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) prep_s2s_kernel(KParams p, long long crow) {
+__global__ void __launch_bounds__(256) prep_s2s_kernel(KParams p) {
   const int im = p.im0 + blockIdx.y, m = p.mval[im];
   const int lmax = p.lmax - 2, l0 = max(m, 2);
   const int j = blockIdx.x * blockDim.x + threadIdx.x, lj = m + 2 * j;
   const int J = (p.lmax - m) / 2 + 1;
   const int npad = (J + 7) & ~7;
   if (j >= npad) return;
-  TileS0 e[2] = {{0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}};
+  TileS0<2> e{0.0, 0.0, {{0.0, 0.0, 0.0, 0.0}, {0.0, 0.0, 0.0, 0.0}}};
   if (j < J) {
     const double *aE = p.alm0, *aB = p.alm1;
     const long long mvs = p.mvstart[im];
@@ -1437,16 +1460,14 @@ __global__ void __launch_bounds__(256) prep_s2s_kernel(KParams p, long long crow
     }
     const double2 rc = reinterpret_cast<const double2 *>(p.coef + p.cofs[im])[j];        // {A_j, B_j}
     const double4 mx = reinterpret_cast<const double4 *>(p.coef2 + 2 * p.cofs[im])[j];   // {u_j, v_j, h_j, v_{j-1}}
+    e.A = rc.x; e.B = rc.y;
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
-      e[c].A = rc.x; e[c].B = rc.y;
-      e[c].c1r = fma(mx.x, d[c][0][0], mx.y * d[c][2][0]); e[c].c1i = fma(mx.x, d[c][0][1], mx.y * d[c][2][1]);
-      e[c].c2r = mx.z * d[c][1][0]; e[c].c2i = mx.z * d[c][1][1];
+      e.c[c][0] = fma(mx.x, d[c][0][0], mx.y * d[c][2][0]); e.c[c][1] = fma(mx.x, d[c][0][1], mx.y * d[c][2][1]);
+      e.c[c][2] = mx.z * d[c][1][0]; e.c[c][3] = mx.z * d[c][1][1];
     }
   }
-  TileS0 *rows = reinterpret_cast<TileS0 *>(p.trows) + p.tofs[im] + j;
-  rows[0] = e[0];
-  rows[crow] = e[1];
+  reinterpret_cast<TileS0<2> *>(p.trows)[p.tofs[im] + j] = e;
 }
 
 // E, B from the scalar sums T (component c at T + c * ctot, {re, im} of (m, l) at 2 (xcofs[im] + l - m)), added to the
@@ -1601,22 +1622,14 @@ static KParams s2s_params(const LegGeom &g, const LegAlm &a, const KParams &p) {
 // slots' phases.  `p`: the spin-2 parameters with the spin-2 tile rows.
 static void launch_s2s_synth(const LegGeom &g, const LegAlm &a, const KParams &p, int nmr, cudaStream_t st, bool prep) {
   KParams q = s2s_params(g, a, p);
-  const long long crow = a.s2s_trows + TL;   // tile rows per component
-  q.trows = static_cast<double *>(scratch_get("synth_rows_s2s", sizeof(TileS0) * 2 * (size_t)crow));
+  q.trows = static_cast<double *>(scratch_get("synth_rows_s2s", sizeof(TileS0<2>) * (size_t)(a.s2s_trows + TL_S2S)));
   if (prep) {
-    prep_s2s_kernel<<<dim3((a.lmax + 2 + 8 + 255) / 256, nmr), 256, 0, st>>>(q, crow);
+    prep_s2s_kernel<<<dim3((a.lmax + 2 + 8 + 255) / 256, nmr), 256, 0, st>>>(q);
     count_launch();
   }
-  const SeedTab *t = seed_table(g, SEED_S0X, 4, q, a.nm, st);
-  if (t) use_seed(q, t);
-  for (int c = 0; c < 2; ++c) {
-    KParams qc = q;
-    qc.comp0 = p.comp0 + c;
-    qc.trows = q.trows + (size_t)c * crow * (sizeof(TileS0) / sizeof(double));
-    if (t) launch_w<4>(synth0_kernel<4, 16, true>, qc, nmr, st);
-    else launch_w<4>(synth0_kernel<4, 16>, qc, nmr, st);
-    count_launch();
-  }
+  if (const SeedTab *t = seed_table(g, SEED_S0X, 4, q, a.nm, st)) { use_seed(q, t); launch_w<4>(synth0_kernel<2, 4, 12, true>, q, nmr, st); }
+  else launch_w<4>(synth0_kernel<2, 4, 12>, q, nmr, st);
+  count_launch();
   if (g.s2s_npolar > 0) {
     KParams pp = p;
     pp.nslots = min(p.nslots, g.s2s_npolar);
@@ -1669,7 +1682,7 @@ void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *cons
   KParams p = make_params(g, a, const_cast<double *>(alm[0]), (spin && !a.deriv1) ? const_cast<double *>(alm[1]) : nullptr, ph);
   // tile rows {A', [C',] g a_lm} for all local (m, l): written once per transform (`prep`), then
   // streamed by every warp of the Legendre kernel
-  const size_t rowbytes = spin == 0 ? sizeof(TileS0) : (a.deriv1 ? sizeof(TileD1) : sizeof(TileS2));
+  const size_t rowbytes = spin == 0 ? sizeof(TileS0<1>) : (a.deriv1 ? sizeof(TileD1) : sizeof(TileS2));
   p.tofs = a.tofs;
   p.trows = static_cast<double *>(scratch_get(spin == 0 ? "synth_rows0" : "synth_rows2", rowbytes * (size_t)(a.trows + TL)));
   if (s2s_route(g, a)) { launch_s2s_synth(g, a, p, nmr, st, prep); return; }
@@ -1692,14 +1705,14 @@ void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *cons
     }
   } else if (spin == 0) {
     switch (r0 * 100 + b0) {
-      case 216: launch_w<2>(synth0_kernel<2, 16>, p, nmr, st); break;
-      case 412: launch_w<4>(synth0_kernel<4, 12>, p, nmr, st); break;
-      case 612: launch_w<6>(synth0_kernel<6, 12>, p, nmr, st); break;
-      case 812: launch_w<8>(synth0_kernel<8, 12>, p, nmr, st); break;
-      case 808: launch_w<8>(synth0_kernel<8, 8>, p, nmr, st); break;
+      case 216: launch_w<2>(synth0_kernel<1, 2, 16>, p, nmr, st); break;
+      case 412: launch_w<4>(synth0_kernel<1, 4, 12>, p, nmr, st); break;
+      case 612: launch_w<6>(synth0_kernel<1, 6, 12>, p, nmr, st); break;
+      case 812: launch_w<8>(synth0_kernel<1, 8, 12>, p, nmr, st); break;
+      case 808: launch_w<8>(synth0_kernel<1, 8, 8>, p, nmr, st); break;
       default:
-        if (const SeedTab *t = seed_table(g, SEED_S0, 4, p, a.nm, st)) { use_seed(p, t); launch_w<4>(synth0_kernel<4, 16, true>, p, nmr, st); }
-        else launch_w<4>(synth0_kernel<4, 16>, p, nmr, st);
+        if (const SeedTab *t = seed_table(g, SEED_S0, 4, p, a.nm, st)) { use_seed(p, t); launch_w<4>(synth0_kernel<1, 4, 16, true>, p, nmr, st); }
+        else launch_w<4>(synth0_kernel<1, 4, 16>, p, nmr, st);
         break;
     }
   } else {
