@@ -571,6 +571,22 @@ def _view_maps(m: comm_map, info: comm_mapinfo, nm: int) -> comm_map:
 # sqrt(S) / beam / N^-1 passes fused into the transform kernels, dot products reduced on the device.
 # =====================================================================================================
 
+def _draw_args(seed, draw, pixel, prior):
+    """(seed, draw, terms) of cmdr_cr_compute_rhs_draw, after the range checks."""
+    from . import sharp
+    for name, v in (("seed", seed), ("draw", draw)):
+        if not isinstance(v, (int, np.integer)) or not 0 <= int(v) < 2 ** 64:
+            raise ValueError(f"{name} must be an integer in [0, 2^64), got {v!r}")
+    return int(seed), int(draw), (sharp.CMDR_CR_ETA_PIX if pixel else 0) | (sharp.CMDR_CR_ETA_ALM if prior else 0)
+
+
+def _cuda_probe(device=None):
+    """An empty float64 tensor on `device` (default: the current CUDA device): what output buffers follow when no input
+    array says where they live."""
+    import torch
+    return torch.empty(0, dtype=torch.float64, device=device if device is not None else torch.device("cuda", torch.cuda.current_device()))
+
+
 def _ptrs(arrs):
     """Array of column pointers over a list of 1-D views (numpy or torch); returns (ctypes array, keep-alive)."""
     import ctypes as C
@@ -670,6 +686,36 @@ class cr_native_system:
         bp, _d = _ptrs([b[c] for c in range(nm)])
         self.L.cmdr_cr_compute_rhs(self.handle, dp, ep, ap, bp, None)
         return b
+
+    def computeRHS_draw(self, data, seed, draw, pixel=True, prior=True):
+        """cr_computeRHS with the fluctuation terms drawn on the device (cmdr_cr_compute_rhs_draw, stream of
+        commander_b200/csrc/rng.cuh): data as for computeRHS, or None for the fluctuation terms alone (d = 0); seed and
+        draw unsigned 64-bit (draw: e.g. the Gibbs sample index); pixel / prior: the N^-1/2 eta_nu and eta_0 terms (eta_0
+        only with a prior).  b follows data (numpy or torch on its device); with data None it is a torch tensor on the
+        current CUDA device.  Collective."""
+        seed, draw, terms = _draw_args(seed, draw, pixel, prior)
+        nm = self.nmaps
+        b = self._like(data[0] if data is not None else _cuda_probe())
+        dp = None
+        if data is not None:
+            dp, _a = _ptrs([data[q][c] for q in range(self.nbands) for c in range(nm)])
+        bp, _d = _ptrs([b[c] for c in range(nm)])
+        self.L.cmdr_cr_compute_rhs_draw(self.handle, dp, seed, draw, terms, bp, None)
+        return b
+
+    def draw_eta(self, seed, draw, device=None):
+        """The draws of computeRHS_draw written out (cmdr_cr_draw_eta): (eta_pix, eta_alm) in computeRHS's layouts, a
+        list (per band) of (nmaps, np) and one (nmaps, nalm), zeros without a prior; torch tensors on `device` (default:
+        the current CUDA device).  computeRHS(data, *draw_eta(s, d)) equals computeRHS_draw(data, s, d) bit for bit."""
+        import torch
+        seed, draw, _ = _draw_args(seed, draw, True, True)
+        dev = _cuda_probe(device).device
+        eta_pix = [torch.empty((self.nmaps, self.info.np), dtype=torch.float64, device=dev) for _ in range(self.nbands)]
+        eta_alm = torch.empty((self.nmaps, self.info.nalm), dtype=torch.float64, device=dev)
+        ep, _a = _ptrs([e[c] for e in eta_pix for c in range(self.nmaps)])
+        ap, _b = _ptrs([eta_alm[c] for c in range(self.nmaps)])
+        self.L.cmdr_cr_draw_eta(self.handle, seed, draw, ep, ap, None)
+        return eta_pix, eta_alm
 
     def solve(self, b, x0=None, maxiter=300, cg_tol=1e-8, cg_conv_crit="residual", cg_miniter=5, cg_check_conv_freq=1):
         """solve_cr_eqn_by_CG, commander3/src/comm_cr_mod.f90:201-348.  Returns (x, iterations done, residual history)."""
@@ -875,6 +921,35 @@ class cr_native_multi_system:
         bp, _d = self._cols(b)
         self.L.cmdr_cr_compute_rhs(self.handle, dp, ep, ap, bp, None)
         return b
+
+    def computeRHS_draw(self, data, seed, draw, pixel=True, prior=True):
+        """cr_computeRHS with the fluctuation terms drawn on the device (cmdr_cr_compute_rhs_draw, stream of
+        commander_b200/csrc/rng.cuh): data as for computeRHS, or None for the fluctuation terms alone (d = 0); seed and
+        draw unsigned 64-bit; pixel / prior: the N^-1/2 eta_nu and eta_0 terms (eta_0 on the components with a prior).
+        b follows data (numpy or torch on its device); with data None it is a torch tensor on the current CUDA device.
+        Collective."""
+        seed, draw, terms = _draw_args(seed, draw, pixel, prior)
+        b = self._like(data[0] if data is not None else _cuda_probe())
+        dp = None
+        if data is not None:
+            dp, _a = self._band_cols(data, "data")
+        bp, _d = self._cols(b)
+        self.L.cmdr_cr_compute_rhs_draw(self.handle, dp, seed, draw, terms, bp, None)
+        return b
+
+    def draw_eta(self, seed, draw, device=None):
+        """The draws of computeRHS_draw written out (cmdr_cr_draw_eta): (eta_pix, eta_alm) in computeRHS's layouts, a
+        list (per band) of (nmaps_q, np_q) and a flat vector of length ncr (zeros on the components without a prior);
+        torch tensors on `device` (default: the current CUDA device)."""
+        import torch
+        seed, draw, _ = _draw_args(seed, draw, True, True)
+        dev = _cuda_probe(device).device
+        eta_pix = [torch.empty((b.info.nmaps, b.info.np), dtype=torch.float64, device=dev) for b in self.bands]
+        eta_alm = torch.empty(self.ncr, dtype=torch.float64, device=dev)
+        ep, _a = self._band_cols(eta_pix, "eta_pix")
+        ap, _b = self._cols(eta_alm)
+        self.L.cmdr_cr_draw_eta(self.handle, seed, draw, ep, ap, None)
+        return eta_pix, eta_alm
 
     def solve(self, b, x0=None, maxiter=300, cg_tol=1e-8, cg_conv_crit="residual", cg_miniter=5, cg_check_conv_freq=1):
         """solve_cr_eqn_by_CG, commander3/src/comm_cr_mod.f90:201-348.  Returns (x, iterations done, residual history)."""

@@ -54,6 +54,7 @@ struct cmdr_cr_system {
   std::vector<long long> col;  // a_lm per column of a CG vector: nmaps x nalm, or those of every component (multi)
   cmdr::CrMulti *multi = nullptr;   // several components and bands (cmdr_cr_setup_multi, cr_multi.cu)
   double *vs = nullptr;        // M^-1 r of the block or pseudo-inverse preconditioner (multi)
+  CrRing *rings = nullptr;     // local -> global ring table of the drawn fluctuation terms (cr_draw.cu; one-component)
 };
 
 namespace {
@@ -320,6 +321,7 @@ cmdr_cr_system *cmdr_cr_setup(int comm, int nbands, int nmaps, const sharp_geom_
   s->lsc = dalloc<double>(s->h_lsc.size());
   CMDR_CUDA_CHECK(cudaMemcpyAsync(s->lsc, s->h_lsc.data(), sizeof(double) * s->h_lsc.size(), cudaMemcpyHostToDevice, st));
   s->map = dalloc<double>((size_t)nmaps * s->npix);
+  s->rings = cr_ring_table_device(s->gT);
   s->col.assign(nmaps, s->nalm);
   alloc_work(s, st);
   CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
@@ -407,7 +409,7 @@ void cmdr_cr_destroy(cmdr_cr_system *s) {
   cudaDeviceSynchronize();
   cudaFree(s->invN); cudaFree(s->lsc); cudaFree(s->blF); cudaFree(s->Minv); cudaFree(s->map);
   cudaFree(s->vx); cudaFree(s->vr); cudaFree(s->vd); cudaFree(s->vq); cudaFree(s->vb);
-  cudaFree(s->sc); cudaFree(s->partial); cudaFree(s->hist); cudaFree(s->vs);
+  cudaFree(s->sc); cudaFree(s->partial); cudaFree(s->hist); cudaFree(s->vs); cudaFree(s->rings);
   if (s->h_sc) cudaFreeHost(s->h_sc);
   if (s->multi) cr_multi_destroy(s->multi);
   delete s;
@@ -452,13 +454,35 @@ void cmdr_cr_invM(cmdr_cr_system *s, const double *const *r, double *const *z, v
   CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
 }
 
-// data / eta_pix: nbands * nmaps column pointers (n_pix each; eta_pix may be NULL), eta_alm: nmaps pointers or NULL
-void cmdr_cr_compute_rhs(cmdr_cr_system *s, const double *const *data, const double *const *eta_pix,
-                         const double *const *eta_alm, double *const *b, void *stream) {
-  cudaStream_t st = (cudaStream_t)stream;
+}  // extern "C"
+
+namespace {
+
+// The drawn eta_0 of every component with a prior into the device CG vector out (zeros elsewhere)
+void draw_alm(cmdr_cr_system *s, unsigned long long seed, unsigned long long draw, double *out, cudaStream_t st) {
   if (s->multi) {
-    if (eta_alm) copy_in(s, s->vq, eta_alm, st);
-    cr_multi_rhs(s->multi, data, eta_pix, eta_alm ? s->vq : nullptr, s->vb, st);
+    cr_multi_draw_eta(s->multi, seed, draw, nullptr, out, st);
+  } else if (s->prior) {
+    cr_draw_alm(out, s->nalm, s->a, s->nmaps, seed, draw, 0, st);
+  } else {
+    CMDR_CUDA_CHECK(cudaMemsetAsync(out, 0, sizeof(double) * s->n, st));
+  }
+}
+
+// cr_computeRHS into the caller's b.  data: nbands * nmaps column pointers (nullptr: d = 0, drawn terms only); the pixel
+// term from `eta`, the prior term from the caller's eta_alm columns or, with eta.draw, from the stream
+void compute_rhs(cmdr_cr_system *s, const double *const *data, const RhsEta &eta, const double *const *eta_alm, double *const *b,
+                 cudaStream_t st) {
+  const double *alm = nullptr;   // eta_0 as a device CG vector (s->vq), or none
+  if (eta.draw) {
+    const bool prior = s->multi ? true : s->prior;   // cr_multi_rhs adds it on the components with a prior only
+    if ((eta.terms & CMDR_CR_ETA_ALM) && prior) { draw_alm(s, eta.seed, eta.index, s->vq, st); alm = s->vq; }
+  } else if (eta_alm) {
+    copy_in(s, s->vq, eta_alm, st);
+    alm = s->vq;
+  }
+  if (s->multi) {
+    cr_multi_rhs(s->multi, data, eta, alm, s->vb, st);
     copy_out(s, b, s->vb, st);
     CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
     return;
@@ -473,20 +497,73 @@ void cmdr_cr_compute_rhs(cmdr_cr_system *s, const double *const *data, const dou
     for (int c = 0; c < s->nmaps; ++c) {
       const int i = bnd * s->nmaps + c;
       o.lscale[c] = s->lsc + (size_t)i * (s->lmax + 1);
-      if (!s->npix) continue;
-      CMDR_CUDA_CHECK(cudaMemcpyAsync(tmp, data[i], sizeof(double) * s->npix, cudaMemcpyDefault, st));
-      if (eta_pix) CMDR_CUDA_CHECK(cudaMemcpyAsync(tmp + s->npix, eta_pix[i], sizeof(double) * s->npix, cudaMemcpyDefault, st));
-      k_rhs_map<<<NBLK, NTHR, 0, st>>>(mp[c], s->invN + (size_t)i * s->npix, tmp, eta_pix ? tmp + s->npix : nullptr, s->npix);
-      count_launch(1);
+      cr_rhs_column(mp[c], s->invN + (size_t)i * s->npix, data ? data[i] : nullptr, eta, i, bnd, c, s->npix, s->rings,
+                    s->gT->nrings, tmp, st);
     }
     execute_iqu_opts(s->comm, SHARP_Yt, s->nmaps, ba, mp, s->gT, s->gP, s->a, SHARP_DP | SHARP_ADD, &o, st);
   }
-  if (eta_alm) {
-    copy_in(s, s->vq, eta_alm, st);
-    k_add<<<NBLK, NTHR, 0, st>>>(s->vb, s->vq, s->n);
+  if (alm) {
+    k_add<<<NBLK, NTHR, 0, st>>>(s->vb, alm, s->n);
     count_launch(1);
   }
   copy_out(s, b, s->vb, st);
+  CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
+}
+
+// cmdr_cr_compute_rhs_draw's arguments, checked on every rank and compared between them before any of them aborts
+void check_draw_call(const cmdr_cr_system *s, unsigned long long seed, unsigned long long draw, int terms, cudaStream_t st) {
+  const std::string err = check_cr_draw(terms);
+  int w[CR_DRAW_WORDS];
+  cr_draw_words(seed, draw, terms, err.empty(), w);
+  bool same = true;
+  for (int i = 0; i < CR_DRAW_WORDS; ++i) same = comm_all_equal(s->comm, w[i], st) && same;
+  if (!err.empty()) { fprintf(stderr, "cmdr_sht: cmdr_cr_compute_rhs_draw: %s\n", err.c_str()); abort(); }
+  if (!same) {
+    fprintf(stderr, "cmdr_sht: cmdr_cr_compute_rhs_draw: the ranks passed different (seed, draw, terms) or one of them an "
+                    "invalid argument; every rank of the communicator must make the same call\n");
+    abort();
+  }
+}
+
+}  // namespace
+
+extern "C" {
+
+// data / eta_pix: nbands * nmaps column pointers (n_pix each; eta_pix may be NULL), eta_alm: nmaps pointers or NULL
+void cmdr_cr_compute_rhs(cmdr_cr_system *s, const double *const *data, const double *const *eta_pix,
+                         const double *const *eta_alm, double *const *b, void *stream) {
+  RhsEta eta;
+  eta.pix = eta_pix;
+  compute_rhs(s, data, eta, eta_alm, b, (cudaStream_t)stream);
+}
+
+void cmdr_cr_compute_rhs_draw(cmdr_cr_system *s, const double *const *data, unsigned long long seed, unsigned long long draw,
+                              int terms, double *const *b, void *stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  check_draw_call(s, seed, draw, terms, st);
+  RhsEta eta;
+  eta.draw = true;
+  eta.seed = seed;
+  eta.index = draw;
+  eta.terms = terms;
+  compute_rhs(s, data, eta, nullptr, b, st);
+}
+
+void cmdr_cr_draw_eta(cmdr_cr_system *s, unsigned long long seed, unsigned long long draw, double *const *eta_pix,
+                      double *const *eta_alm, void *stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (s->multi) {
+    cr_multi_draw_eta(s->multi, seed, draw, eta_pix, nullptr, st);
+  } else if (eta_pix) {
+    for (int bnd = 0; bnd < s->nbands; ++bnd)
+      for (int c = 0; c < s->nmaps; ++c)
+        cr_draw_pix(eta_pix[bnd * s->nmaps + c], s->rings, s->gT->nrings, s->npix, seed, draw, bnd, c, st);
+  }
+  if (eta_alm) {
+    draw_alm(s, seed, draw, s->vq, st);
+    copy_out(s, eta_alm, s->vq, st);
+  }
+  CMDR_CUDA_CHECK(cudaGetLastError());
   CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
 }
 

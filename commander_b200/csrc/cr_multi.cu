@@ -259,6 +259,7 @@ struct CrMulti {
   std::vector<bool> own_xa;              // built here (L_q < lmax_q)
   std::vector<long long> npix;
   std::vector<double *> invN, buf;       // per band: [nmaps_q][npix_q], [nmaps_q][nalm at L_q]
+  std::vector<CrRing *> rings;           // per band: local -> global ring table of the drawn fluctuation terms (cr_draw.cu)
   double *map = nullptr;                 // [3][max npix]
   CrDev D;
   int *d_mval = nullptr, *d_cnm = nullptr, *d_clmax = nullptr, *d_bnm = nullptr, *d_L = nullptr;
@@ -353,6 +354,7 @@ CrMulti *cr_multi_create(int comm, const CrPlan &plan, const sharp_alm_info *con
     for (int j = 0; j < S->bnm[q]; ++j)
       if (np) CMDR_CUDA_CHECK(cudaMemcpyAsync(d + (size_t)j * np, invN[bofs[q] + j], sizeof(double) * np, cudaMemcpyDefault, st));
     S->invN.push_back(d);
+    S->rings.push_back(cr_ring_table_device(S->gT[q]));
     S->buf.push_back(dalloc<double>((size_t)S->bnm[q] * p.nalm[p.xform(q)]));
   }
   S->map = dalloc<double>((size_t)3 * maxpix);
@@ -403,7 +405,7 @@ CrMulti *cr_multi_create(int comm, const CrPlan &plan, const sharp_alm_info *con
 void cr_multi_destroy(CrMulti *S) {
   for (size_t q = 0; q < S->xa.size(); ++q) {
     if (S->own_xa[q]) sharp_destroy_alm_info(S->xa[q]);
-    cudaFree(S->invN[q]); cudaFree(S->buf[q]);
+    cudaFree(S->invN[q]); cudaFree(S->buf[q]); cudaFree(S->rings[q]);
   }
   for (size_t i = 0; i < S->F.size(); ++i) { cudaFree(S->F[i]); cudaFree(S->mix[i]); }
   for (double *n : S->Ncov) cudaFree(n);
@@ -524,9 +526,9 @@ void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st) {
   comp_gather(S, x, y, st);                                        // :926-1008, + P x
 }
 
-// b = sum_q g Y^t (N^-1 d_q + N^-1/2 eta_q) (+ eta_alm on the components with a prior); eta_alm: device vector or nullptr
-void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *eta_pix, const double *eta_alm, double *b,
-                  cudaStream_t st) {
+// b = sum_q g Y^t (N^-1 d_q + N^-1/2 eta_q) (+ eta_alm on the components with a prior); eta_q from the caller or drawn
+// (RhsEta), data nullptr: d = 0; eta_alm: device vector or nullptr
+void cr_multi_rhs(CrMulti *S, const double *const *data, const RhsEta &eta, const double *eta_alm, double *b, cudaStream_t st) {
   double *alm[3], *map[3];
   long long maxpix = 1;
   for (long long np : S->npix) maxpix = std::max(maxpix, np);
@@ -535,15 +537,27 @@ void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *et
   for (int q = 0; q < S->p.nbands; ++q) {
     band_cols(S, q, alm, map);
     const long long np = S->npix[q];
-    for (int j = 0; j < S->bnm[q]; ++j, ++col) {
-      if (!np) continue;
-      CMDR_CUDA_CHECK(cudaMemcpyAsync(tmp, data[col], sizeof(double) * np, cudaMemcpyDefault, st));
-      if (eta_pix) CMDR_CUDA_CHECK(cudaMemcpyAsync(tmp + np, eta_pix[col], sizeof(double) * np, cudaMemcpyDefault, st));
-      cr_rhs_map(map[j], S->invN[q] + (size_t)j * np, tmp, eta_pix ? tmp + np : nullptr, np, st);
-    }
+    for (int j = 0; j < S->bnm[q]; ++j, ++col)
+      cr_rhs_column(map[j], S->invN[q] + (size_t)j * np, data ? data[col] : nullptr, eta, col, q, j, np, S->rings[q],
+                    S->gT[q]->nrings, tmp, st);
     band_back(S, q, alm, map, st);
   }
   comp_gather(S, eta_alm, b, st);
+}
+
+void cr_multi_draw_eta(CrMulti *S, unsigned long long seed, unsigned long long draw, double *const *eta_pix, double *eta_alm,
+                       cudaStream_t st) {
+  if (eta_pix)
+    for (int q = 0, col = 0; q < S->p.nbands; ++q)
+      for (int j = 0; j < S->bnm[q]; ++j, ++col)
+        cr_draw_pix(eta_pix[col], S->rings[q], S->gT[q]->nrings, S->npix[q], seed, draw, q, j, st);
+  if (!eta_alm) return;
+  for (int k = 0; k < S->p.ncomp; ++k) {
+    double *out = eta_alm + S->off[k];
+    const long long na = S->p.nalm[S->p.comp(k)];
+    if ((S->prior >> k) & 1u) cr_draw_alm(out, na, S->ca[k], S->cnm[k], seed, draw, k, st);
+    else if (na) CMDR_CUDA_CHECK(cudaMemsetAsync(out, 0, sizeof(double) * S->cnm[k] * na, st));
+  }
 }
 
 // Installs (F != nullptr) or removes the per-pixel mixing map of pair (band, comp); the arguments are checked

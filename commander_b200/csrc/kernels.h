@@ -6,6 +6,7 @@
 #include <cstdlib>
 #include <vector>
 
+#include "cr_draw.h"
 #include "cr_plan.h"
 #include "job.h"
 #include "sht_internal.h"
@@ -202,6 +203,24 @@ void execute_iqu_opts(int comm, int type, int nmaps, double *const *alm, double 
 // constrained-realisation pieces shared by the one-component system (cr.cu) and the multi-component one (cr_multi.cu)
 // m = N^-1 d (+ sqrt(N^-1) eta): the map of one band and map column in cr_computeRHS
 void cr_rhs_map(double *m, const double *invN, const double *d, const double *eta, long long n, cudaStream_t st);
+// Where the fluctuation terms of cr_computeRHS come from: the caller's columns, or the device stream of rng.cuh
+struct RhsEta {
+  const double *const *pix = nullptr;   // caller eta_pix columns (per band and map), nullptr: no pixel term (draw = false)
+  bool draw = false;                    // draw on the device: (seed, index) of the stream, `terms` CMDR_CR_ETA_PIX | _ALM
+  unsigned long long seed = 0, index = 0;
+  int terms = 0;
+};
+// The RHS map of band q, map j (column `col` of data and eta_pix) into m: N^-1 d (data_col nullptr: d = 0) plus the pixel
+// term of `eta`.  `rings`, `nrings`: the band's table (cr_ring_table_device); tmp: 2 np doubles of device scratch (cr_draw.cu)
+void cr_rhs_column(double *m, const double *invN, const double *data_col, const RhsEta &eta, int col, int q, int j, long long np,
+                   const CrRing *rings, int nrings, double *tmp, cudaStream_t st);
+CrRing *cr_ring_table_device(const sharp_geom_info *g);   // the caller frees it
+// eta of band q, map j at every local pixel into dst (np doubles, host or device)
+void cr_draw_pix(double *dst, const CrRing *rings, int nrings, long long np, unsigned long long seed, unsigned long long draw,
+                 int q, int j, cudaStream_t st);
+// eta_0 of component k at every local slot of `a` into out[j * stride + slot], j < nmaps (device)
+void cr_draw_alm(double *out, long long stride, sharp_alm_info *a, int nmaps, unsigned long long seed, unsigned long long draw,
+                 int k, cudaStream_t st);
 // nlm ([nmaps][nalm] device) = N^-1_{lm,lm} of one band from its N^-1 maps ([nmaps][npix] device): compute_invN_lm
 void cr_invn_lm(int comm, int nmaps, double *invN, sharp_geom_info *gT, sharp_geom_info *gP, sharp_alm_info *a, double *nlm,
                 cudaStream_t st);
@@ -216,8 +235,11 @@ long long cr_multi_length(const CrMulti *S);
 void cr_multi_columns(const CrMulti *S, std::vector<long long> &len);   // a_lm per column of a CG vector
 bool cr_multi_has_precond(const CrMulti *S);   // a preconditioner other than the identity is selected
 void cr_multi_matmulA(CrMulti *S, const double *x, double *y, cudaStream_t st);
-void cr_multi_rhs(CrMulti *S, const double *const *data, const double *const *eta_pix, const double *eta_alm, double *b,
-                  cudaStream_t st);
+void cr_multi_rhs(CrMulti *S, const double *const *data, const RhsEta &eta, const double *eta_alm, double *b, cudaStream_t st);
+// The draws of the stream for this handle: eta_pix (per band and map, host or device; nullptr: none) and eta_alm (a device
+// CG vector, zeros on the components without a prior; nullptr: none)
+void cr_multi_draw_eta(CrMulti *S, unsigned long long seed, unsigned long long draw, double *const *eta_pix, double *eta_alm,
+                       cudaStream_t st);
 // z = M^-1 r with the selected preconditioner (pseudo-inverse or block diagonal; collective with the pseudo-inverse)
 void cr_multi_precond(CrMulti *S, const double *r, double *z, cudaStream_t st);
 // cmdr_cr_set_pseudoinv on a multi-component handle: checks (collectively), builds the tables on first use, selects

@@ -22,6 +22,7 @@ SHARP_DP = 1 << 4
 SHARP_ADD = 1 << 5
 SHARP_REAL_HARMONICS = 1 << 6
 SHARP_NO_FFT = 1 << 7
+CMDR_CR_ETA_PIX, CMDR_CR_ETA_ALM = 1, 2   # `terms` of cmdr_cr_compute_rhs_draw
 
 _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libcmdr_sht.so")
 _lib = None
@@ -42,7 +43,7 @@ ABI_SYMBOLS = [
     "cmdr_sht_set_spin2_scalar",
     "cmdr_cr_setup", "cmdr_cr_destroy", "cmdr_cr_matmulA", "cmdr_cr_invM", "cmdr_cr_set_precond_diag",
     "cmdr_cr_get_precond_diag", "cmdr_cr_compute_rhs", "cmdr_cr_solve", "cmdr_cr_matmul_count", "cmdr_cr_setup_multi",
-    "cmdr_cr_set_mixing_map", "cmdr_cr_set_pseudoinv",
+    "cmdr_cr_set_mixing_map", "cmdr_cr_set_pseudoinv", "cmdr_cr_compute_rhs_draw", "cmdr_cr_draw_eta",
 ]
 
 
@@ -116,6 +117,8 @@ def lib() -> C.CDLL:
     L.cmdr_cr_set_precond_diag.argtypes = [vp, vp]
     L.cmdr_cr_get_precond_diag.argtypes = [vp, vp]
     L.cmdr_cr_compute_rhs.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.cmdr_cr_compute_rhs_draw.argtypes = [vp, vp, C.c_ulonglong, C.c_ulonglong, ci, vp, vp]
+    L.cmdr_cr_draw_eta.argtypes = [vp, C.c_ulonglong, C.c_ulonglong, vp, vp, vp]
     L.cmdr_cr_solve.argtypes = [vp, vp, vp, ci, ci, C.c_double, ci, ci, ci, vp, vp]
     L.cmdr_cr_solve.restype = ci
     L.cmdr_cr_matmul_count.argtypes = [vp]
