@@ -5,6 +5,7 @@
 // (SURVEY.md 8b).  Multi-GPU entry points live in dist.cu.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <cmath>
@@ -438,6 +439,28 @@ LegAlm make_legalm(sharp_alm_info *a, const Job &job, const double *const *lscal
   return A;
 }
 
+__global__ void __launch_bounds__(256) add_into_kernel(double *__restrict__ a, const double *__restrict__ r, long long n) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) a[i] = a[i] + r[i];
+}
+
+double *const *det_add_begin(bool add, double *const *alm, int ncols, size_t nd, cudaStream_t st) {
+  if (!add || !deterministic() || nd == 0) return alm;
+  static thread_local double *cols[4];
+  double *buf = static_cast<double *>(scratch_get("det_add", sizeof(double) * nd * ncols));
+  CMDR_CUDA_CHECK(cudaMemsetAsync(buf, 0, sizeof(double) * nd * ncols, st));
+  for (int c = 0; c < ncols; ++c) cols[c] = buf + (size_t)c * nd;
+  return cols;
+}
+void det_add_end(double *const *out, double *const *alm, int ncols, size_t nd, cudaStream_t st) {
+  if (out == alm) return;
+  for (int c = 0; c < ncols; ++c) {
+    add_into_kernel<<<(unsigned)std::min<size_t>((nd + 255) / 256, 148 * 8), 256, 0, st>>>(alm[c], out[c], (long long)nd);
+    count_launch();
+  }
+  CMDR_CUDA_CHECK(cudaGetLastError());
+}
+
 // Single-GPU transform with device pointers.  `ph` holds ncomp_tot components; this call
 // handles components [comp0, comp0+ncomp) of it.
 void run_single(const Job &job, double *const *alm, double *const *map, sharp_geom_info *g, sharp_alm_info *a,
@@ -483,12 +506,15 @@ void run_single(const Job &job, double *const *alm, double *const *map, sharp_ge
     prof_begin(100 + spin, 1, st);
     ringfft_anal(g, ncomp, L, ph, map, job.weighted, st);
     prof_end(st);
+    const size_t nd = (size_t)a->nalm * (a->real_packed ? 1 : 2);
+    double *const *out = det_add_begin(job.add, alm, ncomp, nd, st);
     if (!job.add)
       for (int c = 0; c < ncomp; ++c)
-        CMDR_CUDA_CHECK(cudaMemsetAsync(alm[c], 0, sizeof(double) * a->nalm * (a->real_packed ? 1 : 2), st));
+        CMDR_CUDA_CHECK(cudaMemsetAsync(alm[c], 0, sizeof(double) * nd, st));
     prof_begin(spin, 1, st);
-    launch_legendre_anal(G, A, alm, ph, st);
+    launch_legendre_anal(G, A, out, ph, st);
     prof_end(st);
+    det_add_end(out, alm, ncomp, nd, st);
   }
 }
 
@@ -604,6 +630,9 @@ static bool try_pipelined(const Job &job, double *const *alm, double *const *map
   static const bool disabled = getenv("CMDR_SHT_NO_PIPELINE") != nullptr;
   const int spin = job.spin, nca = job.alm_cols, ncomp = job.map_cols;
   if (disabled || job.add || g->npix < (1 << 21) || a->nm == 0) return false;
+  // Deterministic analysis takes the staged path: the chunks below run spin 2 on the spin-2 kernels without seed tables,
+  // while a transform of device arrays runs the scalar-sum route, so only the staged path gives the device path's bits.
+  if (!job.synth && deterministic()) return false;
   // host arrays of either kind: pinned ones are copied in place, pageable ones (what sharp.f90:219-224 passes)
   // go through the library's pinned arena and the copy threads (hostio.cu)
   for (int c = 0; c < nca; ++c)

@@ -26,6 +26,7 @@
 #include <map>
 #include <tuple>
 
+#include "det.h"
 #include "kernels.h"
 #include "legendre_core.cuh"
 
@@ -496,11 +497,13 @@ static void run_dist(DistComm *C, const Part *parts, int nparts, int ncomp_tot, 
       LegAlm A = make_legalm(a, p.job, p.lscale);
       G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.job.spin);
       const size_t nd = (size_t)a->nalm * (a->real_packed ? 1 : 2);
+      double *const *out = det_add_begin(add, p.alm, p.job.alm_cols, nd, st);
       if (!add && nd)
         for (int c = 0; c < p.job.alm_cols; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(p.alm[c], 0, sizeof(double) * nd, st));
       prof_begin(p.job.spin, 1, st);
-      launch_legendre_anal(G, A, p.alm, reinterpret_cast<const double4 *>(B.mine), st);
+      launch_legendre_anal(G, A, out, reinterpret_cast<const double4 *>(B.mine), st);
       prof_end(st);
+      det_add_end(out, p.alm, p.job.alm_cols, nd, st);
     }
     return;
   }
@@ -548,11 +551,13 @@ static void run_dist(DistComm *C, const Part *parts, int nparts, int ncomp_tot, 
       LegAlm A = make_legalm(a, p.job, p.lscale);
       G.comp0 = p.comp0; G.mlim = plan_mlim(P, a->lmax, p.job.spin);
       const size_t nd = (size_t)a->nalm * (a->real_packed ? 1 : 2);
+      double *const *out = det_add_begin(add, p.alm, p.job.alm_cols, nd, st);
       if (!add && nd)
         for (int c = 0; c < p.job.alm_cols; ++c) CMDR_CUDA_CHECK(cudaMemsetAsync(p.alm[c], 0, sizeof(double) * nd, st));
       prof_begin(p.job.spin, 1, st);
-      launch_legendre_anal(G, A, p.alm, reinterpret_cast<const double4 *>(bufB), st);
+      launch_legendre_anal(G, A, out, reinterpret_cast<const double4 *>(bufB), st);
       prof_end(st);
+      det_add_end(out, p.alm, p.job.alm_cols, nd, st);
     }
   }
 }
@@ -667,6 +672,7 @@ static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, 
     CMDR_CUDA_CHECK(cudaStreamSynchronize(cs));
     CMDR_CUDA_CHECK(cudaStreamSynchronize(st));
   } else {
+    const bool det = deterministic();
     cudaEvent_t e0 = pooled_event(ev0 + K);                // staging rows may still be read by earlier work on `st`
     CMDR_CUDA_CHECK(cudaEventRecord(e0, st));
     CMDR_CUDA_CHECK(cudaStreamWaitEvent(cs, e0, 0));
@@ -689,11 +695,15 @@ static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, 
       }
       stream_barrier(C, st);                               // chunk c is complete on every rank
       G.slot_begin = P->wcut[c]; G.slot_end = P->wcut[c + 1];
+      // deterministic mode: whole warp blocks per launch (a block that straddles two chunks waits for the later one, whose
+      // barrier completes its phases) and one ordered reduce per m range after the last chunk, before its download
+      if (det) det_cut(P->wcut[c], P->wcut[c + 1], c == K - 1, P->nslots, det_block_slots(spin), G.slot_begin, G.slot_end);
       if (c == K - 1 && nmch > 1) {
         for (int j = 0; j < nmch; ++j) {
           LegAlm Aj = A;
           Aj.im_begin = mcut[j]; Aj.im_end = mcut[j + 1];
-          launch_legendre_anal(G, Aj, alm_dev, reinterpret_cast<const double4 *>(B.mine), st);
+          launch_legendre_anal(G, Aj, alm_dev, reinterpret_cast<const double4 *>(B.mine), st, !det);
+          legendre_anal_reduce(G, Aj, alm_dev, st);
           cudaEvent_t ej = pooled_event(evm + NMCH + j);
           CMDR_CUDA_CHECK(cudaEventRecord(ej, st));
           CMDR_CUDA_CHECK(cudaStreamWaitEvent(cs, ej, 0));
@@ -702,7 +712,8 @@ static bool try_dist_pipelined(DistComm *C, const Job &job, double *const *alm, 
           ioA.commit(cs);
         }
       } else {
-        launch_legendre_anal(G, A, alm_dev, reinterpret_cast<const double4 *>(B.mine), st);
+        launch_legendre_anal(G, A, alm_dev, reinterpret_cast<const double4 *>(B.mine), st, !det);
+        if (c == K - 1) legendre_anal_reduce(G, A, alm_dev, st);
       }
     }
     if (nmch == 1) {
@@ -792,6 +803,15 @@ void comm_allgather(int comm, const void *in, void *out, size_t bytes, cudaStrea
   DistComm *C = find_comm(comm);
   CMDR_NCCL_CHECK(nccl_api()->AllGather(in, out, bytes, ncclChar, C->nccl, st));
   count_launch(1);
+}
+
+// out[i] = sum over ranks r in ascending order of all[r n + i]: the deterministic form of cmdr_sht_allreduce_sum
+__global__ void __launch_bounds__(256) rank_order_sum_kernel(double *out, const double *all, int n, int nranks) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  double s = all[i];
+  for (int r = 1; r < nranks; ++r) s += all[(size_t)r * n + i];
+  out[i] = s;
 }
 
 // map *= F, the pixel-space mixing step between Y and YtW (HBM-bound: 24 bytes per pixel)
@@ -885,6 +905,16 @@ void cmdr_sht_allreduce_sum(int comm, double *dev_buf, int n, void *stream) {
     abort();
   }
   if (!C || C->nranks == 1) return;
+  if (deterministic()) {
+    // NCCL fixes no reduction order: gather every rank's n values and sum them in rank order, the same bits on every rank
+    cudaStream_t st = (cudaStream_t)stream;
+    double *all = static_cast<double *>(scratch_get("det_allreduce", sizeof(double) * (size_t)std::max(n, 1) * C->nranks));
+    CMDR_NCCL_CHECK(nccl_api()->AllGather(dev_buf, all, n, ncclDouble, C->nccl, st));
+    if (n > 0) rank_order_sum_kernel<<<(n + 255) / 256, 256, 0, st>>>(dev_buf, all, n, C->nranks);
+    count_launch(2);
+    CMDR_CUDA_CHECK(cudaGetLastError());
+    return;
+  }
   CMDR_NCCL_CHECK(nccl_api()->AllReduce(dev_buf, dev_buf, n, ncclDouble, ncclSum, C->nccl, (cudaStream_t)stream));
   count_launch(1);
 }

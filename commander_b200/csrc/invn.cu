@@ -13,11 +13,13 @@
 // squared accumulate.  No 3j recursion, O(lmax^3) FMAs on the FP64 pipe instead of on 16 host threads.
 //
 // One warp per (local m, block of 32*R nodes); x -> -x symmetry folds the nodes to the positive half.
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <thread>
 #include <vector>
 
+#include "det.h"
 #include "kernels.h"
 #include "legendre_core.cuh"
 
@@ -37,11 +39,16 @@ struct InvNParams {
   const double *f;         // nmaps * nnodes: folded weight * profile, see cmdr_sht_invn_diag
   double *out[3];
   long long nalm;
+  // deterministic mode (det.h): partials of component c at det + c * dl.comp_stride(), one value per l (part 0), local m's
+  // from dl.im0; every (node block, m, l) is stored, so no records are needed
+  double *det;
+  DetLayout dl;
 };
 
-template <int R, int NM>
+// DET: lane 0 stores each l's sum of the warp (0.0 where the warp is below the threshold) instead of adding it to out
+template <int R, int NM, bool DET = false>
 __global__ void __launch_bounds__(32, 16) invn_kernel(InvNParams p) {
-  const int im = blockIdx.y, m = p.mval[im];
+  const int im = (DET ? p.dl.im0 : 0) + blockIdx.y, m = p.mval[im];
   const int lane = threadIdx.x;
   const int node0 = blockIdx.x * (32 * R);
   double x[R], cur[R], prev[R], f[R][NM];
@@ -73,6 +80,9 @@ __global__ void __launch_bounds__(32, 16) invn_kernel(InvNParams p) {
     for (int j = 0; j < nl; ++j) {
       const int l = l0 + j;
       const double2 cg = coef[l - m];
+      if (DET && skip && lane == 0)
+#pragma unroll
+        for (int c = 0; c < NM; ++c) p.det[c * p.dl.comp_stride() + p.dl.index(0, blockIdx.x, im, l, 0)] = 0.0;
       if (!skip) {
         double s[NM];
 #pragma unroll
@@ -94,7 +104,9 @@ __global__ void __launch_bounds__(32, 16) invn_kernel(InvNParams p) {
 #pragma unroll
           for (int c = 0; c < NM; ++c) {
             const double val = g2 * s[c];
-            if (m == 0) {
+            if (DET) {
+              p.det[c * p.dl.comp_stride() + p.dl.index(0, blockIdx.x, im, l, 0)] = val;
+            } else if (m == 0) {
               atomicAdd(p.out[c] + mvs + l, val);
             } else {
               atomicAdd(p.out[c] + mvs + 2 * (long long)l, val);
@@ -112,6 +124,29 @@ __global__ void __launch_bounds__(32, 16) invn_kernel(InvNParams p) {
 #pragma unroll
     for (int r = 0; r < R; ++r)
       if (k[r] < 0 && needs_rescale(cur[r])) { cur[r] *= SCALE_DOWN_D; prev[r] *= SCALE_DOWN_D; ++k[r]; }
+  }
+}
+
+// Ordered reduce of the deterministic mode: out = out + (sum over node blocks in ascending order), both entries of an
+// m > 0 pair getting the same value as with the atomics
+template <int NM>
+__global__ void __launch_bounds__(256) invn_reduce_kernel(InvNParams p) {
+  const int im = p.dl.im0 + blockIdx.y, m = p.mval[im];
+  const int l = blockIdx.x * blockDim.x + threadIdx.x;
+  if (l < m || l > p.lmax) return;
+  const long long mvs = p.mvstart[im];
+  const size_t bstride = (size_t)p.dl.nm * p.dl.row();
+#pragma unroll
+  for (int c = 0; c < NM; ++c) {
+    const double *src = p.det + c * p.dl.comp_stride() + p.dl.index(0, 0, im, l, 0);
+    double s = 0.0;
+    for (int b = 0; b < p.dl.nb; ++b) s += src[(size_t)b * bstride];
+    if (m == 0) {
+      p.out[c][mvs + l] = p.out[c][mvs + l] + s;
+    } else {
+      p.out[c][mvs + 2 * (long long)l] = p.out[c][mvs + 2 * (long long)l] + s;
+      p.out[c][mvs + 2 * (long long)l + 1] = p.out[c][mvs + 2 * (long long)l + 1] + s;
+    }
   }
 }
 
@@ -231,12 +266,33 @@ void cmdr_sht_invn_diag(int nmaps, const double *const *a_l0, double npix, const
   }
   constexpr int R = 4;
   dim3 grid((h + 32 * R - 1) / (32 * R), a->nm);
-  switch (nmaps) {
-    case 1: invn_kernel<R, 1><<<grid, 32, 0, st>>>(p); break;
-    case 2: invn_kernel<R, 2><<<grid, 32, 0, st>>>(p); break;
-    default: invn_kernel<R, 3><<<grid, 32, 0, st>>>(p); break;
+  p.det = nullptr;
+  if (deterministic()) {
+    // partials of at most 1/16 of the device memory per launch: several launches over m ranges beyond that
+    static size_t cap = 0;
+    if (!cap) { size_t fr, tot; CMDR_CUDA_CHECK(cudaMemGetInfo(&fr, &tot)); cap = tot / 16; }
+    p.dl.nb = (int)grid.x; p.dl.lmax = lmax;
+    const size_t per_m = (size_t)grid.x * p.dl.row() * sizeof(double) * nmaps;
+    const int mpl = (int)std::max<size_t>(1, std::min<size_t>(cap / per_m, a->nm));
+    for (int i0 = 0; i0 < a->nm; i0 += mpl) {
+      p.dl.im0 = i0; p.dl.nm = std::min(mpl, a->nm - i0);
+      p.det = static_cast<double *>(scratch_get("det_part", sizeof(double) * p.dl.comp_stride() * nmaps));
+      const dim3 gi(grid.x, p.dl.nm), gr((lmax + 1 + 255) / 256, p.dl.nm);
+      switch (nmaps) {
+        case 1: invn_kernel<R, 1, true><<<gi, 32, 0, st>>>(p); invn_reduce_kernel<1><<<gr, 256, 0, st>>>(p); break;
+        case 2: invn_kernel<R, 2, true><<<gi, 32, 0, st>>>(p); invn_reduce_kernel<2><<<gr, 256, 0, st>>>(p); break;
+        default: invn_kernel<R, 3, true><<<gi, 32, 0, st>>>(p); invn_reduce_kernel<3><<<gr, 256, 0, st>>>(p); break;
+      }
+      count_launch(2);
+    }
+  } else {
+    switch (nmaps) {
+      case 1: invn_kernel<R, 1><<<grid, 32, 0, st>>>(p); break;
+      case 2: invn_kernel<R, 2><<<grid, 32, 0, st>>>(p); break;
+      default: invn_kernel<R, 3><<<grid, 32, 0, st>>>(p); break;
+    }
+    count_launch(1);
   }
-  count_launch(1);
   CMDR_CUDA_CHECK(cudaGetLastError());
   if (!on_dev)
     for (int c = 0; c < nmaps; ++c)

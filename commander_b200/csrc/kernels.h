@@ -101,7 +101,20 @@ __host__ __device__ inline size_t ph_index(int block, int ncomp_tot, int comp, i
 // prepared by an earlier launch of this transform (ring-pair chunks of the pipelined host path)
 void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *const *alm, double4 *ph, cudaStream_t st,
                            bool prep = true);
-void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm, const double4 *ph, cudaStream_t st);
+// In deterministic mode (deterministic(), det.h) the analysis kernels store per-warp-block partials and an ordered reduce
+// adds them to the a_lm.  reduce = false: one piece of an analysis that a pipelined caller launches over several cuts of
+// the slot range (det_cut on det_block_slots(spin)); the caller then runs legendre_anal_reduce for each m range once all
+// pieces covering it are queued.  Outside deterministic mode `reduce` is ignored and legendre_anal_reduce does nothing.
+void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm, const double4 *ph, cudaStream_t st,
+                          bool reduce = true);
+void legendre_anal_reduce(const LegGeom &g, const LegAlm &a, double *const *alm, cudaStream_t st);
+bool deterministic();              // cmdr_sht_set_deterministic / CMDR_SHT_DETERMINISTIC
+// SHARP_ADD analysis in deterministic mode (abi.cu): det_add_begin returns zeroed scratch columns for the analysis to
+// write (else `alm` itself), det_add_end adds them once to `alm`, a = a + r, so that an ADD gives the prior values plus
+// the plain result on every route (the spin-2 scalar-sum route adds to the a_lm twice)
+double *const *det_add_begin(bool add, double *const *alm, int ncols, size_t nd, cudaStream_t st);
+void det_add_end(double *const *out, double *const *alm, int ncols, size_t nd, cudaStream_t st);
+int det_block_slots(int spin);     // work slots per warp block of the deterministic analysis kernels
 // Seed tables (legendre.cu): dropped with the geometry or alm handle they were built for, or all at once.
 void seed_forget(const void *h);
 void seed_release();

@@ -20,11 +20,13 @@
 // On one GPU, spin 2 runs as two scalar sums of premixed coefficients everywhere but near the poles (launch_s2s_*).
 // Analysis reduces over the rings of the warp with a select-free, software-pipelined register
 // butterfly and adds the sums to the a_lm with coalesced atomics (DESIGN.md 3.1).
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <map>
 #include <tuple>
 
+#include "det.h"
 #include "kernels.h"
 #include "legendre_core.cuh"
 
@@ -72,6 +74,14 @@ struct KParams {
   double4 *ph;
   int src_rank;                      // fused exchange: block of this rank in the ring owners' buffers (-1: local buffer, block = owner)
   double4 *peer[CMDR_MAX_PEERS];     // phase buffer of each ring owner (all = ph without the fused exchange)
+};
+
+// Partials buffer (component 0 at det), records and their layout of the deterministic analysis kernels (det.h): a
+// parameter of its own, so that KParams and the kernels that do not use it keep their parameter layout
+struct DetArgs {
+  double *det = nullptr;
+  int *drec = nullptr;
+  DetLayout dl;
 };
 
 // one row = two l (l_j = m + 2j, l_j + 1): the shared recurrence coefficients and {c1r, c1i, c2r, c2i} of each of NC
@@ -834,13 +844,17 @@ __device__ __forceinline__ void anal0_step(const TileA0 *tA, const double (&x2)[
 // shuffle latency hides behind FP64 work.  After each tile the reduced sums are read back row-major
 // from shared memory and added to the a_lm with fully coalesced atomics (other warps hold the
 // other rings of the same m).
-template <int R, int MINB, bool SEED = false>
-__global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
+// DET: the tile flush stores into the partials buffer (det.h) instead of adding to the a_lm; lane 0 records the first l
+// the warp stores (DET_EMPTY until the warp knows it stores anything).
+template <int R, int MINB, bool SEED = false, bool DET = false>
+__global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p, DetArgs d) {
   __shared__ __align__(16) TileA0 tile[2][TL];
   __shared__ __align__(16) double red[(TL + 1) * 4];   // row 0: T1 of the last row of the previous tile
   const int im = p.im0 + blockIdx.y, m = p.mval[im];
   const int lane = threadIdx.x;
   const int chunk0 = p.slot_begin + blockIdx.x * (32 * R);
+  [[maybe_unused]] const int blk = chunk0 / (32 * R);   // warp block of the whole geometry (DET launches start on a block boundary)
+  if constexpr (DET) { if (lane == 0) d.drec[d.dl.rec_index(blk, im)] = DET_EMPTY; }
   const int J = p.lmax >= m ? (p.lmax - m) / 2 + 1 : 0;   // rows (steps of two l) of this m
   double x2[R], cur[R], prev[R], w[R][4];
   int k[R];
@@ -884,6 +898,7 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
   // first flush reads from red[0..3] is zero too)
   const int j0 = SEED ? p.sl[(size_t)im * gridDim.x + blockIdx.x] : 0;
   if (SEED && j0 >= J) return;
+  if constexpr (DET) { if (lane == 0) d.drec[d.dl.rec_index(blk, im)] = m + 2 * j0; }
   const double *coef = p.coef + p.cofs[im];
   const double4 *mix = reinterpret_cast<const double4 *>(p.coef2 + 2 * p.cofs[im]);   // {u_j, v_j, h_j, v_{j-1}}
   const long long mvs = p.mvstart[im];
@@ -966,7 +981,8 @@ __global__ void __launch_bounds__(32, MINB) anal0_kernel(KParams p) {
         if (p.lscale0) val *= p.lscale0[l];
         const long long idx = p.s2s_npolar >= 0 ? xofs + 2 * (long long)l + part
                             : p.real_packed ? (m == 0 ? mvs + l : mvs + 2 * (long long)l + part) : 2 * (mvs + l) + part;
-        atomicAdd(&a[idx], val);
+        if constexpr (DET) d.det[d.dl.index(0, blk, im, l, part)] = val;
+        else atomicAdd(&a[idx], val);
       }
     }
     __syncwarp();
@@ -1071,13 +1087,16 @@ __device__ __forceinline__ void anal2_step(const TileA2 *t, const int csign, con
   }
 }
 
-template <int R, int MINB, bool SEED = false>
-__global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
+// DET: as in anal0_kernel, E into component 0 and B into component 1 of the partials buffer
+template <int R, int MINB, bool SEED = false, bool DET = false>
+__global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p, DetArgs d) {
   __shared__ __align__(16) TileA2 tile[2][TL];
   __shared__ __align__(16) double red[TL * 4];
   const int im = p.im0 + blockIdx.y, m = p.mval[im];
   const int lane = threadIdx.x;
   const int chunk0 = p.slot_begin + blockIdx.x * (32 * R);
+  [[maybe_unused]] const int blk = chunk0 / (32 * R);
+  if constexpr (DET) { if (lane == 0) d.drec[d.dl.rec_index(blk, im)] = DET_EMPTY; }
   const int l0 = max(m, p.spin);
   if (l0 > p.lmax) return;
   double x[R], Pa[R], Pap[R], Pb[R], Pbp[R], w[R][8];
@@ -1179,6 +1198,7 @@ __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
     for (int q = 0; q < (int)(TL * sizeof(TileA2)) / 512; ++q) cp_async16(dst + (q * 32 + lane) * 16, src + (q * 32 + lane) * 16);
     cp_async_commit();
   };
+  if constexpr (DET) { if (lane == 0) d.drec[d.dl.rec_index(blk, im)] = l0 + lskip; }
   issue_tile(0, l0 + lskip);
   cp_async_wait_all();
   __syncwarp();
@@ -1246,8 +1266,13 @@ __global__ void __launch_bounds__(32, MINB) anal2_kernel(KParams p) {
         if (p.lscale0) E *= p.lscale0[l];
         if (p.lscale1) B *= p.lscale1[l];
         const long long idx = p.real_packed ? (m == 0 ? mvs + l : mvs + 2 * (long long)l + part) : 2 * (mvs + l) + part;
-        atomicAdd(&aE[idx], E);
-        atomicAdd(&aB[idx], B);
+        if constexpr (DET) {
+          d.det[d.dl.index(0, blk, im, l, part)] = E;
+          d.det[d.dl.index(1, blk, im, l, part)] = B;
+        } else {
+          atomicAdd(&aE[idx], E);
+          atomicAdd(&aB[idx], B);
+        }
       }
     }
     __syncwarp();
@@ -1497,6 +1522,24 @@ __global__ void __launch_bounds__(256) post_s2s_kernel(KParams p, const double *
   if (m > 0) { aE[i0 + 1] += fE * ei; aB[i0 + 1] += fB * bi; }
 }
 
+// Ordered reduce of a deterministic analysis (det.h): for each (l, part) of the local m's of `p`, a = a + (the sum of the
+// partials of every warp block in ascending block order), component c of the partials into alm0 (c = 0) / alm1 (c = 1).
+// The a_lm slots and the destination index are those of the kernels' tile flush.
+__global__ void __launch_bounds__(256) det_reduce_kernel(KParams p, DetArgs d, int ncomp) {
+  const int im = p.im0 + blockIdx.y, m = p.mval[im];
+  const int e = blockIdx.x * blockDim.x + threadIdx.x, l = e >> 1, part = e & 1;
+  if (l < max(m, p.spin) || l > p.lmax || (m == 0 && part)) return;
+  const long long idx = det_dst_index(p.s2s_npolar >= 0, p.real_packed, m, p.mvstart[im], 2 * (p.cofs[im] - m), l, part);
+  const int *rec = d.drec + d.dl.rec_index(0, im);
+  const size_t bstride = (size_t)d.dl.nm * d.dl.row();
+  for (int c = 0; c < ncomp; ++c) {
+    const double *src = d.det + d.dl.index(c, 0, im, l, part);
+    const double s = det_sum(rec, 1, d.dl.nb, l, [&](int b) { return src[(size_t)b * bstride]; });
+    double *a = c ? p.alm1 : p.alm0;
+    a[idx] = a[idx] + s;
+  }
+}
+
 // ------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------
@@ -1527,12 +1570,12 @@ static KParams make_params(const LegGeom &g, const LegAlm &a, double *alm0, doub
   return p;
 }
 
-template <int R, typename K>
-static void launch_w(K kernel, const KParams &p, int nm, cudaStream_t st) {   // one warp per CTA
+template <int R, typename K, typename... A>
+static void launch_w(K kernel, const KParams &p, int nm, cudaStream_t st, A... args) {   // one warp per CTA
   const int n = p.nslots - p.slot_begin;
   if (n <= 0) return;
   dim3 grid((n + 32 * R - 1) / (32 * R), nm);
-  kernel<<<grid, 32, 0, st>>>(p);
+  kernel<<<grid, 32, 0, st>>>(p, args...);
 }
 
 // ---- seed tables: one per (geometry handle, alm handle, kernel), built on first use ----
@@ -1602,6 +1645,52 @@ static const SeedTab *seed_table(const LegGeom &g, SeedKind kind, int R, const K
 }
 static void use_seed(KParams &p, const SeedTab *t) { p.sl = t->sl; p.ss = t->ss; p.sk = t->sk; }
 
+// ---- deterministic analysis (det.h): on with cmdr_sht_set_deterministic or CMDR_SHT_DETERMINISTIC=1 at load ----
+static bool g_det = getenv("CMDR_SHT_DETERMINISTIC") && atoi(getenv("CMDR_SHT_DETERMINISTIC")) != 0;
+bool deterministic() { return g_det; }
+// slots per warp block of the deterministic kernels: anal0_kernel<8, ...>, anal2_kernel<4, ...> (the defaults; the
+// CMDR_SHT_R_A0 / _A2 tuning overrides do not apply in this mode)
+int det_block_slots(int spin) { return spin == 0 ? 32 * 8 : 32 * 4; }
+
+// Partials of a launch whose blocks cover work slots [0, nslots) and local m's [im0, im0 + nm), ncomp components, in
+// the library's scratch arena (one buffer: the kernels and the reduce of a transform run in stream order)
+static DetArgs det_use(const KParams &p, int nslots, int im0, int nm, int ncomp) {
+  DetArgs d;
+  d.dl.nb = (nslots + det_block_slots(p.spin) - 1) / det_block_slots(p.spin);
+  d.dl.nm = nm; d.dl.im0 = im0; d.dl.lmax = p.lmax;
+  d.det = static_cast<double *>(scratch_get("det_part", sizeof(double) * d.dl.comp_stride() * ncomp));
+  d.drec = static_cast<int *>(scratch_get("det_rec", sizeof(int) * (size_t)d.dl.nb * nm));
+  return d;
+}
+// local m's per launch so that the partials take at most 1/16 of the device memory (decided once, as seed_table does);
+// a launch over more m's runs as several launches over m ranges
+static int det_m_per_launch(int nslots, int spin, int lmax, int ncomp) {
+  static size_t cap = 0;
+  if (!cap) { size_t fr, tot; CMDR_CUDA_CHECK(cudaMemGetInfo(&fr, &tot)); cap = tot / 16; }
+  const size_t nb = (nslots + det_block_slots(spin) - 1) / det_block_slots(spin);
+  const size_t per_m = nb * (sizeof(double) * 2 * (size_t)(lmax + 1) * ncomp + sizeof(int));
+  return (int)std::max<size_t>(1, std::min<size_t>(cap / per_m, 1 << 30));
+}
+static void det_reduce(const KParams &p, const DetArgs &d, int nmr, int ncomp, cudaStream_t st) {
+  det_reduce_kernel<<<dim3((unsigned)((d.dl.row() + 255) / 256), nmr), 256, 0, st>>>(p, d, ncomp);
+  count_launch();
+}
+// the deterministic Legendre analysis kernel of `p` (partials set), seeded where the plain launch would be
+static void det_anal_kernel(const LegGeom &g, const LegAlm &a, KParams p, const DetArgs &d, SeedKind kind, int nmr,
+                            cudaStream_t st) {
+  if (p.spin == 0) {
+    if (const SeedTab *t = seed_table(g, kind, 8, p, a.nm, st)) { use_seed(p, t); launch_w<8>(anal0_kernel<8, 12, true, true>, p, nmr, st, d); }
+    else launch_w<8>(anal0_kernel<8, 12, false, true>, p, nmr, st, d);
+  } else {
+    if (const SeedTab *t = p.spin == 2 ? seed_table(g, SEED_A2, 4, p, a.nm, st) : nullptr) {
+      use_seed(p, t); launch_w<4>(anal2_kernel<4, 12, true, true>, p, nmr, st, d);
+    } else {
+      launch_w<4>(anal2_kernel<4, 12, false, true>, p, nmr, st, d);
+    }
+  }
+  count_launch();
+}
+
 // ---- spin 2 as scalar sums (prep_s2s_kernel / post_s2s_kernel above) ----
 static bool g_s2s_on = true;
 bool spin2_scalar_on() { return g_s2s_on; }
@@ -1651,21 +1740,41 @@ static void launch_s2s_anal(const LegGeom &g, const LegAlm &a, const KParams &p,
   const long long ctot = 2 * a.s2s_nl;   // doubles per component
   double *T = static_cast<double *>(scratch_get("anal_s2s", sizeof(double) * 2 * (size_t)ctot));
   CMDR_CUDA_CHECK(cudaMemsetAsync(T, 0, sizeof(double) * 2 * (size_t)ctot, st));
-  const SeedTab *t = seed_table(g, SEED_A0X, 8, q, a.nm, st);
-  if (t) use_seed(q, t);
-  for (int c = 0; c < 2; ++c) {
-    KParams qc = q;
-    qc.comp0 = p.comp0 + c;
-    qc.alm0 = T + (size_t)c * ctot;
-    if (t) launch_w<8>(anal0_kernel<8, 12, true>, qc, nmr, st);
-    else launch_w<8>(anal0_kernel<8, 12>, qc, nmr, st);
-    count_launch();
-  }
-  if (g.s2s_npolar > 0) {
-    KParams pp = p;
-    pp.nslots = min(p.nslots, g.s2s_npolar);
-    launch_w<4>(anal2_kernel<4, 12>, pp, nmr, st);
-    count_launch();
+  if (g_det) {   // both scalar sums through the partials and the reduce into T, then the polar rings into the a_lm
+    const DetArgs d = det_use(q, q.nslots, q.im0, nmr, 2);
+    for (int c = 0; c < 2; ++c) {   // the two launches store the same records
+      KParams qc = q;
+      qc.comp0 = p.comp0 + c;
+      DetArgs dc = d;
+      dc.det = d.det + (size_t)c * d.dl.comp_stride();
+      det_anal_kernel(g, a, qc, dc, SEED_A0X, nmr, st);
+    }
+    q.alm0 = T; q.alm1 = T + ctot;
+    det_reduce(q, d, nmr, 2, st);
+    if (g.s2s_npolar > 0) {
+      KParams pp = p;
+      pp.nslots = min(p.nslots, g.s2s_npolar);
+      const DetArgs dp = det_use(pp, pp.nslots, pp.im0, nmr, 2);
+      det_anal_kernel(g, a, pp, dp, SEED_A2, nmr, st);
+      det_reduce(pp, dp, nmr, 2, st);
+    }
+  } else {
+    const SeedTab *t = seed_table(g, SEED_A0X, 8, q, a.nm, st);
+    if (t) use_seed(q, t);
+    for (int c = 0; c < 2; ++c) {
+      KParams qc = q;
+      qc.comp0 = p.comp0 + c;
+      qc.alm0 = T + (size_t)c * ctot;
+      if (t) launch_w<8>(anal0_kernel<8, 12, true>, qc, nmr, st, DetArgs{});
+      else launch_w<8>(anal0_kernel<8, 12>, qc, nmr, st, DetArgs{});
+      count_launch();
+    }
+    if (g.s2s_npolar > 0) {
+      KParams pp = p;
+      pp.nslots = min(p.nslots, g.s2s_npolar);
+      launch_w<4>(anal2_kernel<4, 12>, pp, nmr, st, DetArgs{});
+      count_launch();
+    }
   }
   post_s2s_kernel<<<dim3((a.lmax + 1 + 255) / 256, nmr), 256, 0, st>>>(p, T, a.s2s_cofs, ctot);
   count_launch();
@@ -1736,12 +1845,37 @@ void launch_legendre_synth(const LegGeom &g, const LegAlm &a, const double *cons
   CMDR_CUDA_CHECK(cudaGetLastError());
 }
 
-void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm, const double4 *ph, cudaStream_t st) {
+void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm, const double4 *ph, cudaStream_t st,
+                          bool reduce) {
   if (a.nm == 0 || g.nslots == 0) return;
   const int nmr = (a.im_end >= 0 ? a.im_end : a.nm) - a.im_begin;   // local m's of this launch
   if (nmr <= 0) return;
   const int spin = a.spin;
   KParams p = make_params(g, a, alm[0], spin ? alm[1] : nullptr, const_cast<double4 *>(ph));
+  if (g_det) {
+    if (p.slot_begin % det_block_slots(spin) != 0 || (!reduce && s2s_route(g, a)) || (reduce && p.slot_begin != 0)) {
+      fprintf(stderr, "cmdr_sht: deterministic analysis launched over slots [%d, %d), not a cut on warp blocks\n", p.slot_begin, p.nslots);
+      abort();
+    }
+    if (!reduce) {   // one piece of a pipelined analysis: partials of the whole geometry and every local m
+      det_anal_kernel(g, a, p, det_use(p, g.nslots, 0, a.nm, spin ? 2 : 1), SEED_A0, nmr, st);
+      CMDR_CUDA_CHECK(cudaGetLastError());
+      return;
+    }
+    const int s2s = s2s_route(g, a);
+    const int mpl = det_m_per_launch(p.nslots, s2s ? 0 : spin, s2s ? a.lmax + 2 : a.lmax, spin ? 2 : 1);
+    for (int i0 = a.im_begin; i0 < a.im_begin + nmr; i0 += mpl) {
+      const int n = std::min(mpl, a.im_begin + nmr - i0);
+      KParams pi = p;
+      pi.im0 = i0;
+      if (s2s) { launch_s2s_anal(g, a, pi, n, st); continue; }
+      const DetArgs d = det_use(pi, pi.nslots, i0, n, spin ? 2 : 1);
+      det_anal_kernel(g, a, pi, d, SEED_A0, n, st);
+      det_reduce(pi, d, n, spin ? 2 : 1, st);
+    }
+    CMDR_CUDA_CHECK(cudaGetLastError());
+    return;
+  }
   if (s2s_route(g, a)) { launch_s2s_anal(g, a, p, nmr, st); return; }
   // spin 0: 8 ring pairs per thread since the two-l-per-step kernels (fewer registers per ring pair; the butterfly and the
   // per-tile flush are per warp, so their share halves): 8.71 -> 8.31 ms at nside 2048 / lmax 4000
@@ -1750,35 +1884,44 @@ void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm,
   static const int b0 = env_int("CMDR_SHT_MINB_A0", 12), b2 = env_int("CMDR_SHT_MINB_A2", 12);
   if (spin == 0) {
     switch (r0 * 100 + b0) {
-      case 416: launch_w<4>(anal0_kernel<4, 16>, p, nmr, st); break;
-      case 408: launch_w<4>(anal0_kernel<4, 8>, p, nmr, st); break;
-      case 612: launch_w<6>(anal0_kernel<6, 12>, p, nmr, st); break;
-      case 608: launch_w<6>(anal0_kernel<6, 8>, p, nmr, st); break;
+      case 416: launch_w<4>(anal0_kernel<4, 16>, p, nmr, st, DetArgs{}); break;
+      case 408: launch_w<4>(anal0_kernel<4, 8>, p, nmr, st, DetArgs{}); break;
+      case 612: launch_w<6>(anal0_kernel<6, 12>, p, nmr, st, DetArgs{}); break;
+      case 608: launch_w<6>(anal0_kernel<6, 8>, p, nmr, st, DetArgs{}); break;
       case 812:
-        if (const SeedTab *t = seed_table(g, SEED_A0, 8, p, a.nm, st)) { use_seed(p, t); launch_w<8>(anal0_kernel<8, 12, true>, p, nmr, st); }
-        else launch_w<8>(anal0_kernel<8, 12>, p, nmr, st);
+        if (const SeedTab *t = seed_table(g, SEED_A0, 8, p, a.nm, st)) { use_seed(p, t); launch_w<8>(anal0_kernel<8, 12, true>, p, nmr, st, DetArgs{}); }
+        else launch_w<8>(anal0_kernel<8, 12>, p, nmr, st, DetArgs{});
         break;
-      case 808: launch_w<8>(anal0_kernel<8, 8>, p, nmr, st); break;
-      default: launch_w<4>(anal0_kernel<4, 12>, p, nmr, st); break;
+      case 808: launch_w<8>(anal0_kernel<8, 8>, p, nmr, st, DetArgs{}); break;
+      default: launch_w<4>(anal0_kernel<4, 12>, p, nmr, st, DetArgs{}); break;
     }
   } else {
     switch (r2 * 100 + b2) {
-      case 312: launch_w<3>(anal2_kernel<3, 12>, p, nmr, st); break;
-      case 308: launch_w<3>(anal2_kernel<3, 8>, p, nmr, st); break;
-      case 216: launch_w<2>(anal2_kernel<2, 16>, p, nmr, st); break;
-      case 212: launch_w<2>(anal2_kernel<2, 12>, p, nmr, st); break;
+      case 312: launch_w<3>(anal2_kernel<3, 12>, p, nmr, st, DetArgs{}); break;
+      case 308: launch_w<3>(anal2_kernel<3, 8>, p, nmr, st, DetArgs{}); break;
+      case 216: launch_w<2>(anal2_kernel<2, 16>, p, nmr, st, DetArgs{}); break;
+      case 212: launch_w<2>(anal2_kernel<2, 12>, p, nmr, st, DetArgs{}); break;
       case 412:
         if (const SeedTab *t = spin == 2 ? seed_table(g, SEED_A2, 4, p, a.nm, st) : nullptr) {
-          use_seed(p, t); launch_w<4>(anal2_kernel<4, 12, true>, p, nmr, st);
+          use_seed(p, t); launch_w<4>(anal2_kernel<4, 12, true>, p, nmr, st, DetArgs{});
         } else {
-          launch_w<4>(anal2_kernel<4, 12>, p, nmr, st);
+          launch_w<4>(anal2_kernel<4, 12>, p, nmr, st, DetArgs{});
         }
         break;
-      case 410: launch_w<4>(anal2_kernel<4, 10>, p, nmr, st); break;
-      default: launch_w<4>(anal2_kernel<4, 8>, p, nmr, st); break;
+      case 410: launch_w<4>(anal2_kernel<4, 10>, p, nmr, st, DetArgs{}); break;
+      default: launch_w<4>(anal2_kernel<4, 8>, p, nmr, st, DetArgs{}); break;
     }
   }
   count_launch();
+  CMDR_CUDA_CHECK(cudaGetLastError());
+}
+
+void legendre_anal_reduce(const LegGeom &g, const LegAlm &a, double *const *alm, cudaStream_t st) {
+  if (!g_det || a.nm == 0 || g.nslots == 0) return;
+  const int nmr = (a.im_end >= 0 ? a.im_end : a.nm) - a.im_begin;
+  if (nmr <= 0) return;
+  KParams p = make_params(g, a, alm[0], a.spin ? alm[1] : nullptr, nullptr);
+  det_reduce(p, det_use(p, g.nslots, 0, a.nm, a.spin ? 2 : 1), nmr, a.spin ? 2 : 1, st);
   CMDR_CUDA_CHECK(cudaGetLastError());
 }
 
@@ -1787,5 +1930,7 @@ void launch_legendre_anal(const LegGeom &g, const LegAlm &a, double *const *alm,
 extern "C" {
 void cmdr_sht_set_legendre_seeds(int on) { cmdr::g_seeds_on = on != 0; }
 void cmdr_sht_set_spin2_scalar(int on) { cmdr::g_s2s_on = on != 0; }
+void cmdr_sht_set_deterministic(int on) { cmdr::g_det = on != 0; }
+int cmdr_sht_deterministic(void) { return cmdr::g_det ? 1 : 0; }
 size_t cmdr_sht_legendre_seed_bytes(void) { return cmdr::g_seed_bytes; }
 }

@@ -40,7 +40,7 @@ ABI_SYMBOLS = [
     "cmdr_sht_set_profiling", "cmdr_sht_last_legendre_ms", "cmdr_sht_nominal_flops",
     "cmdr_sht_release_caches", "cmdr_sht_measure_fp64_tflops", "cmdr_sht_measure_fp64_tflops_3op",
     "cmdr_sht_measure_host_copy", "cmdr_sht_host_copy_threads", "cmdr_sht_set_legendre_seeds", "cmdr_sht_legendre_seed_bytes",
-    "cmdr_sht_set_spin2_scalar",
+    "cmdr_sht_set_spin2_scalar", "cmdr_sht_set_deterministic", "cmdr_sht_deterministic",
     "cmdr_cr_setup", "cmdr_cr_destroy", "cmdr_cr_matmulA", "cmdr_cr_invM", "cmdr_cr_set_precond_diag",
     "cmdr_cr_get_precond_diag", "cmdr_cr_compute_rhs", "cmdr_cr_solve", "cmdr_cr_matmul_count", "cmdr_cr_setup_multi",
     "cmdr_cr_set_mixing_map", "cmdr_cr_set_pseudoinv", "cmdr_cr_compute_rhs_draw", "cmdr_cr_draw_eta",
@@ -105,6 +105,8 @@ def lib() -> C.CDLL:
     L.cmdr_sht_set_legendre_seeds.argtypes = [ci]
     L.cmdr_sht_legendre_seed_bytes.restype = C.c_size_t
     L.cmdr_sht_set_spin2_scalar.argtypes = [ci]
+    L.cmdr_sht_set_deterministic.argtypes = [ci]
+    L.cmdr_sht_deterministic.restype = ci
     L.cmdr_cr_setup.argtypes = [ci, ci, ci, vp, vp, vp, vp, vp, vp, ci]
     L.cmdr_cr_setup.restype = vp
     L.cmdr_cr_setup_multi.argtypes = [ci, ci, vp, vp, vp, ci, vp, vp, vp, vp, vp, vp, vp, ci]
@@ -418,6 +420,16 @@ def set_legendre_seeds(on: bool) -> None:
 def set_spin2_scalar(on: bool) -> None:
     """Spin-2 transforms as scalar sums on (default) or off; see cmdr_sht.h."""
     lib().cmdr_sht_set_spin2_scalar(1 if on else 0)
+
+
+def set_deterministic(on: bool) -> None:
+    """Deterministic analysis on or off (default off, or on with CMDR_SHT_DETERMINISTIC=1); see cmdr_sht.h."""
+    lib().cmdr_sht_set_deterministic(1 if on else 0)
+
+
+def deterministic() -> bool:
+    """Whether the deterministic mode is on in this process."""
+    return bool(lib().cmdr_sht_deterministic())
 
 
 def legendre_seed_bytes() -> int:
